@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Detection_3D sparse backbone path (BASELINE.json north_star).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--math tf32|bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--math tf32|bf16|fp32] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one `FPN_Net.forward` of the sw_4c_fpn432 backbone (BASELINE.json configs[1]) on the
@@ -9,6 +9,9 @@ synthetic 470 m^2 building "B470" (1,177,224 input rows / 1,155,656 active voxel
 Metadata / rulebook build, which the reference redoes every forward (sparseconvnet/ioLayers.py:52-55).
 Prints ONE JSON line (rank 0).  `value`: inputs resident in HBM.  `e2e`: same metric through the
 public API with HOST (pinned) coords + features, H2D and D2H copies inside the timed region.
+`--dump-outputs DIR`: the maps the last timed step returned, as DIR/<map>_features.npy (float32) and
+DIR/<map>_locations.npy (float64: x, y, z, batch index per row); the inputs are seeded, so two builds
+can be compared output for output.
 """
 import argparse
 import json
@@ -18,6 +21,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -134,6 +138,20 @@ def parity_of(maps, ref_maps, tol):
             "against": "reference CPU forward of the same full B470 building in this run (cpu_baseline leg)"}
 
 
+def dump_outputs(out_dir, rpn, roi):
+    """The maps FPN_Net.forward returned: features [rows, C] as float32, locations [rows, 4] as float64."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    for tag, maps in (("rpn", rpn), ("roi", roi)):
+        for i, m in enumerate(maps):
+            arrays[f"{tag}{i}_features"] = m.features.detach().float().cpu().numpy()
+            arrays[f"{tag}{i}_locations"] = m.get_spatial_locations().numpy().astype(np.float64)
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20, "outputs exceed 64 MB"
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def make_model(cfg, device):
     import torch
     import fpn_util
@@ -187,7 +205,7 @@ def run_reference_arm(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
-def leg_batch64(args, rank, world, dev, net, n_build=64):
+def leg_batch64(args, rank, world, dev, net, n_build=64, steps=3):
     """BASELINE.json config 4: batched inference over 64 DISTINCT synthetic buildings (B470 footprint jittered +-15 %, seeds 0..63)
     sharded by building across the ranks (longest first, no collective on the data path).  Every rank streams its shard from
     pinned host memory through the backbone (Metadata built two buildings ahead) and copies every returned map back to pinned
@@ -261,11 +279,11 @@ def leg_batch64(args, rank, world, dev, net, n_build=64):
                 dist.all_reduce(tp, op=dist.ReduceOp.MAX)
             return tp.item(), d2h, outs
 
-        # the whole batch three times: the first pass of a fresh process is occasionally 2-3x slower (cold host pages) and the host
+        # the whole batch `steps` times (three by default): the first pass of a fresh process is occasionally 2-3x slower (cold host pages) and the host
         # side of this leg (5 GB of pinned uploads per pass) is sensitive to whatever else the box is doing; the best pass is reported,
         # all are listed
         passes = []
-        for _ in range(3):
+        for _ in range(steps):
             ms_p, d2h, outs = one_pass()
             passes.append(ms_p)
     t = torch.tensor([min(passes)], device=dev, dtype=torch.float64)
@@ -276,7 +294,7 @@ def leg_batch64(args, rank, world, dev, net, n_build=64):
     ms = t.item()
     from detection_3d_b200._lib import lib
     pool = {"chunk_mallocs": lib().scn_debug_counter(0), "chunk_waits": lib().scn_debug_counter(1), "pool_mib": lib().scn_debug_counter(2)}
-    return {"pool": pool, "ms_passes": passes, "metric": "batched_inference_buildings_per_s", "value": n_build / (ms * 1e-3), "unit": "buildings/s", "buildings": n_build, "ms_total": ms,
+    return {"pool": pool, "ms_passes": passes, "steps": steps, "metric": "batched_inference_buildings_per_s", "value": n_build / (ms * 1e-3), "unit": "buildings/s", "buildings": n_build, "ms_total": ms,
             "ms_per_building": ms / n_build, "scaling": "strong", "buildings_done": int(counts.item()), "finite": ok,
             "h2d_bytes_rank0": h2d, "d2h_bytes_rank0": d2h, "shard_sizes": [len(distributed.shard_buildings(sizes, world, r)) for r in range(world)],
             "note": "64 distinct buildings (B470 +-15 %), host pinned inputs, sharded longest-first, Metadata built two buildings ahead, outputs copied to pinned host memory"}
@@ -397,7 +415,7 @@ def leg_train(args, rank, world, dev, scn, steps=8, warmup=4):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 400 for our arm = a >= 2 s steady-state window, 3 for the reference arm)")
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 400 for the headline = a >= 2 s steady-state window, 3 for the reference arm; --config rpn / train / batch64: 20 steps / 8 steps / 3 passes over the batch)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--math", default=os.environ.get("SCN_MATH", "auto"), choices=["auto", "fp32", "tf32", "bf16"])
@@ -407,9 +425,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the sustained leg and the tf32 / fp32 sub-results")
     ap.add_argument("--sustain-steps", type=int, default=400, help="steps of the steady-state leg (>= 2 s of back-to-back forwards)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the maps returned by the last timed step of the headline as DIR/<map>_{features,locations}.npy")
     args = ap.parse_args()
+    steps_given = args.steps is not None  # configs rpn / batch64 / train keep their own step counts unless --steps is passed
     if args.steps is None:
         args.steps = 400 if args.impl == "ours" else 3
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "backbone"):
+        ap.error("--dump-outputs writes the outputs of the headline (--impl ours --config backbone)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -456,11 +480,12 @@ def main():
     cfg = scn.sw4c_fpn432_config()
     net, state = make_model(cfg, dev)
     if args.config != "backbone":  # configs 4 / 5 on their own: one JSON line in the same format
+        leg_steps = {"steps": args.steps} if steps_given else {}
         if args.config == "rpn":
             c_np = synthetic.building_coords()
-            sub = leg_rpn(args, rank, world, dev, net, torch.from_numpy(c_np).pin_memory(), torch.from_numpy(fpn_util.features_for(c_np)).pin_memory())
+            sub = leg_rpn(args, rank, world, dev, net, torch.from_numpy(c_np).pin_memory(), torch.from_numpy(fpn_util.features_for(c_np)).pin_memory(), **leg_steps)
         else:
-            sub = leg_batch64(args, rank, world, dev, net) if args.config == "batch64" else leg_train(args, rank, world, dev, scn)
+            sub = leg_batch64(args, rank, world, dev, net, **leg_steps) if args.config == "batch64" else leg_train(args, rank, world, dev, scn, **leg_steps)
         line = {"metric": sub.pop("metric"), "value": sub.pop("value"), "unit": sub.pop("unit"), "n_gpus": world, "steps": sub.get("steps", 1), "warmup": args.warmup,
                 "ms_per_step": sub.get("ms_per_step", sub.get("ms_total")), "higher_is_better": True, "scaling": sub.pop("scaling"), "vs_baseline": None,
                 "dtype": {"fp32": "f32", "tf32": "tf32", "bf16": "bf16"}[math], "data": "synthetic",
@@ -524,7 +549,8 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return t.item(), launches
 
-    def timed(fn, steps, warmup):
+    def timed(fn, steps, warmup, keep=None):
+        """`keep`, a list, receives what the last timed step returned."""
         for _ in range(warmup):
             fn()
         torch.cuda.synchronize()
@@ -533,10 +559,13 @@ def main():
         torch.cuda.synchronize()
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         l0 = scn.kernel_launch_count()
-        for a, b in ev:
+        for i, (a, b) in enumerate(ev):
             flush.fill_(1)  # L2 flush between timed iterations (outside the event pair)
             a.record()
-            fn()
+            if keep is not None and i == steps - 1:
+                keep[:] = [fn()]
+            else:
+                fn()  # (outputs and their Metadata are released before the next step, as a caller's would be)
             b.record()
         torch.cuda.synchronize()
         launches = scn.kernel_launch_count() - l0
@@ -551,8 +580,12 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     scn.forward_pass_multiplyAdd_count = 0
-    total_ms, launches = timed(step_resident, args.steps, args.warmup)
+    last = []
+    total_ms, launches = timed(step_resident, args.steps, args.warmup, keep=last)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:  # before any other forward can reuse the returned buffers
+        dump_outputs(args.dump_outputs, *last[0])
+    del last
     macs_per_step = scn.forward_pass_multiplyAdd_count / (args.steps + args.warmup)
     e2e_ms, _ = timed(step_e2e, args.steps, 1)
     # streaming variant (FPN_Net.prefetch builds the Metadata two buildings ahead); reported beside the headline, which

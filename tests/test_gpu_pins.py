@@ -588,15 +588,9 @@ def _roi_case(rs, ext, n_rois, batch):
     return np.stack([b, cw, ch, cz, w, h, z, th], 1).astype(np.float32)
 
 
-@pytest.mark.parametrize("case", ["small2", "level4"])
-@pytest.mark.parametrize("sampling", [2, 0])
-def test_roi_align_rotated_3d_vs_reference_kernel(case, sampling):
-    """detection_3d_b200.roi_align.ROIAlignRotated3D (samples the SPARSE map) against (a) the reference's own CUDA kernels compiled
-    unmodified (oracle/_ref/libroialign3d_ref.so) on the densified, cropped map -- exactly the reference module's data flow -- and (b)
-    the CPU restatement (oracle).  Forward and backward; rois inside, straddling and outside the map, degenerate sizes, sampling
-    ratio 2 and adaptive.  Tolerance 2e-5 of max|ref|: fp32, the order of the 8-corner sum and FMA contraction differ."""
-    scn = _scn()
-    from detection_3d_b200.roi_align import ROIAlignRotated3D
+def _roi_inputs(case, sampling):
+    """The seeded inputs of one ROIAlignRotated3D case (also read by tests/golden/make_golden_roialign.py): coordinates, features,
+    map size, channels, pooled size, spatial scale, cropped extent, batch size, rois and the gradient of the output."""
     rs = np.random.RandomState(17 + sampling)
     if case == "small2":
         coords = np.concatenate([synthetic.small_building(20, 18, 8, 2, seed=4), synthetic.small_building(16, 22, 6, 2, seed=5, batch_index=1)])
@@ -606,22 +600,39 @@ def test_roi_align_rotated_3d_vs_reference_kernel(case, sampling):
         coords = np.unique(np.concatenate([c0[:, :3] >> 4, c0[:, 3:]], 1), axis=0)
         sz, C_, n_rois, pooled, scale = [128, 128, 32], 128, 24, (7, 7, 7), 0.25
     feats = rs.randn(coords.shape[0], C_).astype(np.float32)
+    ext = (coords[:, :3].max(0) + 1).tolist()
+    batch = int(coords[:, 3].max()) + 1
+    rois = _roi_case(rs, [e / scale for e in ext], n_rois, batch)  # roi coordinates are in input units: the kernel multiplies by spatial_scale
+    g = rs.randn(n_rois, C_, *pooled).astype(np.float32)
+    return coords, feats, sz, C_, pooled, scale, ext, batch, rois, g
+
+
+def _close_golden(got, gold, key, rtol, atol):
+    """_close on the entries of `got` stored under `key` of the golden file, scaled by the max|.| of the whole stored array."""
+    got = np.asarray(got)
+    assert got.shape == tuple(gold[key + "_shape"])
+    scale = max(1.0, float(gold[key + "_absmax"]))
+    np.testing.assert_allclose(got.ravel()[gold[key + "_idx"]], gold[key], rtol=rtol, atol=atol * scale)
+    np.testing.assert_allclose(np.abs(got).max(), gold[key + "_absmax"], rtol=rtol, atol=atol * scale)
+
+
+def _roi_align_vs_restatement(case, sampling):
+    """detection_3d_b200.roi_align.ROIAlignRotated3D (samples the SPARSE map) against the CPU restatement (oracle) of the reference's
+    kernels on the densified, cropped map -- exactly the reference module's data flow.  Forward and backward (down to the input
+    features).  Returns what the reference comparison needs: output, restated output, restated map gradient, dense map, inputs."""
+    scn = _scn()
+    from detection_3d_b200.roi_align import ROIAlignRotated3D
+    coords, feats, sz, C_, pooled, scale, ext, batch, rois, g = _roi_inputs(case, sampling)
     inp = scn.InputLayer(3, sz, mode=4)
     ft = T(feats).requires_grad_(True)
     x = inp([torch.from_numpy(coords.astype(np.int64)), ft])
-    ext = (coords[:, :3].max(0) + 1).tolist()
-    batch = int(coords[:, 3].max()) + 1
-    rois = _roi_case(rs, [e / scale for e in ext], n_rois, batch)
-    rois[:, 1:7] = rois[:, 1:7]  # roi coordinates are in input units: the kernel multiplies by spatial_scale
     layer = ROIAlignRotated3D(pooled, scale, sampling)
     out = layer(x, T(rois))
-    g = rs.randn(*out.shape).astype(np.float32)
+    assert tuple(out.shape) == g.shape
     out.backward(T(g))
     torch.cuda.synchronize()
     dense = scn.sparse_3d_to_dense_2d(x).detach().contiguous()          # what the reference module samples
     assert list(dense.shape[2:]) == ext
-    d_rows = torch.autograd.grad  # (silence linters)
-    # (b) CPU restatement
     want = so.o_roi_align_rotated_3d_forward(dense.cpu().numpy(), rois, scale, pooled, sampling)
     _close(out.detach().cpu().numpy(), want, 1e-5, 2e-5)
     dd = so.o_roi_align_rotated_3d_backward(g, rois, scale, pooled, sampling, tuple(dense.shape))
@@ -632,10 +643,36 @@ def test_roi_align_rotated_3d_vs_reference_kernel(case, sampling):
     hdr, tab = O.input_rules()
     want_g = so.o_input_layer_backward(so.o_sparse_to_dense_backward(full, O.sparse_to_dense_rules(sz), n), hdr, tab)
     _close(ft.grad.cpu().numpy(), want_g, 1e-4, 5e-5)
-    # (a) the reference's own kernels
+    return out, want, dd, dense, (C_, pooled, scale, ext, batch, rois, g)
+
+
+@pytest.mark.parametrize("case", ["small2", "level4"])
+@pytest.mark.parametrize("sampling", [2, 0])
+def test_roi_align_rotated_3d_vs_restatement_and_golden(case, sampling):
+    """ROIAlignRotated3D against the CPU restatement (_roi_align_vs_restatement), and both against tests/golden/roi_align_rotated_3d.npz:
+    a regression pin of the restatement's outputs for these inputs (a seeded sample of every output, tests/golden/
+    make_golden_roialign.py), so that the product and the restatement cannot drift together.  Rois inside, straddling and outside the
+    map, degenerate sizes, sampling ratio 2 and adaptive.  Tolerance 2e-5 of max|ref|: fp32, the order of the 8-corner sum and FMA
+    contraction differ."""
+    out, want, dd, _, _ = _roi_align_vs_restatement(case, sampling)
+    gold = np.load(os.path.join(GOLD, "roi_align_rotated_3d.npz"))
+    key = f"{case}_s{sampling}"
+    _close_golden(out.detach().cpu().numpy(), gold, key + "_fwd", 1e-5, 2e-5)
+    _close_golden(want, gold, key + "_fwd", 1e-5, 2e-5)
+    _close_golden(dd, gold, key + "_bwd", 1e-4, 5e-5)
+
+
+@pytest.mark.skipif(not os.path.exists(os.path.join(os.path.dirname(so.__file__), "_ref", "libroialign3d_ref.so")),
+                    reason="needs the reference's ROIAlignRotated3D kernels built into oracle/_ref (make -C oracle ref, from the reference's sources)")
+@pytest.mark.parametrize("case", ["small2", "level4"])
+@pytest.mark.parametrize("sampling", [2, 0])
+def test_roi_align_rotated_3d_vs_reference_kernel(case, sampling):
+    """ROIAlignRotated3D and the CPU restatement against the reference's own CUDA kernels compiled unmodified
+    (oracle/_ref/libroialign3d_ref.so) on the densified, cropped map.  Same cases and tolerances as above."""
+    out, want, dd, dense, (C_, pooled, scale, ext, batch, rois, g) = _roi_align_vs_restatement(case, sampling)
     ref = so.roi_align_ref_lib()
-    assert ref is not None, "oracle/_ref/libroialign3d_ref.so missing (make -C oracle ref)"
     p = lambda t: C.c_void_p(t.data_ptr())
+    n_rois = rois.shape[0]
     r_t = T(rois)
     out_ref = torch.empty_like(out)
     assert ref.ref_roi_align_rotated_3d_forward(p(dense), batch, C_, ext[0], ext[1], ext[2], p(r_t), n_rois, scale, pooled[0], pooled[1], pooled[2], sampling, p(out_ref)) == 0
