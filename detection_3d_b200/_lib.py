@@ -6,10 +6,13 @@ import of any operator fails loudly -- there is no CPU or PyTorch fallback.
 import ctypes as C
 import os
 
+import torch
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libscn_b200.so")
 
 _lib = None
+_det = None  # the deterministic-mode flag last handed to the library
 L3 = C.c_long * 3
 
 # every symbol include/scn_b200.h declares: (restype, argtypes)
@@ -83,6 +86,8 @@ SYMBOLS = {
     "scn_voxelize": (_i, [_vp, _vp, _l, _i, _pd, _pd, _d, _pd, _i, _l, _i, _vp, _vp, _pl, _vp]),
     "scn_set_math_mode": (_i, [_i]),
     "scn_get_math_mode": (_i, []),
+    "scn_set_deterministic": (_i, [_i]),
+    "scn_get_deterministic": (_i, []),
     "scn_tensor_core_path_available": (_i, []),
     "scn_kernel_launch_count": (_l, []),
     "scn_debug_counter": (_l, [_i]),
@@ -94,8 +99,11 @@ SYMBOLS = {
 
 
 def lib():
-    """Load libscn_b200.so (built by detection_3d_b200/csrc/Makefile or __graft_entry__.build())."""
-    global _lib
+    """Load libscn_b200.so (built by detection_3d_b200/csrc/Makefile or __graft_entry__.build()).
+
+    Every native call goes through here, so this is also where torch.are_deterministic_algorithms_enabled() is copied into the
+    library (scn_set_deterministic) before the call: torch's flag is the package's only switch for the deterministic mode."""
+    global _lib, _det
     if _lib is None:
         if not os.path.exists(LIB_PATH):
             raise RuntimeError(
@@ -107,6 +115,10 @@ def lib():
             fn.restype = res
             fn.argtypes = args
         _lib = handle
+    det = torch.are_deterministic_algorithms_enabled()
+    if det is not _det:
+        _lib.scn_set_deterministic(int(det))
+        _det = det
     return _lib
 
 

@@ -81,6 +81,8 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
 int to_bf16(const float *x, void *y, long n, cudaStream_t s);
 int dense_rows_dw(const float *in, const float *d_out, float *dW, float *d_bias, long n, int Cin, int Cout, cudaStream_t s);
 static int g_math_mode = 0;
+static std::atomic<int> g_deterministic{0};
+bool deterministic() { return g_deterministic.load(std::memory_order_relaxed) != 0; }
 } // namespace scn
 
 // The caller's thread and the prefetch worker (scn_metadata_prefetch) build into the same lazily
@@ -151,6 +153,11 @@ int scn_set_math_mode(int mode) {
   return 0;
 }
 int scn_get_math_mode(void) { return scn::g_math_mode; }
+int scn_set_deterministic(int on) {
+  scn::g_deterministic = on ? 1 : 0;
+  return 0;
+}
+int scn_get_deterministic(void) { return scn::g_deterministic.load(); }
 int scn_tensor_core_path_available(void) { return scn::tc_available(); }
 
 int scn_metadata_create(scn_metadata **out, void *stream) {

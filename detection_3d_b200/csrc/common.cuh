@@ -56,11 +56,23 @@ enum DebugCounter {
   kCntTrainReplay = 11,    // backward passes run by the program executor (scn_program_backward)
   kCntDwPlanLaunch = 13,   // weight-gradient launches driven by the output-stationary plan (conv_dw_plan_tc)
   kCntBwdOperandReused = 12, // bf16 operand copies the weight-gradient kernel took from its caller instead of converting again
+  kCntFloatAtomic = 14,    // launches that accumulated floats with atomics, i.e. whose result depends on the order the atomics land in
   kCntCounters = 16
 };
 extern std::atomic<long> g_counters[kCntCounters];
 
 static inline int cdiv(long a, long b) { return (int)((a + b - 1) / b); }
+
+// ---------------------------------------------------------------- deterministic mode (scn_set_deterministic)
+// On: every launcher that would accumulate floats with atomics writes per-work-item partials to fixed slots instead and sums them
+// in index order, so that results do not depend on which CTA ran first.  Read at launch time.
+bool deterministic();
+// grow-only scratch of the deterministic mode's partial sums, one per (device, stream); uses on one stream are ordered
+int det_scratch(cudaStream_t s, size_t bytes, void **out);
+// out[map(j)] = sum over p = 0 .. nPart-1 of part[p * width + j] for j < width, in an order fixed by (nPart, width) alone;
+// map(j) = j, or (j / seg) * segStride + j % seg when seg > 0.  T = float or double (accumulated in double).
+template <class T>
+int ordered_sum(const T *part, int nPart, long width, T *out, cudaStream_t s, long seg = 0, long segStride = 0);
 
 // ---------------------------------------------------------------- programmatic dependent launch (sm_90+)
 // The layer kernels of a forward sit back to back on one stream, ~100 of them, half of them a few microseconds long.  Launched with

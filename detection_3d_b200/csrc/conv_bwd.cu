@@ -5,7 +5,8 @@
 //          (dOut, W^T) with the pair columns swapped, lists back to back (a source row occurs at
 //          most once per list, so the read-modify-write is race free, as in the reference).
 //   dW[k] = gather(in, rules_k.src)^T @ gather(dOut, rules_k.dst) -> split over rule chunks, fp32
-//          atomics into dW (replaces dConvolution_KMxKN_backward_dW_A/B, SCN/CUDA/Convolution.cu:249-410).
+//          atomics into dW (replaces dConvolution_KMxKN_backward_dW_A/B, SCN/CUDA/Convolution.cu:249-410); in deterministic mode
+//          each chunk stores its partial dW[k] into its own slot and ordered_sum adds the chunks in chunk order.
 // Reference semantics: SCN/CPU/Convolution.cpp:81-115,152-185, SCN/CPU/Deconvolution.cpp:43-77.
 #include "common.cuh"
 
@@ -34,7 +35,7 @@ int transpose_weights(const float *W, float *Wt, int K, int Cin, int Cout, int r
 
 constexpr int BM = 64, BN = 64, BK = 16, BPAD = 4;
 __global__ void __launch_bounds__(256) k_dw(const float *__restrict__ in, const float *__restrict__ dOut, float *__restrict__ dW, const int2 *__restrict__ pairs,
-                                            int start, int len, int chunk, int Cin, int Cout, int srcIsY) {
+                                            int start, int len, int chunk, int Cin, int Cout, int srcIsY, float *__restrict__ part) {
   __shared__ __align__(16) float A_s[BK][BM + BPAD];
   __shared__ __align__(16) float B_s[BK][BN];
   __shared__ int s_src[BK], s_dst[BK];
@@ -85,15 +86,44 @@ __global__ void __launch_bounds__(256) k_dw(const float *__restrict__ in, const 
 #pragma unroll
     for (int j = 0; j < 4; j++) {
       int ci = ci0 + ty * 4 + i, co = co0 + tx * 4 + j;
-      if (ci < Cin && co < Cout) atomicAdd(dW + (long)ci * Cout + co, acc[i][j]);
+      if (ci < Cin && co < Cout) {
+        if (part) part[((long)blockIdx.x * Cin + ci) * Cout + co] = acc[i][j];
+        else atomicAdd(dW + (long)ci * Cout + co, acc[i][j]);
+      }
     }
 }
-__global__ void k_colsum(const float *__restrict__ x, long n, int C, float *__restrict__ out) {
+__global__ void k_colsum(const float *__restrict__ x, long n, int C, float *__restrict__ out, float *__restrict__ part) {
   int c = blockIdx.y * blockDim.x + threadIdx.x;
   if (c >= C) return;
   float s = 0.f;
   for (long r = blockIdx.x; r < n; r += gridDim.x) s += x[r * C + c];
-  atomicAdd(out + c, s);
+  if (part) part[(long)blockIdx.x * C + c] = s;
+  else atomicAdd(out + c, s);
+}
+// d_bias = column sums of d_out (zeroed by the caller)
+static int column_sums(const float *d_out, long n, int C, float *d_bias, cudaStream_t s) {
+  if (!n) return 0;
+  const int parts = kSMs * 2;
+  float *part = nullptr;
+  if (deterministic()) SCN_TRY(det_scratch(s, (size_t)parts * C * 4, (void **)&part));
+  else ++g_counters[kCntFloatAtomic];
+  k_colsum<<<dim3(parts, cdiv(C, 128)), 128, 0, LS(s)>>>(d_out, n, C, d_bias, part);
+  if (part) SCN_TRY(ordered_sum(part, parts, (long)C, d_bias, s));
+  SCN_CUDA(cudaGetLastError());
+  return 0;
+}
+// dW (zeroed by the caller) += the chunks of one rule list (pairs == nullptr: dense rows, row i pairs with row i)
+static int dw_chunks(const float *in, const float *d_out, float *dW, const int2 *pairs, int start, int len, int Cin, int Cout, int srcIsY, cudaStream_t s) {
+  int chunk = std::max(256, cdiv(len, kSMs * 4));
+  chunk = (chunk + BK - 1) / BK * BK;
+  dim3 grid(cdiv(len, chunk), cdiv(Cin, BM), cdiv(Cout, BN));
+  float *part = nullptr;
+  if (deterministic()) SCN_TRY(det_scratch(s, (size_t)grid.x * Cin * Cout * 4, (void **)&part));
+  else ++g_counters[kCntFloatAtomic];
+  k_dw<<<grid, 256, 0, LS(s)>>>(in, d_out, dW, pairs, start, len, chunk, Cin, Cout, srcIsY, part);
+  if (part) SCN_TRY(ordered_sum(part, (int)grid.x, (long)Cin * Cout, dW, s));
+  SCN_CUDA(cudaGetLastError());
+  return 0;
 }
 
 // NetworkInNetwork_accGradParameters (SCN/CPU/NetworkInNetwork.cpp:36-46): dW = in^T @ d_out over dense rows (row i pairs with row i),
@@ -102,15 +132,10 @@ int dense_rows_dw(const float *in, const float *d_out, float *dW, float *d_bias,
   SCN_CUDA(cudaMemsetAsync(dW, 0, (size_t)Cin * Cout * 4, s));
   if (d_bias) {
     SCN_CUDA(cudaMemsetAsync(d_bias, 0, (size_t)Cout * 4, s));
-    if (n) k_colsum<<<dim3(kSMs * 2, cdiv(Cout, 128)), 128, 0, LS(s)>>>(d_out, n, Cout, d_bias);
+    SCN_TRY(column_sums(d_out, n, Cout, d_bias, s));
   }
   if (n == 0) return 0;
-  int chunk = std::max(256, cdiv(n, kSMs * 4));
-  chunk = (chunk + BK - 1) / BK * BK;
-  dim3 grid(cdiv(n, chunk), cdiv(Cin, BM), cdiv(Cout, BN));
-  k_dw<<<grid, 256, 0, LS(s)>>>(in, d_out, dW, nullptr, 0, (int)n, chunk, Cin, Cout, 0);
-  SCN_CUDA(cudaGetLastError());
-  return 0;
+  return dw_chunks(in, d_out, dW, nullptr, 0, (int)n, Cin, Cout, 0, s);
 }
 
 // skipDIn: the caller computes d_in itself (tensor-core forward kernel on (d_out, W^T)); only dW / d_bias here
@@ -121,7 +146,7 @@ int conv_backward_simt(const float *in, float *d_in, const float *d_out, const f
   SCN_CUDA(cudaMemsetAsync(dW, 0, (size_t)K * Cin * Cout * 4, s));
   if (d_bias) {
     SCN_CUDA(cudaMemsetAsync(d_bias, 0, (size_t)Cout * 4, s));
-    if (nOutRows) k_colsum<<<dim3(kSMs * 2, cdiv(Cout, 128)), 128, 0, LS(s)>>>(d_out, nOutRows, Cout, d_bias);
+    SCN_TRY(column_sums(d_out, nOutRows, Cout, d_bias, s));
   }
   // pairs == nullptr: the caller did not build the rule lists (input gradient done / not wanted, weight gradient from the plan)
   if (pairs && offHost[K] == 0) return 0;
@@ -143,10 +168,7 @@ int conv_backward_simt(const float *in, float *d_in, const float *d_out, const f
   for (int L_ = 0; L_ < K; L_++) {
     int len = offHost[L_ + 1] - offHost[L_];
     if (!len) continue;
-    int chunk = std::max(256, cdiv(len, kSMs * 4));
-    chunk = (chunk + BK - 1) / BK * BK;
-    dim3 grid(cdiv(len, chunk), cdiv(Cin, BM), cdiv(Cout, BN));
-    k_dw<<<grid, 256, 0, LS(s)>>>(in, d_out, dW + (long)L_ * Cin * Cout, pairs, offHost[L_], len, chunk, Cin, Cout, srcIsY);
+    SCN_TRY(dw_chunks(in, d_out, dW + (long)L_ * Cin * Cout, pairs, offHost[L_], len, Cin, Cout, srcIsY, s));
   }
   SCN_CUDA(cudaGetLastError());
   return 0;

@@ -66,6 +66,8 @@ struct TcParams {
   int dbg;    // developer switches (SCN_TC_DBG): 1 = skip A gathers, 2 = skip B copies, 4 = skip MMAs
   int kSplit; // > 1: the filter offsets of a work item are split over kSplit CTAs, epilogue accumulates atomically
   unsigned *sched; // dynamic work distribution: [0] next work item, [1] CTAs that have drawn their last item (self-resetting); null = static stride
+  double *statsPart; // deterministic mode, with stats: [work item][epilogue warp][2][Cout] per-item sums instead of atomics into `stats`
+  float *part;       // deterministic mode, kSplit > 1: [kSplit][nOut][Cout] per-split partial outputs instead of atomics into `out`
 };
 
 // ------------------------------------------------------------------ PTX helpers
@@ -253,7 +255,8 @@ __device__ __forceinline__ void sched_publish(const Sched &S, int n, int wi) {
 // barrier hand-offs.
 // CTAS = CTAs per SM the variant is built for (register cap: 65536 / (CTAS x threads)): <PW 8, CTAS 2> caps the kernel at 72
 // registers (a few spilled words in the epilogue) and doubles the gather issue rate of the two-CTA configuration.
-template <bool BF16, int PW, int G, int CTAS>
+// DET = deterministic mode (P.part / P.statsPart may be set): a separate instantiation, so that the default kernels stay as they are.
+template <bool BF16, int PW, int G, int CTAS, bool DET>
 __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_COLS == 16 ? 384 : 320)), CTAS) conv_plan_tc(const TcParams P) {
   constexpr int TM = G == 4 ? 2 : kMaxT; // tiles per item the producers keep neighbour ids for (G ids per row and tile)
   constexpr int kProdWarps = PW;
@@ -319,7 +322,7 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
       for (int t = 0; t < kMaxT; t++) {
         if (t >= P.T || I.st * P.T + t >= P.nTiles) continue;
         const bool started = I.m[t] != 0ull;
-        if (!started && P.kSplit > 1 && !((P.addend || P.bias) && I.part == 0)) continue; // nothing to add
+        if (!started && P.kSplit > 1 && !(DET && P.part) && !((P.addend || P.bias) && I.part == 0)) continue; // nothing to add (a partial slot is written even then)
         int rows[NI];
 #pragma unroll
         for (int i = 0; i < NI; i++) rows[i] = __shfl_sync(0xffffffffu, myRow[t], i * RPI + rsub);
@@ -393,6 +396,10 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
                   *reinterpret_cast<uint2 *>(static_cast<unsigned char *>(P.out16) + ((size_t)rows[i] * P.Cout + c0 + cc) * 2) = pk;
                 }
               }
+          } else if (DET && P.part) { // offsets split over CTAs, deterministic mode: this split's partial rows into its own slot
+#pragma unroll
+            for (int i = 0; i < NI; i++)
+              if (rows[i] >= 0) *reinterpret_cast<float4 *>(P.part + ((size_t)I.part * P.nOut + rows[i]) * P.Cout + c0 + cc) = o[i];
           } else { // offsets split over CTAs: accumulate into the launcher-zeroed output
 #pragma unroll
             for (int i = 0; i < NI; i++)
@@ -406,8 +413,19 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(accEmpty + a));
+      if (DET && P.statsPart) { // deterministic mode: this item's sums of this warp's rows into slot (item, warp); the launcher adds the slots in order
+        const int c = rsub * EC + cc;
+        if (c < P.Cout) {
+          double *dst = P.statsPart + ((size_t)wi * 4 + warp) * 2 * P.Cout + c;
+          dst[0] = sAcc.x; dst[1] = sAcc.y; dst[2] = sAcc.z; dst[3] = sAcc.w;
+          dst += P.Cout;
+          dst[0] = qAcc.x; dst[1] = qAcc.y; dst[2] = qAcc.z; dst[3] = qAcc.w;
+        }
+        sAcc = make_float4(0.f, 0.f, 0.f, 0.f);
+        qAcc = sAcc;
+      }
     }
-    if (P.stats) { // one double atomic per (warp, channel) into one of kBnReplicas accumulators
+    if (P.stats && !(DET && P.statsPart)) { // one double atomic per (warp, channel) into one of kBnReplicas accumulators
       const int c = rsub * EC + cc;
       if (c < P.Cout) {
         double *rep = P.stats + (size_t)(blockIdx.x % kBnReplicas) * 2 * kFusedStatsC;
@@ -780,6 +798,27 @@ int to_bf16(const float *x, void *y, long n, cudaStream_t s) {
   SCN_CUDA(cudaGetLastError());
   return 0;
 }
+// deterministic mode, split filter offsets: out = partial of split 0 + split 1 + ... in that order (bias and addend are in split 0's),
+// with the bf16 copy of the finished rows (what the memset + atomic epilogue + k_to_bf16 do otherwise)
+__global__ void __launch_bounds__(256) k_split_sum(const float4 *__restrict__ part, int kSplit, long n4, float4 *__restrict__ out, uint2 *__restrict__ out16) {
+  pdl_launch_dependents();
+  pdl_wait();
+  for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
+    float4 a = part[i];
+    for (int k = 1; k < kSplit; k++) {
+      const float4 b = part[(long)k * n4 + i];
+      a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
+    }
+    out[i] = a;
+    if (out16) {
+      __nv_bfloat162 lo = __floats2bfloat162_rn(a.x, a.y), hi = __floats2bfloat162_rn(a.z, a.w);
+      uint2 pk;
+      pk.x = *reinterpret_cast<unsigned int *>(&lo);
+      pk.y = *reinterpret_cast<unsigned int *>(&hi);
+      out16[i] = pk;
+    }
+  }
+}
 static int stream_scratch(cudaStream_t s, int slot, size_t bytes, void **out);
 // bf16 copy of a backward call's d_out, made once and read by both the input-gradient and the weight-gradient kernel
 int dout_bf16_copy(const float *d_out, long n, cudaStream_t s, const void **out) {
@@ -798,7 +837,8 @@ const void *bwd_in16_take() { const void *p = tl_bwd_in16; tl_bwd_in16 = nullptr
 // narrow input; slot 1: bf16 copy of an input that arrived without one -- one launch can need both, the second derived
 // from the first, so they must not share a buffer; slot 2: the operand pair of the weight-gradient kernel).  Uses of a
 // slot on one stream are ordered; cudaMallocAsync took milliseconds for these 150-300 MB blocks.
-enum ScratchSlot { kScratchPad = 0, kScratchBf16 = 1, kScratchDw = 2, kScratchDout = 3 }; // 3: bf16 copy of d_out shared by the two gradient kernels of a backward call
+// 3: bf16 copy of d_out shared by the two gradient kernels of a backward call; 4: partial sums of the deterministic mode (det_scratch)
+enum ScratchSlot { kScratchPad = 0, kScratchBf16 = 1, kScratchDw = 2, kScratchDout = 3, kScratchDet = 4 };
 static std::mutex g_scratch_mu;
 static std::map<std::tuple<int, cudaStream_t, int>, std::pair<void *, size_t>> g_scratch;
 static int stream_scratch(cudaStream_t s, int slot, size_t bytes, void **out) {
@@ -814,6 +854,7 @@ static int stream_scratch(cudaStream_t s, int slot, size_t bytes, void **out) {
   *out = e.first;
   return 0;
 }
+int det_scratch(cudaStream_t s, size_t bytes, void **out) { return stream_scratch(s, kScratchDet, bytes, out); }
 // Work-item counters of the dynamic distribution: two zero-initialised words per (device, stream); launches on one stream are
 // ordered and every launch leaves them zeroed again (sched_draw).
 static int sched_counters(cudaStream_t s, unsigned **out) {
@@ -849,6 +890,32 @@ static thread_local bool tl_lat_done = false;
 void lateral_arm(const float *in, const void *in16, const float *w, long long tag, int Cin, long rows) { tl_lat = Lateral{in, in16, w, tag, Cin, rows}; tl_lat_done = false; }
 bool lateral_take() { bool d = tl_lat_done; tl_lat.in = nullptr; tl_lat_done = false; return d; }
 bool epilogue_stats_take() { bool d = tl_stats_done; tl_stats = nullptr; tl_stats_done = false; return d; }
+template <bool DET>
+static int set_plan_attributes() {
+  const int half = (233472 - kBuildRoom) / 2 - 1024;
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<false, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<false, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 4, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 4, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<false, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  return 0;
+}
+template <bool DET>
+static cudaError_t launch_plan_variant(const TcParams &P, int packG, bool pw8, int ctas, int grid, int th2, size_t smem, cudaStream_t s) {
+  if (packG == 2) return pw8 ? launch_pdl(conv_plan_tc<true, 8, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<true, 4, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+  if (packG == 4) return pw8 ? launch_pdl(conv_plan_tc<true, 8, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<true, 4, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+  if (ctas == 2) {
+    if (P.bf16) return pw8 ? launch_pdl(conv_plan_tc<true, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<true, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+    return pw8 ? launch_pdl(conv_plan_tc<false, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<false, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+  }
+  if (P.bf16) return launch_pdl(conv_plan_tc<true, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
+  return launch_pdl(conv_plan_tc<false, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
+}
 // in16: optional bf16 copy of `in` (same layout); used in math mode 2 when Cin is a multiple of 64
 int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
                         int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, const int *tileW, int nWeights,
@@ -942,8 +1009,15 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   if (kSplitMaxItems < 0) kSplitMaxItems = getenv("SCN_TC_SPLIT_MAX") ? atoi(getenv("SCN_TC_SPLIT_MAX")) : 40;
   if (P.nSuper <= kSplitMaxItems && !tileW) P.kSplit = std::max(1, std::min(packG > 1 ? P.KG : K, kSMs * ctas / P.nSuper));
   P.stats = nullptr;
+  P.statsPart = nullptr;
+  P.part = nullptr;
+  const bool det = deterministic();
   if (tl_stats && P.kSplit == 1 && Cout <= kFusedStatsC && Cout % 32 == 0) { P.stats = tl_stats; tl_stats_done = true; ++g_counters[kCntEpilogueStats]; }
   tl_stats = nullptr;
+  if (P.stats) { // deterministic mode: per-(item, epilogue warp) sums, added in item order after the launch
+    if (det) SCN_TRY(det_scratch(s, (size_t)P.nSuper * 4 * 2 * Cout * sizeof(double), (void **)&P.statsPart));
+    else ++g_counters[kCntFloatAtomic];
+  }
   const size_t stageBytes = (size_t)P.T * kAtomBytes + (size_t)Cout * 128;
   P.S = (int)std::min<size_t>(envS > 0 ? envS : 6, (smemBudget - fixed) / stageBytes);
   SCN_CHECK(P.S >= 2, "tcgen05 path: shared memory budget exceeded");
@@ -955,7 +1029,8 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   SCN_CHECK(out || (P.kSplit == 1 && out16), "tcgen05 path: fp32 output dropped on a launch that needs it");
   ++g_counters[kCntTcLaunch];
   if (P.kSplit > 1) ++g_counters[kCntSplitLaunch];
-  if (P.kSplit > 1) SCN_CUDA(cudaMemsetAsync(out, 0, (size_t)nOut * Cout * 4, s));
+  if (P.kSplit > 1 && det) SCN_TRY(det_scratch(s, (size_t)P.kSplit * nOut * Cout * 4, (void **)&P.part)); // (k_split_sum writes every output row)
+  else if (P.kSplit > 1) { ++g_counters[kCntFloatAtomic]; SCN_CUDA(cudaMemsetAsync(out, 0, (size_t)nOut * Cout * 4, s)); }
   unsigned char *wimg = nullptr;
   bool wimgOwned = false;
   SCN_TRY(get_wimg(W, wTag, nWeights, Cin, CinW, Cout, packG > 1 ? 1 + 16 * packG : P.bf16, s, &wimg, &wimgOwned, wT));
@@ -979,17 +1054,8 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   tl_lat.in = nullptr;
   static bool attr = false;
   if (!attr) {
-    const int half = (233472 - kBuildRoom) / 2 - 1024;
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<false, 8, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<false, 4, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 4, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 4, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 4, 4, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<false, 8, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-    SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 4, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+    SCN_TRY(set_plan_attributes<false>());
+    SCN_TRY(set_plan_attributes<true>());
     attr = true;
   }
   static int envSms = -1;
@@ -1009,15 +1075,8 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   if (envPw8 < 0) envPw8 = getenv("SCN_TC_PW8") ? atoi(getenv("SCN_TC_PW8")) : 0;
   const bool pw8 = ctas == 2 && ((packG > 1 && (envPw8 & 1)) || (packG == 1 && (envPw8 & 2)));
   const int th2 = 32 * (pw8 ? 14 : 10);
-  if (packG == 2) { if (pw8) SCN_CUDA(launch_pdl(conv_plan_tc<true, 8, 2, 2>, dim3(grid), dim3(th2), (size_t)smem, LS(s), P)); else SCN_CUDA(launch_pdl(conv_plan_tc<true, 4, 2, 2>, dim3(grid), dim3(th2), (size_t)smem, LS(s), P)); }
-  else if (packG == 4) { if (pw8) SCN_CUDA(launch_pdl(conv_plan_tc<true, 8, 4, 2>, dim3(grid), dim3(th2), (size_t)smem, LS(s), P)); else SCN_CUDA(launch_pdl(conv_plan_tc<true, 4, 4, 2>, dim3(grid), dim3(th2), (size_t)smem, LS(s), P)); }
-  else if (ctas == 2) {
-    if (P.bf16) { if (pw8) SCN_CUDA(launch_pdl(conv_plan_tc<true, 8, 1, 2>, dim3(grid), dim3(th2), (size_t)smem, LS(s), P)); else SCN_CUDA(launch_pdl(conv_plan_tc<true, 4, 1, 2>, dim3(grid), dim3(th2), (size_t)smem, LS(s), P)); }
-    else { if (pw8) SCN_CUDA(launch_pdl(conv_plan_tc<false, 8, 1, 2>, dim3(grid), dim3(th2), (size_t)smem, LS(s), P)); else SCN_CUDA(launch_pdl(conv_plan_tc<false, 4, 1, 2>, dim3(grid), dim3(th2), (size_t)smem, LS(s), P)); }
-  } else {
-    if (P.bf16) SCN_CUDA(launch_pdl(conv_plan_tc<true, 8, 1, 1>, dim3(grid), dim3(32 * 14), (size_t)smem, LS(s), P));
-    else SCN_CUDA(launch_pdl(conv_plan_tc<false, 8, 1, 1>, dim3(grid), dim3(32 * 14), (size_t)smem, LS(s), P));
-  }
+  if (det) SCN_CUDA(launch_plan_variant<true>(P, packG, pw8, ctas, grid, th2, smem, s));
+  else SCN_CUDA(launch_plan_variant<false>(P, packG, pw8, ctas, grid, th2, smem, s));
   SCN_CUDA(cudaGetLastError());
   if (envProf) { // developer aid: mean stall cycles per role over the CTAs of this launch
     static long long h[2 * kSMs * 32];
@@ -1029,7 +1088,11 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
             ctas, grid, P.T, K, Cin, Cout, P.S, P.nAcc, P.kSplit, m[0], m[1], m[4], m[5], m[6], m[7], m[10], m[11], m[12], m[13], m[14], m[15], m[16], m[17]);
     cudaFreeAsync(P.prof, s);
   }
-  if (out16 && P.kSplit > 1 && nOutRows > 0) // partial sums were accumulated atomically: the bf16 copy needs the finished rows
+  if (P.statsPart) SCN_TRY(ordered_sum(P.statsPart, P.nSuper * 4, 2l * Cout, P.stats, s, Cout, kFusedStatsC)); // into replica 0
+  if (P.part) // the split partials in split order, and the bf16 copy from the same registers
+    SCN_CUDA(launch_pdl(k_split_sum, dim3(stream_grid((long)nOut * Cout / 4, 256)), dim3(256), 0, LS(s), reinterpret_cast<const float4 *>(P.part), P.kSplit,
+                        (long)nOut * Cout / 4, reinterpret_cast<float4 *>(out), static_cast<uint2 *>(out16)));
+  else if (out16 && P.kSplit > 1 && nOutRows > 0) // partial sums were accumulated atomically: the bf16 copy needs the finished rows
     SCN_CUDA(launch_pdl(k_to_bf16, dim3(stream_grid(nOutRows * Cout / 4, 256)), dim3(256), 0, LS(s), out, static_cast<uint2 *>(out16), nOutRows * Cout / 4));
   if (wimgOwned) cudaFreeAsync(wimg, s);
   if (wimg2Owned) cudaFreeAsync(wimg2, s);
@@ -1137,6 +1200,7 @@ struct DwParams {
   const int2 *pairs;
   const int *d_off;           // K + 1 list offsets
   float *dW;
+  float *part;                // deterministic mode: [item][Cin][Cout], item w's partial dW[w % K] (plain stores), summed in part order afterwards
   int K, Cin, Cout, nC, srcIsY, rowBytesA, rowBytesB, R, S, nAcc; // nC: parts per rule list
 };
 __device__ __forceinline__ uint64_t smem_desc_mn_sw128(uint32_t addr, uint32_t lboBytes) {
@@ -1188,19 +1252,27 @@ __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwPara
     for (int w = blockIdx.x; w < nItems; w += gridDim.x) {
       int k, r0, cnt;
       item(w, k, r0, cnt);
-      if (cnt <= 0) continue;
+      if (cnt <= 0) {
+        if (P.part) // (an empty part still owns a slot of the ordered sum)
+          for (long i = tid; i < (long)P.Cin * P.Cout; i += 128) P.part[(size_t)w * P.Cin * P.Cout + i] = 0.f;
+        continue;
+      }
       const int it = itN++;
       const int a = P.nAcc == 2 ? (it & 1) : 0, use = P.nAcc == 2 ? (it >> 1) : it;
       mbar_wait(smem_u32(accFull + a), use & 1);
       tc_fence_after();
       for (int mh = 0; mh < nMh; mh++) {
         const int ci = mh * 128 + warp * 32 + lane;
-        float *dst = P.dW + ((size_t)k * P.Cin + ci) * P.Cout;
+        float *dst = P.part ? P.part + ((size_t)w * P.Cin + ci) * P.Cout : P.dW + ((size_t)k * P.Cin + ci) * P.Cout;
         if (mh * 128 + warp * 32 >= P.Cin) continue; // rows of the channel padding (warp-uniform)
         for (int c0 = 0; c0 < P.Cout; c0 += 32) {
           uint32_t v[32];
           tmem_ld(tmemBase + ((uint32_t)(warp * 32) << 16) + (uint32_t)(a * accCols + mh * P.Cout + c0), v);
-          if (ci < P.Cin) {
+          if (ci < P.Cin && P.part) {
+#pragma unroll
+            for (int j = 0; j < 32; j += 4)
+              *reinterpret_cast<float4 *>(dst + c0 + j) = make_float4(__uint_as_float(v[j]), __uint_as_float(v[j + 1]), __uint_as_float(v[j + 2]), __uint_as_float(v[j + 3]));
+          } else if (ci < P.Cin) {
 #pragma unroll
             for (int j = 0; j < 32; j++) atomicAdd(dst + c0 + j, __uint_as_float(v[j]));
           }
@@ -1527,7 +1599,7 @@ int from_bf16(const void *x, float *y, long n, cudaStream_t s) {
 bool dw_plan_ok(int Cin, int Cout, int K, int mathMode) {
   static int planOn = -1;
   if (planOn < 0) planOn = getenv("SCN_DW_PLAN") ? atoi(getenv("SCN_DW_PLAN")) : 0;
-  if (!planOn || mathMode != 2 || !tc_available()) return false;
+  if (!planOn || mathMode != 2 || !tc_available() || deterministic()) return false; // (its partial sums are not indexed by work item)
   return !((Cin % 32 != 0 && Cin > 32) || Cin > 256 || (Cin > 128 && Cin % 128 != 0) || Cout % 32 != 0 || Cout > 256 || ((Cin + 127) / 128) * Cout > 512 || K > 64);
 }
 // dW must be zero on entry.  Returns 1 when the configuration is not supported (the caller then uses the CUDA-core kernel).
@@ -1545,7 +1617,7 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
   // (100 % row fill, equal work items) against 0.69 ms with the plan (row fill 89 %, items of unequal cost), all 39 launches of a
   // step 2.6 against 4.2 ms -- the list kernel is the default, SCN_DW_PLAN=1 selects the plan-driven one.
   if (planOn < 0) planOn = getenv("SCN_DW_PLAN") ? atoi(getenv("SCN_DW_PLAN")) : 0;
-  const bool usePlan = planOn && planNbr && planMask && planPos > 0;
+  const bool usePlan = planOn && planNbr && planMask && planPos > 0 && !deterministic();
   SCN_CHECK(usePlan || offHost, "weight gradient: neither a plan nor rule lists");
   const long total = usePlan ? 1 : offHost[K];
   if (total == 0) return 0;
@@ -1599,6 +1671,7 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
     Q.prof = nullptr;
     if (envProf) { SCN_CUDA(cudaMalloc((void **)&Q.prof, kSMs * 8 * 8)); SCN_CUDA(cudaMemsetAsync(Q.prof, 0, kSMs * 8 * 8, s)); }
     SCN_TRY(sched_counters(s, &Q.sched));
+    ++g_counters[kCntFloatAtomic];
     conv_dw_plan_tc<true><<<gridQ, 32 * (6 + kDwProd), smemQ, LS(s)>>>(Q);
     SCN_CUDA(cudaGetLastError());
     if (envProf) { // developer aid: per-role cycle counters, mean and max over the CTAs
@@ -1622,6 +1695,15 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
   long nC = std::max<long>(1, avgLen / envPart);
   if (K * nC < 3 * kSMs) nC = std::max<long>(nC, std::min<long>(cdiv(3 * kSMs, K), std::max<long>(1, avgLen / (4 * P.R))));
   P.nC = (int)std::min<long>(nC, 4096);
+  P.part = nullptr;
+  if (deterministic()) { // one dW-sized slot per work item, at most kDetDwBytes in all (fewer, longer parts beyond that)
+    constexpr size_t kDetDwBytes = 256u << 20;
+    const size_t perItem = (size_t)Cin * Cout * 4;
+    P.nC = (int)std::max<size_t>(1, std::min<size_t>((size_t)P.nC, kDetDwBytes / (perItem * K)));
+    SCN_TRY(det_scratch(s, (size_t)K * P.nC * perItem, (void **)&P.part));
+  } else {
+    ++g_counters[kCntFloatAtomic];
+  }
   const long nItems = (long)K * P.nC;
   const size_t smemBytes = (size_t)P.S * stageBytes + 64 * 8 + 64;
   static bool attr = false;
@@ -1634,6 +1716,7 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
   if (bf16) conv_dw_tc<true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(P);
   else conv_dw_tc<false><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(P);
   SCN_CUDA(cudaGetLastError());
+  if (P.part) SCN_TRY(ordered_sum(P.part, P.nC, (long)K * Cin * Cout, dW, s)); // item c K + k = part c of list k: rows [nC][K][Cin][Cout]
   return 0;
 }
 

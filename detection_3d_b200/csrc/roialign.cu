@@ -142,6 +142,7 @@ int run(scn_metadata *m, const long sz[3], const float *feats, float *dFeats, in
   SCN_CHECK(smem <= 200 * 1024, "pooled output too large for the staging buffer");
   if (smem > 48 * 1024) SCN_CUDA(cudaFuncSetAttribute(k_roi_align<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const unsigned grid = (unsigned)(nRois * PH);
+  if (backward) ++g_counters[kCntFloatAtomic]; // (no deterministic variant: the Python layer raises or warns under torch.use_deterministic_algorithms)
   if (backward) k_roi_align<true><<<grid, 256, 0, LS(s)>>>(v, g->p2id, nullptr, dFeats, C, ext[0], ext[1], ext[2], rois, scale, PH, PW, PZ, sampling, nullptr, dOut);
   else k_roi_align<false><<<grid, 256, smem, LS(s)>>>(v, g->p2id, feats, nullptr, C, ext[0], ext[1], ext[2], rois, scale, PH, PW, PZ, sampling, out, nullptr);
   SCN_CUDA(cudaGetLastError());

@@ -45,14 +45,43 @@ __device__ __forceinline__ void bn_finalize_channel(const BnFin &F, int c, doubl
   F.scale[c] = w;
   F.shift[c] = -mean * w + (F.bias ? F.bias[c] : 0.f);
 }
+// ------------------------------------------------------------------ ordered sums (deterministic mode)
+// Column j of a [nPart][width] matrix of partial sums: 32 row lanes each add the rows lane, lane + 32, ... in ascending order, then
+// one thread adds the 32 lane sums in lane order.  The order depends on nPart and width only, never on the scheduling.
+template <class T>
+__global__ void __launch_bounds__(1024) k_ordered_sum(const T *__restrict__ part, int nPart, long width, T *__restrict__ out, long seg, long segStride) {
+  __shared__ double red[32][33];
+  const long j = (long)blockIdx.x * 32 + threadIdx.x;
+  double a = 0.0;
+  if (j < width)
+    for (int p = threadIdx.y; p < nPart; p += 32) a += (double)part[(long)p * width + j];
+  red[threadIdx.y][threadIdx.x] = a;
+  __syncthreads();
+  if (threadIdx.y == 0 && j < width) {
+    double t = 0.0;
+    for (int l = 0; l < 32; l++) t += red[l][threadIdx.x];
+    out[seg > 0 ? (j / seg) * segStride + j % seg : j] = (T)t;
+  }
+}
+template <class T>
+int ordered_sum(const T *part, int nPart, long width, T *out, cudaStream_t s, long seg, long segStride) {
+  if (width <= 0) return 0;
+  k_ordered_sum<T><<<cdiv(width, 32), dim3(32, 32), 0, LS(s)>>>(part, nPart, width, out, seg, segStride);
+  SCN_CUDA(cudaGetLastError());
+  return 0;
+}
+template int ordered_sum<float>(const float *, int, long, float *, cudaStream_t, long, long);
+template int ordered_sum<double>(const double *, int, long, double *, cudaStream_t, long, long);
+
 // ------------------------------------------------------------------ BN statistics
 // stats[0..C) = sum x, stats[C..2C) = sum x^2 (or sum of (x-shift)^2 terms), in double.
 // Each thread owns one float4 column group and strides over rows; per-CTA partials are reduced
 // in shared memory and added with one double atomic per channel per CTA.
 // The CTA that finishes last (ticket) turns the sums into scale / shift and re-zeroes sums and ticket:
 // statistics + finalize are one launch.
+// part (deterministic mode): the CTA's sums go to row blockIdx.x of part [grid][2][C] instead; ordered_sum + k_bn_finalize follow.
 __global__ void __launch_bounds__(256) k_bn_stats(const float *__restrict__ x, long n, int C, int rowsPerCta, double *__restrict__ stats,
-                                                  unsigned *ticket, BnFin F) {
+                                                  unsigned *ticket, BnFin F, double *__restrict__ part) {
   extern __shared__ float s_red[]; // [2][256][4]
   const int cv = C >> 2;           // float4 groups per row
   const int tid = threadIdx.x;
@@ -90,13 +119,20 @@ __global__ void __launch_bounds__(256) k_bn_stats(const float *__restrict__ x, l
       a[0] += u.x; a[1] += u.y; a[2] += u.z; a[3] += u.w;
       b[0] += w.x; b[1] += w.y; b[2] += w.z; b[3] += w.w;
     }
-    double *rep = stats + (size_t)(blockIdx.x % kBnReplicas) * 2 * kBnMaxC; // same-address double atomics cost ~45 ns each: spread them
+    if (part) {
+      double *row = part + (size_t)blockIdx.x * 2 * C;
 #pragma unroll
-    for (int j = 0; j < 4; j++) {
-      atomicAdd(rep + tid * 4 + j, a[j]);
-      atomicAdd(rep + C + tid * 4 + j, b[j]);
+      for (int j = 0; j < 4; j++) { row[tid * 4 + j] = a[j]; row[C + tid * 4 + j] = b[j]; }
+    } else {
+      double *rep = stats + (size_t)(blockIdx.x % kBnReplicas) * 2 * kBnMaxC; // same-address double atomics cost ~45 ns each: spread them
+#pragma unroll
+      for (int j = 0; j < 4; j++) {
+        atomicAdd(rep + tid * 4 + j, a[j]);
+        atomicAdd(rep + C + tid * 4 + j, b[j]);
+      }
     }
   }
+  if (part) return; // (uniform over the grid)
   __shared__ bool last;
   __threadfence();
   __syncthreads();
@@ -171,7 +207,8 @@ __global__ void __launch_bounds__(256) k_bn_small(const float *__restrict__ x, f
   }
 }
 // scalar fallback for C % 4 != 0 (C <= 256)
-__global__ void __launch_bounds__(256) k_bn_stats_scalar(const float *__restrict__ x, long n, int C, int rowsPerCta, double *__restrict__ stats) {
+__global__ void __launch_bounds__(256) k_bn_stats_scalar(const float *__restrict__ x, long n, int C, int rowsPerCta, double *__restrict__ stats,
+                                                         double *__restrict__ part) {
   __shared__ float S[256], Q[256];
   const int tid = threadIdx.x;
   const int rowLanes = 256 / C;
@@ -185,8 +222,8 @@ __global__ void __launch_bounds__(256) k_bn_stats_scalar(const float *__restrict
   if (tid < C) {
     double a = 0, b = 0;
     for (int l = 0; l < rowLanes; l++) { a += S[l * C + tid]; b += Q[l * C + tid]; }
-    atomicAdd(stats + tid, a);
-    atomicAdd(stats + C + tid, b);
+    if (part) { part[(size_t)blockIdx.x * 2 * C + tid] = a; part[(size_t)blockIdx.x * 2 * C + C + tid] = b; }
+    else { atomicAdd(stats + tid, a); atomicAdd(stats + C + tid, b); }
   }
 }
 
@@ -311,14 +348,18 @@ int bn_forward(const float *x, float *y, long n, int C, float *saveMean, float *
     // 1073 CTAs -> 48 us for a 17 MB input): at most 4 CTAs per SM, >= 256 rows each, spread over kBnReplicas accumulators
     int rowsPerCta = (int)std::max<long>(256, (n + kSMs * 4 - 1) / (kSMs * 4));
     int grid = cdiv(n, rowsPerCta);
+    double *part = nullptr; // deterministic mode: per-CTA sums, added in CTA order into replica 0 (k_bn_finalize reads it)
+    if (deterministic()) SCN_TRY(det_scratch(s, (size_t)grid * 2 * C * sizeof(double), (void **)&part));
+    else ++g_counters[kCntFloatAtomic];
     if (C % 4 == 0) {
       SCN_CHECK(C / 4 <= 256, "BatchNorm: more than 1024 channels not supported");
-      k_bn_stats<<<grid, 256, 2 * 256 * 16, LS(s)>>>(x, n, C, rowsPerCta, stats, ticket, F); // last CTA finalizes
-      finalized = true;
+      k_bn_stats<<<grid, 256, 2 * 256 * 16, LS(s)>>>(x, n, C, rowsPerCta, stats, ticket, F, part); // last CTA finalizes
+      finalized = !part;
     } else {
       SCN_CHECK(C <= 256, "BatchNorm: channel count not a multiple of 4 must be <= 256");
-      k_bn_stats_scalar<<<grid, 256, 0, LS(s)>>>(x, n, C, rowsPerCta, stats);
+      k_bn_stats_scalar<<<grid, 256, 0, LS(s)>>>(x, n, C, rowsPerCta, stats, part);
     }
+    if (part) SCN_TRY(ordered_sum(part, grid, 2l * C, stats, s));
   }
   if (!finalized) k_bn_finalize<<<cdiv(C, 128), 128, 0, LS(s)>>>(stats, F);
   if (n) {
@@ -335,7 +376,8 @@ int bn_forward(const float *x, float *y, long n, int C, float *saveMean, float *
 // written back into dy (the reference rewrites d_output in place, :79-82), per-channel sum d and
 // sum (x-mean)*d.  Pass 2: dx = (d - mean(d) - (x-mean)*k) * invstd * gamma.
 __global__ void __launch_bounds__(256) k_bn_bwd_stats(const float *__restrict__ x, const float *__restrict__ y, float *__restrict__ dy, long n, int C,
-                                                      int rowsPerCta, const float *__restrict__ saveMean, float leak, double *__restrict__ stats) {
+                                                      int rowsPerCta, const float *__restrict__ saveMean, float leak, double *__restrict__ stats,
+                                                      double *__restrict__ part) {
   __shared__ float S[256], Q[256];
   const int tid = threadIdx.x;
   const int cols = min(C, 256), rowLanes = 256 / cols;
@@ -358,8 +400,8 @@ __global__ void __launch_bounds__(256) k_bn_bwd_stats(const float *__restrict__ 
     if (tid < cols && cb + tid < C) {
       double a = 0, b = 0;
       for (int l = 0; l < rowLanes; l++) { a += S[l * cols + tid]; b += Q[l * cols + tid]; }
-      atomicAdd(stats + cb + tid, a);
-      atomicAdd(stats + C + cb + tid, b);
+      if (part) { part[(size_t)blockIdx.x * 2 * C + cb + tid] = a; part[(size_t)blockIdx.x * 2 * C + C + cb + tid] = b; }
+      else { atomicAdd(stats + cb + tid, a); atomicAdd(stats + C + cb + tid, b); }
     }
     __syncthreads();
   }
@@ -392,7 +434,8 @@ __device__ __forceinline__ float4 bn_y4(const float4 *y, const uint2 *y16, long 
   return make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xffff0000u), __uint_as_float(v.y << 16), __uint_as_float(v.y & 0xffff0000u));
 }
 __global__ void __launch_bounds__(256) k_bn_bwd_stats4(const float4 *__restrict__ x, const float4 *__restrict__ y, const uint2 *__restrict__ y16, float4 *__restrict__ dy, long n, int C4,
-                                                       int rowsPerCta, const float *__restrict__ saveMean, float leak, double *__restrict__ stats) {
+                                                       int rowsPerCta, const float *__restrict__ saveMean, float leak, double *__restrict__ stats,
+                                                       double *__restrict__ part) {
   __shared__ float4 S[256], Q[256];
   const int tid = threadIdx.x;
   const int cols = min(C4, 256), rowLanes = 256 / cols;
@@ -428,7 +471,10 @@ __global__ void __launch_bounds__(256) k_bn_bwd_stats4(const float4 *__restrict_
       }
       const int ch = (cb + tid) * 4, C = C4 * 4;
 #pragma unroll
-      for (int j = 0; j < 4; j++) { atomicAdd(stats + ch + j, a[j]); atomicAdd(stats + C + ch + j, b[j]); }
+      for (int j = 0; j < 4; j++) {
+        if (part) { part[(size_t)blockIdx.x * 2 * C + ch + j] = a[j]; part[(size_t)blockIdx.x * 2 * C + C + ch + j] = b[j]; }
+        else { atomicAdd(stats + ch + j, a[j]); atomicAdd(stats + C + ch + j, b[j]); }
+      }
     }
     __syncthreads();
   }
@@ -460,10 +506,15 @@ int bn_backward(const float *x, float *dx, const float *y, float *dy, long n, in
                                   reinterpret_cast<uintptr_t>(saveMean) | reinterpret_cast<uintptr_t>(saveInvStd) | reinterpret_cast<uintptr_t>(weight)) & 15) == 0;
   if (n) {
     int rowsPerCta = (int)std::max<long>(64, (n + kSMs * 16 - 1) / (kSMs * 16));
+    const int grid = cdiv(n, rowsPerCta);
     SCN_CHECK(vec || y, "BatchNorm backward: the bf16-only output path needs 16-byte aligned rows of a multiple of 4 channels");
-    if (vec) k_bn_bwd_stats4<<<cdiv(n, rowsPerCta), 256, 0, LS(s)>>>(reinterpret_cast<const float4 *>(x), reinterpret_cast<const float4 *>(y), y ? nullptr : static_cast<const uint2 *>(y16),
-                                                                     reinterpret_cast<float4 *>(dy), n, C / 4, rowsPerCta, saveMean, leak, stats);
-    else k_bn_bwd_stats<<<cdiv(n, rowsPerCta), 256, 0, LS(s)>>>(x, y, dy, n, C, rowsPerCta, saveMean, leak, stats);
+    double *part = nullptr; // deterministic mode: per-CTA sums, added in CTA order
+    if (deterministic()) SCN_TRY(det_scratch(s, (size_t)grid * 2 * C * sizeof(double), (void **)&part));
+    else ++g_counters[kCntFloatAtomic];
+    if (vec) k_bn_bwd_stats4<<<grid, 256, 0, LS(s)>>>(reinterpret_cast<const float4 *>(x), reinterpret_cast<const float4 *>(y), y ? nullptr : static_cast<const uint2 *>(y16),
+                                                      reinterpret_cast<float4 *>(dy), n, C / 4, rowsPerCta, saveMean, leak, stats, part);
+    else k_bn_bwd_stats<<<grid, 256, 0, LS(s)>>>(x, y, dy, n, C, rowsPerCta, saveMean, leak, stats, part);
+    if (part) SCN_TRY(ordered_sum(part, grid, 2l * C, stats, s));
   }
   k_bn_bwd_finalize<<<cdiv(C, 128), 128, 0, LS(s)>>>(stats, n, C, saveInvStd, dWeight, dBias, gradMean, kk);
   if (n && vec) k_bn_bwd_apply4<<<stream_grid(n * C / 4, 256), 256, 0, LS(s)>>>(reinterpret_cast<const float4 *>(x), reinterpret_cast<const float4 *>(dy), reinterpret_cast<float4 *>(dx),

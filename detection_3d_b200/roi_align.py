@@ -4,6 +4,7 @@ maskrcnn_benchmark/layers/roi_align_rotated_3d.py:56-94 (`ROIAlignRotated3D(outp
 (sparse_3d_to_dense_2d) and samples the dense tensor (csrc/cuda/ROIAlignRotated3D_cuda.cu); here the CUDA kernel samples the
 sparse grid directly (detection_3d_b200/csrc/roialign.cu) -- same values, no 268 MB zero fill per call."""
 import ctypes as C
+import warnings
 
 import torch
 from torch import nn
@@ -17,6 +18,19 @@ def _extent(input_s3d):
     md, sz = input_s3d.metadata, input_s3d.spatial_size
     loc = md.getSpatialLocations(sz, device="cuda") if hasattr(md, "getSpatialLocations") else input_s3d.get_spatial_locations()
     return [int(v) for v in (loc[:, :3].max(0)[0] + 1).tolist()]
+
+
+def _alert_not_deterministic(op):
+    """torch's convention for an op without a deterministic implementation under torch.use_deterministic_algorithms(True): raise, or
+    warn in warn-only mode."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    msg = (f"{op} does not have a deterministic implementation, but you set 'torch.use_deterministic_algorithms(True)'. You can turn off "
+           "determinism just for this operation, or you can use the 'warn_only=True' option, if that's acceptable for your application.")
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        warnings.warn(msg)
+    else:
+        raise RuntimeError(msg)
 
 
 class _ROIAlignRotated3D(Function):
@@ -36,6 +50,7 @@ class _ROIAlignRotated3D(Function):
 
     @staticmethod
     def backward(ctx, grad_output):
+        _alert_not_deterministic("ROIAlignRotated3D backward")  # (gradients are scattered into the feature rows with float atomics)
         roi, = ctx.saved_tensors
         metadata, sz, extent, (ph, pw, pz), scale, sampling, shape = ctx.args
         g = grad_output.contiguous()

@@ -258,6 +258,7 @@ int scn_rpn_grid_anchors(const long *locations, long n_rows, float voxel_scale, 
  * (zero where no sample touches a site).  Both run on the Metadata's compute stream. */
 int scn_roi_align_rotated_3d_forward(scn_metadata *m, const long spatial_size[3], const float *feats, int n_planes, const int extent[3], const float *rois,
                                      long n_rois, float spatial_scale, int pooled_h, int pooled_w, int pooled_z, int sampling_ratio, float *out);
+/* (accumulates with float atomics in every mode: not reproducible bit for bit, see scn_set_deterministic) */
 int scn_roi_align_rotated_3d_backward(scn_metadata *m, const long spatial_size[3], float *d_feats, int n_planes, const int extent[3], const float *rois,
                                       long n_rois, float spatial_scale, int pooled_h, int pooled_w, int pooled_z, int sampling_ratio, const float *d_out);
 
@@ -299,6 +300,14 @@ int scn_voxelize(const float *xyz, const float *feats, long n, int n_feat, const
  * channel counts allow), 2 = tcgen05 BF16 inputs / fp32 accumulate. */
 int scn_set_math_mode(int mode);
 int scn_get_math_mode(void);
+/* Deterministic mode for this process (0 = off, the default): with 1, every float result of the calls above except
+ * scn_roi_align_rotated_3d_backward is bitwise reproducible from run to run for a fixed build, GPU model, math mode and
+ * inputs.  Launches that would accumulate floats with atomics (split filter offsets, BatchNorm statistics, weight and bias
+ * gradients) write per-work-item partial sums to fixed slots of a per-stream workspace instead and add them in index
+ * order.  Read by every launch, so a change applies from the next call on, recorded programs included.  The Python
+ * package follows torch.are_deterministic_algorithms_enabled(). */
+int scn_set_deterministic(int on);
+int scn_get_deterministic(void);
 /* 1 when the tcgen05 kernels are compiled in and the device is sm_100 */
 int scn_tensor_core_path_available(void);
 /* number of kernels this library has launched since load (for bench.py's gpu_launches) */
@@ -309,7 +318,9 @@ long scn_kernel_launch_count(void);
  * written as bf16 only, 6 = laterals run as a separate convolution + add (fallback), 7 = tcgen05 convolution launches,
  * 8 = BatchNorm ops applied from epilogue statistics, 9 = launches that split the filter offsets over CTAs (atomic
  * epilogue), 10 = CUDA-core convolution launches, 11 = backward passes run by scn_program_backward, 12 = bf16 operand copies the
- * weight-gradient kernel took from its caller (forward shadow / shared d_out copy) instead of converting again. */
+ * weight-gradient kernel took from its caller (forward shadow / shared d_out copy) instead of converting again, 13 = weight-gradient
+ * launches driven by the output-stationary plan, 14 = float-atomic launches: launches whose float result depends on the order in
+ * which atomics land (0 in deterministic mode except for scn_roi_align_rotated_3d_backward). */
 long scn_debug_counter(int which);
 /* Hands the library's idle device memory back to the driver: Metadata chunks not owned by a live Metadata, cached weight operand
  * images, per-stream scratch buffers (the library recycles these itself instead of returning them; torch.cuda.empty_cache() cannot
@@ -324,7 +335,8 @@ long scn_release_cached_memory(void);
  *  lateral: out = conv(in) [+ add_in] + lat_in[row] @ lat_weight ([n_in][n_out], one filter offset), lat_in_bf16 = bf16
  *           copy of lat_in (needed in math mode 2);
  *  stats:   sums = [8 replicas][2][128] doubles, zeroed by the caller; the launch adds per-channel sum (first 128) and sum
- *           of squares (second 128) of the rows it stores, spread over the replicas.
+ *           of squares (second 128) of the rows it stores, spread over the replicas (deterministic mode: written into replica
+ *           0 after the launch, in a fixed order).
  * A launch that cannot honour a request (CUDA-core path, packed rows, split offsets, > 128 channels) ignores it;
  * scn_fuse_result reports what the last call did and disarms both requests. */
 int scn_fuse_next_lateral(const float *lat_in, const void *lat_in_bf16, const float *lat_weight, long long weight_tag, int n_in, long rows);
