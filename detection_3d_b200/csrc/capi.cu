@@ -148,7 +148,7 @@ int scn_fuse_result(int *lateral_taken, int *stats_taken) {
   return 0;
 }
 int scn_set_math_mode(int mode) {
-  if (mode < 0 || mode > 2) { scn::set_error("math mode must be 0 (fp32), 1 (tf32) or 2 (bf16)"); return -2; }
+  if (mode < 0 || mode > 3) { scn::set_error("math mode must be 0 (fp32), 1 (tf32), 2 (bf16) or 3 (tf32x3)"); return -2; }
   scn::g_math_mode = mode;
   return 0;
 }

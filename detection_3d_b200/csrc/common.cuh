@@ -57,6 +57,7 @@ enum DebugCounter {
   kCntDwPlanLaunch = 13,   // weight-gradient launches driven by the output-stationary plan (conv_dw_plan_tc)
   kCntBwdOperandReused = 12, // bf16 operand copies the weight-gradient kernel took from its caller instead of converting again
   kCntFloatAtomic = 14,    // launches that accumulated floats with atomics, i.e. whose result depends on the order the atomics land in
+  kCntTf32x3Launch = 15,   // conv_plan_tc launches with TF32X3 operands (math mode 3)
   kCntCounters = 16
 };
 extern std::atomic<long> g_counters[kCntCounters];

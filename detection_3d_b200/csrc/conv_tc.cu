@@ -43,6 +43,11 @@ constexpr int kLateralBit = 63; // mask bit of the lateral stage (real filter of
 constexpr int kEpiCols = SCN_EPI_COLS;           // output columns per epilogue round: 32 (16 KB of staging per CTA) or 16 (8 KB)
 constexpr int kEpiBytes = 4 * 32 * kEpiCols * 4; // 4 epilogue warps x (32 rows x kEpiCols floats), XOR-swizzled
 constexpr int kBuildRoom = SCN_EPI_COLS == 16 ? 12 * 1024 : 0; // shared memory per SM left to the build kernels that run beside this one
+// Operand type of conv_plan_tc (template parameter OP).  TF32X3 ("3xTF32", math mode 3): every fp32 operand x = hi + lo with
+// both parts exact TF32 values, and out += A_hi W_lo + A_lo W_hi + A_hi W_hi in the same fp32 accumulator (the dropped
+// A_lo W_lo and the rounding of lo leave ~2^-21 relative error per product).
+enum TcOperand { kOpTF32 = 0, kOpBF16 = 1, kOpTF32X3 = 2 };
+constexpr int kSplitWarps = 4; // TF32X3: warps that split the gathered A atoms of a stage into hi / lo parts
 
 struct TcParams {
   const unsigned char *in; // activations, row-major, rowBytes per row (fp32 or bf16 elements)
@@ -150,6 +155,17 @@ __device__ __forceinline__ void tc_mma(uint32_t dTmem, uint64_t aDesc, uint64_t 
         "l"(aDesc), "l"(bDesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+// fp32 -> the nearest TF32 value (ties away from zero), as an fp32 number whose low 13 mantissa bits are zero
+__device__ __forceinline__ float tf32_rna(float x) {
+  uint32_t r;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+  return __uint_as_float(r & 0xffffe000u);
+}
+// x = hi + lo, hi = tf32(x), lo = tf32(x - hi) (x - hi is exact in fp32)
+__device__ __forceinline__ void tf32_split(float x, float &hi, float &lo) {
+  hi = tf32_rna(x);
+  lo = tf32_rna(x - hi);
+}
 // K-major, 128-byte swizzle: rows of 128 B, 8-row groups 1024 B apart (SBO), version 1 (sm_100)
 __device__ __forceinline__ uint64_t smem_desc_sw128(uint32_t addr) {
   return (uint64_t)((addr >> 4) & 0x3fffu) | (1ull << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
@@ -256,28 +272,39 @@ __device__ __forceinline__ void sched_publish(const Sched &S, int n, int wi) {
 // CTAS = CTAs per SM the variant is built for (register cap: 65536 / (CTAS x threads)): <PW 8, CTAS 2> caps the kernel at 72
 // registers (a few spilled words in the epilogue) and doubles the gather issue rate of the two-CTA configuration.
 // DET = deterministic mode (P.part / P.statsPart may be set): a separate instantiation, so that the default kernels stay as they are.
-template <bool BF16, int PW, int G, int CTAS, bool DET>
+// OP = operand type (TcOperand).  TF32X3 is built for the one-CTA configuration only (PW 8, CTAS 1): its stage is twice as large
+// ([T A_hi atoms][T A_lo atoms][W_hi atom][W_lo atom]), and kSplitWarps more warps (warps 14-17, 576 threads = the launch bound)
+// split each landed stage: they wait on full[slot], write hi in place and lo into the lo atom at the same swizzled offset, fence
+// the generic-proxy stores against the tensor core's reads and arrive on split[slot], which the MMA warp waits on.  Separate
+// warps rather than the producers: the producers never wait for their own copies (cp.async.mbarrier.arrive.noinc), and that is
+// what keeps their gathers in flight; a producer that split its rows would have to drain them first.
+template <int OP, int PW, int G, int CTAS, bool DET>
 __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_COLS == 16 ? 384 : 320)), CTAS) conv_plan_tc(const TcParams P) {
+  constexpr bool BF16 = OP == kOpBF16, X3 = OP == kOpTF32X3;
+  static_assert(!X3 || (PW == 8 && G == 1 && CTAS == 1), "TF32X3: one-CTA configuration only");
   constexpr int TM = G == 4 ? 2 : kMaxT; // tiles per item the producers keep neighbour ids for (G ids per row and tile)
   constexpr int kProdWarps = PW;
   constexpr int kRowsPerWarp = kTileM / PW; // rows of a tile one producer warp gathers
+  constexpr int kTakers = 4 + kProdWarps + 1 + (X3 ? kSplitWarps : 0); // warps that take work items from the schedule ring
   extern __shared__ __align__(1024) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int nWork = P.nSuper * P.kSplit;
   const uint32_t bBytes = (uint32_t)P.Cout * 128u;
-  const uint32_t stageBytes = (uint32_t)P.T * kAtomBytes + bBytes; // [T A atoms][B atom]
+  const uint32_t stageBytes = X3 ? 2u * ((uint32_t)P.T * kAtomBytes + bBytes) : (uint32_t)P.T * kAtomBytes + bBytes; // [T A atoms][B atom] (TF32X3: [T A_hi][T A_lo][W_hi][W_lo])
   unsigned char *sStage = smem;
   float *sEpi = reinterpret_cast<float *>(sStage + (size_t)P.S * stageBytes);
   uint64_t *bars = reinterpret_cast<uint64_t *>(sEpi + kEpiBytes / 4);
   uint64_t *full = bars, *empty = bars + P.S, *accFull = bars + 2 * P.S, *accEmpty = accFull + 2;
   uint32_t *tmemSlot = reinterpret_cast<uint32_t *>(accEmpty + 2);
-  Sched SC{bars + 24, bars + 24 + kSchedSlots, reinterpret_cast<volatile int *>(bars + 24 + 2 * kSchedSlots)}; // (64 barrier words are reserved; 2 S + 5 <= 17 are used above)
+  uint64_t *split = accEmpty + 3; // TF32X3: [S] stage split into hi / lo (after the TMEM slot word)
+  Sched SC{bars + 24, bars + 24 + kSchedSlots, reinterpret_cast<volatile int *>(bars + 24 + 2 * kSchedSlots)}; // (64 barrier words are reserved; 2 S + 5 <= 17 are used above, 3 S + 5 <= 23 with TF32X3)
   const bool dyn = P.sched != nullptr;
 
   if (tid == 0) {
     for (int i = 0; i < P.S; i++) { mbar_init(smem_u32(full + i), kProdWarps * 32 + 1); mbar_init(smem_u32(empty + i), 1); }
+    if constexpr (X3) for (int i = 0; i < P.S; i++) mbar_init(smem_u32(split + i), kSplitWarps * 32);
     for (int i = 0; i < 2; i++) { mbar_init(smem_u32(accFull + i), 1); mbar_init(smem_u32(accEmpty + i), 4); }
-    for (int i = 0; i < kSchedSlots; i++) { mbar_init(smem_u32(SC.full + i), 1); mbar_init(smem_u32(SC.empty + i), 4 + kProdWarps + 1); } // takers: epilogue + producer warps + MMA warp (the loader keeps its own copy)
+    for (int i = 0; i < kSchedSlots; i++) { mbar_init(smem_u32(SC.full + i), 1); mbar_init(smem_u32(SC.empty + i), kTakers); } // takers: epilogue + producer warps + MMA warp (+ split warps; the loader keeps its own copy)
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   constexpr int kMmaWarp = 4 + PW;
@@ -556,9 +583,10 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
           for (int c = 0; c < nA; c++) {
             n++;
             mbar_wait_t(full0 + slot * 8u, round & 1u, pw1, prof);
+            if constexpr (X3) mbar_wait_t(smem_u32(split + slot), round & 1u, pw1, prof); // (full: the weight atoms; split: the A atoms, split and fenced)
             tc_fence_after();
             const uint32_t sbase = sStage0 + slot * stageBytes;
-            const uint64_t bDesc = smem_desc_sw128(sbase + (uint32_t)P.T * kAtomBytes);
+            const uint64_t bDesc = smem_desc_sw128(sbase + (X3 ? 2u * (uint32_t)P.T * kAtomBytes : (uint32_t)P.T * kAtomBytes));
             const long long tI0 = prof ? clock64() : 0;
             if (elect_one()) {
               if (!(P.dbg & 4)) {
@@ -567,9 +595,19 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
                   if (!((I.m[t] >> k) & 1ull)) continue;
                   const uint64_t aDesc = smem_desc_sw128(sbase + t * kAtomBytes);
                   const uint32_t d = tmemBase + (uint32_t)(a * accCols + t * P.Cout);
+                  if constexpr (X3) {
+                    const uint64_t aLoDesc = smem_desc_sw128(sbase + (uint32_t)(P.T + t) * kAtomBytes), bLoDesc = smem_desc_sw128(sbase + 2u * (uint32_t)P.T * kAtomBytes + bBytes);
 #pragma unroll
-                  for (int j = 0; j < 4; j++) // 4 x 32 bytes of K inside the 128-byte swizzle atom
-                    tc_mma<BF16>(d, aDesc + (uint64_t)(j * 2), bDesc + (uint64_t)(j * 2), idesc, ((started >> t) & 1u) | (j > 0));
+                    for (int j = 0; j < 4; j++) { // per 32 bytes of K: the two small terms first, then A_hi W_hi
+                      tc_mma<false>(d, aDesc + (uint64_t)(j * 2), bLoDesc + (uint64_t)(j * 2), idesc, ((started >> t) & 1u) | (j > 0));
+                      tc_mma<false>(d, aLoDesc + (uint64_t)(j * 2), bDesc + (uint64_t)(j * 2), idesc, 1u);
+                      tc_mma<false>(d, aDesc + (uint64_t)(j * 2), bDesc + (uint64_t)(j * 2), idesc, 1u);
+                    }
+                  } else {
+#pragma unroll
+                    for (int j = 0; j < 4; j++) // 4 x 32 bytes of K inside the 128-byte swizzle atom
+                      tc_mma<BF16>(d, aDesc + (uint64_t)(j * 2), bDesc + (uint64_t)(j * 2), idesc, ((started >> t) & 1u) | (j > 0));
+                  }
                 }
               }
               const long long tI1 = prof ? clock64() : 0;
@@ -591,7 +629,7 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
         if (pw2 | pw3) { q[4] = pw2; q[5] = pw3; }
       }
     }
-  } else {
+  } else if (!X3 || warp == kMmaWarp + 1) {
     // ============================ B loader ============================
     if (lane == 0) {
       uint32_t n = 0, slot = 0, round = 0;
@@ -625,14 +663,60 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
             const uint32_t bar = smem_u32(full + slot);
             if (P.dbg & 2) { mbar_arrive(bar); }
             else {
-              mbar_arrive_expect_tx(bar, bBytes);
-              bulk_g2s(smem_u32(sStage) + slot * stageBytes + (uint32_t)P.T * kAtomBytes, wsrc + ((size_t)w * nA + c) * bBytes, bBytes, bar);
+              if constexpr (X3) { // the W_hi and W_lo atoms lie side by side in the image and in the stage
+                mbar_arrive_expect_tx(bar, 2u * bBytes);
+                bulk_g2s(smem_u32(sStage) + slot * stageBytes + 2u * (uint32_t)P.T * kAtomBytes, wsrc + ((size_t)w * nA + c) * 2u * bBytes, 2u * bBytes, bar);
+              } else {
+                mbar_arrive_expect_tx(bar, bBytes);
+                bulk_g2s(smem_u32(sStage) + slot * stageBytes + (uint32_t)P.T * kAtomBytes, wsrc + ((size_t)w * nA + c) * bBytes, bBytes, bar);
+              }
             }
             if (++slot == (uint32_t)P.S) { slot = 0; round++; }
           }
         }
       }
       if (prof) { long long *q = P.prof + blockIdx.x * 32 + 16; q[0] = clock64() - tStart; q[1] = pw0; q[2] = n; }
+    }
+  } else if constexpr (X3) {
+    // ============================ operand split (TF32X3) ============================
+    // The 128 threads walk the stages in the MMA warp's order; of every live tile each thread rewrites 8 of the 1024 16-byte
+    // chunks (consecutive threads, consecutive chunks: conflict-free): hi = tf32(x) in place, lo = tf32(x - hi) at the same
+    // offset of the lo atom (the 128-byte swizzle depends on the offset within the 1024-aligned atom only, so the lo atom
+    // needs no swizzle of its own).  Zero-filled rows (no neighbour) split into zeros.
+    const int st = tid - (kMmaWarp + 2) * 32;
+    uint32_t slot = 0, round = 0;
+    const uint32_t full0 = smem_u32(full), split0 = smem_u32(split);
+    for (int it = 0;; it++) {
+      const int wi = dyn ? sched_take(SC, it, lane == 0) : (int)(blockIdx.x + (long)it * gridDim.x < nWork ? blockIdx.x + it * gridDim.x : -1);
+      if (wi < 0) break;
+      const Item I = load_item<G>(P, wi);
+      unsigned long long rest = I.uni;
+      while (rest) {
+        const int k = __ffsll((long long)rest) - 1;
+        rest &= rest - 1;
+        const int nA = (G == 1 && k == kLateralBit) ? P.nAtoms2 : P.nAtoms;
+        for (int c = 0; c < nA; c++) {
+          mbar_wait(full0 + slot * 8u, round & 1u);
+          unsigned char *sb = sStage + (size_t)slot * stageBytes;
+#pragma unroll
+          for (int t = 0; t < kMaxT; t++) {
+            if (!((I.m[t] >> k) & 1ull)) continue;
+            float4 *hi = reinterpret_cast<float4 *>(sb + t * kAtomBytes), *lo = reinterpret_cast<float4 *>(sb + (size_t)(P.T + t) * kAtomBytes);
+#pragma unroll
+            for (int i = 0; i < kAtomBytes / 16 / (kSplitWarps * 32); i++) {
+              const int q = i * kSplitWarps * 32 + st;
+              const float4 x = hi[q];
+              float4 h, l;
+              tf32_split(x.x, h.x, l.x); tf32_split(x.y, h.y, l.y); tf32_split(x.z, h.z, l.z); tf32_split(x.w, h.w, l.w);
+              hi[q] = h;
+              lo[q] = l;
+            }
+          }
+          fence_proxy_async(); // generic-proxy stores -> the tensor core's (async proxy) reads
+          mbar_arrive(split0 + slot * 8u);
+          if (++slot == (uint32_t)P.S) { slot = 0; round++; }
+        }
+      }
     }
   }
   tc_fence_before();
@@ -671,6 +755,27 @@ __global__ void k_prep_wimg(const float *__restrict__ W, unsigned char *__restri
   }
 }
 
+// TF32X3 operands: the same image twice per (k, K atom), [W_hi atom][W_lo atom] side by side (one bulk copy per stage),
+// W_hi = tf32(w) and W_lo = tf32(w - W_hi), both exact TF32 values.  Same arguments as k_prep_wimg.
+__global__ void k_prep_wimg_split(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int Cin, int CinW, int Cout, int wT) {
+  const long n = (long)K * Cin * Cout;
+  const int nAtoms = Cin / 32;
+  for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
+    const int co = (int)(i % Cout);
+    const long t = i / Cout;
+    const int ci = (int)(t % Cin), k = (int)(t / Cin);
+    const int c = ci / 32, j = ci % 32;
+    const int byte = j * 4, chunk = byte >> 4, within = byte & 15;
+    unsigned char *dst = img + ((long)k * nAtoms + c) * 2 * Cout * 128 + (long)co * 128 + ((chunk ^ (co & 7)) << 4) + within;
+    const int ks = wT == 2 ? K - 1 - k : k;
+    const float w = ci < CinW ? (wT ? W[((long)ks * Cout + co) * CinW + ci] : W[((long)k * CinW + ci) * Cout + co]) : 0.f;
+    float hi, lo;
+    tf32_split(w, hi, lo);
+    *reinterpret_cast<float *>(dst) = hi;
+    *reinterpret_cast<float *>(dst + (long)Cout * 128) = lo;
+  }
+}
+
 // Packed layers (bf16 rows of 128 / G bytes, G = 2 or 4): the K atom of offset group kg holds, for output channel co,
 // [offset kg G | offset kg G + 1 | ...] x Cin input channels -- the same order in which the producers lay the G
 // gathered neighbour rows side by side.  Offsets beyond K and channels beyond CinW are zero.
@@ -706,16 +811,19 @@ static size_t g_wimg_bytes = 0;
 static unsigned long long g_wimg_clock = 0;
 constexpr size_t kWimgBudget = 768u << 20;
 // Returns the image; *owned = true when the caller must cudaFreeAsync it (uncached).
-// fmt: 0 = tf32, 1 = bf16, 1 + 16 G = packed bf16 (G offsets per atom)
+// fmt: 0 = tf32, 1 = bf16, 1 + 16 G = packed bf16 (G offsets per atom), kWimgSplit = tf32 hi / lo pairs (TF32X3).  The format is
+// part of the cache key: the images of one weight tensor in different modes are separate entries.
+constexpr int kWimgSplit = 2;
 static void launch_prep_wimg(const float *W, unsigned char *img, int K, int Cin, int CinW, int Cout, int fmt, cudaStream_t s, int wT) {
   const int G = fmt >> 4;
   if (G > 1) k_prep_wimg_packed<<<stream_grid((long)((K + G - 1) / G) * G * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, G, Cin, CinW, Cout, wT);
+  else if (fmt == kWimgSplit) k_prep_wimg_split<<<stream_grid((long)K * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, Cin, CinW, Cout, wT);
   else k_prep_wimg<<<stream_grid((long)K * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, Cin, CinW, Cout, fmt & 1, wT);
 }
 static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int Cout, int bf16, cudaStream_t s, unsigned char **img, bool *owned, int wT = 0) {
   if (wT) tag = 0; // (transposed operands belong to the backward pass of a training step: the weights change every step, nothing to cache)
   const int packG = bf16 >> 4;
-  const size_t bytes = packG > 1 ? (size_t)((K + packG - 1) / packG) * Cout * 128 : (size_t)K * Cin * Cout * (bf16 ? 2 : 4);
+  const size_t bytes = packG > 1 ? (size_t)((K + packG - 1) / packG) * Cout * 128 : (size_t)K * Cin * Cout * (bf16 == kWimgSplit ? 8 : bf16 ? 2 : 4);
   *owned = false;
   if (tag != 0) {
     int dev = 0;
@@ -893,30 +1001,33 @@ bool epilogue_stats_take() { bool d = tl_stats_done; tl_stats = nullptr; tl_stat
 template <bool DET>
 static int set_plan_attributes() {
   const int half = (233472 - kBuildRoom) / 2 - 1024;
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<false, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<false, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 4, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 4, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<false, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<true, 8, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpTF32, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpTF32, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 4, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 4, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpTF32, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpTF32X3, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
   return 0;
 }
 template <bool DET>
-static cudaError_t launch_plan_variant(const TcParams &P, int packG, bool pw8, int ctas, int grid, int th2, size_t smem, cudaStream_t s) {
-  if (packG == 2) return pw8 ? launch_pdl(conv_plan_tc<true, 8, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<true, 4, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
-  if (packG == 4) return pw8 ? launch_pdl(conv_plan_tc<true, 8, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<true, 4, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+static cudaError_t launch_plan_variant(const TcParams &P, int packG, bool pw8, int ctas, int grid, int th2, size_t smem, cudaStream_t s, bool x3) {
+  if (x3) return launch_pdl(conv_plan_tc<kOpTF32X3, 8, 1, 1, DET>, dim3(grid), dim3(32 * (14 + kSplitWarps)), smem, LS(s), P);
+  if (packG == 2) return pw8 ? launch_pdl(conv_plan_tc<kOpBF16, 8, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpBF16, 4, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+  if (packG == 4) return pw8 ? launch_pdl(conv_plan_tc<kOpBF16, 8, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpBF16, 4, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
   if (ctas == 2) {
-    if (P.bf16) return pw8 ? launch_pdl(conv_plan_tc<true, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<true, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
-    return pw8 ? launch_pdl(conv_plan_tc<false, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<false, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+    if (P.bf16) return pw8 ? launch_pdl(conv_plan_tc<kOpBF16, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpBF16, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+    return pw8 ? launch_pdl(conv_plan_tc<kOpTF32, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpTF32, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
   }
-  if (P.bf16) return launch_pdl(conv_plan_tc<true, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
-  return launch_pdl(conv_plan_tc<false, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
+  if (P.bf16) return launch_pdl(conv_plan_tc<kOpBF16, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
+  return launch_pdl(conv_plan_tc<kOpTF32, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
 }
-// in16: optional bf16 copy of `in` (same layout); used in math mode 2 when Cin is a multiple of 64
+// in16: optional bf16 copy of `in` (same layout); used in math mode 2 when Cin is a multiple of 64.
+// mathMode 1 = TF32 operands, 2 = BF16 where the channel counts allow (TF32 elsewhere), 3 = TF32X3 (the fp32 rows as hi / lo TF32 pairs)
 int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
                         int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, const int *tileW, int nWeights,
                         long nInRows, const void *in16, long long wTag, const float *addend, void *out16, long nOutRows, int CinW = 0, int wT = 0) {
@@ -960,6 +1071,7 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   // filter offsets side by side in one atom: half / a quarter of the stages, gather bytes and MMAs of the 128-byte-row layout
   const int packG = (canPack && (Cin == 32 || Cin == 16)) ? 64 / Cin : 1;
   P.bf16 = (mathMode == 2 && (Cin % 64 == 0 || packG > 1)) ? 1 : 0; // other narrow layers keep TF32 operands
+  const bool x3 = mathMode == 3 && !P.bf16; // TF32X3: the fp32 rows split into two TF32 operands (one-CTA configuration, stages twice as large)
   void *tmp16 = nullptr;
   if (P.bf16) {
     if (!in16) {
@@ -987,11 +1099,13 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   static int smallOne = -1;
   if (smallOne < 0) smallOne = getenv("SCN_TC_SMALL_ONE") ? atoi(getenv("SCN_TC_SMALL_ONE")) : 1;
   if (smallOne && !envCtas && packG == 1 && cdiv(nOut, kTileM) <= kSMs) ctas = 1;
+  if (x3) ctas = 1; // (with half the shared memory, a 128-channel layer would not even fit two stages of one tile)
   P.tmemCols = ctas == 2 ? 256 : 512;
   const size_t smemBudget = ctas == 2 ? ((233472 - kBuildRoom) / 2 - 1024) : (227 * 1024 - kBuildRoom);
   const int Tcap = std::min(packG == 4 ? 2 : kMaxT, P.tmemCols / Cout);
   const size_t fixed = kEpiBytes + 64 * 8 + 64;
-  auto ring = [&](int t) { return (int)((smemBudget - fixed) / ((size_t)t * kAtomBytes + (size_t)Cout * 128)); };
+  const size_t stageMul = x3 ? 2 : 1; // TF32X3: hi and lo atoms of A and of W
+  auto ring = [&](int t) { return (int)((smemBudget - fixed) / (stageMul * ((size_t)t * kAtomBytes + (size_t)Cout * 128))); };
   int T = Tcap;
   if (ctas == 1) while (T > 2 && ring(T) < 3) T--; // a 2-slot ring exposes the gather latency (measured: T=3/S=3 beats T=4/S=2 by 12 %)
   while (T > 1 && ring(T) < 2) T--;
@@ -1018,7 +1132,7 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
     if (det) SCN_TRY(det_scratch(s, (size_t)P.nSuper * 4 * 2 * Cout * sizeof(double), (void **)&P.statsPart));
     else ++g_counters[kCntFloatAtomic];
   }
-  const size_t stageBytes = (size_t)P.T * kAtomBytes + (size_t)Cout * 128;
+  const size_t stageBytes = stageMul * ((size_t)P.T * kAtomBytes + (size_t)Cout * 128);
   P.S = (int)std::min<size_t>(envS > 0 ? envS : 6, (smemBudget - fixed) / stageBytes);
   SCN_CHECK(P.S >= 2, "tcgen05 path: shared memory budget exceeded");
   static int envLag = -2;
@@ -1028,12 +1142,13 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   const size_t smem = (size_t)P.S * stageBytes + fixed;
   SCN_CHECK(out || (P.kSplit == 1 && out16), "tcgen05 path: fp32 output dropped on a launch that needs it");
   ++g_counters[kCntTcLaunch];
+  if (x3) ++g_counters[kCntTf32x3Launch];
   if (P.kSplit > 1) ++g_counters[kCntSplitLaunch];
   if (P.kSplit > 1 && det) SCN_TRY(det_scratch(s, (size_t)P.kSplit * nOut * Cout * 4, (void **)&P.part)); // (k_split_sum writes every output row)
   else if (P.kSplit > 1) { ++g_counters[kCntFloatAtomic]; SCN_CUDA(cudaMemsetAsync(out, 0, (size_t)nOut * Cout * 4, s)); }
   unsigned char *wimg = nullptr;
   bool wimgOwned = false;
-  SCN_TRY(get_wimg(W, wTag, nWeights, Cin, CinW, Cout, packG > 1 ? 1 + 16 * packG : P.bf16, s, &wimg, &wimgOwned, wT));
+  SCN_TRY(get_wimg(W, wTag, nWeights, Cin, CinW, Cout, packG > 1 ? 1 + 16 * packG : x3 ? kWimgSplit : P.bf16, s, &wimg, &wimgOwned, wT));
   P.wimg = wimg;
   P.in2 = nullptr; P.wimg2 = nullptr; P.rowBytes2 = 0; P.nAtoms2 = 0;
   unsigned char *wimg2 = nullptr;
@@ -1042,7 +1157,7 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
     const int esz = P.bf16 ? 2 : 4, per = 128 / esz, C2 = tl_lat.Cin; // per = channels of one K atom
     if ((C2 * esz) % 16 == 0) {
       const int C2p = (C2 + per - 1) / per * per;
-      SCN_TRY(get_wimg(tl_lat.w, tl_lat.tag, 1, C2p, C2, Cout, P.bf16, s, &wimg2, &wimg2Owned));
+      SCN_TRY(get_wimg(tl_lat.w, tl_lat.tag, 1, C2p, C2, Cout, x3 ? kWimgSplit : P.bf16, s, &wimg2, &wimg2Owned));
       P.in2 = static_cast<const unsigned char *>(P.bf16 ? tl_lat.in16 : static_cast<const void *>(tl_lat.in));
       P.rowBytes2 = C2 * esz;
       P.nAtoms2 = C2p / per;
@@ -1075,8 +1190,8 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   if (envPw8 < 0) envPw8 = getenv("SCN_TC_PW8") ? atoi(getenv("SCN_TC_PW8")) : 0;
   const bool pw8 = ctas == 2 && ((packG > 1 && (envPw8 & 1)) || (packG == 1 && (envPw8 & 2)));
   const int th2 = 32 * (pw8 ? 14 : 10);
-  if (det) SCN_CUDA(launch_plan_variant<true>(P, packG, pw8, ctas, grid, th2, smem, s));
-  else SCN_CUDA(launch_plan_variant<false>(P, packG, pw8, ctas, grid, th2, smem, s));
+  if (det) SCN_CUDA(launch_plan_variant<true>(P, packG, pw8, ctas, grid, th2, smem, s, x3));
+  else SCN_CUDA(launch_plan_variant<false>(P, packG, pw8, ctas, grid, th2, smem, s, x3));
   SCN_CUDA(cudaGetLastError());
   if (envProf) { // developer aid: mean stall cycles per role over the CTAs of this launch
     static long long h[2 * kSMs * 32];

@@ -448,8 +448,11 @@ def add_features(a, b):
 
 
 def set_math_mode(mode):
-    """'fp32' (CUDA cores, exact), 'tf32' or 'bf16' (tcgen05 tensor cores, fp32 accumulate)."""
-    code = {"fp32": 0, "tf32": 1, "bf16": 2}[mode] if isinstance(mode, str) else int(mode)
+    """'fp32' (CUDA cores, exact), 'tf32' or 'bf16' (tcgen05 tensor cores, fp32 accumulate), or 'tf32x3' (tcgen05, every fp32
+    operand split into two TF32 values hi + lo, three products per step in one fp32 accumulator: fp32-class accuracy at tensor-core
+    speed; weight gradients and the convolutions the tensor-core kernel cannot take run on the exact CUDA-core kernels, as in
+    'tf32').  math_mode() returns the code: 0, 1, 2 or 3."""
+    code = {"fp32": 0, "tf32": 1, "bf16": 2, "tf32x3": 3}[mode] if isinstance(mode, str) else int(mode)
     check(lib().scn_set_math_mode(code))
     _MATH["mode"] = lib().scn_get_math_mode()
 

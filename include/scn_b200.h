@@ -297,7 +297,10 @@ int scn_voxelize(const float *xyz, const float *feats, long n, int n_feat, const
 
 /* Selects the arithmetic of the gather-GEMM kernels for this process: 0 = fp32 CUDA cores
  * (exact-fp32 anchor), 1 = tcgen05 tensor cores, TF32 inputs / fp32 accumulate (default where the
- * channel counts allow), 2 = tcgen05 BF16 inputs / fp32 accumulate. */
+ * channel counts allow), 2 = tcgen05 BF16 inputs / fp32 accumulate, 3 = tcgen05 "3xTF32": each fp32
+ * operand split into two exact TF32 values hi + lo, three TF32 products (hi*lo, lo*hi, hi*hi) in one fp32
+ * accumulator, fp32-class accuracy.  In modes 1 and 3 every convolution the tensor-core kernel cannot take,
+ * and every weight gradient, runs on the exact fp32 CUDA-core kernels. */
 int scn_set_math_mode(int mode);
 int scn_get_math_mode(void);
 /* Deterministic mode for this process (0 = off, the default): with 1, every float result of the calls above except

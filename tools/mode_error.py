@@ -16,7 +16,7 @@ GOLD = os.path.join(ROOT, "tests", "golden")
 for name, cfg, bld in (("mini4", fpn_util.mini4_config(), dict(nx=60, ny=56, nz=24, n_walls=3, seed=3)),
                        ("sw4c_mid", scn.sw4c_fpn432_config(), dict(nx=300, ny=280, nz=40, n_walls=5, seed=5))):
     g = np.load(os.path.join(GOLD, f"fpn_{name}.npz"))
-    for mode in ("fp32", "tf32", "bf16"):
+    for mode in ("fp32", "tf32", "tf32x3", "bf16"):
         scn.set_math_mode(mode)
         net = scn.FPN_Net(**cfg)
         net.load_state_dict(fpn_util.deterministic_state(net, seed=1))
