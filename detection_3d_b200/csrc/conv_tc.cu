@@ -36,7 +36,7 @@ namespace scn {
 constexpr int kTileM = 128;
 constexpr int kAtomBytes = kTileM * 128; // 128 rows x 128 B
 constexpr int kMaxT = 4;
-constexpr int kLateralBit = 63; // mask bit of the lateral stage (real filter offsets use bits 0..K-1, K <= 63 then)
+constexpr int kLateralBit = 63; // mask bit of the lateral stage (launches with a lateral stage have K <= 63; a K = 64 plan uses bit 63 for offset 63)
 #ifndef SCN_EPI_COLS
 #define SCN_EPI_COLS 32
 #endif
@@ -227,6 +227,10 @@ __device__ __forceinline__ Item load_item(const TcParams &P, int wi) {
   }
   return I;
 }
+
+// whether mask bit k of a work item is the lateral stage: only in a launch that carries one (a plan with K = 64 uses bit 63 for its
+// last filter offset; the launcher folds a lateral stage into plans with K < 64 only)
+__device__ __forceinline__ bool is_lateral(const TcParams &P, int k) { return k == kLateralBit && P.in2 != nullptr; }
 
 // ------------------------------------------------------------------ dynamic work distribution
 // Work items are handed out by a global counter instead of a static stride: a CTA that starts late (its SM was still running a
@@ -483,7 +487,7 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
         for (int g = 0; g < G; g++)
 #pragma unroll
           for (int t = 0; t < TM; t++) {
-            if (G == 1 && k == kLateralBit) { // lateral stage: the input row of an output site is its own output row
+            if (G == 1 && is_lateral(P, k)) { // lateral stage: the input row of an output site is its own output row
               const long p = (long)(I.st * P.T + t) * kTileM + pw * kRowsPerWarp + (lane & (kRowsPerWarp - 1));
               dst[g][t] = (((I.m[t] >> k) & 1ull) && p < P.nOut) ? (P.outRow ? __ldg(P.outRow + p) : (int)p) : -1;
             } else if (!P.nbr) { // dense rows: site p reads row p
@@ -507,7 +511,7 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
         const unsigned long long rest = (k + 1 < 64) ? (I.uni >> (k + 1)) : 0ull;
         const int kNext = rest ? k + 1 + (__ffsll((long long)rest) - 1) : -1;
         if (kNext >= 0) load_ids(kNext, idn);
-        const bool lat = G == 1 && k == kLateralBit;
+        const bool lat = G == 1 && is_lateral(P, k);
         const unsigned char *srcBase = lat ? P.in2 : P.in;
         const int srcRowBytes = lat ? P.rowBytes2 : P.rowBytes, nA = lat ? P.nAtoms2 : P.nAtoms;
         for (int c = 0; c < nA; c++) {
@@ -579,7 +583,7 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
         while (rest) {
           const int k = __ffsll((long long)rest) - 1;
           rest &= rest - 1;
-          const int nA = (G == 1 && k == kLateralBit) ? P.nAtoms2 : P.nAtoms;
+          const int nA = (G == 1 && is_lateral(P, k)) ? P.nAtoms2 : P.nAtoms;
           for (int c = 0; c < nA; c++) {
             n++;
             mbar_wait_t(full0 + slot * 8u, round & 1u, pw1, prof);
@@ -653,7 +657,7 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
         while (rest) {
           const int k = __ffsll((long long)rest) - 1;
           rest &= rest - 1;
-          const bool lat = G == 1 && k == kLateralBit;
+          const bool lat = G == 1 && is_lateral(P, k);
           const int w = lat ? 0 : (P.tileW ? __ldg(P.tileW + I.st) : k / G); // packed: one weight atom per offset group
           const unsigned char *wsrc = lat ? P.wimg2 : P.wimg;
           const int nA = lat ? P.nAtoms2 : P.nAtoms;
@@ -694,7 +698,7 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
       while (rest) {
         const int k = __ffsll((long long)rest) - 1;
         rest &= rest - 1;
-        const int nA = (G == 1 && k == kLateralBit) ? P.nAtoms2 : P.nAtoms;
+        const int nA = (G == 1 && is_lateral(P, k)) ? P.nAtoms2 : P.nAtoms;
         for (int c = 0; c < nA; c++) {
           mbar_wait(full0 + slot * 8u, round & 1u);
           unsigned char *sb = sStage + (size_t)slot * stageBytes;
@@ -1111,7 +1115,7 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   while (T > 1 && ring(T) < 2) T--;
   while (T > 1 && cdiv(P.nTiles, T) < 2 * kSMs * ctas) T--;
   if (tileW) T = 1;
-  if (envT > 0 && envT <= Tcap && !tileW) T = envT;
+  if (envT > 0 && envT <= Tcap && !tileW && ring(envT) >= 2) T = envT; // (a forced T must leave room for a 2-stage ring)
   P.T = T;
   P.nAcc = 2 * T * Cout <= P.tmemCols ? 2 : 1;
   P.nSuper = cdiv(P.nTiles, P.T);
@@ -1199,8 +1203,8 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
     SCN_CUDA(cudaStreamSynchronize(s));
     double m[32] = {0};
     for (int b = 0; b < grid; b++) for (int i = 0; i < 32; i++) m[i] += (double)h[b * 32 + i] / grid;
-    fprintf(stderr, "[tcprof] ctas=%d grid=%d T=%d K=%d Cin=%d Cout=%d S=%d nAcc=%d kSplit=%d | epi total %.0f waitAcc %.0f | prod total %.0f empty %.0f cpwait %.0f stages %.0f | mma total %.0f accEmpty %.0f full %.0f stages %.0f issue %.0f commit %.0f | bld total %.0f empty %.0f\n",
-            ctas, grid, P.T, K, Cin, Cout, P.S, P.nAcc, P.kSplit, m[0], m[1], m[4], m[5], m[6], m[7], m[10], m[11], m[12], m[13], m[14], m[15], m[16], m[17]);
+    fprintf(stderr, "[tcprof] ctas=%d pw=%d grid=%d T=%d K=%d Cin=%d Cout=%d S=%d lag=%d nAcc=%d kSplit=%d | epi total %.0f waitAcc %.0f | prod total %.0f empty %.0f cpwait %.0f stages %.0f | mma total %.0f accEmpty %.0f full %.0f stages %.0f issue %.0f commit %.0f | bld total %.0f empty %.0f\n",
+            ctas, x3 || ctas == 1 || pw8 ? 8 : 4, grid, P.T, K, Cin, Cout, P.S, P.lag, P.nAcc, P.kSplit, m[0], m[1], m[4], m[5], m[6], m[7], m[10], m[11], m[12], m[13], m[14], m[15], m[16], m[17]);
     cudaFreeAsync(P.prof, s);
   }
   if (P.statsPart) SCN_TRY(ordered_sum(P.statsPart, P.nSuper * 4, 2l * Cout, P.stats, s, Cout, kFusedStatsC)); // into replica 0

@@ -393,8 +393,9 @@ def test_tc_submanifold_forward(cin, cout, f, math):
 def test_tc_input_gradients(math):
     """tf32 / bf16 mode: the input gradient of all three convolution kinds runs on the tcgen05 forward kernel with transposed
     weights (submanifold: symmetric plan with reversed offsets; strided convolution: a deconvolution; deconvolution: the
-    strided convolution); d_weight runs on the tcgen05 MN-major kernel (conv_dw_tc) for 128 / 256 input channels and on the
-    fp32 CUDA cores otherwise.  Checked against the oracle's backward."""
+    strided convolution); d_weight runs on the tcgen05 kernel conv_dw_tc in bf16 mode (every shape here, 9 / 32 / 64 input channels
+    included: tests/test_gpu_tc_exact.py reads which kernel ran) and on the fp32 CUDA cores in tf32 mode.  Checked against the
+    oracle's backward."""
     scn, G, O = _setup_levels()
     _tc_or_skip(scn)
     L = torch.LongTensor
