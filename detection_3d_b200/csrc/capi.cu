@@ -678,7 +678,7 @@ int scn_iteration_order(scn_metadata *m, const long sz[3], int *dst) {
 }
 
 static bool tc_ok(int Cin, int Cout, int K) {
-  return scn::g_math_mode != 0 && scn::tc_available() && Cout % 32 == 0 && Cout >= 32 && Cout <= 256 && K <= 64 && Cin >= 4 && Cin <= 1024;
+  return scn::g_math_mode != 0 && scn::tc_available() && Cout % 32 == 0 && Cout >= 32 && Cout <= 256 && K <= scn::kMaxFilterVolume && Cin >= 4 && Cin <= 1024;
 }
 // out += addend (optional) and the bf16 copy of out (optional), for the paths whose kernels do not fuse them
 static int plain_epilogue(float *out, const float *addend, void *out16, long rows, int C, cudaStream_t s) {

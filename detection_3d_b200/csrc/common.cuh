@@ -58,7 +58,8 @@ enum DebugCounter {
   kCntBwdOperandReused = 12, // bf16 operand copies the weight-gradient kernel took from its caller instead of converting again
   kCntFloatAtomic = 14,    // launches that accumulated floats with atomics, i.e. whose result depends on the order the atomics land in
   kCntTf32x3Launch = 15,   // conv_plan_tc launches with TF32X3 operands (math mode 3)
-  kCntCounters = 16
+  kCntChunkedLaunch = 16,  // conv_plan_tc launches over one offset chunk of a plan with more than 64 filter offsets
+  kCntCounters = 17
 };
 extern std::atomic<long> g_counters[kCntCounters];
 
@@ -124,7 +125,18 @@ static inline int stream_grid(long n, int threads, int per_sm = 8) {
 // (see NbrPlan in metadata.cuh) tiles of 128 output sites, ids of one filter offset contiguous
 constexpr int kPlanPad = 512;
 __host__ __device__ __forceinline__ long nbr_index(long p, int k, int K) { return ((p >> 7) * K + k) * 128 + (p & 127); }
-static inline long plan_padded(long n) { return (n + kPlanPad - 1) / kPlanPad * kPlanPad; }
+__host__ __device__ __forceinline__ long plan_padded(long n) { return (n + kPlanPad - 1) / kPlanPad * kPlanPad; }
+// Wide plans (K > 64 filter offsets, up to kMaxFilterVolume) are stored CHUNK-MAJOR: chunk c holds offsets [63 c, 63 c + Kc),
+// Kc = min(63, K - 63 c), as an ordinary plan of Kc offsets over the same nPad = plan_padded(nOut) sites, at nbr + 63 c nPad; its
+// per-tile offset masks (bit j = offset 63 c + j) are at tileMask + c nPad / 128.  A chunk is then exactly what the tensor-core
+// kernel takes, with bit 63 of its masks left free for the lateral stage.  Plans of K <= 64 keep the single-chunk layout above.
+constexpr int kMaxFilterVolume = 512;
+constexpr int kChunkOffsets = 63;
+__host__ __device__ __forceinline__ int plan_chunks(int K) { return K <= 64 ? 1 : (K + kChunkOffsets - 1) / kChunkOffsets; }
+__host__ __device__ __forceinline__ long nbr_index_wide(long p, int k, int K, long nPad) {
+  const int c = k / kChunkOffsets, k0 = c * kChunkOffsets, Kc = K - k0 < kChunkOffsets ? K - k0 : kChunkOffsets;
+  return (long)k0 * nPad + nbr_index(p, k - k0, Kc);
+}
 
 // ---------------------------------------------------------------- single-pass scan
 // Decoupled look-back exclusive scan (int32) with a fused consumer.  One launch:

@@ -61,7 +61,8 @@ __device__ __forceinline__ void mma_chunk(const float (*A_s)[TM + APAD], const f
   }
 }
 
-template <bool VEC>
+// WIDE: a plan of more than 64 filter offsets (chunk-major, nbr_index_wide); one launch still sums all offsets in order
+template <bool VEC, bool WIDE = false>
 __global__ void __launch_bounds__(256) conv_plan_simt(const float *__restrict__ in, float *__restrict__ out, const float *__restrict__ W,
                                                       const int *__restrict__ nbr, const int *__restrict__ outRow, int nOut, int K, int Cin, int Cout,
                                                       const float *__restrict__ bias) {
@@ -77,7 +78,8 @@ __global__ void __launch_bounds__(256) conv_plan_simt(const float *__restrict__ 
     for (int j = 0; j < 4; j++) acc[i][j] = 0.f;
   for (int k = 0; k < K; k++) {
     int id = -1;
-    if (tid < TM && p0 + tid < nOut) id = nbr ? __ldg(nbr + nbr_index(p0 + tid, k, K)) : p0 + tid; // no plan: dense rows (NetworkInNetwork)
+    if (tid < TM && p0 + tid < nOut)
+      id = nbr ? __ldg(nbr + (WIDE ? nbr_index_wide(p0 + tid, k, K, plan_padded(nOut)) : nbr_index(p0 + tid, k, K))) : p0 + tid; // no plan: dense rows (NetworkInNetwork)
     __syncthreads(); // previous offset's readers of s_ids / tiles are done
     if (tid < TM) s_ids[tid] = id;
     if (!__syncthreads_or(id >= 0)) continue;
@@ -280,7 +282,11 @@ int launch_conv_plan_simt(const float *in, float *out, const float *W, const int
     return 0;
   }
   dim3 grid(cdiv(nOut, TM), cdiv(Cout, TN));
-  if (Cin % 4 == 0 && Cout % 4 == 0)
+  if (K > 64 && Cin % 4 == 0 && Cout % 4 == 0)
+    conv_plan_simt<true, true><<<grid, 256, 0, LS(s)>>>(in, out, W, nbr, outRow, nOut, K, Cin, Cout, bias);
+  else if (K > 64)
+    conv_plan_simt<false, true><<<grid, 256, 0, LS(s)>>>(in, out, W, nbr, outRow, nOut, K, Cin, Cout, bias);
+  else if (Cin % 4 == 0 && Cout % 4 == 0)
     conv_plan_simt<true><<<grid, 256, 0, LS(s)>>>(in, out, W, nbr, outRow, nOut, K, Cin, Cout, bias);
   else
     conv_plan_simt<false><<<grid, 256, 0, LS(s)>>>(in, out, W, nbr, outRow, nOut, K, Cin, Cout, bias);

@@ -950,7 +950,8 @@ const void *bwd_in16_take() { const void *p = tl_bwd_in16; tl_bwd_in16 = nullptr
 // from the first, so they must not share a buffer; slot 2: the operand pair of the weight-gradient kernel).  Uses of a
 // slot on one stream are ordered; cudaMallocAsync took milliseconds for these 150-300 MB blocks.
 // 3: bf16 copy of d_out shared by the two gradient kernels of a backward call; 4: partial sums of the deterministic mode (det_scratch)
-enum ScratchSlot { kScratchPad = 0, kScratchBf16 = 1, kScratchDw = 2, kScratchDout = 3, kScratchDet = 4 };
+// 5: running sums of a chunked launch (launch_conv_plan_tc_chunked)
+enum ScratchSlot { kScratchPad = 0, kScratchBf16 = 1, kScratchDw = 2, kScratchDout = 3, kScratchDet = 4, kScratchChunk = 5 };
 static std::mutex g_scratch_mu;
 static std::map<std::tuple<int, cudaStream_t, int>, std::pair<void *, size_t>> g_scratch;
 static int stream_scratch(cudaStream_t s, int slot, size_t bytes, void **out) {
@@ -1030,6 +1031,9 @@ static cudaError_t launch_plan_variant(const TcParams &P, int packG, bool pw8, i
   if (P.bf16) return launch_pdl(conv_plan_tc<kOpBF16, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
   return launch_pdl(conv_plan_tc<kOpTF32, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
 }
+static int launch_conv_plan_tc_chunked(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
+                                       int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, long nInRows, const void *in16,
+                                       long long wTag, const float *addend, void *out16, long nOutRows, int CinW, int wT);
 // in16: optional bf16 copy of `in` (same layout); used in math mode 2 when Cin is a multiple of 64.
 // mathMode 1 = TF32 operands, 2 = BF16 where the channel counts allow (TF32 elsewhere), 3 = TF32X3 (the fp32 rows as hi / lo TF32 pairs)
 int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
@@ -1037,6 +1041,10 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
                         long nInRows, const void *in16, long long wTag, const float *addend, void *out16, long nOutRows, int CinW = 0, int wT = 0) {
   if (nOut == 0) return 0;
   if (CinW == 0) CinW = Cin;
+  if (K > 64 && !tileW) {
+    SCN_CHECK(nbr && tileMask && nWeights == K && K <= kMaxFilterVolume, "tcgen05 path: wide plan");
+    return launch_conv_plan_tc_chunked(in, out, W, nbr, outRow, tileMask, nOut, K, Cin, Cout, bias, mathMode, s, nInRows, in16, wTag, addend, out16, nOutRows, CinW, wT);
+  }
   const bool canPack = mathMode == 2 && !tileW && Cout <= 128; // packed narrow rows: two-CTA configuration only
   if (canPack && CinW == Cin && Cin != 16 && Cin % 32 != 0) {
     // bf16 mode, odd channel counts (e.g. the 9-channel network input): bf16 rows zero-padded to 16 channels (packed, G = 4),
@@ -1216,6 +1224,45 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   if (wimgOwned) cudaFreeAsync(wimg, s);
   if (wimg2Owned) cudaFreeAsync(wimg2, s);
 
+  return 0;
+}
+
+// A plan of more than 64 filter offsets (chunk-major, common.cuh) runs as one launch per chunk of <= 63 offsets.  Chunk c is an
+// ordinary plan -- its own block of neighbour ids and mask array, the weights of its offsets -- and takes the running sum of the
+// chunks before it as its fused addend.  Bias and the caller's addend go into chunk 0; the lateral stage, the epilogue statistics
+// and the bf16 copy into the last chunk, the only one that sees finished rows.  The running sums alternate between two scratch
+// buffers, so no launch reads rows it writes (an offset-split launch zeroes its output first).  Each chunk boundary adds one fp32
+// rounding of the partial sum (DESIGN.md section 7).
+static int launch_conv_plan_tc_chunked(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
+                                       int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, long nInRows, const void *in16,
+                                       long long wTag, const float *addend, void *out16, long nOutRows, int CinW, int wT) {
+  const int nC = plan_chunks(K);
+  const long nPad = plan_padded(nOut);
+  float *run = nullptr;
+  SCN_TRY(stream_scratch(s, kScratchChunk, (size_t)std::min(nC - 1, 2) * nOutRows * Cout * 4 + 16, (void **)&run));
+  // the side channels are consumed by the first launch that can take them: hold them back for the chunk they belong to
+  const Lateral lat = tl_lat;
+  double *const stats = tl_stats;
+  const void *const pre = tl_prepad;
+  const int preC = tl_prepad_c;
+  tl_lat.in = nullptr;
+  tl_stats = nullptr;
+  const float *prev = addend;
+  for (int c = 0; c < nC; c++) {
+    const int k0 = c * kChunkOffsets, Kc = std::min(kChunkOffsets, K - k0);
+    const bool last = c == nC - 1;
+    float *dst = last ? out : run + (size_t)(c & 1) * nOutRows * Cout;
+    // W: [K][CinW][Cout] (or [K][Cout][CinW] transposed): CinW x Cout floats per offset.  Offset-reversed operands (wT = 2): offset j
+    // of this chunk is W[K - 1 - k0 - j], i.e. the reversal of the block W[K - k0 - Kc, K - k0)
+    const float *Wc = W + (size_t)(wT == 2 ? K - k0 - Kc : k0) * CinW * Cout;
+    if (last) { tl_lat = lat; tl_stats = stats; }
+    tl_prepad = pre;
+    tl_prepad_c = preC;
+    ++g_counters[kCntChunkedLaunch];
+    SCN_TRY(launch_conv_plan_tc(in, dst, Wc, nbr + (size_t)k0 * nPad, outRow, tileMask + (size_t)c * (nPad / 128), nOut, Kc, Cin, Cout, c == 0 ? bias : nullptr,
+                                mathMode, s, nullptr, Kc, nInRows, in16, wTag, prev, last ? out16 : nullptr, nOutRows, CinW, wT));
+    prev = dst;
+  }
   return 0;
 }
 

@@ -920,6 +920,48 @@ static int build_rule_lists(Metadata &M, int n, int K, MaskF maskf, PairF pairf,
   SCN_CUDA(cudaGetLastError());
   return 0;
 }
+// More than 64 lists (filter volumes up to kMaxFilterVolume): the same count / scan / write kernels, one pass per 64 lists.  F::word(r, k0)
+// gives bits [k0, k0 + 64) of rank r's events; pass w keeps its per-tile prefix table at tileCnt + w nTiles 64.  Each list is
+// numbered exactly as above (its position only depends on the earlier ranks with an event in it).
+template <class F> struct ChunkMask { F f; int k0; __device__ unsigned long long operator()(int r) const { return f.word(r, k0); } };
+template <class F> struct ShiftPair { F f; int k0; __device__ int2 operator()(int r, int L) const { return f(r, L + k0); } };
+template <class MaskF, class PairF>
+static int write_rule_lists_wide(Metadata &M, int n, int K, MaskF maskf, PairF pairf, const int *tileCnt, const int *d_off, int2 *pairs) {
+  const int nTiles = cdiv(std::max(n, 1), kRuleTile);
+  for (int k0 = 0; n > 0 && k0 < K; k0 += 64)
+    k_rule_write<<<nTiles, kRuleTile, 0, LS(M.cur().stream)>>>(n, std::min(64, K - k0), ChunkMask<MaskF>{maskf, k0}, ShiftPair<PairF>{pairf, k0},
+                                                              tileCnt + (long)(k0 / 64) * nTiles * 64, d_off + k0, pairs);
+  SCN_CUDA(cudaGetLastError());
+  return 0;
+}
+template <class MaskF, class PairF>
+static int build_rule_lists_wide(Metadata &M, int n, int K, MaskF maskf, PairF pairf, RuleBookDev &rb, int extraScalars, bool write = true, int **tileCntOut = nullptr) {
+  SCN_CHECK(K > 64 && K <= kMaxFilterVolume, "filter volume must be <= 512");
+  cudaStream_t s = M.cur().stream;
+  rb.nLists = K;
+  rb.off.assign(K + 1, 0);
+  rb.d_off = M.alloc_n<int>(K + 1);
+  const int nTiles = cdiv(std::max(n, 1), kRuleTile);
+  int *tileCnt = M.alloc_n<int>((long)cdiv(K, 64) * nTiles * 64);
+  int *totals = M.alloc_n<int>(K);
+  SCN_CHECK(rb.d_off && tileCnt && totals, "alloc");
+  for (int k0 = 0; k0 < K; k0 += 64) {
+    const int Lw = std::min(64, K - k0);
+    int *tc = tileCnt + (long)(k0 / 64) * nTiles * 64;
+    k_rule_count<<<nTiles, kRuleTile, 0, LS(s)>>>(n, Lw, ChunkMask<MaskF>{maskf, k0}, tc);
+    k_rule_scan<<<Lw, 1024, 0, LS(s)>>>(nTiles, Lw, tc, totals + k0);
+  }
+  k_list_offsets<<<1, 32, 0, LS(s)>>>(K, totals, rb.d_off);
+  SCN_CUDA(cudaMemcpyAsync(rb.off.data(), rb.d_off, (K + 1) * 4, cudaMemcpyDeviceToHost, s));
+  if (extraScalars) SCN_CUDA(cudaMemcpyAsync(M.cur().h_scalars, M.cur().d_scalars, extraScalars * 4, cudaMemcpyDeviceToHost, s));
+  SCN_CUDA(cudaStreamSynchronize(s));
+  rb.total = rb.off[K];
+  if (tileCntOut) *tileCntOut = tileCnt;
+  if (!write) return 0;
+  rb.pairs = M.alloc_n<int2>(std::max(1l, rb.total));
+  SCN_CHECK(rb.pairs, "alloc");
+  return write_rule_lists_wide(M, n, K, maskf, pairf, tileCnt, rb.d_off, rb.pairs);
+}
 
 // ------------------------------------------------------------------ per-tile offset masks
 __global__ void __launch_bounds__(128) k_tile_masks(const int *__restrict__ nbr, int nOut, int K, unsigned long long *__restrict__ masks) {
@@ -934,7 +976,29 @@ __global__ void __launch_bounds__(128) k_tile_masks(const int *__restrict__ nbr,
   __syncthreads();
   if (threadIdx.x == 0) masks[tile] = s[0] | s[1] | s[2] | s[3];
 }
+// wide plans: block (tile, chunk) -> the chunk's mask word of the tile (bit j = offset 63 chunk + j), for every tile of the padded plan
+__global__ void __launch_bounds__(128) k_tile_masks_wide(const int *__restrict__ nbr, int nOut, int K, long nPad, unsigned long long *__restrict__ masks) {
+  const int tile = blockIdx.x, c = blockIdx.y, k0 = c * kChunkOffsets, Kc = min(kChunkOffsets, K - k0);
+  const long p = (long)tile * 128 + threadIdx.x;
+  unsigned long long m = 0;
+  if (p < nOut)
+    for (int j = 0; j < Kc; j++) m |= (unsigned long long)(nbr[(long)k0 * nPad + nbr_index(p, j, Kc)] >= 0) << j;
+  for (int d = 16; d > 0; d >>= 1) m |= __shfl_xor_sync(0xffffffffu, m, d);
+  __shared__ unsigned long long s[4];
+  if ((threadIdx.x & 31) == 0) s[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) masks[(long)c * (nPad / 128) + tile] = s[0] | s[1] | s[2] | s[3];
+}
 int Metadata::build_tile_masks(NbrPlan &plan) {
+  if (plan.K > 64) {
+    const long nPad = plan_padded(plan.nOut);
+    plan.tileMask = alloc_n<unsigned long long>(plan_chunks(plan.K) * (nPad / 128) + 8);
+    SCN_CHECK(plan.tileMask, "alloc");
+    if (plan.nOut > 0)
+      k_tile_masks_wide<<<dim3((unsigned)(nPad / 128), plan_chunks(plan.K)), 128, 0, LS(cur().stream)>>>(plan.nbr, plan.nOut, plan.K, nPad, plan.tileMask);
+    SCN_CUDA(cudaGetLastError());
+    return 0;
+  }
   int nTiles = cdiv(std::max(plan.nOut, 1), 128);
   plan.tileMask = alloc_n<unsigned long long>(nTiles + 8);
   SCN_CHECK(plan.tileMask, "alloc");
@@ -1131,6 +1195,50 @@ __global__ void __launch_bounds__(128) k_subm_nbr(GridView g, const int4 *coords
   for (int d = 16; d > 0; d >>= 1) cntv += __shfl_xor_sync(0xffffffffu, cntv, d);
   if ((threadIdx.x & 31) == 0 && cntv) atomicAdd(nValid, cntv);
 }
+// Filters of more than 64 offsets: the same probes into a chunk-major plan (nbr_index_wide); the tile masks are derived from the
+// finished plan (k_tile_masks_wide), one word per chunk.
+__global__ void __launch_bounds__(128) k_subm_nbr_wide(GridView g, const int4 *coords, const int *p2id, int n, int f0, int f1, int f2, long nPad, int *nbr,
+                                                       int *nValid, const int *__restrict__ perm, int *__restrict__ outRow) {
+  const int K = f0 * f1 * f2;
+  int cntv = 0;
+  for (long p = blockIdx.x * (long)blockDim.x + threadIdx.x; p < n; p += (long)gridDim.x * blockDim.x) { // p = plan slot
+    const int site = perm ? perm[p] : (int)p;
+    const int id = p2id[site];
+    if (outRow) outRow[p] = id;
+    const int4 c = coords[id];
+    int k = 0;
+    for (int a = 0; a < f0; a++)
+      for (int b = 0; b < f1; b++)
+        for (int d = 0; d < f2; d++, k++) {
+          const int x = c.x - f0 / 2 + a, y = c.y - f1 / 2 + b, z = c.z - f2 / 2 + d;
+          const int q = (x == c.x && y == c.y && z == c.z) ? site : grid_lookup(g, x, y, z, c.w);
+          const int v = q >= 0 ? p2id[q] : -1;
+          nbr[nbr_index_wide(p, k, K, nPad)] = v;
+          cntv += v >= 0;
+        }
+  }
+  for (int d = 16; d > 0; d >>= 1) cntv += __shfl_xor_sync(0xffffffffu, cntv, d);
+  if ((threadIdx.x & 31) == 0 && cntv) atomicAdd(nValid, cntv);
+}
+struct SubmMaskWide {
+  const int *rank2id, *id2p, *nbr; int K; const int *slot; long nPad;
+  __device__ unsigned long long word(int r, int k0) const {
+    long p = id2p[rank2id[r]];
+    if (slot) p = slot[p];
+    unsigned long long m = 0;
+    for (int k = k0; k < min(K, k0 + 64); k++) m |= (unsigned long long)(nbr[nbr_index_wide(p, k, K, nPad)] >= 0) << (k - k0);
+    return m;
+  }
+};
+struct SubmPairWide {
+  const int *rank2id, *id2p, *nbr; int K; const int *slot; long nPad;
+  __device__ int2 operator()(int r, int L) const {
+    int id = rank2id[r];
+    long p = id2p[id];
+    if (slot) p = slot[p];
+    return make_int2(nbr[nbr_index_wide(p, L, K, nPad)], id);
+  }
+};
 struct SubmMask {
   const int *rank2id, *id2p, *nbr; int K; const int *slot;
   __device__ unsigned long long operator()(int r) const {
@@ -1156,7 +1264,7 @@ struct SubmPair {
 int Metadata::get_submanifold(const long *sz, const long *f, SubmEntry **out) {
   SubmKey key{P3{sz[0], sz[1], sz[2]}, P3{f[0], f[1], f[2]}};
   long K = f[0] * f[1] * f[2];
-  SCN_CHECK(K >= 1 && K <= 64 && f[0] > 0 && f[1] > 0 && f[2] > 0, "unsupported submanifold filter size");
+  SCN_CHECK(f[0] > 0 && f[1] > 0 && f[2] > 0 && K <= kMaxFilterVolume, "unsupported submanifold filter size: the filter volume must be <= 512");
   Grid *g = tl_prefetch_worker ? find_grid_wait(sz) : find_grid(sz);
   SCN_CHECK(g, "no active sites recorded for this spatial size");
   SubmEntry *ep;
@@ -1179,13 +1287,18 @@ int Metadata::get_submanifold(const long *sz, const long *f, SubmEntry **out) {
   const long nPad = plan_padded(g->n);
   e.plan.nbr = alloc_n<int>(std::max(1l, nPad * K));
   SCN_CHECK(e.plan.nbr, "alloc");
-  { // -1 in every slot of the last (partial) work item: whole tiles from the first incomplete one
+  const bool wide = K > 64;
+  if (wide) { // (every chunk has its own partial last work item)
+    SCN_CUDA(cudaMemsetAsync(e.plan.nbr, 0xff, nPad * K * 4, cur().stream));
+  } else { // -1 in every slot of the last (partial) work item: whole tiles from the first incomplete one
     const long t0 = (long)g->n / 128;
     SCN_CUDA(cudaMemsetAsync(e.plan.nbr + t0 * K * 128, 0xff, (nPad / 128 - t0) * K * 128 * 4, cur().stream));
   }
   SCN_CUDA(cudaMemsetAsync(cur().d_scalars, 0, 4, cur().stream));
-  e.plan.tileMask = alloc_n<unsigned long long>(cdiv(std::max(g->n, 1), 128) + 8);
-  SCN_CHECK(e.plan.tileMask, "alloc");
+  if (!wide) {
+    e.plan.tileMask = alloc_n<unsigned long long>(cdiv(std::max(g->n, 1), 128) + 8);
+    SCN_CHECK(e.plan.tileMask, "alloc");
+  }
   static int sortOn = -1;
   if (sortOn < 0) sortOn = getenv("SCN_PLAN_SORT") ? atoi(getenv("SCN_PLAN_SORT")) : 1;
   int *perm = nullptr, *outRowSorted = nullptr;
@@ -1207,7 +1320,11 @@ int Metadata::get_submanifold(const long *sz, const long *f, SubmEntry **out) {
     e.plan.outRow = outRowSorted;
     e.plan.slot = slot;
   }
-  if (g->n) k_subm_nbr<<<stream_grid(g->n, 128, 16), 128, 0, LS(cur().stream)>>>(view(*g), g->coords, g->p2id, g->n, (int)f[0], (int)f[1], (int)f[2], e.plan.nbr, cur().d_scalars, e.plan.tileMask, perm, outRowSorted, nmask);
+  if (wide) {
+    if (g->n) k_subm_nbr_wide<<<stream_grid(g->n, 128, 16), 128, 0, LS(cur().stream)>>>(view(*g), g->coords, g->p2id, g->n, (int)f[0], (int)f[1], (int)f[2], nPad, e.plan.nbr,
+                                                                                  cur().d_scalars, perm, outRowSorted);
+    SCN_TRY(build_tile_masks(e.plan));
+  } else if (g->n) k_subm_nbr<<<stream_grid(g->n, 128, 16), 128, 0, LS(cur().stream)>>>(view(*g), g->coords, g->p2id, g->n, (int)f[0], (int)f[1], (int)f[2], e.plan.nbr, cur().d_scalars, e.plan.tileMask, perm, outRowSorted, nmask);
   // The forward pass only needs the plan and the rule COUNT (the reference's multiply-add counter);
   // the per-offset (in,out) lists in the reference's hash-iteration order are materialised on demand
   // (ensure_subm_rules: backward pass, rulebook inspection).
@@ -1231,7 +1348,13 @@ int Metadata::ensure_subm_rules(SubmEntry &e) {
   SCN_TRY(need(e.rdy));
   SCN_TRY(ensure_rank(*g));
   const int K = e.plan.K;
-  SCN_TRY(build_rule_lists(*this, g->n, K, SubmMask{g->rank2id, g->id2p, e.plan.nbr, K, e.plan.slot}, SubmPair{g->rank2id, g->id2p, e.plan.nbr, K, e.plan.slot}, e.rb, 0));
+  if (K > 64) {
+    const long nPad = plan_padded(e.plan.nOut);
+    SCN_TRY(build_rule_lists_wide(*this, g->n, K, SubmMaskWide{g->rank2id, g->id2p, e.plan.nbr, K, e.plan.slot, nPad},
+                                  SubmPairWide{g->rank2id, g->id2p, e.plan.nbr, K, e.plan.slot, nPad}, e.rb, 0));
+  } else {
+    SCN_TRY(build_rule_lists(*this, g->n, K, SubmMask{g->rank2id, g->id2p, e.plan.nbr, K, e.plan.slot}, SubmPair{g->rank2id, g->id2p, e.plan.nbr, K, e.plan.slot}, e.rb, 0));
+  }
   SCN_CHECK(e.plan.nValid == e.rb.total, "internal: rule count mismatch");
   return mark_ready(e.rulesRdy);
 }
@@ -1293,6 +1416,12 @@ struct ConvMask {
     for (int e = 0; e < G.M; e++) { int off; if (conv_event(G, c, e, j, off)) m |= 1ull << off; }
     return m;
   }
+  __device__ unsigned long long word(int r, int k0) const { // filters of more than 64 offsets: offsets [k0, k0 + 64)
+    int4 c = coords[rank2id[r]], j;
+    unsigned long long m = 0;
+    for (int e = 0; e < G.M; e++) { int off; if (conv_event(G, c, e, j, off) && (unsigned)(off - k0) < 64u) m |= 1ull << (off - k0); }
+    return m;
+  }
 };
 struct ConvPair {
   ConvGeom G; const int *rank2id; const int4 *coords; const int *evQ; const int *outP2id;
@@ -1312,6 +1441,17 @@ __global__ void k_conv_plan(ConvGeom G, const int *rank2id, const int4 *coords, 
     int4 j; int off;
     conv_event(G, coords[id], m, j, off);
     nbr[nbr_index(q, off, G.K)] = id;
+  }
+}
+__global__ void k_conv_plan_wide(ConvGeom G, const int *rank2id, const int4 *coords, const int *evQ, int n, long nPad, int *nbr) {
+  for (long e = blockIdx.x * (long)blockDim.x + threadIdx.x; e < (long)n * G.M; e += (long)gridDim.x * blockDim.x) {
+    int q = evQ[e];
+    if (q < 0) continue;
+    int r = (int)(e / G.M), m = (int)(e % G.M);
+    int id = rank2id[r];
+    int4 j; int off;
+    conv_event(G, coords[id], m, j, off);
+    nbr[nbr_index_wide(q, off, G.K, nPad)] = id;
   }
 }
 
@@ -1555,7 +1695,7 @@ int Metadata::get_conv(const long *inS, const long *outS, const long *f, const l
     if (G.cnt[d] < 1) G.cnt[d] = 1;
     G.M *= G.cnt[d]; G.K *= (int)f[d];
   }
-  SCN_CHECK(G.K <= 64 && G.M <= 64, "unsupported convolution filter size");
+  SCN_CHECK(G.K <= kMaxFilterVolume && G.M <= 64, "unsupported convolution filter size: the filter volume must be <= 512 and the output cells per input site <= 64");
   Grid *gop;
   { std::lock_guard<std::mutex> lk(mapMu); gop = &grids[okey]; }
   ConvEntry &e = *ep;
@@ -1567,7 +1707,7 @@ int Metadata::get_conv(const long *inS, const long *outS, const long *f, const l
   go.batch = gi->batch;
   static int smallOn = -1;
   if (smallOn < 0) smallOn = getenv("SCN_SMALL_FUSED") ? atoi(getenv("SCN_SMALL_FUSED")) : 1;
-  if (smallOn && G.M == 1 && gi->batch == 1 && gi->n > 0 && gi->n <= kSmallSites && gi->itemCtr.size() == 1 && gi->itemCtr[0] >= 0 &&
+  if (smallOn && G.M == 1 && G.K <= 64 && gi->batch == 1 && gi->n > 0 && gi->n <= kSmallSites && gi->itemCtr.size() == 1 && gi->itemCtr[0] >= 0 &&
       ((outS[0] + 7) / 8) * ((outS[1] + 7) / 8) * ((outS[2] + 7) / 8) <= (1 << 16)) {
     SCN_TRY(get_conv_small(*gi, go, e, G));
     SCN_TRY(mark_ready(e.rulesRdy)); // the one-launch build writes the lists as well
@@ -1601,8 +1741,12 @@ int Metadata::get_conv(const long *inS, const long *outS, const long *f, const l
     SCN_TRY(run_scan(*this, E, EvFirstIn{evQ, firstEv}, EvFirstOut{evQ, evPts, go.p2id, go.id2p, go.coords, go.batch > 1 ? sc + 8 : nullptr}, sc + 3));
   }
   // rule lists (one sync: list offsets + nOut + per-item counts)
-  SCN_TRY(build_rule_lists(*this, n, G.K, ConvMask{G, gi->rank2id, gi->coords},
-                           ConvPair{G, gi->rank2id, gi->coords, evQ, go.p2id}, e.rb, 64, /*write=*/false, &e.tileCnt));
+  if (G.K > 64)
+    SCN_TRY(build_rule_lists_wide(*this, n, G.K, ConvMask{G, gi->rank2id, gi->coords},
+                                  ConvPair{G, gi->rank2id, gi->coords, evQ, go.p2id}, e.rb, 64, /*write=*/false, &e.tileCnt));
+  else
+    SCN_TRY(build_rule_lists(*this, n, G.K, ConvMask{G, gi->rank2id, gi->coords},
+                             ConvPair{G, gi->rank2id, gi->coords, evQ, go.p2id}, e.rb, 64, /*write=*/false, &e.tileCnt));
   e.evQ = evQ;
   go.n = cur().h_scalars[3];
   SCN_CHECK(cur().h_scalars[1] == go.n, "internal: unique count mismatch (conv)");
@@ -1616,7 +1760,8 @@ int Metadata::get_conv(const long *inS, const long *outS, const long *f, const l
   e.plan.nbr = alloc_n<int>(std::max(1l, nPadOut * G.K));
   SCN_CHECK(e.plan.nbr, "alloc");
   SCN_CUDA(cudaMemsetAsync(e.plan.nbr, 0xff, std::max(1l, nPadOut * G.K) * 4, s));
-  if (E) k_conv_plan<<<stream_grid(E, 256), 256, 0, LS(s)>>>(G, gi->rank2id, gi->coords, evQ, n, e.plan.nbr);
+  if (E && G.K > 64) k_conv_plan_wide<<<stream_grid(E, 256), 256, 0, LS(s)>>>(G, gi->rank2id, gi->coords, evQ, n, nPadOut, e.plan.nbr);
+  else if (E) k_conv_plan<<<stream_grid(E, 256), 256, 0, LS(s)>>>(G, gi->rank2id, gi->coords, evQ, n, e.plan.nbr);
   SCN_CUDA(cudaGetLastError());
   SCN_TRY(build_tile_masks(e.plan));
   SCN_TRY(mark_ready(go.rdy)); // the event first: a thread that sees `built` must also see the event to wait for
@@ -1638,7 +1783,10 @@ int Metadata::ensure_conv_rules(ConvEntry &e) {
   const int n = gi->n, K = e.geom.K;
   e.rb.pairs = alloc_n<int2>(std::max(1l, e.rb.total));
   SCN_CHECK(e.rb.pairs, "alloc");
-  if (n > 0)
+  if (K > 64)
+    SCN_TRY(write_rule_lists_wide(*this, n, K, ConvMask{e.geom, gi->rank2id, gi->coords}, ConvPair{e.geom, gi->rank2id, gi->coords, e.evQ, go->p2id},
+                                  e.tileCnt, e.rb.d_off, e.rb.pairs));
+  else if (n > 0)
     k_rule_write<<<cdiv(n, kRuleTile), kRuleTile, 0, LS(cur().stream)>>>(n, K, ConvMask{e.geom, gi->rank2id, gi->coords},
                                                                          ConvPair{e.geom, gi->rank2id, gi->coords, e.evQ, go->p2id}, e.tileCnt, e.rb.d_off, e.rb.pairs);
   SCN_CUDA(cudaGetLastError());
@@ -1651,6 +1799,10 @@ struct DeconvMask {
   __device__ unsigned long long operator()(int p) const {
     int4 j; int off;
     return conv_event(G, coords[p2id[p]], 0, j, off) ? 1ull << off : 0ull;
+  }
+  __device__ unsigned long long word(int p, int k0) const {
+    int4 j; int off;
+    return conv_event(G, coords[p2id[p]], 0, j, off) && (unsigned)(off - k0) < 64u ? 1ull << (off - k0) : 0ull;
   }
 };
 struct DeconvPair {
@@ -1676,8 +1828,9 @@ __global__ void k_deconv_pad(const int2 *__restrict__ pairs, const int *__restri
   }
 }
 // tile -> filter offset table, from the list offsets already on the device (no host round trip)
+template <int KMAX>
 __global__ void k_deconv_tiles(const int *__restrict__ off, int K, int *__restrict__ tileW, int *__restrict__ tileFirst) {
-  __shared__ int first[65];
+  __shared__ int first[KMAX + 1];
   if (threadIdx.x == 0) {
     int a = 0;
     for (int k = 0; k < K; k++) { first[k] = a; a += (off[k + 1] - off[k] + 127) / 128; }
@@ -1707,9 +1860,20 @@ int Metadata::get_deconv_plan(ConvEntry &e) {
   SCN_CHECK(tileCnt && dpairs, "alloc");
   DeconvMask mf{e.geom, gf->p2id, gf->coords};
   DeconvPair pf{e.geom, gf->p2id, gf->coords, view(*gc), gc->p2id};
-  k_rule_count<<<nT, kRuleTile, 0, LS(s)>>>(n, K, mf, tileCnt);
-  k_rule_scan<<<K, 1024, 0, LS(s)>>>(nT, K, tileCnt, cur().d_scalars + 128);
-  if (n > 0) k_rule_write<<<nT, kRuleTile, 0, LS(s)>>>(n, K, mf, pf, tileCnt, e.rb.d_off, dpairs);
+  if (K > 64) { // one pass per 64 lists (build_rule_lists_wide); the totals are known already (e.rb.off)
+    int *totals = alloc_n<int>(K), *tc = alloc_n<int>((long)cdiv(K, 64) * nT * 64);
+    SCN_CHECK(totals && tc, "alloc");
+    for (int k0 = 0; k0 < K; k0 += 64) {
+      const int Lw = std::min(64, K - k0);
+      k_rule_count<<<nT, kRuleTile, 0, LS(s)>>>(n, Lw, ChunkMask<DeconvMask>{mf, k0}, tc + (long)(k0 / 64) * nT * 64);
+      k_rule_scan<<<Lw, 1024, 0, LS(s)>>>(nT, Lw, tc + (long)(k0 / 64) * nT * 64, totals + k0);
+    }
+    SCN_TRY(write_rule_lists_wide(*this, n, K, mf, pf, tc, e.rb.d_off, dpairs));
+  } else {
+    k_rule_count<<<nT, kRuleTile, 0, LS(s)>>>(n, K, mf, tileCnt);
+    k_rule_scan<<<K, 1024, 0, LS(s)>>>(nT, K, tileCnt, cur().d_scalars + 128);
+    if (n > 0) k_rule_write<<<nT, kRuleTile, 0, LS(s)>>>(n, K, mf, pf, tileCnt, e.rb.d_off, dpairs);
+  }
   DeconvPlan &d = e.deconv;
   d.nTiles = 0;
   for (int k = 0; k < K; k++) d.nTiles += cdiv(e.rb.off[k + 1] - e.rb.off[k], 128);
@@ -1720,7 +1884,8 @@ int Metadata::get_deconv_plan(ConvEntry &e) {
   int *dFirst = alloc_n<int>(K + 1);
   SCN_CHECK(d.nbr && d.outRow && d.tileW && d.tileMask && dFirst, "alloc");
   if (d.nTiles) {
-    k_deconv_tiles<<<1, 256, 0, LS(s)>>>(e.rb.d_off, K, d.tileW, dFirst);
+    if (K > 64) k_deconv_tiles<kMaxFilterVolume><<<1, 256, 0, LS(s)>>>(e.rb.d_off, K, d.tileW, dFirst);
+    else k_deconv_tiles<64><<<1, 256, 0, LS(s)>>>(e.rb.d_off, K, d.tileW, dFirst);
     k_deconv_pad<<<stream_grid(d.nTiles * 128l, 256), 256, 0, LS(s)>>>(dpairs, e.rb.d_off, d.tileW, dFirst, d.nTiles, d.nbr, d.outRow, d.tileMask);
   }
   SCN_CUDA(cudaGetLastError());

@@ -171,7 +171,7 @@ class Metadata_3(object):
 
     def _rulebook(self, kind, a, b, c):
         nl = C.c_int()
-        lens = (C.c_long * 128)()
+        lens = (C.c_long * 512)()  # one entry per list: filter volumes up to 512 (8^3, [1, 1, 512])
         check(lib().scn_rulebook_info(self._h, kind, a, b, c, C.byref(nl), lens))
         out = []
         for i in range(nl.value):
