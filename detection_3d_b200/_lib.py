@@ -37,7 +37,7 @@ SYMBOLS = {
     "scn_program_backward": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _pi, _vp]),
     "scn_metadata_set_internal_numbering": (_i, [_vp, _i]),
     "scn_get_batch_size": (_i, [_vp, L3, _pi]),
-    "scn_metadata_build_reference_grids": (_i, [_vp, L3, _vp, _i, _l, _i, _i, _i, _i, _vp, _vp]),
+    "scn_metadata_build_reference_grids": (_i, [_vp, _vp, L3, _i, _vp]),
     "scn_metadata_wait_jobs": (_i, [_vp]),
     "scn_rows_to_reference_order": (_i, [_vp, _vp, L3, _vp, _vp, _i]),
     "scn_program_output_copy": (_i, [_vp, _vp, _i, L3, _vp]),

@@ -96,8 +96,7 @@ struct scn_metadata {
   int pending = 0;
   std::atomic<bool> stop{false};
   std::vector<PrefetchOp> ops, ops2; // chain worker (strided convolutions = the grid pyramid) / everything else
-  // input-layer arguments of a job that starts with the input layer itself (kind 0, scn_metadata_build_reference_grids)
-  long inSz[3] = {0, 0, 0}; const long *inCoords = nullptr; int inOnDevice = 0; long inRows = 0; int inCols = 0, inBatch = 0, inMode = 0;
+  scn_metadata *internal = nullptr;   // twin job (scn_metadata_build_reference_grids): the internally numbered Metadata
   int device = 0;
   std::map<scn::P3, scn::RuleBookDev> s2d; // SparseToDense rulebooks (parity / inspection only: the scatter kernel does not need them)
 };
@@ -199,9 +198,7 @@ static void prefetch_worker(scn_metadata *m, int which) {
     if (m->stop) break;
     const long *a = op.v + 1, *b = op.v + 4, *f = op.v + 7, *s = op.v + 10;
     struct Mark { const PrefetchOp &o; ~Mark() { scn::timeline_mark("worker", (int)o.v[0], o.v[1], o.v[7]); } } mark{op};
-    if (op.v[0] == 0) {
-      if (m->md.input_layer(m->inSz, m->inCoords, m->inOnDevice, m->inRows, m->inCols, m->inBatch, m->inMode)) break;
-    } else if (op.v[0] == 1) {
+    if (op.v[0] == 1) {
       scn::SubmEntry *e;
       if (m->md.get_submanifold(a, f, &e)) break;
     } else if (op.v[0] == 2) {
@@ -217,7 +214,17 @@ static void prefetch_worker(scn_metadata *m, int which) {
     }
   }
 }
-// Two process-wide worker threads (chain / everything else) serve the prefetch jobs of all Metadata objects: a thread per
+// The twin job: the numbering overlay of m over m->internal, level by level (input layer first).
+static void twin_worker(scn_metadata *m) {
+  struct Done { scn_metadata *m; ~Done() { m->md.set_chain_done(true); } } done{m};
+  for (const PrefetchOp &op : m->ops) {
+    if (m->stop) break;
+    struct Mark { const PrefetchOp &o; ~Mark() { scn::timeline_mark("twin", (int)o.v[0], o.v[1], o.v[7]); } } mark{op};
+    const long *a = op.v + 1, *b = op.v + 4, *f = op.v + 7, *s = op.v + 10;
+    if (op.v[0] == 0 ? m->md.overlay_input(m->internal->md, a) : m->md.overlay_conv(m->internal->md, a, b, f, s)) break;
+  }
+}
+// Three process-wide worker threads (chain / everything else / twin jobs) serve the prefetch jobs of all Metadata objects: a thread per
 // forward cost ~0.2 ms before its first kernel (creation + binding the CUDA context), on the critical path of the forward.
 namespace {
 struct WorkerPool {
@@ -239,7 +246,8 @@ void pool_main(int which) {
       g_pool->q[which].pop_front();
     }
     if (dev != m->device) { cudaSetDevice(m->device); dev = m->device; }
-    prefetch_worker(m, which == 2 ? 0 : which);
+    if (which == 2) twin_worker(m);
+    else prefetch_worker(m, which);
     { std::lock_guard<std::mutex> lk(m->jobMu); m->pending--; }
     m->jobCv.notify_all();
   }
@@ -313,22 +321,21 @@ int scn_metadata_prefetch(scn_metadata *m, int n_ops, const long *ops) {
   return 0;
 }
 
-// Reference-numbered grids beside an internally numbered forward (program.cu): input layer + the given strided convolutions
-// (ops: n_ops x 13 longs, kind 2), all on a worker thread; scn_metadata_wait_jobs blocks until they are built.
-int scn_metadata_build_reference_grids(scn_metadata *m, const long sz[3], const long *coords, int on_device, long nrows, int ncols, int batch_size,
-                                       int mode, int n_ops, const long *ops, void *coords_ready_event) {
+// Reference-numbered grids beside an internally numbered forward (program.cu): the numbering overlay of the input layer and of
+// the given strided convolutions' output grids, on a worker thread; scn_metadata_wait_jobs blocks until they are built.
+int scn_metadata_build_reference_grids(scn_metadata *m, scn_metadata *internal, const long sz[3], int n_ops, const long *ops) {
   M_OR_FAIL(m);
+  M_OR_FAIL(internal);
   m->md.set_chain_done(true);
   wait_jobs(m);
-  for (int d = 0; d < 3; d++) m->inSz[d] = sz[d];
-  m->inCoords = coords; m->inOnDevice = on_device; m->inRows = nrows; m->inCols = ncols; m->inBatch = batch_size; m->inMode = mode;
-  m->md.coordsReady = static_cast<cudaEvent_t>(coords_ready_event);
   // (stream priorities do not help: normal-priority streams for this job measured 5.39 vs 5.27 ms in round 1; in round 2 the layers on
   // a high-priority stream of their own with this job on lowest-priority streams: 5.19 vs 5.05 ms)
+  m->internal = internal;
   m->ops.clear();
   m->ops2.clear();
   PrefetchOp in;
   for (int j = 0; j < 13; j++) in.v[j] = 0;
+  for (int d = 0; d < 3; d++) in.v[1 + d] = sz[d];
   m->ops.push_back(in);
   for (int i = 0; i < n_ops; i++) {
     PrefetchOp op;
@@ -343,6 +350,7 @@ int scn_metadata_build_reference_grids(scn_metadata *m, const long sz[3], const 
 int scn_metadata_wait_jobs(scn_metadata *m) {
   M_OR_FAIL(m);
   wait_jobs(m);
+  m->md.to_compute();
   return 0;
 }
 int scn_input_layer_build(scn_metadata *m, const long sz[3], const long *coords, int on_device, long nrows, int ncols,

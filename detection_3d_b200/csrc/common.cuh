@@ -59,7 +59,8 @@ enum DebugCounter {
   kCntFloatAtomic = 14,    // launches that accumulated floats with atomics, i.e. whose result depends on the order the atomics land in
   kCntTf32x3Launch = 15,   // conv_plan_tc launches with TF32X3 operands (math mode 3)
   kCntChunkedLaunch = 16,  // conv_plan_tc launches over one offset chunk of a plan with more than 64 filter offsets
-  kCntCounters = 17
+  kCntCoordUpload = 17,    // host -> device copies of input-layer coordinates
+  kCntCounters = 18
 };
 extern std::atomic<long> g_counters[kCntCounters];
 

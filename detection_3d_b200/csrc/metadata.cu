@@ -138,13 +138,7 @@ Metadata::~Metadata() {
   // blocked, so that the next Metadata (which recycles them, possibly while this forward still computes: streaming
   // inference with FPN_Net.prefetch) can start building at once.
   std::lock_guard<std::mutex> lk(g_pool_mu);
-  for (int i = 0; i < nCtx; i++) {
-    BuildCtx &c = cx[i];
-    if (evCompute && c.stream != cstream) {
-      cudaEventRecord(evCompute, c.stream);
-      cudaStreamWaitEvent(cstream, evCompute, 0);
-    }
-  }
+  to_compute();
   for (int i = 0; i < nCtx; i++) {
     BuildCtx &c = cx[i];
     for (Chunk &k : c.chunks) {
@@ -192,6 +186,15 @@ int Metadata::from_compute() {
   SCN_CUDA(cudaEventRecord(evCompute, cstream));
   SCN_CUDA(cudaStreamWaitEvent(cur().stream, evCompute, 0));
   return 0;
+}
+void Metadata::to_compute() {
+  for (int i = 0; i < nCtx; i++) {
+    BuildCtx &c = cx[i];
+    if (evCompute && c.stream != cstream) {
+      cudaEventRecord(evCompute, c.stream);
+      cudaStreamWaitEvent(cstream, evCompute, 0);
+    }
+  }
 }
 void *Metadata::alloc_in(BuildCtx &c, size_t bytes) {
   void *p = nullptr;
@@ -528,15 +531,13 @@ int Metadata::input_layer(const long *sz, const long *coords, int onDevice, long
   Grid &g = *gp;
   g.sz = key;
   cudaStream_t s = cur().stream;
-  if (onDevice == 1) { // the coordinates were produced on the caller's stream (2: already complete, no dependency)
-    if (coordsReady) SCN_CUDA(cudaStreamWaitEvent(s, coordsReady, 0));
-    else SCN_TRY(from_compute());
-  }
+  if (onDevice == 1) SCN_TRY(from_compute()); // the coordinates were produced on the caller's stream (2: already complete, no dependency)
   const long *dcoords = coords;
   if (!onDevice && nrows) {
     long *tmp = alloc_n<long>(nrows * ncols);
     SCN_CHECK(tmp, "alloc");
     SCN_CUDA(cudaMemcpyAsync(tmp, coords, nrows * ncols * 8, cudaMemcpyHostToDevice, s));
+    ++g_counters[kCntCoordUpload];
     dcoords = tmp;
   }
   int4 *pts = alloc_n<int4>(std::max(1l, nrows));
@@ -584,24 +585,108 @@ int Metadata::input_layer(const long *sz, const long *coords, int onDevice, long
   }
   { std::lock_guard<std::mutex> lk(mapMu); g.built = true; }
   SCN_TRY(mark_ready(g.rdy));
-  // rules
   input.mode = mode; input.nIn = (int)nrows; input.nOut = g.n; input.valid = true;
   input.maxActive = (mode == 3 || mode == 4) ? maxActive : 1;
-  if (mode == 0) { input.tab = nullptr; return mark_ready(input.rdy); }
+  input.rowP = rowP; input.firstRow = firstRow; input.lastRow = lastRow; input.pts = pts;
+  return input_rules(g);
+}
+// The rule table of the input layer in the numbering of g (input.mode / maxActive / nIn / rowP / firstRow / lastRow are set).
+int Metadata::input_rules(const Grid &g) {
+  if (input.mode == 0) { input.tab = nullptr; return mark_ready(input.rdy); }
+  cudaStream_t s = cur().stream;
   int w = 1 + input.maxActive;
   input.tab = alloc_n<int>(std::max(1l, (long)g.n * w));
   SCN_CHECK(input.tab, "alloc");
   if (g.n == 0) return mark_ready(input.rdy);
-  if (mode == 3 || mode == 4) {
+  if (input.mode == 3 || input.mode == 4) {
     SCN_CUDA(cudaMemsetAsync(input.tab, 0, (long)g.n * w * 4, s));
-    k_input_rules_fill<<<stream_grid(nrows, 256), 256, 0, LS(s)>>>(rowP, g.p2id, nrows, input.tab, w);
-    if (maxActive > 1) k_input_rules_sort<<<stream_grid(g.n, 256), 256, 0, LS(s)>>>(input.tab, g.n, w);
+    k_input_rules_fill<<<stream_grid(input.nIn, 256), 256, 0, LS(s)>>>(input.rowP, g.p2id, input.nIn, input.tab, w);
+    if (input.maxActive > 1) k_input_rules_sort<<<stream_grid(g.n, 256), 256, 0, LS(s)>>>(input.tab, g.n, w);
   } else {
     // IOLayersRules.h:100-110: mode 1 keeps the FIRST row of a voxel, mode 2 the LAST
-    k_input_rules_pick<<<stream_grid(g.n, 256), 256, 0, LS(s)>>>(mode == 1 ? firstRow : lastRow, g.id2p, g.n, input.tab);
+    k_input_rules_pick<<<stream_grid(g.n, 256), 256, 0, LS(s)>>>(input.mode == 1 ? input.firstRow : input.lastRow, g.id2p, g.n, input.tab);
   }
   SCN_CUDA(cudaGetLastError());
   return mark_ready(input.rdy);
+}
+
+// ------------------------------------------------------------------ numbering overlay
+// copies the block structure of `src` (same spatial size and sites) into g's own buffers; only the nblocks * 8 live occupancy
+// words are copied -- maxBlocks is bounded by the input rows, at level 0 many times the live blocks
+__global__ void k_copy_words(const unsigned long long *__restrict__ bmask, const int *__restrict__ wbase, const int *__restrict__ nblocks,
+                             unsigned long long *__restrict__ bOut, int *__restrict__ wOut) {
+  const long n = (long)(*nblocks) * 8;
+  for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) { bOut[i] = bmask[i]; wOut[i] = wbase[i]; }
+}
+static int copy_blocks(Metadata &M, Grid &g, const Grid &src) {
+  for (int d = 0; d < 3; d++) g.dd[d] = src.dd[d];
+  g.dirCells = src.dirCells;
+  g.maxBlocks = src.maxBlocks;
+  const long cells = g.dirCells * g.batch;
+  g.dir = M.alloc_n<int>(cells);
+  g.d_nblocks = M.alloc_n<int>(4);
+  g.bmask = M.alloc_n<unsigned long long>(g.maxBlocks * 8);
+  g.wbase = M.alloc_n<int>(g.maxBlocks * 8);
+  SCN_CHECK(g.dir && g.bmask && g.wbase && g.d_nblocks, "alloc");
+  cudaStream_t s = M.cur().stream;
+  SCN_CUDA(cudaMemcpyAsync(g.dir, src.dir, cells * 4, cudaMemcpyDeviceToDevice, s));
+  SCN_CUDA(cudaMemcpyAsync(g.d_nblocks, src.d_nblocks, 4, cudaMemcpyDeviceToDevice, s));
+  k_copy_words<<<stream_grid(g.maxBlocks * 8, 256), 256, 0, LS(s)>>>(src.bmask, src.wbase, src.d_nblocks, g.bmask, g.wbase);
+  SCN_CUDA(cudaGetLastError());
+  return 0;
+}
+// The internally numbered grid of size sz once `in`'s chain worker has made it (nullptr: the chain worker has finished without it);
+// this build stream waits for it.
+static Grid *internal_grid(Metadata &M, Metadata &in, const long *sz) {
+  Grid *gq = in.find_grid_wait(sz);
+  if (gq && gq->rdy.ev && cudaStreamWaitEvent(M.cur().stream, gq->rdy.ev, 0) != cudaSuccess) return nullptr;
+  return gq;
+}
+static Grid *new_grid(Metadata &M, const long *sz) {
+  std::lock_guard<std::mutex> lk(M.mapMu);
+  const P3 key{sz[0], sz[1], sz[2]};
+  if (M.grids.find(key) != M.grids.end()) return nullptr;
+  Grid *g = &M.grids[key];
+  g->sz = key;
+  return g;
+}
+static int publish_grid(Metadata &M, Grid &g) {
+  g.itemCount.assign(1, g.n);
+  g.itemCtr.assign(1, 0);
+  SCN_TRY(M.mark_ready(g.rdy)); // the event first: a thread that sees `built` must also see the event to wait for
+  { std::lock_guard<std::mutex> lk(M.mapMu); g.built = true; }
+  M.cv.notify_all();
+  return 0;
+}
+// Input level: the reference id of a site is the rank of its first input row among the first rows of all sites (FirstIn /
+// FirstOut, as in input_layer), read from the internal input layer's arrays -- no coordinate upload, no block build.
+int Metadata::overlay_input(Metadata &in, const long *sz) {
+  Grid *gq = in.find_grid(sz);
+  SCN_CHECK(gq && in.input.valid && gq->batch == 1, "numbering overlay: the internal input layer is missing");
+  BuildLock bl(*this);
+  SCN_CHECK(!input.valid, "input layer already built for this Metadata");
+  Grid *gp = new_grid(*this, sz);
+  SCN_CHECK(gp, "input layer already built for this Metadata");
+  Grid &g = *gp;
+  cudaStream_t s = cur().stream;
+  if (gq->rdy.ev) SCN_CUDA(cudaStreamWaitEvent(s, gq->rdy.ev, 0));
+  g.batch = 1;
+  g.n = gq->n;
+  SCN_TRY(copy_blocks(*this, g, *gq));
+  const long nrows = in.input.nIn, cap = std::max(1, g.n);
+  g.coords = alloc_n<int4>(cap);
+  g.p2id = alloc_n<int>(cap);
+  g.id2p = alloc_n<int>(cap);
+  SCN_CHECK(g.coords && g.p2id && g.id2p, "alloc");
+  const InputRules &I = in.input;
+  SCN_TRY(run_scan(*this, nrows, FirstIn{I.rowP, I.firstRow}, FirstOut{I.rowP, I.pts, g.p2id, g.id2p, g.coords}, nullptr));
+  SCN_TRY(publish_grid(*this, g));
+  input.mode = I.mode; input.nIn = I.nIn; input.nOut = g.n; input.maxActive = I.maxActive; input.valid = true;
+  input.rowP = I.rowP; input.firstRow = I.firstRow; input.lastRow = I.lastRow; input.pts = I.pts;
+  SCN_TRY(input_rules(g));
+  input.rowP = input.firstRow = input.lastRow = nullptr; // `in`'s buffers: not kept beyond this build
+  input.pts = nullptr;
+  return 0;
 }
 
 // ------------------------------------------------------------------ dense_hash_map order
@@ -1669,6 +1754,26 @@ int Metadata::get_conv_small(Grid &gi, Grid &go, ConvEntry &e, const ConvGeomHos
   return 0;
 }
 
+static int conv_geom(const long *f, const long *st, const long *outS, ConvGeom &G) {
+  G.M = 1; G.K = 1;
+  for (int d = 0; d < 3; d++) {
+    SCN_CHECK(f[d] >= 1 && st[d] >= 1 && outS[d] >= 1, "bad filter geometry");
+    G.f[d] = (int)f[d]; G.s[d] = (int)st[d]; G.outS[d] = (int)outS[d];
+    G.cnt[d] = (int)std::min<long>(outS[d], (f[d] + st[d] - 1) / st[d]);
+    if (G.cnt[d] < 1) G.cnt[d] = 1;
+    G.M *= G.cnt[d]; G.K *= (int)f[d];
+  }
+  SCN_CHECK(G.K <= kMaxFilterVolume && G.M <= 64, "unsupported convolution filter size: the filter volume must be <= 512 and the output cells per input site <= 64");
+  return 0;
+}
+// get_conv_small serves this convolution (one launch builds the output grid, its numbering, the lists and the plan)
+static bool small_conv(const Grid &gi, const ConvGeom &G, const long *outS) {
+  static int smallOn = -1;
+  if (smallOn < 0) smallOn = getenv("SCN_SMALL_FUSED") ? atoi(getenv("SCN_SMALL_FUSED")) : 1;
+  return smallOn && G.M == 1 && G.K <= 64 && gi.batch == 1 && gi.n > 0 && gi.n <= kSmallSites && gi.itemCtr.size() == 1 && gi.itemCtr[0] >= 0 &&
+         ((outS[0] + 7) / 8) * ((outS[1] + 7) / 8) * ((outS[2] + 7) / 8) <= (1 << 16);
+}
+
 // getRuleBook (Metadata.cpp:484-510) -> Convolution_InputSgToRulesAndOutputSg (ConvolutionRules.h:11-34)
 int Metadata::get_conv(const long *inS, const long *outS, const long *f, const long *st, ConvEntry **out) {
   ConvKey key{P3{inS[0], inS[1], inS[2]}, P3{f[0], f[1], f[2]}, P3{st[0], st[1], st[2]}};
@@ -1682,33 +1787,25 @@ int Metadata::get_conv(const long *inS, const long *outS, const long *f, const l
   struct Guard { Metadata &m; Ready &r; ~Guard() { if (!r.ready) m.unclaim(r); } } guard{*this, ep->rdy};
   BuildLock bl(*this);
   SCN_TRY(need(gi->rdy));
+  ConvEntry &e = *ep;
+  // gridGiven: overlay_conv made the output grid (numbering included) and the events' spatial indices evQ; what is left are the
+  // rule counts, the plan and the tile masks over that grid
+  const bool given = e.gridGiven;
   {
     std::lock_guard<std::mutex> lk(mapMu);
-    SCN_CHECK(grids.find(okey) == grids.end(), "output spatial size already has a grid (each spatial size may occur once per Metadata)");
+    SCN_CHECK(given ? e.out == okey : grids.find(okey) == grids.end(), "output spatial size already has a grid (each spatial size may occur once per Metadata)");
   }
   ConvGeom G;
-  G.M = 1; G.K = 1;
-  for (int d = 0; d < 3; d++) {
-    SCN_CHECK(f[d] >= 1 && st[d] >= 1 && outS[d] >= 1, "bad filter geometry");
-    G.f[d] = (int)f[d]; G.s[d] = (int)st[d]; G.outS[d] = (int)outS[d];
-    G.cnt[d] = (int)std::min<long>(outS[d], (f[d] + st[d] - 1) / st[d]);
-    if (G.cnt[d] < 1) G.cnt[d] = 1;
-    G.M *= G.cnt[d]; G.K *= (int)f[d];
-  }
-  SCN_CHECK(G.K <= kMaxFilterVolume && G.M <= 64, "unsupported convolution filter size: the filter volume must be <= 512 and the output cells per input site <= 64");
+  SCN_TRY(conv_geom(f, st, outS, G));
   Grid *gop;
   { std::lock_guard<std::mutex> lk(mapMu); gop = &grids[okey]; }
-  ConvEntry &e = *ep;
   e.out = okey;
   e.in = key.in;
   e.geom = G;
   Grid &go = *gop;
-  go.sz = okey;
-  go.batch = gi->batch;
-  static int smallOn = -1;
-  if (smallOn < 0) smallOn = getenv("SCN_SMALL_FUSED") ? atoi(getenv("SCN_SMALL_FUSED")) : 1;
-  if (smallOn && G.M == 1 && G.K <= 64 && gi->batch == 1 && gi->n > 0 && gi->n <= kSmallSites && gi->itemCtr.size() == 1 && gi->itemCtr[0] >= 0 &&
-      ((outS[0] + 7) / 8) * ((outS[1] + 7) / 8) * ((outS[2] + 7) / 8) <= (1 << 16)) {
+  if (!given && small_conv(*gi, G, outS)) {
+    go.sz = okey;
+    go.batch = gi->batch;
     SCN_TRY(get_conv_small(*gi, go, e, G));
     SCN_TRY(mark_ready(e.rulesRdy)); // the one-launch build writes the lists as well
     SCN_TRY(mark_ready(go.rdy));
@@ -1721,39 +1818,49 @@ int Metadata::get_conv(const long *inS, const long *outS, const long *f, const l
   cudaStream_t s = cur().stream;
   const int n = gi->n;
   const long E = (long)n * G.M;
-  int4 *evPts = alloc_n<int4>(std::max(1l, E));
-  int *evQ = alloc_n<int>(std::max(1l, E));
-  SCN_CHECK(evPts && evQ, "alloc");
-  int *sc = cur().d_scalars; // [1] nunique [3] nOut [8..56) per-item counts
-  SCN_CUDA(cudaMemsetAsync(sc, 0, 64 * 4, s));
-  if (E) k_conv_events<<<stream_grid(E, 256), 256, 0, LS(s)>>>(G, gi->rank2id, gi->coords, n, evPts);
-  SCN_TRY(build_blocks(*this, go, evPts, E, evQ, sc + 1));
-  long cap = std::max(1l, E);
-  go.coords = alloc_n<int4>(cap); go.p2id = alloc_n<int>(cap); go.id2p = alloc_n<int>(cap);
-  int *firstEv = alloc_n<int>(cap);
-  SCN_CHECK(go.coords && go.p2id && go.id2p && firstEv, "alloc");
-  if (spatialIds) {
-    if (E) k_spatial_conv_ids<<<stream_grid(E, 256), 256, 0, LS(s)>>>(evQ, evPts, E, go.coords, go.p2id, go.id2p);
-    k_copy_scalar<<<1, 1, 0, LS(s)>>>(sc + 1, sc + 3);
-  } else {
-    SCN_CUDA(cudaMemsetAsync(firstEv, 0x7f, cap * 4, s));
-    if (E) k_first_event<<<stream_grid(E, 256), 256, 0, LS(s)>>>(evQ, E, firstEv);
-    SCN_TRY(run_scan(*this, E, EvFirstIn{evQ, firstEv}, EvFirstOut{evQ, evPts, go.p2id, go.id2p, go.coords, go.batch > 1 ? sc + 8 : nullptr}, sc + 3));
+  const int *evQ = e.evQ;
+  if (given) SCN_TRY(need(go.rdy));
+  else {
+    go.sz = okey;
+    go.batch = gi->batch;
+    int4 *evPts = alloc_n<int4>(std::max(1l, E));
+    int *q = alloc_n<int>(std::max(1l, E));
+    SCN_CHECK(evPts && q, "alloc");
+    int *sc = cur().d_scalars; // [1] nunique [3] nOut [8..56) per-item counts
+    SCN_CUDA(cudaMemsetAsync(sc, 0, 64 * 4, s));
+    if (E) k_conv_events<<<stream_grid(E, 256), 256, 0, LS(s)>>>(G, gi->rank2id, gi->coords, n, evPts);
+    SCN_TRY(build_blocks(*this, go, evPts, E, q, sc + 1));
+    long cap = std::max(1l, E);
+    go.coords = alloc_n<int4>(cap); go.p2id = alloc_n<int>(cap); go.id2p = alloc_n<int>(cap);
+    int *firstEv = alloc_n<int>(cap);
+    SCN_CHECK(go.coords && go.p2id && go.id2p && firstEv, "alloc");
+    if (spatialIds) {
+      if (E) k_spatial_conv_ids<<<stream_grid(E, 256), 256, 0, LS(s)>>>(q, evPts, E, go.coords, go.p2id, go.id2p);
+      k_copy_scalar<<<1, 1, 0, LS(s)>>>(sc + 1, sc + 3);
+    } else {
+      SCN_CUDA(cudaMemsetAsync(firstEv, 0x7f, cap * 4, s));
+      if (E) k_first_event<<<stream_grid(E, 256), 256, 0, LS(s)>>>(q, E, firstEv);
+      SCN_TRY(run_scan(*this, E, EvFirstIn{q, firstEv}, EvFirstOut{q, evPts, go.p2id, go.id2p, go.coords, go.batch > 1 ? sc + 8 : nullptr}, sc + 3));
+    }
+    evQ = q;
   }
   // rule lists (one sync: list offsets + nOut + per-item counts)
+  const int extra = given ? 0 : 64;
   if (G.K > 64)
     SCN_TRY(build_rule_lists_wide(*this, n, G.K, ConvMask{G, gi->rank2id, gi->coords},
-                                  ConvPair{G, gi->rank2id, gi->coords, evQ, go.p2id}, e.rb, 64, /*write=*/false, &e.tileCnt));
+                                  ConvPair{G, gi->rank2id, gi->coords, evQ, go.p2id}, e.rb, extra, /*write=*/false, &e.tileCnt));
   else
     SCN_TRY(build_rule_lists(*this, n, G.K, ConvMask{G, gi->rank2id, gi->coords},
-                             ConvPair{G, gi->rank2id, gi->coords, evQ, go.p2id}, e.rb, 64, /*write=*/false, &e.tileCnt));
+                             ConvPair{G, gi->rank2id, gi->coords, evQ, go.p2id}, e.rb, extra, /*write=*/false, &e.tileCnt));
   e.evQ = evQ;
-  go.n = cur().h_scalars[3];
-  SCN_CHECK(cur().h_scalars[1] == go.n, "internal: unique count mismatch (conv)");
-  go.itemCount.assign(go.batch, 0);
-  go.itemCtr.assign(go.batch, 0);
-  int ctr = 0;
-  for (int b = 0; b < go.batch; b++) { go.itemCount[b] = go.batch > 1 ? cur().h_scalars[8 + b] : go.n; go.itemCtr[b] = ctr; ctr += go.itemCount[b]; }
+  if (!given) {
+    go.n = cur().h_scalars[3];
+    SCN_CHECK(cur().h_scalars[1] == go.n, "internal: unique count mismatch (conv)");
+    go.itemCount.assign(go.batch, 0);
+    go.itemCtr.assign(go.batch, 0);
+    int ctr = 0;
+    for (int b = 0; b < go.batch; b++) { go.itemCount[b] = go.batch > 1 ? cur().h_scalars[8 + b] : go.n; go.itemCtr[b] = ctr; ctr += go.itemCount[b]; }
+  }
   // output-stationary plan
   e.plan.K = G.K; e.plan.nOut = go.n; e.plan.outRow = go.p2id; e.plan.nValid = e.rb.total;
   const long nPadOut = plan_padded(go.n);
@@ -1764,11 +1871,72 @@ int Metadata::get_conv(const long *inS, const long *outS, const long *f, const l
   else if (E) k_conv_plan<<<stream_grid(E, 256), 256, 0, LS(s)>>>(G, gi->rank2id, gi->coords, evQ, n, e.plan.nbr);
   SCN_CUDA(cudaGetLastError());
   SCN_TRY(build_tile_masks(e.plan));
-  SCN_TRY(mark_ready(go.rdy)); // the event first: a thread that sees `built` must also see the event to wait for
-  { std::lock_guard<std::mutex> lk(mapMu); go.built = true; }
-  cv.notify_all();
+  if (!given) {
+    SCN_TRY(mark_ready(go.rdy)); // the event first: a thread that sees `built` must also see the event to wait for
+    { std::lock_guard<std::mutex> lk(mapMu); go.built = true; }
+    cv.notify_all();
+  }
   SCN_TRY(mark_ready(e.rdy));
   return 0;
+}
+
+// Output level of a strided convolution, numbered as get_conv numbers it: the events of the input sites in hash-iteration order
+// find their spatial index in the internal output grid (whose block structure this grid copies) and the first-touch scan turns
+// them into reference ids.  Rule lists and plan are left to get_conv (entry.gridGiven), which nothing in a replayed forward
+// calls.  Small levels take the one-launch get_conv as they are.
+int Metadata::overlay_conv(Metadata &in, const long *inS, const long *outS, const long *f, const long *st) {
+  Grid *gi = find_grid(inS);
+  SCN_CHECK(gi, "numbering overlay: no grid of the input spatial size");
+  ConvGeom G;
+  SCN_TRY(conv_geom(f, st, outS, G));
+  if (small_conv(*gi, G, outS)) {
+    ConvEntry *e;
+    return get_conv(inS, outS, f, st, &e);
+  }
+  SCN_CHECK(gi->batch == 1, "numbering overlay: one batch item");
+  BuildLock bl(*this);
+  SCN_TRY(need(gi->rdy));
+  SCN_TRY(ensure_rank(*gi)); // first: the hash-order emulation does not need the internal output grid
+  Grid *gq = internal_grid(*this, in, outS);
+  if (!gq) { // not made by `in`'s chain worker (a leaf of the pyramid, built later by another thread): the complete build
+    ConvEntry *e;
+    return get_conv(inS, outS, f, st, &e);
+  }
+  ConvEntry *ep;
+  {
+    std::lock_guard<std::mutex> lk(mapMu);
+    ep = &conv[ConvKey{P3{inS[0], inS[1], inS[2]}, P3{f[0], f[1], f[2]}, P3{st[0], st[1], st[2]}}];
+  }
+  SCN_CHECK(!ep->rdy.ready && !ep->rdy.building && !ep->gridGiven, "numbering overlay: convolution already built");
+  Grid *gop = new_grid(*this, outS);
+  SCN_CHECK(gop, "output spatial size already has a grid (each spatial size may occur once per Metadata)");
+  Grid &go = *gop;
+  cudaStream_t s = cur().stream;
+  go.batch = 1;
+  go.n = gq->n;
+  SCN_TRY(copy_blocks(*this, go, *gq));
+  const int n = gi->n;
+  const long E = (long)n * G.M, cap = std::max(1, go.n);
+  int4 *evPts = alloc_n<int4>(std::max(1l, E));
+  int *evQ = alloc_n<int>(std::max(1l, E)), *firstEv = alloc_n<int>(cap);
+  go.coords = alloc_n<int4>(cap); go.p2id = alloc_n<int>(cap); go.id2p = alloc_n<int>(cap);
+  SCN_CHECK(evPts && evQ && firstEv && go.coords && go.p2id && go.id2p, "alloc");
+  SCN_CUDA(cudaMemsetAsync(firstEv, 0x7f, cap * 4, s));
+  if (E) {
+    k_conv_events<<<stream_grid(E, 256), 256, 0, LS(s)>>>(G, gi->rank2id, gi->coords, n, evPts);
+    k_lookup_pts<<<stream_grid(E, 256), 256, 0, LS(s)>>>(view(go), evPts, E, evQ);
+    k_first_event<<<stream_grid(E, 256), 256, 0, LS(s)>>>(evQ, E, firstEv);
+  }
+  SCN_TRY(run_scan(*this, E, EvFirstIn{evQ, firstEv}, EvFirstOut{evQ, evPts, go.p2id, go.id2p, go.coords, nullptr}, nullptr));
+  {
+    std::lock_guard<std::mutex> lk(mapMu);
+    ep->in = P3{inS[0], inS[1], inS[2]};
+    ep->out = go.sz;
+    ep->geom = G;
+    ep->evQ = evQ;
+    ep->gridGiven = true;
+  }
+  return publish_grid(*this, go);
 }
 
 // The (in,out) lists of a strided convolution in the reference's order (ConvolutionRules.h:11-34), written on demand.

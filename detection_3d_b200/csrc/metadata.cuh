@@ -89,11 +89,16 @@ struct SubmEntry { RuleBookDev rb; NbrPlan plan; Ready rdy, rulesRdy; P3 sz; boo
 struct ConvEntry {
   RuleBookDev rb; NbrPlan plan; P3 out; P3 in; ConvGeomHost geom; DeconvPlan deconv; Ready rdy, deconvRdy, rulesRdy;
   const int *evQ = nullptr; int *tileCnt = nullptr; // kept for the deferred list write
+  bool gridGiven = false; // the output grid and evQ came from overlay_conv: get_conv builds the lists and the plan over that grid
 };
 
 struct InputRules {
   int mode = 0, maxActive = 0, nIn = 0, nOut = 0;
   int *tab = nullptr;  // [nOut*(1+maxActive)] device
+  // per input row: spatial index and coordinates; per site (spatial index): first / last input row (lastRow: mode 2 only).
+  // Numbering-independent: overlay_input numbers a twin's input level from them.
+  const int *rowP = nullptr, *firstRow = nullptr, *lastRow = nullptr;
+  const int4 *pts = nullptr;
   bool valid = false;
   Ready rdy;
 };
@@ -136,9 +141,9 @@ struct Metadata {
   int nCtx = 1;
   BuildCtx &cur();           // build context of the calling thread
   cudaEvent_t evCompute = nullptr;
-  cudaEvent_t coordsReady = nullptr; // optional (not owned): device coordinates are complete once this event has fired (input_layer, on_device == 1)
   int use_low_priority_streams(); // builds of this Metadata are not urgent: move its build contexts to normal-priority streams
   int from_compute();        // the current build stream waits for everything the caller has queued so far
+  void to_compute();         // the caller's stream waits for everything the build streams have queued so far
   // `mapMu` guards the structure of the caches and the ready / building flags; `cv` wakes threads
   // that wait for an entry another thread is building.
   std::mutex mapMu;
@@ -175,6 +180,12 @@ struct Metadata {
 
   int input_layer(const long *sz, const long *coords, int coordsOnDevice, long nrows, int ncols,
                   int batchHint, int mode);
+  int input_rules(const Grid &g);
+  // Reference numbering over the grids of an internally numbered Metadata `in` built from the same input (one batch item):
+  // the input level, and the output grid of one strided convolution, take the block structure of `in`'s grid of the same
+  // size and compute only the reference row ids (and the hash-iteration order that induces them).
+  int overlay_input(Metadata &in, const long *sz);
+  int overlay_conv(Metadata &in, const long *inS, const long *outS, const long *f, const long *st);
   Grid *find_grid(const long *sz);
   int ensure_rank(Grid &g);
   int get_submanifold(const long *sz, const long *f, SubmEntry **out);

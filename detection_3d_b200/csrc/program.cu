@@ -67,7 +67,6 @@ struct scn_program {
   std::vector<char> statsDone;
   scn_metadata *ms = nullptr;   // internally numbered Metadata of the current / last run (see scn_program_run)
   bool internal = false;        // the registers of the last run are in internal row order
-  cudaEvent_t evCoords = nullptr;
   cudaEvent_t evEnd[2] = {nullptr, nullptr}; // end of the last two runs on `stream` (throttle of scn_program_prepare)
   long nRuns = 0;
   cudaStream_t stream = nullptr;
@@ -128,7 +127,6 @@ void scn_program_destroy(scn_program *p) {
   if (p->stats) cudaFree(p->stats);
   for (cudaEvent_t e : p->evEnd) if (e) cudaEventDestroy(e);
   if (p->ms) scn_metadata_destroy(p->ms);
-  if (p->evCoords) cudaEventDestroy(p->evCoords);
   delete p;
 }
 int scn_program_set_training(scn_program *p, int on) {
@@ -357,9 +355,10 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
   // ---- Which Metadata do the layers run on?
   // A forward whose Metadata arrives unprepared runs on an INTERNALLY NUMBERED Metadata of its own (rows = spatial order):
   // the reference's hash-iteration order and first-touch numbering -- ~40 % of the grid-pyramid latency, all of it on the
-  // critical path -- are not needed to compute anything, only to NAME the rows.  The caller's Metadata `m` is built beside
-  // it on a worker thread (input layer + the strided convolutions that lead to the output grids, in the reference's
-  // numbering) and the output rows are handed out in that numbering (scn_program_output_copy).  A Metadata prepared ahead
+  // critical path -- are not needed to compute anything, only to NAME the rows.  The caller's Metadata `m` is numbered beside
+  // it on a worker thread (input layer + the strided convolutions that lead to the output grids: reference row ids over the
+  // block structure of the internal grids, scn_metadata_build_reference_grids) and the output rows are handed out in that
+  // numbering (scn_program_output_copy).  The layers' rulebooks on `m` are built on first use.  A Metadata prepared ahead
   // (scn_program_prepare) or an input mode / batch the internal numbering does not cover uses `m` for everything, as before.
   static int internalOn = -1;
   if (internalOn < 0) internalOn = getenv("SCN_INTERNAL_IDS") ? atoi(getenv("SCN_INTERNAL_IDS")) : 1;
@@ -376,10 +375,6 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
   static int trainInternal = -1; // training runs on the internally numbered Metadata too (rows in spatial order: every gather of the
   if (trainInternal < 0) trainInternal = getenv("SCN_TRAIN_INTERNAL") ? atoi(getenv("SCN_TRAIN_INTERNAL")) : 1; // forward AND backward pass stays local)
   if ((!train || trainInternal) && internalOn && inOp && inOp->a[4] != 0 && !scn_input_layer_built(m, nullptr, nullptr)) {
-    if (coords_on_device == 1) {
-      if (!p->evCoords) SCN_CUDA(cudaEventCreateWithFlags(&p->evCoords, cudaEventDisableTiming));
-      SCN_CUDA(cudaEventRecord(p->evCoords, s));
-    }
     SCN_TRY(scn_metadata_create(&p->ms, stream));
     SCN_TRY(scn_metadata_set_internal_numbering(p->ms, 1));
     SCN_TRY(scn_program_prepare(p, p->ms, coords, coords_on_device, nrows, ncols));
@@ -408,8 +403,7 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
     }
     static const bool skipTwin = getenv("SCN_SKIP_TWIN") && atoi(getenv("SCN_SKIP_TWIN")); // developer timing experiment only: outputs stay in internal row order
     if (batch == 1 && !skipTwin)
-    SCN_TRY(scn_metadata_build_reference_grids(m, inOp->a + 1, coords, coords_on_device, nrows, ncols, (int)inOp->a[5], (int)inOp->a[4],
-                                               (int)(hints.size() / 13), hints.data(), coords_on_device == 1 ? p->evCoords : nullptr));
+    SCN_TRY(scn_metadata_build_reference_grids(m, p->ms, inOp->a + 1, (int)(hints.size() / 13), hints.data()));
     if (batch == 1) {
       M = p->ms;
       p->internal = true;
@@ -599,6 +593,7 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
     scn::epilogue_stats_take();
     scn::prepadded_disarm();
     release_regs(p, true);
+    if (p->internal) scn_metadata_wait_jobs(m); // the twin reads p->ms, which the next run destroys
     return rc;
   }
   if (macs_out) *macs_out = macs;

@@ -200,8 +200,13 @@ int scn_program_backward(scn_program *p, int n_out, const int *out_regs, const f
  * emulation from the critical path.  scn_rows_to_reference_order hands a feature matrix computed under such a Metadata
  * out in the reference numbering of an ordinary Metadata built from the same input. */
 int scn_metadata_set_internal_numbering(scn_metadata *m, int on);
-int scn_metadata_build_reference_grids(scn_metadata *m, const long spatial_size[3], const long *coords, int coords_on_device, long nrows, int ncols,
-                                       int batch_size, int mode, int n_ops, const long *ops, void *coords_ready_event);
+/* Makes the empty Metadata m the reference-numbered twin of `internal` (one batch item, input layer already built): on a worker
+ * thread, m's input layer (grid of spatial_size) and the output grids of the given strided convolutions (ops: n_ops x 13 longs,
+ * kind 2, in the order they follow from each other) take their block structure from internal's grids and compute only the
+ * reference row ids.  Their rulebooks are built on first use.  `internal` must stay alive until scn_metadata_wait_jobs(m)
+ * returns. */
+int scn_metadata_build_reference_grids(scn_metadata *m, scn_metadata *internal, const long spatial_size[3], int n_ops, const long *ops);
+/* blocks until the Metadata's worker jobs are done; its compute stream then waits for what they queued */
 int scn_metadata_wait_jobs(scn_metadata *m);
 /* batch items of the grid of this spatial size (0 when there is none) */
 int scn_get_batch_size(scn_metadata *m, const long spatial_size[3], int *batch);
@@ -323,7 +328,8 @@ long scn_kernel_launch_count(void);
  * epilogue), 10 = CUDA-core convolution launches, 11 = backward passes run by scn_program_backward, 12 = bf16 operand copies the
  * weight-gradient kernel took from its caller (forward shadow / shared d_out copy) instead of converting again, 13 = weight-gradient
  * launches driven by the output-stationary plan, 14 = float-atomic launches: launches whose float result depends on the order in
- * which atomics land (0 in deterministic mode except for scn_roi_align_rotated_3d_backward). */
+ * which atomics land (0 in deterministic mode except for scn_roi_align_rotated_3d_backward), 17 = host -> device copies of
+ * input-layer coordinates. */
 long scn_debug_counter(int which);
 /* Hands the library's idle device memory back to the driver: Metadata chunks not owned by a live Metadata, cached weight operand
  * images, per-stream scratch buffers (the library recycles these itself instead of returning them; torch.cuda.empty_cache() cannot
