@@ -63,7 +63,7 @@ int conv_backward_simt(const float *in, float *d_in, const float *d_out, const f
                        const int *d_off, const int *offHost, int K, long nInRows, long nOutRows, int Cin, int Cout, int srcIsY, cudaStream_t s, int skipDIn = 0, int mathMode = 0,
                        const void *in16 = nullptr, const void *dout16 = nullptr, const int *planNbr = nullptr, const int *planOutRow = nullptr,
                        const unsigned long long *planMask = nullptr, int planPos = 0);
-int dout_bf16_copy(const float *d_out, long n, cudaStream_t s, const void **out);
+int dout16_copy(const float *d_out, long n, cudaStream_t s, const void **out);
 bool dw_plan_ok(int Cin, int Cout, int K, int mathMode);
 void bwd_in16_arm(const void *in16);
 const void *bwd_in16_take();
@@ -78,9 +78,10 @@ long release_conv_caches();
 int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
                         int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, const int *tileW, int nWeights,
                         long nInRows, const void *in16, long long wTag, const float *addend, void *out16, long nOutRows, int CinW = 0, int wT = 0);
-int to_bf16(const float *x, void *y, long n, cudaStream_t s);
+int to_16(const float *x, void *y, long n, cudaStream_t s);
 int dense_rows_dw(const float *in, const float *d_out, float *dW, float *d_bias, long n, int Cin, int Cout, cudaStream_t s);
 static int g_math_mode = 0;
+int math_mode() { return g_math_mode; }
 static std::atomic<int> g_deterministic{0};
 bool deterministic() { return g_deterministic.load(std::memory_order_relaxed) != 0; }
 } // namespace scn
@@ -147,7 +148,7 @@ int scn_fuse_result(int *lateral_taken, int *stats_taken) {
   return 0;
 }
 int scn_set_math_mode(int mode) {
-  if (mode < 0 || mode > 3) { scn::set_error("math mode must be 0 (fp32), 1 (tf32), 2 (bf16) or 3 (tf32x3)"); return -2; }
+  if (mode < 0 || mode > 5 || mode == 4) { scn::set_error("math mode must be 0 (fp32), 1 (tf32), 2 (bf16), 3 (tf32x3) or 5 (fp16)"); return -2; }
   scn::g_math_mode = mode;
   return 0;
 }
@@ -688,11 +689,11 @@ int scn_iteration_order(scn_metadata *m, const long sz[3], int *dst) {
 static bool tc_ok(int Cin, int Cout, int K) {
   return scn::g_math_mode != 0 && scn::tc_available() && Cout % 32 == 0 && Cout >= 32 && Cout <= 256 && K <= scn::kMaxFilterVolume && Cin >= 4 && Cin <= 1024;
 }
-// out += addend (optional) and the bf16 copy of out (optional), for the paths whose kernels do not fuse them
+// out += addend (optional) and the 16-bit copy of out (optional), for the paths whose kernels do not fuse them
 static int plain_epilogue(float *out, const float *addend, void *out16, long rows, int C, cudaStream_t s) {
   if (rows <= 0) return 0;
   if (addend) return scn::add_rows(out, addend, out, rows * C, s, out16);
-  if (out16) return scn::to_bf16(out, out16, rows * C, s);
+  if (out16) return scn::to_16(out, out16, rows * C, s);
   return 0;
 }
 static int run_plan(Metadata &M, const scn::NbrPlan &plan, const float *in, float *out, const float *w, const float *bias, int Cin, int Cout,
@@ -767,11 +768,11 @@ static int dIn_tensor_core(Metadata &M, const float *d_out, float *d_in, const f
   return scn::launch_conv_plan_tc(d_out, d_in, W, nbr, outRow, tileMask, nOutPlan, tileW ? 1 : K, /*Cin=*/Cout, /*Cout=*/Cin, nullptr, scn::g_math_mode, s, tileW, K,
                                   nSrcRows, dout16, 0, nullptr, nullptr, nDstRows, 0, reverse ? 2 : 1);
 }
-// bf16 mode: one bf16 copy of d_out serves both gradient kernels of a backward call (each used to make its own)
+// bf16 / fp16 mode: one 16-bit copy of d_out serves both gradient kernels of a backward call (each used to make its own)
 static int shared_dout16(cudaStream_t s, const float *d_out, long rows, int Cin, int Cout, const void **out) {
   *out = nullptr;
-  if (scn::g_math_mode != 2 || !scn::tc_available() || rows == 0 || Cout % 32 != 0 || !tc_ok(Cout, Cin, 1)) return 0;
-  return scn::dout_bf16_copy(d_out, rows * Cout, s, out);
+  if (!scn::half_mode(scn::g_math_mode) || !scn::tc_available() || rows == 0 || Cout % 32 != 0 || !tc_ok(Cout, Cin, 1)) return 0;
+  return scn::dout16_copy(d_out, rows * Cout, s, out);
 }
 int scn_submanifold_convolution_backward(scn_metadata *m, const long sz[3], const long f[3], const float *in, float *d_in, const float *d_out,
                                          const float *w, float *dw, float *d_bias, int Cin, int Cout) {

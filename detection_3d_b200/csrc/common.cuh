@@ -60,7 +60,8 @@ enum DebugCounter {
   kCntTf32x3Launch = 15,   // conv_plan_tc launches with TF32X3 operands (math mode 3)
   kCntChunkedLaunch = 16,  // conv_plan_tc launches over one offset chunk of a plan with more than 64 filter offsets
   kCntCoordUpload = 17,    // host -> device copies of input-layer coordinates
-  kCntCounters = 18
+  kCntF16Launch = 18,      // tensor-core launches with fp16 operands (math mode 5): conv_plan_tc and the weight-gradient kernels
+  kCntCounters = 19
 };
 extern std::atomic<long> g_counters[kCntCounters];
 
@@ -76,6 +77,41 @@ int det_scratch(cudaStream_t s, size_t bytes, void **out);
 // map(j) = j, or (j / seg) * segStride + j % seg when seg > 0.  T = float or double (accumulated in double).
 template <class T>
 int ordered_sum(const T *part, int nPart, long width, T *out, cudaStream_t s, long seg = 0, long segStride = 0);
+
+// ---------------------------------------------------------------- 16-bit operand modes (scn_set_math_mode)
+// Math modes 2 (bf16) and 5 (fp16) give the tensor cores 16-bit operands on the same layers: rows of a multiple of 64 channels
+// and the packed 16- / 32-channel rows; the other layers keep TF32 operands.  Every 16-bit copy of a feature matrix -- the
+// "bf16" arguments of the C ABI, the shadows of a recorded program, the operand copies the launchers make -- is written and read
+// in the format of the current mode: fp16 in mode 5, bf16 in every other mode (as before mode 5 existed).
+constexpr int kModeBF16 = 2, kModeF16 = 5;
+static inline bool half_mode(int mathMode) { return mathMode == kModeBF16 || mathMode == kModeF16; }
+int math_mode(); // the current mode (capi.cu)
+static inline bool f16_copies() { return math_mode() == kModeF16; }
+#if defined(__CUDACC__)
+} // namespace scn
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+namespace scn {
+// fp32 -> 16 bits, round to nearest even; fp16 overflows to +-inf (no saturation) and keeps subnormals, as torch's .half() does
+template <bool F16>
+__device__ __forceinline__ unsigned short to16(float x) {
+  if (F16) return __half_as_ushort(__float2half_rn(x));
+  return __bfloat16_as_ushort(__float2bfloat16_rn(x));
+}
+template <bool F16>
+__device__ __forceinline__ unsigned int pack16x2(float a, float b) {
+  if (F16) { __half2 h = __floats2half2_rn(a, b); return *reinterpret_cast<unsigned int *>(&h); }
+  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<unsigned int *>(&h);
+}
+template <bool F16>
+__device__ __forceinline__ uint2 pack16x4(float4 v) {
+  uint2 pk;
+  pk.x = pack16x2<F16>(v.x, v.y);
+  pk.y = pack16x2<F16>(v.z, v.w);
+  return pk;
+}
+#endif
 
 // ---------------------------------------------------------------- programmatic dependent launch (sm_90+)
 // The layer kernels of a forward sit back to back on one stream, ~100 of them, half of them a few microseconds long.  Launched with

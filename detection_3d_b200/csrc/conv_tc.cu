@@ -45,8 +45,10 @@ constexpr int kEpiBytes = 4 * 32 * kEpiCols * 4; // 4 epilogue warps x (32 rows 
 constexpr int kBuildRoom = SCN_EPI_COLS == 16 ? 12 * 1024 : 0; // shared memory per SM left to the build kernels that run beside this one
 // Operand type of conv_plan_tc (template parameter OP).  TF32X3 ("3xTF32", math mode 3): every fp32 operand x = hi + lo with
 // both parts exact TF32 values, and out += A_hi W_lo + A_lo W_hi + A_hi W_hi in the same fp32 accumulator (the dropped
-// A_lo W_lo and the rounding of lo leave ~2^-21 relative error per product).
-enum TcOperand { kOpTF32 = 0, kOpBF16 = 1, kOpTF32X3 = 2 };
+// A_lo W_lo and the rounding of lo leave ~2^-21 relative error per product).  F16 (math mode 5): fp16 operands wherever bf16 mode
+// has bf16 ones -- the same kind::f16 instruction and the same 2-byte rows, only the A / B format field of the instruction
+// descriptor differs (F16 = 0, BF16 = 1).
+enum TcOperand { kOpTF32 = 0, kOpBF16 = 1, kOpTF32X3 = 2, kOpF16 = 3 };
 constexpr int kSplitWarps = 4; // TF32X3: warps that split the gathered A atoms of a stage into hi / lo parts
 
 struct TcParams {
@@ -55,7 +57,7 @@ struct TcParams {
   const unsigned char *wimg;
   const float *bias;
   const float *addend; // optional [output rows][Cout]: out = conv + addend (the residual / lateral add fused into the epilogue)
-  void *out16;         // optional bf16 copy of the result (gather operand of the next convolution in bf16 mode)
+  void *out16;         // optional 16-bit copy of the result (gather operand of the next convolution in bf16 / fp16 mode): bf16, fp16 with OP F16
   const int *nbr;
   const int *outRow;
   const unsigned long long *tileMask;
@@ -73,6 +75,7 @@ struct TcParams {
   unsigned *sched; // dynamic work distribution: [0] next work item, [1] CTAs that have drawn their last item (self-resetting); null = static stride
   double *statsPart; // deterministic mode, with stats: [work item][epilogue warp][2][Cout] per-item sums instead of atomics into `stats`
   float *part;       // deterministic mode, kSplit > 1: [kSplit][nOut][Cout] per-split partial outputs instead of atomics into `out`
+  int f16;           // OP TF32 only: out16 is fp16 (a narrow layer that keeps TF32 operands in fp16 mode), else bf16
 };
 
 // ------------------------------------------------------------------ PTX helpers
@@ -284,7 +287,7 @@ __device__ __forceinline__ void sched_publish(const Sched &S, int n, int wi) {
 // what keeps their gathers in flight; a producer that split its rows would have to drain them first.
 template <int OP, int PW, int G, int CTAS, bool DET>
 __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_COLS == 16 ? 384 : 320)), CTAS) conv_plan_tc(const TcParams P) {
-  constexpr bool BF16 = OP == kOpBF16, X3 = OP == kOpTF32X3;
+  constexpr bool BF16 = OP == kOpBF16 || OP == kOpF16, X3 = OP == kOpTF32X3; // (BF16: 16-bit operands, kind::f16)
   static_assert(!X3 || (PW == 8 && G == 1 && CTAS == 1), "TF32X3: one-CTA configuration only");
   constexpr int TM = G == 4 ? 2 : kMaxT; // tiles per item the producers keep neighbour ids for (G ids per row and tile)
   constexpr int kProdWarps = PW;
@@ -420,11 +423,9 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
               if (rows[i] >= 0) {
                 if (P.out) *reinterpret_cast<float4 *>(P.out + (size_t)rows[i] * P.Cout + c0 + cc) = o[i]; // null: only the bf16 copy is consumed
                 if (P.out16) {
-                  __nv_bfloat162 lo = __floats2bfloat162_rn(o[i].x, o[i].y), hi = __floats2bfloat162_rn(o[i].z, o[i].w);
-                  uint2 pk;
-                  pk.x = *reinterpret_cast<unsigned int *>(&lo);
-                  pk.y = *reinterpret_cast<unsigned int *>(&hi);
-                  *reinterpret_cast<uint2 *>(static_cast<unsigned char *>(P.out16) + ((size_t)rows[i] * P.Cout + c0 + cc) * 2) = pk;
+                  uint2 *dst16 = reinterpret_cast<uint2 *>(static_cast<unsigned char *>(P.out16) + ((size_t)rows[i] * P.Cout + c0 + cc) * 2);
+                  if (OP == kOpF16 || (OP == kOpTF32 && P.f16)) *dst16 = pack16x4<true>(o[i]);
+                  else *dst16 = pack16x4<false>(o[i]);
                 }
               }
           } else if (DET && P.part) { // offsets split over CTAs, deterministic mode: this split's partial rows into its own slot
@@ -566,8 +567,8 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
     // descriptors in uniform registers and emits straight-line UTCHMMA instead of a per-instruction
     // election loop (measured: ~120 cycles per MMA issued from a divergent `if (lane == 0)` region).
     {
-      // instruction descriptor: D=F32, A/B = TF32 (2) or BF16 (1), K-major both, N=Cout, M=128
-      const uint32_t fmt = BF16 ? 1u : 2u;
+      // instruction descriptor: D=F32, A/B = TF32 (2), BF16 (1) or F16 (0), K-major both, N=Cout, M=128
+      const uint32_t fmt = OP == kOpF16 ? 0u : BF16 ? 1u : 2u;
       const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(P.Cout >> 3) << 17) | ((uint32_t)(kTileM >> 4) << 24);
       uint32_t n = 0, slot = 0, round = 0;
       const uint32_t sStage0 = smem_u32(sStage), full0 = smem_u32(full), empty0 = smem_u32(empty);
@@ -733,11 +734,13 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
 
 // W [K][Cin][Cout] fp32 -> per (k, 128-byte K atom) the exact shared-memory image of the B operand:
 // Cout rows x 128 bytes (32 tf32 / 64 bf16 input channels of one output channel), 16-byte chunks
-// XOR-swizzled by (row & 7); values rounded to nearest (TF32: cvt.rna, BF16: rn).
+// XOR-swizzled by (row & 7); values rounded to nearest (TF32: cvt.rna, BF16 / F16: rn, fp16 overflowing to +-inf).
 // Cin = padded channel count of the image (multiple of the atom width), CinW = channels W really has.
 // wT: 0 = W is [K][CinW][Cout]; 1 / 2 = the operand is the TRANSPOSE of a forward weight tensor stored as [K][Cout][CinW] (the input-gradient
 // convolutions: Wt[k'][co][ci] = W[k][ci][co]), 2 = with the filter offsets reversed as well (k' = K - 1 - k) -- read in place, no transposed copy.
-__global__ void k_prep_wimg(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int Cin, int CinW, int Cout, int bf16, int wT) {
+// el = element format: 0 = tf32, kWimgBF16, kWimgF16.
+__global__ void k_prep_wimg(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int Cin, int CinW, int Cout, int el, int wT) {
+  const bool bf16 = el != 0; // (2-byte elements)
   const long n = (long)K * Cin * Cout;
   const int per = bf16 ? 64 : 32, nAtoms = Cin / per;
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
@@ -749,8 +752,10 @@ __global__ void k_prep_wimg(const float *__restrict__ W, unsigned char *__restri
     unsigned char *dst = img + ((long)k * nAtoms + c) * Cout * 128 + (long)co * 128 + ((chunk ^ (co & 7)) << 4) + within;
     const int ks = wT == 2 ? K - 1 - k : k;
     const float w = ci < CinW ? (wT ? W[((long)ks * Cout + co) * CinW + ci] : W[((long)k * CinW + ci) * Cout + co]) : 0.f;
-    if (bf16) {
-      *reinterpret_cast<unsigned short *>(dst) = __bfloat16_as_ushort(__float2bfloat16_rn(w));
+    if (el == 3) { // (kWimgF16)
+      *reinterpret_cast<unsigned short *>(dst) = to16<true>(w);
+    } else if (bf16) {
+      *reinterpret_cast<unsigned short *>(dst) = to16<false>(w);
     } else {
       uint32_t r;
       asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(w));
@@ -780,10 +785,10 @@ __global__ void k_prep_wimg_split(const float *__restrict__ W, unsigned char *__
   }
 }
 
-// Packed layers (bf16 rows of 128 / G bytes, G = 2 or 4): the K atom of offset group kg holds, for output channel co,
+// Packed layers (16-bit rows of 128 / G bytes, G = 2 or 4; fp16 elements with f16, else bf16): the K atom of offset group kg holds, for output channel co,
 // [offset kg G | offset kg G + 1 | ...] x Cin input channels -- the same order in which the producers lay the G
 // gathered neighbour rows side by side.  Offsets beyond K and channels beyond CinW are zero.
-__global__ void k_prep_wimg_packed(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int G, int Cin, int CinW, int Cout, int wT) {
+__global__ void k_prep_wimg_packed(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int G, int Cin, int CinW, int Cout, int wT, int f16) {
   const int KG = (K + G - 1) / G;
   const long n = (long)KG * G * Cin * Cout;
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
@@ -795,7 +800,7 @@ __global__ void k_prep_wimg_packed(const float *__restrict__ W, unsigned char *_
     unsigned char *dst = img + (long)kg * Cout * 128 + (long)co * 128 + ((chunk ^ (co & 7)) << 4) + within;
     const int ks = wT == 2 ? K - 1 - k : k;
     const float w = (k < K && ci < CinW) ? (wT ? W[((long)ks * Cout + co) * CinW + ci] : W[((long)k * CinW + ci) * Cout + co]) : 0.f;
-    *reinterpret_cast<unsigned short *>(dst) = __bfloat16_as_ushort(__float2bfloat16_rn(w));
+    *reinterpret_cast<unsigned short *>(dst) = f16 ? to16<true>(w) : to16<false>(w);
   }
 }
 
@@ -803,9 +808,9 @@ __global__ void k_prep_wimg_packed(const float *__restrict__ W, unsigned char *_
 // type) -> image.  The tag is how the caller says "same contents as last time" (the Python layer
 // passes a per-Parameter token combined with the tensor's in-place version counter); tag 0 = no caching.
 struct WimgKey {
-  const void *w; long long tag; int K, Cin, CinW, Cout, bf16, dev;
+  const void *w; long long tag; int K, Cin, CinW, Cout, fmt, dev; // fmt: element format and packing of the image (launch_prep_wimg)
   bool operator<(const WimgKey &o) const {
-    return std::tie(w, tag, K, Cin, CinW, Cout, bf16, dev) < std::tie(o.w, o.tag, o.K, o.Cin, o.CinW, o.Cout, o.bf16, o.dev);
+    return std::tie(w, tag, K, Cin, CinW, Cout, fmt, dev) < std::tie(o.w, o.tag, o.K, o.Cin, o.CinW, o.Cout, o.fmt, o.dev);
   }
 };
 struct WimgVal { unsigned char *img; size_t bytes; cudaEvent_t ready; cudaStream_t stream; unsigned long long lastUse; };
@@ -815,25 +820,26 @@ static size_t g_wimg_bytes = 0;
 static unsigned long long g_wimg_clock = 0;
 constexpr size_t kWimgBudget = 768u << 20;
 // Returns the image; *owned = true when the caller must cudaFreeAsync it (uncached).
-// fmt: 0 = tf32, 1 = bf16, 1 + 16 G = packed bf16 (G offsets per atom), kWimgSplit = tf32 hi / lo pairs (TF32X3).  The format is
-// part of the cache key: the images of one weight tensor in different modes are separate entries.
-constexpr int kWimgSplit = 2;
+// fmt: element format (0 = tf32, kWimgBF16, kWimgSplit = tf32 hi / lo pairs (TF32X3), kWimgF16) + 16 G for packed 16-bit images (G
+// offsets per atom).  The format is part of the cache key: the images of one weight tensor in different modes -- bf16 and fp16
+// included -- are separate entries, so a mode switch never hands a kernel an image in the other format.
+constexpr int kWimgBF16 = 1, kWimgSplit = 2, kWimgF16 = 3;
 static void launch_prep_wimg(const float *W, unsigned char *img, int K, int Cin, int CinW, int Cout, int fmt, cudaStream_t s, int wT) {
   const int G = fmt >> 4;
-  if (G > 1) k_prep_wimg_packed<<<stream_grid((long)((K + G - 1) / G) * G * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, G, Cin, CinW, Cout, wT);
+  if (G > 1) k_prep_wimg_packed<<<stream_grid((long)((K + G - 1) / G) * G * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, G, Cin, CinW, Cout, wT, (fmt & 15) == kWimgF16);
   else if (fmt == kWimgSplit) k_prep_wimg_split<<<stream_grid((long)K * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, Cin, CinW, Cout, wT);
-  else k_prep_wimg<<<stream_grid((long)K * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, Cin, CinW, Cout, fmt & 1, wT);
+  else k_prep_wimg<<<stream_grid((long)K * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, Cin, CinW, Cout, fmt & 15, wT);
 }
-static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int Cout, int bf16, cudaStream_t s, unsigned char **img, bool *owned, int wT = 0) {
+static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int Cout, int fmt, cudaStream_t s, unsigned char **img, bool *owned, int wT = 0) {
   if (wT) tag = 0; // (transposed operands belong to the backward pass of a training step: the weights change every step, nothing to cache)
-  const int packG = bf16 >> 4;
-  const size_t bytes = packG > 1 ? (size_t)((K + packG - 1) / packG) * Cout * 128 : (size_t)K * Cin * Cout * (bf16 == kWimgSplit ? 8 : bf16 ? 2 : 4);
+  const int packG = fmt >> 4;
+  const size_t bytes = packG > 1 ? (size_t)((K + packG - 1) / packG) * Cout * 128 : (size_t)K * Cin * Cout * (fmt == kWimgSplit ? 8 : fmt ? 2 : 4);
   *owned = false;
   if (tag != 0) {
     int dev = 0;
     SCN_CUDA(cudaGetDevice(&dev));
     std::lock_guard<std::mutex> lk(g_wimg_mu);
-    WimgKey key{W, tag, K, Cin, CinW, Cout, bf16, dev};
+    WimgKey key{W, tag, K, Cin, CinW, Cout, fmt, dev};
     auto it = g_wimg.find(key);
     if (it != g_wimg.end()) {
       it->second.lastUse = ++g_wimg_clock;
@@ -854,7 +860,7 @@ static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int
     WimgVal v;
     SCN_CUDA(cudaMalloc((void **)&v.img, bytes));
     SCN_CUDA(cudaEventCreateWithFlags(&v.ready, cudaEventDisableTiming));
-    launch_prep_wimg(W, v.img, K, Cin, CinW, Cout, bf16, s, 0);
+    launch_prep_wimg(W, v.img, K, Cin, CinW, Cout, fmt, s, 0);
     SCN_CUDA(cudaEventRecord(v.ready, s));
     v.bytes = bytes; v.stream = s; v.lastUse = ++g_wimg_clock;
     g_wimg[key] = v;
@@ -863,7 +869,7 @@ static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int
     return 0;
   }
   SCN_CUDA(cudaMallocAsync((void **)img, bytes, s));
-  launch_prep_wimg(W, *img, K, Cin, CinW, Cout, bf16, s, wT);
+  launch_prep_wimg(W, *img, K, Cin, CinW, Cout, fmt, s, wT);
   *owned = true;
   return 0;
 }
@@ -884,34 +890,43 @@ __global__ void k_pad_rows(const float *__restrict__ in, float *__restrict__ out
     out[i] = c < C ? __ldg(in + (i / Cp) * C + c) : 0.f;
   }
 }
-// rows of C <= Cp channels -> bf16 rows zero-padded to Cp channels (the 9-channel network input -> 16 channels = 32-byte rows)
-__global__ void k_pad_rows_bf16(const float *__restrict__ in, __nv_bfloat16 *__restrict__ out, long n, int C, int Cp) {
+// rows of C <= Cp channels -> 16-bit rows (bf16, or fp16 with F16) zero-padded to Cp channels (the 9-channel network input -> 16
+// channels = 32-byte rows)
+template <bool F16>
+__global__ void k_pad_rows16(const float *__restrict__ in, unsigned short *__restrict__ out, long n, int C, int Cp) {
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n * Cp; i += (long)gridDim.x * blockDim.x) {
     int c = (int)(i % Cp);
-    out[i] = __float2bfloat16_rn(c < C ? __ldg(in + (i / Cp) * C + c) : 0.f);
+    out[i] = to16<F16>(c < C ? __ldg(in + (i / Cp) * C + c) : 0.f);
   }
 }
-// fp32 -> bf16 (rn) copy of a feature matrix, for inputs that arrive without a bf16 shadow
-__global__ void __launch_bounds__(256) k_to_bf16(const float *__restrict__ x, uint2 *__restrict__ y, long n4) {
+static void launch_pad_rows16(const float *in, void *out, long n, int C, int Cp, bool f16, cudaStream_t s) {
+  if (f16) k_pad_rows16<true><<<stream_grid(n * Cp, 256), 256, 0, LS(s)>>>(in, static_cast<unsigned short *>(out), n, C, Cp);
+  else k_pad_rows16<false><<<stream_grid(n * Cp, 256), 256, 0, LS(s)>>>(in, static_cast<unsigned short *>(out), n, C, Cp);
+}
+// fp32 -> 16-bit (rn) copy of a feature matrix (bf16, or fp16 with F16), for inputs that arrive without a 16-bit shadow
+template <bool F16>
+__global__ void __launch_bounds__(256) k_to_16(const float *__restrict__ x, uint2 *__restrict__ y, long n4) {
   pdl_launch_dependents();
   pdl_wait();
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
     const float4 v = __ldg(reinterpret_cast<const float4 *>(x) + i);
-    __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
-    uint2 pk;
-    pk.x = *reinterpret_cast<unsigned int *>(&lo);
-    pk.y = *reinterpret_cast<unsigned int *>(&hi);
-    y[i] = pk;
+    y[i] = pack16x4<F16>(v);
   }
 }
-int to_bf16(const float *x, void *y, long n, cudaStream_t s) {
-  SCN_CHECK(n % 4 == 0, "bf16 copy needs an element count that is a multiple of 4");
-  if (n) SCN_CUDA(launch_pdl(k_to_bf16, dim3(stream_grid(n / 4, 256)), dim3(256), 0, LS(s), x, static_cast<uint2 *>(y), n / 4));
+static cudaError_t launch_to_16(const float *x, void *y, long n4, bool f16, cudaStream_t s) {
+  if (f16) return launch_pdl(k_to_16<true>, dim3(stream_grid(n4, 256)), dim3(256), 0, LS(s), x, static_cast<uint2 *>(y), n4);
+  return launch_pdl(k_to_16<false>, dim3(stream_grid(n4, 256)), dim3(256), 0, LS(s), x, static_cast<uint2 *>(y), n4);
+}
+// the 16-bit copy of x in the current mode's format (common.cuh)
+int to_16(const float *x, void *y, long n, cudaStream_t s) {
+  SCN_CHECK(n % 4 == 0, "16-bit copy needs an element count that is a multiple of 4");
+  if (n) SCN_CUDA(launch_to_16(x, y, n / 4, f16_copies(), s));
   SCN_CUDA(cudaGetLastError());
   return 0;
 }
 // deterministic mode, split filter offsets: out = partial of split 0 + split 1 + ... in that order (bias and addend are in split 0's),
-// with the bf16 copy of the finished rows (what the memset + atomic epilogue + k_to_bf16 do otherwise)
+// with the 16-bit copy of the finished rows (what the memset + atomic epilogue + k_to_16 do otherwise)
+template <bool F16>
 __global__ void __launch_bounds__(256) k_split_sum(const float4 *__restrict__ part, int kSplit, long n4, float4 *__restrict__ out, uint2 *__restrict__ out16) {
   pdl_launch_dependents();
   pdl_wait();
@@ -922,21 +937,15 @@ __global__ void __launch_bounds__(256) k_split_sum(const float4 *__restrict__ pa
       a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
     }
     out[i] = a;
-    if (out16) {
-      __nv_bfloat162 lo = __floats2bfloat162_rn(a.x, a.y), hi = __floats2bfloat162_rn(a.z, a.w);
-      uint2 pk;
-      pk.x = *reinterpret_cast<unsigned int *>(&lo);
-      pk.y = *reinterpret_cast<unsigned int *>(&hi);
-      out16[i] = pk;
-    }
+    if (out16) out16[i] = pack16x4<F16>(a);
   }
 }
 static int stream_scratch(cudaStream_t s, int slot, size_t bytes, void **out);
-// bf16 copy of a backward call's d_out, made once and read by both the input-gradient and the weight-gradient kernel
-int dout_bf16_copy(const float *d_out, long n, cudaStream_t s, const void **out) {
+// 16-bit copy of a backward call's d_out, made once and read by both the input-gradient and the weight-gradient kernel
+int dout16_copy(const float *d_out, long n, cudaStream_t s, const void **out) {
   void *p = nullptr;
   SCN_TRY(stream_scratch(s, 3, (size_t)n * 2 + 16, &p));
-  SCN_TRY(to_bf16(d_out, p, n, s));
+  SCN_TRY(to_16(d_out, p, n, s));
   *out = p;
   return 0;
 }
@@ -1017,10 +1026,26 @@ static int set_plan_attributes() {
   SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
   SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
   SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpTF32X3, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 4, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 4, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 8, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 8, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
   return 0;
 }
+// H = the 16-bit operand type (kOpBF16 or kOpF16) of a launch with P.bf16 set
+template <bool DET, int H>
+static cudaError_t launch_plan_variant16(const TcParams &P, int packG, bool pw8, int ctas, int grid, int th2, size_t smem, cudaStream_t s) {
+  if (packG == 2) return pw8 ? launch_pdl(conv_plan_tc<H, 8, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<H, 4, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+  if (packG == 4) return pw8 ? launch_pdl(conv_plan_tc<H, 8, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<H, 4, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+  if (ctas == 2) return pw8 ? launch_pdl(conv_plan_tc<H, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<H, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
+  return launch_pdl(conv_plan_tc<H, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
+}
 template <bool DET>
-static cudaError_t launch_plan_variant(const TcParams &P, int packG, bool pw8, int ctas, int grid, int th2, size_t smem, cudaStream_t s, bool x3) {
+static cudaError_t launch_plan_variant(const TcParams &P, int packG, bool pw8, int ctas, int grid, int th2, size_t smem, cudaStream_t s, bool x3, bool f16) {
+  if (f16 && P.bf16) return launch_plan_variant16<DET, kOpF16>(P, packG, pw8, ctas, grid, th2, smem, s);
   if (x3) return launch_pdl(conv_plan_tc<kOpTF32X3, 8, 1, 1, DET>, dim3(grid), dim3(32 * (14 + kSplitWarps)), smem, LS(s), P);
   if (packG == 2) return pw8 ? launch_pdl(conv_plan_tc<kOpBF16, 8, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpBF16, 4, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
   if (packG == 4) return pw8 ? launch_pdl(conv_plan_tc<kOpBF16, 8, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpBF16, 4, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
@@ -1034,8 +1059,9 @@ static cudaError_t launch_plan_variant(const TcParams &P, int packG, bool pw8, i
 static int launch_conv_plan_tc_chunked(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
                                        int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, long nInRows, const void *in16,
                                        long long wTag, const float *addend, void *out16, long nOutRows, int CinW, int wT);
-// in16: optional bf16 copy of `in` (same layout); used in math mode 2 when Cin is a multiple of 64.
-// mathMode 1 = TF32 operands, 2 = BF16 where the channel counts allow (TF32 elsewhere), 3 = TF32X3 (the fp32 rows as hi / lo TF32 pairs)
+// in16: optional 16-bit copy of `in` (same layout, the mode's format); used in math modes 2 / 5 when Cin is a multiple of 64.
+// mathMode 1 = TF32 operands, 2 = BF16 where the channel counts allow (TF32 elsewhere), 3 = TF32X3 (the fp32 rows as hi / lo TF32 pairs),
+// 5 = F16 where mode 2 has BF16 (TF32 elsewhere).  out16 (optional) receives the result in the mode's 16-bit format.
 int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
                         int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, const int *tileW, int nWeights,
                         long nInRows, const void *in16, long long wTag, const float *addend, void *out16, long nOutRows, int CinW = 0, int wT = 0) {
@@ -1045,17 +1071,18 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
     SCN_CHECK(nbr && tileMask && nWeights == K && K <= kMaxFilterVolume, "tcgen05 path: wide plan");
     return launch_conv_plan_tc_chunked(in, out, W, nbr, outRow, tileMask, nOut, K, Cin, Cout, bias, mathMode, s, nInRows, in16, wTag, addend, out16, nOutRows, CinW, wT);
   }
-  const bool canPack = mathMode == 2 && !tileW && Cout <= 128; // packed narrow rows: two-CTA configuration only
+  const bool f16 = mathMode == kModeF16; // 16-bit operands and copies are fp16 (else bf16)
+  const bool canPack = half_mode(mathMode) && !tileW && Cout <= 128; // packed narrow rows: two-CTA configuration only
   if (canPack && CinW == Cin && Cin != 16 && Cin % 32 != 0) {
-    // bf16 mode, odd channel counts (e.g. the 9-channel network input): bf16 rows zero-padded to 16 channels (packed, G = 4),
+    // bf16 / fp16 mode, odd channel counts (e.g. the 9-channel network input): 16-bit rows zero-padded to 16 channels (packed, G = 4),
     // 32 channels (G = 2) or a multiple of 64 (whole atoms), written by one pass; the weight image pads itself
     const int Cp = Cin < 16 ? 16 : (Cin < 32 ? 32 : (Cin + 63) / 64 * 64);
-    __nv_bfloat16 *xp = nullptr;
+    void *xp = nullptr;
     if (tl_prepad && tl_prepad_c == Cp) {
-      xp = const_cast<__nv_bfloat16 *>(static_cast<const __nv_bfloat16 *>(tl_prepad)); // the producer already wrote the padded copy
+      xp = const_cast<void *>(tl_prepad); // the producer already wrote the padded copy
     } else {
-      SCN_TRY(stream_scratch(s, kScratchBf16, (size_t)nInRows * Cp * 2 + 16, (void **)&xp));
-      k_pad_rows_bf16<<<stream_grid(nInRows * Cp, 256), 256, 0, LS(s)>>>(in, xp, nInRows, Cin, Cp);
+      SCN_TRY(stream_scratch(s, kScratchBf16, (size_t)nInRows * Cp * 2 + 16, &xp));
+      launch_pad_rows16(in, xp, nInRows, Cin, Cp, f16, s);
     }
     tl_prepad = nullptr;
     return launch_conv_plan_tc(in, out, W, nbr, outRow, tileMask, nOut, K, Cp, Cout, bias, mathMode, s, tileW, nWeights, nInRows, xp, wTag, addend, out16, nOutRows, Cin, wT);
@@ -1079,16 +1106,17 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   TcParams P;
   P.in = reinterpret_cast<const unsigned char *>(in); P.out = out; P.bias = bias; P.addend = addend; P.out16 = out16; P.nbr = nbr; P.outRow = outRow; P.tileMask = tileMask; P.tileW = tileW;
   P.nOut = nOut; P.K = K; P.Cout = Cout;
-  // bf16 mode: rows of >= 64 channels are whole 128-byte atoms; 32- and 16-channel rows (64 / 32 bytes) are PACKED, G = 2 / 4
+  // bf16 / fp16 mode: rows of >= 64 channels are whole 128-byte atoms; 32- and 16-channel rows (64 / 32 bytes) are PACKED, G = 2 / 4
   // filter offsets side by side in one atom: half / a quarter of the stages, gather bytes and MMAs of the 128-byte-row layout
   const int packG = (canPack && (Cin == 32 || Cin == 16)) ? 64 / Cin : 1;
-  P.bf16 = (mathMode == 2 && (Cin % 64 == 0 || packG > 1)) ? 1 : 0; // other narrow layers keep TF32 operands
+  P.bf16 = (half_mode(mathMode) && (Cin % 64 == 0 || packG > 1)) ? 1 : 0; // 16-bit operands (fp16 in mode 5); other narrow layers keep TF32 operands
+  P.f16 = f16 && !P.bf16; // (a TF32-operand launch in fp16 mode writes its 16-bit copy as fp16)
   const bool x3 = mathMode == 3 && !P.bf16; // TF32X3: the fp32 rows split into two TF32 operands (one-CTA configuration, stages twice as large)
   void *tmp16 = nullptr;
   if (P.bf16) {
     if (!in16) {
       SCN_TRY(stream_scratch(s, kScratchBf16, (size_t)nInRows * Cin * 2 + 16, &tmp16));
-      if (nInRows) SCN_CUDA(launch_pdl(k_to_bf16, dim3(stream_grid(nInRows * Cin / 4, 256)), dim3(256), 0, LS(s), in, static_cast<uint2 *>(tmp16), nInRows * Cin / 4));
+      if (nInRows) SCN_CUDA(launch_to_16(in, tmp16, nInRows * Cin / 4, f16, s));
       in16 = tmp16;
     }
     P.in = static_cast<const unsigned char *>(in16);
@@ -1155,12 +1183,14 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   SCN_CHECK(out || (P.kSplit == 1 && out16), "tcgen05 path: fp32 output dropped on a launch that needs it");
   ++g_counters[kCntTcLaunch];
   if (x3) ++g_counters[kCntTf32x3Launch];
+  if (f16 && P.bf16) ++g_counters[kCntF16Launch];
   if (P.kSplit > 1) ++g_counters[kCntSplitLaunch];
   if (P.kSplit > 1 && det) SCN_TRY(det_scratch(s, (size_t)P.kSplit * nOut * Cout * 4, (void **)&P.part)); // (k_split_sum writes every output row)
   else if (P.kSplit > 1) { ++g_counters[kCntFloatAtomic]; SCN_CUDA(cudaMemsetAsync(out, 0, (size_t)nOut * Cout * 4, s)); }
   unsigned char *wimg = nullptr;
   bool wimgOwned = false;
-  SCN_TRY(get_wimg(W, wTag, nWeights, Cin, CinW, Cout, packG > 1 ? 1 + 16 * packG : x3 ? kWimgSplit : P.bf16, s, &wimg, &wimgOwned, wT));
+  const int el16 = f16 ? kWimgF16 : kWimgBF16; // element format of a 16-bit image
+  SCN_TRY(get_wimg(W, wTag, nWeights, Cin, CinW, Cout, packG > 1 ? el16 + 16 * packG : x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg, &wimgOwned, wT));
   P.wimg = wimg;
   P.in2 = nullptr; P.wimg2 = nullptr; P.rowBytes2 = 0; P.nAtoms2 = 0;
   unsigned char *wimg2 = nullptr;
@@ -1169,7 +1199,7 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
     const int esz = P.bf16 ? 2 : 4, per = 128 / esz, C2 = tl_lat.Cin; // per = channels of one K atom
     if ((C2 * esz) % 16 == 0) {
       const int C2p = (C2 + per - 1) / per * per;
-      SCN_TRY(get_wimg(tl_lat.w, tl_lat.tag, 1, C2p, C2, Cout, x3 ? kWimgSplit : P.bf16, s, &wimg2, &wimg2Owned));
+      SCN_TRY(get_wimg(tl_lat.w, tl_lat.tag, 1, C2p, C2, Cout, x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg2, &wimg2Owned));
       P.in2 = static_cast<const unsigned char *>(P.bf16 ? tl_lat.in16 : static_cast<const void *>(tl_lat.in));
       P.rowBytes2 = C2 * esz;
       P.nAtoms2 = C2p / per;
@@ -1202,8 +1232,8 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   if (envPw8 < 0) envPw8 = getenv("SCN_TC_PW8") ? atoi(getenv("SCN_TC_PW8")) : 0;
   const bool pw8 = ctas == 2 && ((packG > 1 && (envPw8 & 1)) || (packG == 1 && (envPw8 & 2)));
   const int th2 = 32 * (pw8 ? 14 : 10);
-  if (det) SCN_CUDA(launch_plan_variant<true>(P, packG, pw8, ctas, grid, th2, smem, s, x3));
-  else SCN_CUDA(launch_plan_variant<false>(P, packG, pw8, ctas, grid, th2, smem, s, x3));
+  if (det) SCN_CUDA(launch_plan_variant<true>(P, packG, pw8, ctas, grid, th2, smem, s, x3, f16));
+  else SCN_CUDA(launch_plan_variant<false>(P, packG, pw8, ctas, grid, th2, smem, s, x3, f16));
   SCN_CUDA(cudaGetLastError());
   if (envProf) { // developer aid: mean stall cycles per role over the CTAs of this launch
     static long long h[2 * kSMs * 32];
@@ -1216,11 +1246,11 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
     cudaFreeAsync(P.prof, s);
   }
   if (P.statsPart) SCN_TRY(ordered_sum(P.statsPart, P.nSuper * 4, 2l * Cout, P.stats, s, Cout, kFusedStatsC)); // into replica 0
-  if (P.part) // the split partials in split order, and the bf16 copy from the same registers
-    SCN_CUDA(launch_pdl(k_split_sum, dim3(stream_grid((long)nOut * Cout / 4, 256)), dim3(256), 0, LS(s), reinterpret_cast<const float4 *>(P.part), P.kSplit,
-                        (long)nOut * Cout / 4, reinterpret_cast<float4 *>(out), static_cast<uint2 *>(out16)));
-  else if (out16 && P.kSplit > 1 && nOutRows > 0) // partial sums were accumulated atomically: the bf16 copy needs the finished rows
-    SCN_CUDA(launch_pdl(k_to_bf16, dim3(stream_grid(nOutRows * Cout / 4, 256)), dim3(256), 0, LS(s), out, static_cast<uint2 *>(out16), nOutRows * Cout / 4));
+  if (P.part) // the split partials in split order, and the 16-bit copy from the same registers
+    SCN_CUDA(launch_pdl(f16 ? k_split_sum<true> : k_split_sum<false>, dim3(stream_grid((long)nOut * Cout / 4, 256)), dim3(256), 0, LS(s),
+                        reinterpret_cast<const float4 *>(P.part), P.kSplit, (long)nOut * Cout / 4, reinterpret_cast<float4 *>(out), static_cast<uint2 *>(out16)));
+  else if (out16 && P.kSplit > 1 && nOutRows > 0) // partial sums were accumulated atomically: the 16-bit copy needs the finished rows
+    SCN_CUDA(launch_to_16(out, out16, nOutRows * Cout / 4, f16, s));
   if (wimgOwned) cudaFreeAsync(wimg, s);
   if (wimg2Owned) cudaFreeAsync(wimg2, s);
 
@@ -1372,7 +1402,8 @@ struct DwParams {
 __device__ __forceinline__ uint64_t smem_desc_mn_sw128(uint32_t addr, uint32_t lboBytes) {
   return (uint64_t)((addr >> 4) & 0x3fffu) | ((uint64_t)((lboBytes >> 4) & 0x3fffu) << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
-template <bool BF16>
+// BF16: 16-bit operands (kind::f16), fp16 ones with F16 (math mode 5), else TF32
+template <bool BF16, bool F16 = false>
 __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwParams P) {
   extern __shared__ __align__(1024) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -1478,8 +1509,9 @@ __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwPara
       }
     }
   } else {
-    // ---------------- MMA issuer: both operands MN-major (bits 15, 16), M = 128, N = Cout, 32 bytes of K (= 16 bf16 / 8 tf32 rules) per instruction
-    const uint32_t fmt = BF16 ? 1u : 2u;
+    // ---------------- MMA issuer: both operands MN-major (bits 15, 16), M = 128, N = Cout, 32 bytes of K (= 16 bf16 / fp16, 8 tf32 rules) per
+    // instruction (kind::f16 takes MN-major operands in fp16 as in bf16)
+    const uint32_t fmt = F16 ? 0u : BF16 ? 1u : 2u;
     const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(P.Cout >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
     constexpr int kRulesPerMma = BF16 ? 16 : 8;
     const uint32_t aBlkStride16 = ((uint32_t)(nBa / nMh) * blockBytes) >> 4; // second half of M (channels 128..255): descriptor units
@@ -1560,7 +1592,7 @@ struct DwPlanParams {
   unsigned *sched; // [0] next work item, [1] CTAs that have drawn their last item (self-resetting, see sched_counters)
   long long *prof; // developer (SCN_DW_PROF): per CTA [0] total, [1] producer wait-empty, [2] producer stages, [3] mma total, [4] mma wait-full, [5] mma wait-acc, [6] epilogue busy
 };
-template <bool BF16>
+template <bool BF16, bool F16 = false>
 __global__ void __launch_bounds__(32 * (6 + kDwProd), 1) conv_dw_plan_tc(const DwPlanParams P) {
   extern __shared__ __align__(1024) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -1684,8 +1716,8 @@ __global__ void __launch_bounds__(32 * (6 + kDwProd), 1) conv_dw_plan_tc(const D
     }
     if (P.prof && pw == 0 && lane == 0) { long long *q = P.prof + blockIdx.x * 8; q[0] = clock64() - pt0; q[1] = pwait; q[2] = pstages; }
   } else if (warp == kMmaWarp) {
-    // ---------------- MMA issuer: both operands MN-major (bits 15, 16), M = 128, N = Cout, 32 bytes of K (= 16 bf16 / 8 tf32 positions) per instruction
-    const uint32_t fmt = BF16 ? 1u : 2u;
+    // ---------------- MMA issuer: both operands MN-major (bits 15, 16), M = 128, N = Cout, 32 bytes of K (= 16 bf16 / fp16, 8 tf32 positions) per instruction
+    const uint32_t fmt = F16 ? 0u : BF16 ? 1u : 2u;
     const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(P.Cout >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
     constexpr int kRulesPerMma = BF16 ? 16 : 8;
     const uint32_t aBlkStride16 = ((uint32_t)(nBa / nMh) * blockBytes) >> 4; // second half of M (channels 128..255): descriptor units
@@ -1745,19 +1777,26 @@ __global__ void __launch_bounds__(32 * (6 + kDwProd), 1) conv_dw_plan_tc(const D
 }
 // whether launch_conv_dw_tc takes this shape at all (else the caller falls back to the CUDA-core kernel, which needs the fp32 rows)
 bool dw_tc_ok(int Cin, int Cout, int K, int mathMode) {
-  if (mathMode != 2 || !tc_available()) return false;
+  if (!half_mode(mathMode) || !tc_available()) return false;
   return !((Cin % 32 != 0 && Cin > 32) || Cin > 256 || (Cin > 128 && Cin % 128 != 0) || Cout % 32 != 0 || Cout > 256 || ((Cin + 127) / 128) * Cout > 512 || K > 64);
 }
-__global__ void __launch_bounds__(256) k_from_bf16(const uint2 *__restrict__ x, float4 *__restrict__ y, long n4) {
+template <bool F16>
+__global__ void __launch_bounds__(256) k_from_16(const uint2 *__restrict__ x, float4 *__restrict__ y, long n4) {
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
     const uint2 v = x[i];
-    y[i] = make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xffff0000u), __uint_as_float(v.y << 16), __uint_as_float(v.y & 0xffff0000u));
+    if (F16) {
+      const float2 a = __half22float2(*reinterpret_cast<const __half2 *>(&v.x)), b = __half22float2(*reinterpret_cast<const __half2 *>(&v.y));
+      y[i] = make_float4(a.x, a.y, b.x, b.y);
+    } else {
+      y[i] = make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xffff0000u), __uint_as_float(v.y << 16), __uint_as_float(v.y & 0xffff0000u));
+    }
   }
 }
-// bf16 rows -> fp32 rows (exact); n a multiple of 4
-int from_bf16(const void *x, float *y, long n, cudaStream_t s) {
-  SCN_CHECK(n % 4 == 0, "bf16 -> fp32 copy needs an element count that is a multiple of 4");
-  if (n) k_from_bf16<<<stream_grid(n / 4, 256), 256, 0, LS(s)>>>(static_cast<const uint2 *>(x), reinterpret_cast<float4 *>(y), n / 4);
+// 16-bit rows in the current mode's format -> fp32 rows (exact); n a multiple of 4
+int from_16(const void *x, float *y, long n, cudaStream_t s) {
+  SCN_CHECK(n % 4 == 0, "16-bit -> fp32 copy needs an element count that is a multiple of 4");
+  if (n && f16_copies()) k_from_16<true><<<stream_grid(n / 4, 256), 256, 0, LS(s)>>>(static_cast<const uint2 *>(x), reinterpret_cast<float4 *>(y), n / 4);
+  else if (n) k_from_16<false><<<stream_grid(n / 4, 256), 256, 0, LS(s)>>>(static_cast<const uint2 *>(x), reinterpret_cast<float4 *>(y), n / 4);
   SCN_CUDA(cudaGetLastError());
   return 0;
 }
@@ -1765,17 +1804,17 @@ int from_bf16(const void *x, float *y, long n, cudaStream_t s) {
 bool dw_plan_ok(int Cin, int Cout, int K, int mathMode) {
   static int planOn = -1;
   if (planOn < 0) planOn = getenv("SCN_DW_PLAN") ? atoi(getenv("SCN_DW_PLAN")) : 0;
-  if (!planOn || mathMode != 2 || !tc_available() || deterministic()) return false; // (its partial sums are not indexed by work item)
+  if (!planOn || !half_mode(mathMode) || !tc_available() || deterministic()) return false; // (its partial sums are not indexed by work item)
   return !((Cin % 32 != 0 && Cin > 32) || Cin > 256 || (Cin > 128 && Cin % 128 != 0) || Cout % 32 != 0 || Cout > 256 || ((Cin + 127) / 128) * Cout > 512 || K > 64);
 }
 // dW must be zero on entry.  Returns 1 when the configuration is not supported (the caller then uses the CUDA-core kernel).
-// in16 / dout16: optional bf16 copies of `in` / `d_out` ([rows][Cin] / [rows][Cout], same layout) the caller already has.
+// in16 / dout16: optional 16-bit copies (the mode's format) of `in` / `d_out` ([rows][Cin] / [rows][Cout], same layout) the caller already has.
 int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2 *pairs, const int *d_off, const int *offHost, int K, long nInRows,
                       long nOutRows, int Cin, int Cout, int srcIsY, int mathMode, cudaStream_t s, const void *in16, const void *dout16,
                       const int *planNbr, const int *planOutRow, const unsigned long long *planMask, int planPos) {
-  // bf16 mode only: with TF32 operands the MN-major product came out as zeros on B200 (unresolved; tf32 mode keeps the CUDA-core kernel)
-  if (mathMode != 2 || !tc_available()) return 1;
-  const bool bf16 = true;
+  // bf16 / fp16 mode only: with TF32 operands the MN-major product came out as zeros on B200 (unresolved; tf32 mode keeps the CUDA-core kernel)
+  if (!half_mode(mathMode) || !tc_available()) return 1;
+  const bool bf16 = true, f16 = mathMode == kModeF16;
   if ((Cin % 32 != 0 && Cin > 32) || Cin > 256 || (Cin > 128 && Cin % 128 != 0) || Cout % 32 != 0 || Cout > 256 || ((Cin + 127) / 128) * Cout > 512 || K > 64) return 1;
   const int CinP = Cin % 32 == 0 ? Cin : (Cin <= 16 ? 16 : 32); // odd narrow inputs (the 9-channel network input): bf16 rows zero-padded to 16 / 32 channels
   static int planOn = -1;
@@ -1797,10 +1836,10 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
     const size_t na = haveA ? 0 : (((size_t)nInRows * CinP * 2 + 255) & ~(size_t)255);
     if (!haveA || !haveB) SCN_TRY(stream_scratch(s, kScratchDw, na + (haveB ? 0 : (size_t)nOutRows * Cout * 2) + 16, (void **)&scr));
     if (haveA) ++g_counters[kCntBwdOperandReused];
-    else if (CinP == Cin) SCN_TRY(to_bf16(in, scr, nInRows * Cin, s));
-    else if (nInRows) k_pad_rows_bf16<<<stream_grid(nInRows * CinP, 256), 256, 0, LS(s)>>>(in, reinterpret_cast<__nv_bfloat16 *>(scr), nInRows, Cin, CinP);
+    else if (CinP == Cin) SCN_TRY(to_16(in, scr, nInRows * Cin, s));
+    else if (nInRows) launch_pad_rows16(in, scr, nInRows, Cin, CinP, f16, s);
     if (haveB) ++g_counters[kCntBwdOperandReused];
-    else SCN_TRY(to_bf16(d_out, scr + na, nOutRows * Cout, s));
+    else SCN_TRY(to_16(d_out, scr + na, nOutRows * Cout, s));
     P.a = haveA ? static_cast<const unsigned char *>(in16) : scr;
     P.b = haveB ? static_cast<const unsigned char *>(dout16) : scr + na;
   } else {
@@ -1829,6 +1868,7 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
     static bool attrQ = false;
     if (!attrQ) {
       SCN_CUDA(cudaFuncSetAttribute(conv_dw_plan_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
+      SCN_CUDA(cudaFuncSetAttribute(conv_dw_plan_tc<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
       attrQ = true;
     }
     const int gridQ = std::min(K * Q.itemsPerK, kSMs);
@@ -1838,7 +1878,8 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
     if (envProf) { SCN_CUDA(cudaMalloc((void **)&Q.prof, kSMs * 8 * 8)); SCN_CUDA(cudaMemsetAsync(Q.prof, 0, kSMs * 8 * 8, s)); }
     SCN_TRY(sched_counters(s, &Q.sched));
     ++g_counters[kCntFloatAtomic];
-    conv_dw_plan_tc<true><<<gridQ, 32 * (6 + kDwProd), smemQ, LS(s)>>>(Q);
+    if (f16) { ++g_counters[kCntF16Launch]; conv_dw_plan_tc<true, true><<<gridQ, 32 * (6 + kDwProd), smemQ, LS(s)>>>(Q); }
+    else conv_dw_plan_tc<true><<<gridQ, 32 * (6 + kDwProd), smemQ, LS(s)>>>(Q);
     SCN_CUDA(cudaGetLastError());
     if (envProf) { // developer aid: per-role cycle counters, mean and max over the CTAs
       static long long h[kSMs * 8];
@@ -1876,10 +1917,12 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
   if (!attr) {
     SCN_CUDA(cudaFuncSetAttribute(conv_dw_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
     SCN_CUDA(cudaFuncSetAttribute(conv_dw_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
+    SCN_CUDA(cudaFuncSetAttribute(conv_dw_tc<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
     attr = true;
   }
   const int grid = (int)std::min<long>(nItems, kSMs);
-  if (bf16) conv_dw_tc<true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(P);
+  if (f16) { ++g_counters[kCntF16Launch]; conv_dw_tc<true, true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(P); }
+  else if (bf16) conv_dw_tc<true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(P);
   else conv_dw_tc<false><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(P);
   SCN_CUDA(cudaGetLastError());
   if (P.part) SCN_TRY(ordered_sum(P.part, P.nC, (long)K * Cin * Cout, dW, s)); // item c K + k = part c of list k: rows [nC][K][Cin][Cout]

@@ -20,7 +20,7 @@ bool lateral_take();
 void prepadded_arm(const void *rows16, int Cp);
 void bwd_in16_arm(const void *in16);
 bool dw_tc_ok(int Cin, int Cout, int K, int mathMode);
-int from_bf16(const void *x, float *y, long n, cudaStream_t s);
+int from_16(const void *x, float *y, long n, cudaStream_t s);
 int batchnorm_backward_y16(const float *in, float *d_in, const float *out, const void *out_bf16, float *d_out, long n, int C, const float *save_mean,
                            const float *save_invstd, const float *weight, float *d_weight, float *d_bias, float leak, cudaStream_t s);
 void prepadded_disarm();
@@ -40,10 +40,10 @@ struct Op {
 };
 struct Reg {
   float *p = nullptr;
-  void *p16 = nullptr; // bfloat16 copy (math mode 2, written by BatchNorm / add)
+  void *p16 = nullptr; // 16-bit copy (math mode 2: bfloat16, 5: fp16; written by BatchNorm / add)
   long rows = 0;
   int cols = 0;
-  int pad16 = 0; // > 0: p16 holds the rows zero-padded to this many channels (network input in bf16 mode)
+  int pad16 = 0; // > 0: p16 holds the rows zero-padded to this many channels (network input in bf16 / fp16 mode)
 };
 
 } // namespace
@@ -424,7 +424,7 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
     R.p = halfOnly ? nullptr : static_cast<float *>(slot_get(p, (size_t)std::max(1l, rows * cols) * 4));
     if (halfOnly) ++scn::g_counters[scn::kCntHalfOnlyOut];
     if (!R.p && !halfOnly) return -1;
-    if (shadow && mode == 2 && cols % 32 == 0 && rows > 0) {
+    if (shadow && scn::half_mode(mode) && cols % 32 == 0 && rows > 0) {
       R.p16 = slot_get(p, (size_t)rows * cols * 2);
       if (!R.p16) return -1;
     }
@@ -481,7 +481,7 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
         rc = alloc_reg(a[0], nActive, (int)a[6], false);
         p->regs[a[0]].pad16 = 0;
         const int C0 = (int)a[6], Cp = C0 < 16 ? 16 : 32;
-        if (rc == 0 && nActive && mode == 2 && a[4] != 0 && C0 % 32 != 0 && C0 < 32 && scn_tensor_core_path_available()) {
+        if (rc == 0 && nActive && scn::half_mode(mode) && a[4] != 0 && C0 % 32 != 0 && C0 < 32 && scn_tensor_core_path_available()) {
           // bf16 mode: the first convolution gathers bf16 rows zero-padded to 16 / 32 channels; written here, by the same pass
           Reg &R0 = p->regs[a[0]];
           R0.p16 = slot_get(p, (size_t)nActive * Cp * 2);
@@ -499,7 +499,7 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
           if (rc) break;
         }
         rc = scn_get_nactive(M, a + 2, &n);
-        const bool half = !train && a[23] == 1 && mode == 2 && n >= kHalfOnlyRows && scn_tensor_core_path_available();
+        const bool half = !train && a[23] == 1 && scn::half_mode(mode) && n >= kHalfOnlyRows && scn_tensor_core_path_available();
         if (rc == 0) rc = alloc_reg(a[1], n, (int)a[11], half || a[22] >= 0 || a[18] >= 0, half);
         const Reg &I = p->regs[a[0]];
         if (rc == 0) { arm(op); arm_lateral(op); }
@@ -516,7 +516,7 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
       case K_CONV: { // in, out, inS[3], outS[3], f[3], s[3], w, bias, Cin, Cout
         long n = 0, nr = 0;
         rc = scn_convolution_prepare(M, a + 2, a + 5, a + 8, a + 11, &n, &nr);
-        const bool half = !train && a[23] == 1 && mode == 2 && n >= kHalfOnlyRows && scn_tensor_core_path_available();
+        const bool half = !train && a[23] == 1 && scn::half_mode(mode) && n >= kHalfOnlyRows && scn_tensor_core_path_available();
         if (rc == 0) rc = alloc_reg(a[1], n, (int)a[17], half || a[22] >= 0 || a[18] >= 0, half);
         const Reg &I = p->regs[a[0]];
         if (rc == 0) { arm(op); arm_lateral(op); }
@@ -531,7 +531,7 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
       case K_DECONV: {
         long n = 0;
         rc = scn_get_nactive(M, a + 5, &n);
-        const bool half = !train && a[23] == 1 && mode == 2 && n >= kHalfOnlyRows && scn_tensor_core_path_available();
+        const bool half = !train && a[23] == 1 && scn::half_mode(mode) && n >= kHalfOnlyRows && scn_tensor_core_path_available();
         if (rc == 0) rc = alloc_reg(a[1], n, (int)a[17], half || a[22] >= 0 || a[18] >= 0, half);
         const Reg &I = p->regs[a[0]];
         if (rc == 0) { arm(op); arm_lateral(op); }
@@ -550,7 +550,7 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
         // kernels gather from it)
         static int trainHalf = -1;
         if (trainHalf < 0) trainHalf = getenv("SCN_TRAIN_HALF_BN") ? atoi(getenv("SCN_TRAIN_HALF_BN")) : 1;
-        const bool halfOnly = (!train || trainHalf) && fromSums && a[19] == 1 && mode == 2 && scn_tensor_core_path_available();
+        const bool halfOnly = (!train || trainHalf) && fromSums && a[19] == 1 && scn::half_mode(mode) && scn_tensor_core_path_available();
         rc = alloc_reg(a[1], I.rows, (int)a[2], true, halfOnly);
         float *saveM = p->bnScratch, *saveI = p->bnScratch + scn::kBnMaxC;
         if (rc == 0 && train) { // kept for the backward pass
@@ -709,7 +709,7 @@ int scn_program_backward(scn_program *p, int n_out, const int *out_regs, const f
           }
         }
         if (I.rows == 0 || p->regs[outReg].rows == 0) break;
-        SCN_CHECK(I.p || (I.p16 && !I.pad16 && Cin % 32 == 0 && scn_get_math_mode() == 2), "program backward: convolution input was not kept");
+        SCN_CHECK(I.p || (I.p16 && !I.pad16 && Cin % 32 == 0 && scn::half_mode(scn_get_math_mode())), "program backward: convolution input was not kept");
         if ((rc = mark(wi)) || (rc = mark(bi))) break;
         // the gradient of the network input is only computed on request (App. D.13)
         bool inputIsNetworkInput = false;
@@ -728,7 +728,7 @@ int scn_program_backward(scn_program *p, int n_out, const int *out_regs, const f
         }
         // bf16 mode: the forward pass left a bf16 copy of the input rows (same layout: whole rows, no padding) -- the
         // weight-gradient kernel gathers from it instead of converting the fp32 rows again
-        if (I.p16 && !I.pad16 && Cin % 32 == 0 && scn_get_math_mode() == 2) scn::bwd_in16_arm(I.p16);
+        if (I.p16 && !I.pad16 && Cin % 32 == 0 && scn::half_mode(scn_get_math_mode())) scn::bwd_in16_arm(I.p16);
         const float *inRows = I.p;
         float *inTmp = nullptr;
         if (!inRows) { // the forward pass kept only the bf16 copy of these rows (a BatchNorm output read by tensor-core convolutions alone)
@@ -737,7 +737,7 @@ int scn_program_backward(scn_program *p, int n_out, const int *out_regs, const f
           if (!scn::dw_tc_ok(Cin, Cout, (int)Kv, scn_get_math_mode())) { // the CUDA-core weight-gradient kernel reads fp32 rows: widen the copy (exact)
             inTmp = static_cast<float *>(slot_get(p, (size_t)elems(a[0]) * 4));
             if (!inTmp) { rc = -1; break; }
-            if ((rc = scn::from_bf16(I.p16, inTmp, elems(a[0]), s))) break;
+            if ((rc = scn::from_16(I.p16, inTmp, elems(a[0]), s))) break;
             inRows = inTmp;
           }
         }

@@ -155,6 +155,8 @@ __global__ void __launch_bounds__(256) k_bn_stats(const float *__restrict__ x, l
 }
 // One launch for small inputs: CTA b owns channels [32 b, 32 b + 32); statistics, scale / shift and the
 // normalised output (the rows come back out of L1/L2 for the second pass).
+// y16 (optional): the output rows rounded to 16 bits (bf16, or fp16 with F16), the gather operand of a following convolution
+template <bool F16>
 __global__ void __launch_bounds__(256) k_bn_small(const float *__restrict__ x, float *__restrict__ y, int n, int C, BnFin F, float leak, void *__restrict__ y16) {
   __shared__ float4 S[256], Q[256];
   __shared__ float sScale[32], sShift[32];
@@ -197,13 +199,7 @@ __global__ void __launch_bounds__(256) k_bn_small(const float *__restrict__ x, f
     o.x = fmaf(v.x, a.x, b.x); o.y = fmaf(v.y, a.y, b.y); o.z = fmaf(v.z, a.z, b.z); o.w = fmaf(v.w, a.w, b.w);
     o.x = o.x > 0 ? o.x : o.x * leak; o.y = o.y > 0 ? o.y : o.y * leak; o.z = o.z > 0 ? o.z : o.z * leak; o.w = o.w > 0 ? o.w : o.w * leak;
     reinterpret_cast<float4 *>(y)[i] = o;
-    if (y16) {
-      __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
-      uint2 pk;
-      pk.x = *reinterpret_cast<unsigned int *>(&lo);
-      pk.y = *reinterpret_cast<unsigned int *>(&hi);
-      reinterpret_cast<uint2 *>(y16)[i] = pk;
-    }
+    if (y16) reinterpret_cast<uint2 *>(y16)[i] = pack16x4<F16>(o);
   }
 }
 // scalar fallback for C % 4 != 0 (C <= 256)
@@ -237,14 +233,10 @@ __global__ void k_bn_finalize(double *__restrict__ stats, BnFin F) {
 }
 
 // y = leaky(x*scale + shift)   (:53-61)
-// y16 (optional): the same values rounded to bf16, the gather operand of a following bf16 convolution
-__device__ __forceinline__ void store_bf16x4(void *base, long i, float4 o) {
-  __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
-  uint2 pk;
-  pk.x = *reinterpret_cast<unsigned int *>(&lo);
-  pk.y = *reinterpret_cast<unsigned int *>(&hi);
-  reinterpret_cast<uint2 *>(base)[i] = pk;
-}
+// y16 (optional): the same values rounded to 16 bits (bf16, or fp16 with F16), the gather operand of a following convolution
+template <bool F16>
+__device__ __forceinline__ void store16x4(void *base, long i, float4 o) { reinterpret_cast<uint2 *>(base)[i] = pack16x4<F16>(o); }
+template <bool F16>
 __global__ void __launch_bounds__(256) k_bn_apply(const float *__restrict__ x, float *__restrict__ y, long total4, int cv, const float *__restrict__ scale,
                                                   const float *__restrict__ shift, float leak, void *__restrict__ y16) {
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < total4; i += (long)gridDim.x * blockDim.x) {
@@ -255,7 +247,7 @@ __global__ void __launch_bounds__(256) k_bn_apply(const float *__restrict__ x, f
     o.x = fmaf(v.x, a.x, b.x); o.y = fmaf(v.y, a.y, b.y); o.z = fmaf(v.z, a.z, b.z); o.w = fmaf(v.w, a.w, b.w);
     o.x = o.x > 0 ? o.x : o.x * leak; o.y = o.y > 0 ? o.y : o.y * leak; o.z = o.z > 0 ? o.z : o.z * leak; o.w = o.w > 0 ? o.w : o.w * leak;
     reinterpret_cast<float4 *>(y)[i] = o;
-    if (y16) store_bf16x4(y16, i, o);
+    if (y16) store16x4<F16>(y16, i, o);
   }
 }
 __global__ void __launch_bounds__(256) k_bn_apply_scalar(const float *__restrict__ x, float *__restrict__ y, long total, int C, const float *__restrict__ scale,
@@ -271,6 +263,7 @@ __global__ void __launch_bounds__(256) k_bn_apply_scalar(const float *__restrict
 // PRODUCER of x accumulated in its epilogue (conv_plan_tc, P.stats): the statistics pass over x disappears.
 // sums: [kBnReplicas][2][kFusedStatsC] doubles.  Block 0 also writes saveMean / saveInvStd and (train mode) the
 // running statistics, exactly once.
+template <bool F16>
 __global__ void __launch_bounds__(256) k_bn_apply_sums(const float *__restrict__ x, float *__restrict__ y, long total4, int cv, const double *__restrict__ sums,
                                                        BnFin F, float leak, void *__restrict__ y16) {
   __shared__ __align__(16) float sScale[kFusedStatsC], sShift[kFusedStatsC];
@@ -314,8 +307,8 @@ __global__ void __launch_bounds__(256) k_bn_apply_sums(const float *__restrict__
       float4 o;
       o.x = fmaf(v[u].x, a.x, b.x); o.y = fmaf(v[u].y, a.y, b.y); o.z = fmaf(v[u].z, a.z, b.z); o.w = fmaf(v[u].w, a.w, b.w);
       o.x = o.x > 0 ? o.x : o.x * leak; o.y = o.y > 0 ? o.y : o.y * leak; o.z = o.z > 0 ? o.z : o.z * leak; o.w = o.w > 0 ? o.w : o.w * leak;
-      if (y) reinterpret_cast<float4 *>(y)[i] = o; // y == nullptr: only the bf16 copy is consumed downstream
-      if (y16) store_bf16x4(y16, i, o);
+      if (y) reinterpret_cast<float4 *>(y)[i] = o; // y == nullptr: only the 16-bit copy is consumed downstream
+      if (y16) store16x4<F16>(y16, i, o);
     }
   }
 }
@@ -324,7 +317,7 @@ int bn_forward_from_sums(const float *x, float *y, long n, int C, const double *
   SCN_CHECK(C % 4 == 0 && C <= kFusedStatsC && (mode == 0 || mode == 2) && n > 0, "bn_forward_from_sums: unsupported configuration");
   BnFin F{n, C, mode, eps, momentum, saveMean, saveInvStd, runningMean, runningVar, weight, bias, nullptr, nullptr};
   const long total4 = n * C / 4;
-  SCN_CUDA(launch_pdl(k_bn_apply_sums, dim3(stream_grid(total4, 256)), dim3(256), 0, LS(s), x, y, total4, C / 4, sums, F, leak, y16));
+  SCN_CUDA(launch_pdl(f16_copies() ? k_bn_apply_sums<true> : k_bn_apply_sums<false>, dim3(stream_grid(total4, 256)), dim3(256), 0, LS(s), x, y, total4, C / 4, sums, F, leak, y16));
   SCN_CUDA(cudaGetLastError());
   return 0;
 }
@@ -336,9 +329,9 @@ int bn_forward(const float *x, float *y, long n, int C, float *saveMean, float *
   float *scale = reinterpret_cast<float *>(stats + (size_t)kBnReplicas * 2 * kBnMaxC), *shift = scale + kBnMaxC; // fixed layout: the statistics area stays zero between calls
   unsigned *ticket = reinterpret_cast<unsigned *>(shift + kBnMaxC);
   BnFin F{n, C, mode, eps, momentum, saveMean, saveInvStd, runningMean, runningVar, weight, bias, scale, shift};
-  SCN_CHECK(!y16 || C % 4 == 0, "bf16 shadow needs a channel count that is a multiple of 4");
+  SCN_CHECK(!y16 || C % 4 == 0, "16-bit shadow needs a channel count that is a multiple of 4");
   if (C % 4 == 0 && n > 0 && n <= 2048) { // small levels: statistics, finalize and apply in ONE launch
-    SCN_CUDA(launch_pdl(k_bn_small, dim3(cdiv(C, 32)), dim3(256), 0, LS(s), x, y, (int)n, C, F, leak, y16));
+    SCN_CUDA(launch_pdl(f16_copies() ? k_bn_small<true> : k_bn_small<false>, dim3(cdiv(C, 32)), dim3(256), 0, LS(s), x, y, (int)n, C, F, leak, y16));
     SCN_CUDA(cudaGetLastError());
     return 0;
   }
@@ -364,7 +357,8 @@ int bn_forward(const float *x, float *y, long n, int C, float *saveMean, float *
   if (!finalized) k_bn_finalize<<<cdiv(C, 128), 128, 0, LS(s)>>>(stats, F);
   if (n) {
     long total = n * C;
-    if (C % 4 == 0) k_bn_apply<<<stream_grid(total / 4, 256), 256, 0, LS(s)>>>(x, y, total / 4, C / 4, scale, shift, leak, y16);
+    if (C % 4 == 0 && f16_copies()) k_bn_apply<true><<<stream_grid(total / 4, 256), 256, 0, LS(s)>>>(x, y, total / 4, C / 4, scale, shift, leak, y16);
+    else if (C % 4 == 0) k_bn_apply<false><<<stream_grid(total / 4, 256), 256, 0, LS(s)>>>(x, y, total / 4, C / 4, scale, shift, leak, y16);
     else k_bn_apply_scalar<<<stream_grid(total, 256), 256, 0, LS(s)>>>(x, y, total, C, scale, shift, leak);
   }
   SCN_CUDA(cudaGetLastError());
@@ -426,11 +420,15 @@ __global__ void __launch_bounds__(256) k_bn_bwd_apply(const float *__restrict__ 
 }
 // float4 versions (C % 4 == 0): four channels per thread, two rows in flight -- the scalar kernels above ran at well under half of
 // the HBM rate (one 4-byte access in flight per thread, an integer modulo per element in the apply pass).
-// y16 (optional): the BatchNorm output as bf16 rows -- only its sign is needed (the leaky-ReLU mask), and a replayed training step in
-// bf16 mode never writes the fp32 output rows of a BatchNorm whose only readers are tensor-core convolutions.
+// y16 (optional): the BatchNorm output as 16-bit rows -- only its sign is needed (the leaky-ReLU mask), and a replayed training step in
+// bf16 / fp16 mode never writes the fp32 output rows of a BatchNorm whose only readers are tensor-core convolutions.
+// Nothing here decodes the value: each 16-bit pattern goes to the top half of an fp32 pattern, whose sign is then the 16-bit sign
+// bit (bit 15 in bf16 and in fp16) and which is zero exactly when the 16-bit value is +-0, so `> 0` agrees with the 16-bit value in
+// both formats (a bf16 pattern becomes its exact value; an fp16 pattern becomes some other number of the same sign).  The one
+// difference: an fp16 NaN lands on a finite fp32 number and takes the mask of its sign bit.
 __device__ __forceinline__ float4 bn_y4(const float4 *y, const uint2 *y16, long i) {
   if (!y16) return y[i];
-  const uint2 v = y16[i]; // bf16 = the upper half of the fp32 pattern: the sign survives a plain shift
+  const uint2 v = y16[i]; // the sign survives a plain shift
   return make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xffff0000u), __uint_as_float(v.y << 16), __uint_as_float(v.y & 0xffff0000u));
 }
 __global__ void __launch_bounds__(256) k_bn_bwd_stats4(const float4 *__restrict__ x, const float4 *__restrict__ y, const uint2 *__restrict__ y16, float4 *__restrict__ dy, long n, int C4,
@@ -548,11 +546,12 @@ __global__ void __launch_bounds__(256) k_input_bwd(float *__restrict__ din, cons
     for (int j = 1; j <= na; j++) din[(long)r[j] * C + c] = g; // an input row feeds exactly one voxel: plain store
   }
 }
-// Same, plus a bf16 copy of the output rows zero-padded to Cp channels (the packed operand of the first convolution in
-// bf16 mode, which otherwise needs a separate padding pass over the rows).
+// Same, plus a 16-bit copy (bf16, or fp16 with F16) of the output rows zero-padded to Cp channels (the packed operand of the first
+// convolution in bf16 / fp16 mode, which otherwise needs a separate padding pass over the rows).
 // One thread per output row: the rule-table entries are read once per row (not once per channel) and the bf16 row
 // (Cp <= 32 channels) leaves as 16-byte stores.
-__global__ void __launch_bounds__(256) k_input_fwd_pad16(const float *__restrict__ in, float *__restrict__ out, __nv_bfloat16 *__restrict__ out16, int nOut, int w,
+template <bool F16>
+__global__ void __launch_bounds__(256) k_input_fwd_pad16(const float *__restrict__ in, float *__restrict__ out, unsigned short *__restrict__ out16, int nOut, int w,
                                                          int C, int Cp, const int *__restrict__ tab, int average) {
   for (long row = blockIdx.x * (long)blockDim.x + threadIdx.x; row < nOut; row += (long)gridDim.x * blockDim.x) {
     const int *r = tab + row * w;
@@ -574,18 +573,17 @@ __global__ void __launch_bounds__(256) k_input_fwd_pad16(const float *__restrict
 #pragma unroll
     for (int q = 0; q < 4; q++) {
       if (q * 8 >= Cp) break;
-      __nv_bfloat162 v0 = __floats2bfloat162_rn(acc[q * 8], acc[q * 8 + 1]), v1 = __floats2bfloat162_rn(acc[q * 8 + 2], acc[q * 8 + 3]);
-      __nv_bfloat162 v2 = __floats2bfloat162_rn(acc[q * 8 + 4], acc[q * 8 + 5]), v3 = __floats2bfloat162_rn(acc[q * 8 + 6], acc[q * 8 + 7]);
       uint4 pk;
-      pk.x = *reinterpret_cast<unsigned int *>(&v0); pk.y = *reinterpret_cast<unsigned int *>(&v1);
-      pk.z = *reinterpret_cast<unsigned int *>(&v2); pk.w = *reinterpret_cast<unsigned int *>(&v3);
+      pk.x = pack16x2<F16>(acc[q * 8], acc[q * 8 + 1]); pk.y = pack16x2<F16>(acc[q * 8 + 2], acc[q * 8 + 3]);
+      pk.z = pack16x2<F16>(acc[q * 8 + 4], acc[q * 8 + 5]); pk.w = pack16x2<F16>(acc[q * 8 + 6], acc[q * 8 + 7]);
       dst[q] = pk;
     }
   }
 }
 int input_forward_pad16(const float *in, float *out, void *out16, int nOut, int maxActive, int C, int Cp, const int *tab, int average, cudaStream_t s) {
   SCN_CHECK(C <= 32 && Cp <= 32 && Cp % 8 == 0 && Cp >= C, "input_forward_pad16: at most 32 channels");
-  if (nOut) k_input_fwd_pad16<<<stream_grid(nOut, 256, 16), 256, 0, LS(s)>>>(in, out, static_cast<__nv_bfloat16 *>(out16), nOut, 1 + maxActive, C, Cp, tab, average);
+  if (nOut && f16_copies()) k_input_fwd_pad16<true><<<stream_grid(nOut, 256, 16), 256, 0, LS(s)>>>(in, out, static_cast<unsigned short *>(out16), nOut, 1 + maxActive, C, Cp, tab, average);
+  else if (nOut) k_input_fwd_pad16<false><<<stream_grid(nOut, 256, 16), 256, 0, LS(s)>>>(in, out, static_cast<unsigned short *>(out16), nOut, 1 + maxActive, C, Cp, tab, average);
   SCN_CUDA(cudaGetLastError());
   return 0;
 }
@@ -602,19 +600,21 @@ int input_backward(float *din, const float *dout, long nIn, int nOut, int maxAct
 }
 
 // ------------------------------------------------------------------ add_feature_planes / AddTable
+template <bool F16>
 __global__ void __launch_bounds__(256) k_add(const float *__restrict__ a, const float *__restrict__ b, float *__restrict__ o, long n, void *__restrict__ o16) {
   long n4 = n >> 2;
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
     float4 u = __ldg(reinterpret_cast<const float4 *>(a) + i), v = __ldg(reinterpret_cast<const float4 *>(b) + i);
     float4 r = make_float4(u.x + v.x, u.y + v.y, u.z + v.z, u.w + v.w);
     reinterpret_cast<float4 *>(o)[i] = r;
-    if (o16) store_bf16x4(o16, i, r);
+    if (o16) store16x4<F16>(o16, i, r);
   }
   for (long i = (n4 << 2) + blockIdx.x * (long)blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) o[i] = a[i] + b[i];
 }
 int add_rows(const float *a, const float *b, float *o, long n, cudaStream_t s, void *o16) {
-  SCN_CHECK(!o16 || n % 4 == 0, "bf16 shadow needs an element count that is a multiple of 4");
-  if (n) k_add<<<stream_grid(n / 4 + 1, 256), 256, 0, LS(s)>>>(a, b, o, n, o16);
+  SCN_CHECK(!o16 || n % 4 == 0, "16-bit shadow needs an element count that is a multiple of 4");
+  if (n && f16_copies()) k_add<true><<<stream_grid(n / 4 + 1, 256), 256, 0, LS(s)>>>(a, b, o, n, o16);
+  else if (n) k_add<false><<<stream_grid(n / 4 + 1, 256), 256, 0, LS(s)>>>(a, b, o, n, o16);
   SCN_CUDA(cudaGetLastError());
   return 0;
 }

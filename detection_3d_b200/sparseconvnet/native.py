@@ -42,19 +42,23 @@ def _opt(t, what):
     return None if t is None or t.numel() == 0 else _dev_f32(t, what)
 
 
-# ---- bf16 shadows (math mode 'bf16' only).  A BatchNorm / add output carries a bfloat16 copy of
-# itself as a Python attribute of the tensor object, written by the same kernel that wrote the
-# fp32 values; the next convolution gathers from that copy (half the bytes).  The attribute dies
-# with the tensor object and is ignored once the tensor has been modified in place (_version).
+# ---- 16-bit shadows (math modes 'bf16' and 'fp16' only).  A BatchNorm / add output carries a 16-bit
+# copy of itself (bfloat16 in 'bf16' mode, float16 in 'fp16' mode) as a Python attribute of the tensor
+# object, written by the same kernel that wrote the fp32 values; the next convolution gathers from that
+# copy (half the bytes).  The attribute dies with the tensor object and is ignored once the tensor has
+# been modified in place (_version) or when the current mode uses the other 16-bit format (the
+# convolution then converts the fp32 rows itself), so switching between 'bf16' and 'fp16' is safe.
 _MATH = {"mode": 0}
 _WEIGHT_IMAGES_DROPPED = [0]  # (statistics only)
+_SHADOW_DTYPE = {2: torch.bfloat16, 5: torch.float16}  # math mode -> format of the 16-bit copies
 
 
 def _new_shadow(t):
-    """bf16 buffer for the fp32 feature matrix `t` (or None when the mode / shape does not use one)."""
-    if _MATH["mode"] != 2 or t.dim() != 2 or t.size(1) % 32 != 0 or t.size(0) == 0:
+    """16-bit buffer for the fp32 feature matrix `t` (or None when the mode / shape does not use one)."""
+    dt = _SHADOW_DTYPE.get(_MATH["mode"])
+    if dt is None or t.dim() != 2 or t.size(1) % 32 != 0 or t.size(0) == 0:
         return None
-    return torch.empty(t.shape, dtype=torch.bfloat16, device=t.device)
+    return torch.empty(t.shape, dtype=dt, device=t.device)
 
 
 def _attach_shadow(t, sh):
@@ -102,7 +106,7 @@ _EPOCH = 0
 
 def _shadow_ptr(t):
     sh = getattr(t, "_scn_bf16", None)
-    if sh is None or _MATH["mode"] != 2 or sh[1] != t._version or sh[0].shape != t.shape:
+    if sh is None or sh[0].dtype != _SHADOW_DTYPE.get(_MATH["mode"]) or sh[1] != t._version or sh[0].shape != t.shape:
         return None
     return C.c_void_p(sh[0].data_ptr())
 
@@ -448,11 +452,13 @@ def add_features(a, b):
 
 
 def set_math_mode(mode):
-    """'fp32' (CUDA cores, exact), 'tf32' or 'bf16' (tcgen05 tensor cores, fp32 accumulate), or 'tf32x3' (tcgen05, every fp32
+    """'fp32' (CUDA cores, exact), 'tf32' or 'bf16' (tcgen05 tensor cores, fp32 accumulate), 'tf32x3' (tcgen05, every fp32
     operand split into two TF32 values hi + lo, three products per step in one fp32 accumulator: fp32-class accuracy at tensor-core
     speed; weight gradients and the convolutions the tensor-core kernel cannot take run on the exact CUDA-core kernels, as in
-    'tf32').  math_mode() returns the code: 0, 1, 2 or 3."""
-    code = {"fp32": 0, "tf32": 1, "bf16": 2, "tf32x3": 3}[mode] if isinstance(mode, str) else int(mode)
+    'tf32'), or 'fp16' (as 'bf16', with fp16 operands wherever 'bf16' has bf16 ones: 11 significant bits instead of 8, but a range
+    of +-65504 -- a larger value becomes inf, as with .half() -- so training needs loss scaling, e.g. torch.amp.GradScaler).
+    math_mode() returns the code: 0, 1, 2, 3 or 5."""
+    code = {"fp32": 0, "tf32": 1, "bf16": 2, "tf32x3": 3, "fp16": 5}[mode] if isinstance(mode, str) else int(mode)
     check(lib().scn_set_math_mode(code))
     _MATH["mode"] = lib().scn_get_math_mode()
 

@@ -50,7 +50,8 @@ int scn_input_layer_build(scn_metadata *m, const long spatial_size[3], const lon
 int scn_input_layer_built(scn_metadata *m, long *n_active, int *max_active);
 /* InputLayer_ForwardPass / InputLayer_fp  (CPU/IOLayers.cpp:11-29, CUDA/IOLayers.cu:31-41) */
 int scn_input_layer_forward(scn_metadata *m, const float *in_features, float *out_features, int n_planes);
-/* scn_input_layer_forward that also writes the rows as bfloat16 zero-padded to `padded` channels (first convolution of a bf16 program) */
+/* scn_input_layer_forward that also writes the rows as 16-bit values (bfloat16; float16 in math mode 5) zero-padded to `padded`
+ * channels (first convolution of a bf16 / fp16 program) */
 int scn_input_layer_forward_padded_bf16(scn_metadata *m, const float *in_features, float *out_features, void *out_bf16, int n_planes, int padded);
 /* InputLayer_updateGradInput (pybind.cpp:159-162; CPU/IOLayers.cpp:30-47) */
 int scn_input_layer_backward(scn_metadata *m, float *d_in_features, const float *d_out_features, int n_planes);
@@ -94,15 +95,17 @@ int scn_iteration_order(scn_metadata *m, const long spatial_size[3], int *dst);
 /* SubmanifoldConvolution_updateOutput (pybind.cpp:134-138; CPU/Convolution.cpp:117-150;
  * CUDA/Convolution.cpp:95-125).  weight [K][Cin][Cout] (= (K,1,Cin,Cout) with groups 1),
  * bias NULL or [Cout].  *macs = sum_k nRules_k*Cin*Cout, the value the reference returns.
- * in_bf16 (all three forward calls): NULL, or a device copy of `in` rounded to bfloat16 (same
+ * in_bf16 (all three forward calls): NULL, or a device copy of `in` rounded to 16 bits (same
  * [rows][n_in] layout) that a preceding scn_batchnorm_forward / scn_add_features produced; it is
- * only read in math mode 2, where a NULL makes the call convert `in` itself.
+ * only read in math modes 2 and 5, where a NULL makes the call convert `in` itself.  Every "bf16"
+ * argument of this header (in_bf16, out_bf16, lat_in_bf16) holds a 16-bit copy in the format of the
+ * current math mode: float16 in mode 5, bfloat16 in every other mode.
  * weight_tag: 0, or a value that identifies the CONTENTS of `weight` (same pointer + same tag =
  * same values as in an earlier call): the tensor-core paths then reuse the operand image they
  * derived from it (rounded, swizzled copy) instead of rebuilding it on every call.
  * add_in: NULL, or [output rows][n_out] float32 added to the result (out = conv(in) + add_in): the
  * residual / lateral AddTable that follows the convolution in the network, fused into its epilogue.
- * out_bf16: NULL, or [output rows][n_out] bfloat16 that receives the (summed) result rounded to nearest. */
+ * out_bf16: NULL, or [output rows][n_out] 16-bit values (the mode's format) that receive the (summed) result rounded to nearest. */
 int scn_submanifold_convolution_forward(scn_metadata *m, const long spatial_size[3], const long filter_size[3],
                                         const float *in, float *out, const float *weight, const float *bias,
                                         int n_in, int n_out, double *macs, const void *in_bf16, long long weight_tag,
@@ -136,8 +139,8 @@ int scn_deconvolution_backward(scn_metadata *m, const long in_size[3], const lon
  * mode 0 = train, 1 = eval with the given running stats, 2 = eval with
  * track_running_stats=False (batchNormalization.py:51-56: mean(0) / unbiased var(0) of this input).
  * weight / bias may be NULL.  leakiness 0 = ReLU, 1 = no activation.
- * out_bf16: NULL, or [n_rows][n_planes] bfloat16 that receives `out` rounded to nearest (the gather
- * operand of a following convolution in math mode 2; n_planes % 4 == 0). */
+ * out_bf16: NULL, or [n_rows][n_planes] 16-bit values (bfloat16; float16 in math mode 5) that receive `out`
+ * rounded to nearest (the gather operand of a following convolution in math mode 2 / 5; n_planes % 4 == 0). */
 int scn_batchnorm_forward(const float *in, float *out, long n_rows, int n_planes, float *save_mean, float *save_invstd,
                           float *running_mean, float *running_var, const float *weight, const float *bias, float eps,
                           float momentum, int mode, float leakiness, void *stream, void *out_bf16);
@@ -304,8 +307,11 @@ int scn_voxelize(const float *xyz, const float *feats, long n, int n_feat, const
  * (exact-fp32 anchor), 1 = tcgen05 tensor cores, TF32 inputs / fp32 accumulate (default where the
  * channel counts allow), 2 = tcgen05 BF16 inputs / fp32 accumulate, 3 = tcgen05 "3xTF32": each fp32
  * operand split into two exact TF32 values hi + lo, three TF32 products (hi*lo, lo*hi, hi*hi) in one fp32
- * accumulator, fp32-class accuracy.  In modes 1 and 3 every convolution the tensor-core kernel cannot take,
- * and every weight gradient, runs on the exact fp32 CUDA-core kernels. */
+ * accumulator, fp32-class accuracy, 5 = tcgen05 FP16 inputs / fp32 accumulate wherever mode 2 has BF16 inputs
+ * (everything else as in mode 2): 11 significant bits instead of 8, range +-65504 -- conversions round to nearest
+ * even with IEEE overflow (a larger value becomes +-inf and propagates) and keep subnormals.  Code 4 is not a mode.
+ * In modes 1 and 3 every convolution the tensor-core kernel cannot take, and every weight gradient, runs on the
+ * exact fp32 CUDA-core kernels. */
 int scn_set_math_mode(int mode);
 int scn_get_math_mode(void);
 /* Deterministic mode for this process (0 = off, the default): with 1, every float result of the calls above except
@@ -329,7 +335,7 @@ long scn_kernel_launch_count(void);
  * weight-gradient kernel took from its caller (forward shadow / shared d_out copy) instead of converting again, 13 = weight-gradient
  * launches driven by the output-stationary plan, 14 = float-atomic launches: launches whose float result depends on the order in
  * which atomics land (0 in deterministic mode except for scn_roi_align_rotated_3d_backward), 17 = host -> device copies of
- * input-layer coordinates. */
+ * input-layer coordinates, 18 = tensor-core launches with fp16 operands (convolutions and weight gradients, math mode 5). */
 long scn_debug_counter(int which);
 /* Hands the library's idle device memory back to the driver: Metadata chunks not owned by a live Metadata, cached weight operand
  * images, per-stream scratch buffers (the library recycles these itself instead of returning them; torch.cuda.empty_cache() cannot
@@ -341,8 +347,8 @@ long scn_release_cached_memory(void);
  * FPN's lateral 1x1x1 convolution and the statistics of a following BatchNorm into a convolution; no reference counterpart:
  * the reference runs NetworkInNetwork / SubmanifoldConvolution(1), AddTable and BatchNormalization as separate passes,
  * fpn_net.py:166-176, CPU/BatchNormalization.cpp:12-62).
- *  lateral: out = conv(in) [+ add_in] + lat_in[row] @ lat_weight ([n_in][n_out], one filter offset), lat_in_bf16 = bf16
- *           copy of lat_in (needed in math mode 2);
+ *  lateral: out = conv(in) [+ add_in] + lat_in[row] @ lat_weight ([n_in][n_out], one filter offset), lat_in_bf16 = 16-bit
+ *           copy of lat_in in the mode's format (needed in math modes 2 and 5);
  *  stats:   sums = [8 replicas][2][128] doubles, zeroed by the caller; the launch adds per-channel sum (first 128) and sum
  *           of squares (second 128) of the rows it stores, spread over the replicas (deterministic mode: written into replica
  *           0 after the launch, in a fixed order).
