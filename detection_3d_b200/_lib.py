@@ -32,6 +32,8 @@ SYMBOLS = {
     "scn_program_run": (_i, [_vp, _vp, _vp, _i, _l, _i, _vp, _vp, _vp, _i, _vp, _pd]),
     "scn_program_output": (_i, [_vp, _i, C.POINTER(_l), C.POINTER(_i), C.POINTER(_vp)]),
     "scn_program_prepare": (_i, [_vp, _vp, _vp, _i, _l, _i]),
+    "scn_program_prepare_training": (_i, [_vp, _vp, _vp, _i, _l, _i]),
+    "scn_program_drop_prepared": (_i, [_vp]),
     "scn_program_throttle": (_i, [_vp]),
     "scn_program_set_training": (_i, [_vp, _i]),
     "scn_program_backward": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _pi, _vp]),

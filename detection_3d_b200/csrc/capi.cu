@@ -190,7 +190,8 @@ void scn_metadata_destroy(scn_metadata *m) {
 // Builds ahead, on a worker thread and the Metadata's build stream, the rulebooks / plans the caller
 // is about to request (ops: n_ops x 13 longs = kind, a[3], b[3], filter[3], stride[3]; kind 1 =
 // submanifold(a = size), 2 = convolution(a = in, b = out), 3 = deconvolution(a = in (coarse),
-// b = out (fine))).  Purely a hint: results are identical with or without it, entries are built
+// b = out (fine))), and the (in, out) rule lists a backward pass is about to request (kind 4 = those of
+// submanifold(a = size), 5 = those of convolution(a = in, b = out)).  Purely a hint: results are identical with or without it, entries are built
 // in the same lazily-filled caches (Metadata.cpp:429-510) under the same keys; a failing hint is
 // ignored and the error resurfaces when the caller requests that entry itself.
 static void prefetch_worker(scn_metadata *m, int which) {
@@ -212,6 +213,14 @@ static void prefetch_worker(scn_metadata *m, int which) {
       scn::Grid *gf = m->md.find_grid(b);
       if (scn::g_math_mode != 0 && scn::tc_available() && gf && gf->n > 0 && e->geom.M == 1 && e->rb.total == gf->n)
         if (m->md.get_deconv_plan(*e)) break;
+    } else if (op.v[0] == 4) {
+      scn::SubmEntry *e;
+      if (m->md.get_submanifold(a, f, &e) || m->md.ensure_subm_rules(*e, true)) break;
+    } else if (op.v[0] == 5) {
+      scn::ConvEntry *e = which == 1 ? m->md.wait_conv(a, f, s) : nullptr;
+      if (m->stop) break;
+      if (!e && m->md.get_conv(a, b, f, s, &e)) break;
+      if (m->md.ensure_conv_rules(*e, true)) break;
     }
   }
 }
@@ -277,9 +286,11 @@ int scn_metadata_prefetch(scn_metadata *m, int n_ops, const long *ops) {
   auto key3 = [](const long *v) { return (v[0] << 42) ^ (v[1] << 21) ^ v[2]; };
   std::vector<long> usedAsInput;
   for (int i = 0; i < n_ops; i++) usedAsInput.push_back(key3(ops + i * 13 + (ops[i * 13] == 3 ? 4 : 1)));
+  std::vector<PrefetchOp> lists; // rule lists (kinds 4, 5): after every plan, in the order given
   for (int i = 0; i < n_ops; i++) {
     PrefetchOp op;
     for (int j = 0; j < 13; j++) op.v[j] = ops[i * 13 + j];
+    if (op.v[0] >= 4) { lists.push_back(op); continue; }
     bool chain = op.v[0] == 2 && std::find(usedAsInput.begin(), usedAsInput.end(), key3(op.v + 4)) != usedAsInput.end();
     (m->md.nCtx >= 2 && !chain ? m->ops2 : m->ops).push_back(op);
   }
@@ -310,6 +321,8 @@ int scn_metadata_prefetch(scn_metadata *m, int n_ops, const long *ops) {
     if (sx != sy) return sx;
     return sx ? fine(x) > fine(y) : fine(x) < fine(y);
   });
+  std::vector<PrefetchOp> &tail = m->md.nCtx >= 2 ? m->ops2 : m->ops;
+  tail.insert(tail.end(), lists.begin(), lists.end());
   {
     std::lock_guard<std::mutex> lk(m->md.mapMu);
     for (const PrefetchOp &o : m->ops2)
@@ -758,6 +771,31 @@ int scn_deconvolution_forward(scn_metadata *m, const long inS[3], const long out
   return plain_epilogue(out, add_in, out_bf16, gf->n, Cout, s);
 }
 
+// Whether a convolution's backward entry reads the (in, out) rule lists: the CUDA-core weight-gradient kernel does; the
+// tensor-core one reads the execution plan, where the input gradient runs on the tensor cores too (or is not wanted).
+static bool reads_lists(int Cin, int Cout, int K, bool tcInOrNone) { return !(tcInOrNone && scn::dw_plan_ok(Cin, Cout, K, scn::g_math_mode)); }
+// rule lists a backward entry found built ahead by a prefetch worker (program.cu: hinted after the forward's plans)
+static void count_lists_ahead(Metadata &md, const scn::Ready &r) {
+  std::lock_guard<std::mutex> lk(md.mapMu);
+  if (r.ready && r.ahead) ++scn::g_counters[scn::kCntRulesAhead];
+}
+extern "C++" {
+namespace scn {
+// The rule lists the backward entry of a recorded convolution (kind 1 submanifold, 2 strided, 3 deconvolution) will read for a
+// non-empty level, decided from its shape as the entries below decide it from the built rulebook.  A strided convolution's
+// rulebook gives every input site exactly one parent when filter == stride; wantDIn: the input gradient is computed.
+bool backward_reads_lists(int kind, const long *f, const long *st, int Cin, int Cout, bool wantDIn) {
+  const int K = (int)(f[0] * f[1] * f[2]);
+  bool tcIn;
+  if (kind == 1) tcIn = !wantDIn || (tc_ok(Cout, Cin, K) && f[0] % 2 == 1 && f[1] % 2 == 1 && f[2] % 2 == 1);
+  else if (kind == 2) tcIn = tc_ok(Cout, Cin, 1) && f[0] == st[0] && f[1] == st[1] && f[2] == st[2];
+  else tcIn = tc_ok(Cout, Cin, K);
+  return reads_lists(Cin, Cout, K, tcIn);
+}
+cudaStream_t metadata_stream(scn_metadata *m) { return m->md.cstream; }
+} // namespace scn
+} // extern "C++"
+
 // d_in = forward tensor-core convolution of d_out with transposed weights (conv_bwd.cu header).  W: [K][Cin][Cout] of the
 // FORWARD layer; d_out rows have Cout channels (nSrcRows of them), d_in rows Cin channels (nDstRows, all written by the plan).
 static int dIn_tensor_core(Metadata &M, const float *d_out, float *d_in, const float *W, int K, int Cin, int Cout, int reverse, const int *nbr,
@@ -785,8 +823,8 @@ int scn_submanifold_convolution_backward(scn_metadata *m, const long sz[3], cons
   const bool tcIn = d_in && tc_ok(Cout, Cin, e->plan.K) && f[0] % 2 == 1 && f[1] % 2 == 1 && f[2] % 2 == 1 && g->n > 0;
   // the per-offset rule lists (reference order) are only materialised when a CUDA-core kernel needs them: both tensor-core
   // gradient kernels read the execution plan
-  const bool lists = !((tcIn || !d_in) && scn::dw_plan_ok(Cin, Cout, e->plan.K, scn::g_math_mode));
-  if (lists) SCN_TRY(m->md.ensure_subm_rules(*e));
+  const bool lists = reads_lists(Cin, Cout, e->plan.K, tcIn || !d_in);
+  if (lists) { count_lists_ahead(m->md, e->rulesRdy); SCN_TRY(m->md.ensure_subm_rules(*e)); }
   SCN_TRY(m->md.wait_ready(e->rdy));
   if (lists) SCN_TRY(m->md.wait_ready(e->rulesRdy));
   SCN_TRY(shared_dout16(m->md.cstream, d_out, g->n, Cin, Cout, &dout16));
@@ -803,8 +841,8 @@ int scn_convolution_backward(scn_metadata *m, const long inS[3], const long outS
   // d_in (fine rows) on the tensor cores: a deconvolution of d_out with W^T over the single-parent plan
   scn::Grid *gf = m->md.find_grid(inS), *gc = m->md.find_grid(outS);
   const bool tcIn = tc_ok(Cout, Cin, 1) && e->geom.M == 1 && e->rb.total == gf->n && gf->n > 0;
-  const bool lists = !(tcIn && scn::dw_plan_ok(Cin, Cout, e->plan.K, scn::g_math_mode));
-  if (lists) SCN_TRY(m->md.ensure_conv_rules(*e));
+  const bool lists = reads_lists(Cin, Cout, e->plan.K, tcIn);
+  if (lists) { count_lists_ahead(m->md, e->rulesRdy); SCN_TRY(m->md.ensure_conv_rules(*e)); }
   SCN_TRY(m->md.wait_ready(e->rdy));
   if (lists) SCN_TRY(m->md.wait_ready(e->rulesRdy));
   SCN_TRY(shared_dout16(m->md.cstream, d_out, gc->n, Cin, Cout, &dout16));
@@ -826,8 +864,8 @@ int scn_deconvolution_backward(scn_metadata *m, const long inS[3], const long ou
   // d_in (coarse rows) on the tensor cores: the strided convolution fine -> coarse of d_out with W^T
   scn::Grid *gc = m->md.find_grid(inS), *gf = m->md.find_grid(outS);
   const bool tcIn = tc_ok(Cout, Cin, e->plan.K) && gc->n > 0;
-  const bool lists = !(tcIn && scn::dw_plan_ok(Cin, Cout, e->plan.K, scn::g_math_mode));
-  if (lists) SCN_TRY(m->md.ensure_conv_rules(*e));
+  const bool lists = reads_lists(Cin, Cout, e->plan.K, tcIn);
+  if (lists) { count_lists_ahead(m->md, e->rulesRdy); SCN_TRY(m->md.ensure_conv_rules(*e)); }
   SCN_TRY(m->md.wait_ready(e->rdy));
   if (lists) SCN_TRY(m->md.wait_ready(e->rulesRdy));
   SCN_TRY(shared_dout16(m->md.cstream, d_out, gf->n, Cin, Cout, &dout16));

@@ -61,7 +61,9 @@ enum DebugCounter {
   kCntChunkedLaunch = 16,  // conv_plan_tc launches over one offset chunk of a plan with more than 64 filter offsets
   kCntCoordUpload = 17,    // host -> device copies of input-layer coordinates
   kCntF16Launch = 18,      // tensor-core launches with fp16 operands (math mode 5): conv_plan_tc and the weight-gradient kernels
-  kCntCounters = 19
+  kCntRulesAhead = 19,     // rule lists a backward entry found already built (hinted ahead by a training run, program.cu)
+  kCntTrainPrepared = 20,  // training runs that took a Metadata prepared by scn_program_prepare_training
+  kCntCounters = 21
 };
 extern std::atomic<long> g_counters[kCntCounters];
 

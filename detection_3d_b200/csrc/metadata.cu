@@ -1423,7 +1423,7 @@ int Metadata::get_submanifold(const long *sz, const long *f, SubmEntry **out) {
   return 0;
 }
 // SubmanifoldConvolution_SgToRules order (SubmanifoldConvolutionRules.h:26-45): sites in hash-iteration order
-int Metadata::ensure_subm_rules(SubmEntry &e) {
+int Metadata::ensure_subm_rules(SubmEntry &e, bool ahead) {
   if (!claim(e.rulesRdy)) return 0;
   struct Guard { Metadata &m; Ready &r; ~Guard() { if (!r.ready) m.unclaim(r); } } guard{*this, e.rulesRdy};
   BuildLock bl(*this);
@@ -1441,6 +1441,7 @@ int Metadata::ensure_subm_rules(SubmEntry &e) {
     SCN_TRY(build_rule_lists(*this, g->n, K, SubmMask{g->rank2id, g->id2p, e.plan.nbr, K, e.plan.slot}, SubmPair{g->rank2id, g->id2p, e.plan.nbr, K, e.plan.slot}, e.rb, 0));
   }
   SCN_CHECK(e.plan.nValid == e.rb.total, "internal: rule count mismatch");
+  e.rulesRdy.ahead = ahead;
   return mark_ready(e.rulesRdy);
 }
 
@@ -1940,7 +1941,7 @@ int Metadata::overlay_conv(Metadata &in, const long *inS, const long *outS, cons
 }
 
 // The (in,out) lists of a strided convolution in the reference's order (ConvolutionRules.h:11-34), written on demand.
-int Metadata::ensure_conv_rules(ConvEntry &e) {
+int Metadata::ensure_conv_rules(ConvEntry &e, bool ahead) {
   if (!claim(e.rulesRdy)) return 0;
   struct Guard { Metadata &m; Ready &r; ~Guard() { if (!r.ready) m.unclaim(r); } } guard{*this, e.rulesRdy};
   BuildLock bl(*this);
@@ -1958,6 +1959,7 @@ int Metadata::ensure_conv_rules(ConvEntry &e) {
     k_rule_write<<<cdiv(n, kRuleTile), kRuleTile, 0, LS(cur().stream)>>>(n, K, ConvMask{e.geom, gi->rank2id, gi->coords},
                                                                          ConvPair{e.geom, gi->rank2id, gi->coords, e.evQ, go->p2id}, e.tileCnt, e.rb.d_off, e.rb.pairs);
   SCN_CUDA(cudaGetLastError());
+  e.rulesRdy.ahead = ahead;
   return mark_ready(e.rulesRdy);
 }
 

@@ -21,7 +21,10 @@ typedef std::array<long, 3> P3;
 // all its kernels are queued on a build stream (`by`); `building` = some thread has claimed the build;
 // `ev` marks the end of the build on that stream: other build streams (Metadata::need) and the
 // first feature kernel that uses the object (`waited`, Metadata::wait_ready) wait for it.
-struct Ready { bool ready = false, building = false; cudaEvent_t ev = nullptr; cudaStream_t by = nullptr; bool waited = false; };
+struct Ready {
+  bool ready = false, building = false; cudaEvent_t ev = nullptr; cudaStream_t by = nullptr; bool waited = false;
+  bool ahead = false; // rule lists: built by a prefetch worker from a hint (scn_metadata_prefetch kinds 4 / 5), not on demand
+};
 struct Grid {
   Ready rdy;          // active-site structures (directory, masks, numbering)
   Ready rankRdy;      // rank2id (reference hash-iteration order)
@@ -189,10 +192,10 @@ struct Metadata {
   Grid *find_grid(const long *sz);
   int ensure_rank(Grid &g);
   int get_submanifold(const long *sz, const long *f, SubmEntry **out);
-  int ensure_subm_rules(SubmEntry &e);
+  int ensure_subm_rules(SubmEntry &e, bool ahead = false); // ahead: called by a prefetch worker (Ready::ahead)
   int get_conv(const long *inS, const long *outS, const long *f, const long *s, ConvEntry **out);
   int get_conv_small(Grid &gi, Grid &go, ConvEntry &e, const ConvGeomHost &G); // one-launch build for small input grids
-  int ensure_conv_rules(ConvEntry &e);
+  int ensure_conv_rules(ConvEntry &e, bool ahead = false);
   int spatial_locations(const long *sz, long *out, int outOnDevice);
   int build_tile_masks(NbrPlan &plan);
   int get_deconv_plan(ConvEntry &e);

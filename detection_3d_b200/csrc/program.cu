@@ -10,6 +10,8 @@
 #include <algorithm>
 #include <stdlib.h>
 #include <array>
+#include <deque>
+#include <utility>
 #include <vector>
 
 namespace scn {
@@ -27,6 +29,8 @@ void prepadded_disarm();
 int build_subm_on_caller(scn_metadata *m, const long *sz, const long *f);
 int bn_forward_from_sums(const float *x, float *y, long n, int C, const double *sums, float *saveMean, float *saveInvStd, float *runningMean,
                          float *runningVar, const float *weight, const float *bias, float eps, float momentum, int mode, float leak, cudaStream_t s, void *y16);
+bool backward_reads_lists(int kind, const long *f, const long *st, int Cin, int Cout, bool wantDIn);
+cudaStream_t metadata_stream(scn_metadata *m);
 } // namespace scn
 
 namespace {
@@ -77,6 +81,9 @@ struct scn_program {
   std::vector<float *> bnSave;  // per op: [2][C] floats (train mode), from the slot pool
   scn_metadata *lastMd = nullptr; // Metadata the layers of the last training run ran on (the backward pass needs its rulebooks): the caller's, or `ms`
   scn_metadata *lastRef = nullptr; // the caller's Metadata of that run (reference numbering: the order gradients arrive in)
+  // Training steps prepared ahead (scn_program_prepare_training), oldest first: the caller's Metadata and the internally numbered
+  // one its run will take (nullptr: the run uses the caller's Metadata itself, which was prepared instead)
+  std::deque<std::pair<scn_metadata *, scn_metadata *>> prepared;
 };
 
 static void *slot_get(scn_program *p, size_t bytes) {
@@ -97,6 +104,14 @@ static void *slot_get(scn_program *p, size_t bytes) {
 }
 static void slot_put(scn_program *p, void *ptr) {
   for (Slot &s : p->slots) if (s.p == ptr) { s.busy = false; return; }
+}
+// Forgets a prepared training step: its twin job reads the internally numbered Metadata, which goes with it, so the host waits
+// for that job first.  The job waits for nothing but build work -- except when the Metadata chunk pool has grown past its bound
+// (alloc_in): a chunk the running step still owns is then waited for on the GPU.
+static void drop_prepared(const std::pair<scn_metadata *, scn_metadata *> &e) {
+  if (!e.second) return;
+  scn_metadata_wait_jobs(e.first);
+  scn_metadata_destroy(e.second);
 }
 static void release_regs(scn_program *p, bool outputsToo) {
   if (outputsToo) {
@@ -127,6 +142,7 @@ void scn_program_destroy(scn_program *p) {
   if (p->stats) cudaFree(p->stats);
   for (cudaEvent_t e : p->evEnd) if (e) cudaEventDestroy(e);
   if (p->ms) scn_metadata_destroy(p->ms);
+  for (const auto &e : p->prepared) drop_prepared(e);
   delete p;
 }
 int scn_program_set_training(scn_program *p, int on) {
@@ -304,6 +320,51 @@ int scn_program_finish(scn_program *p, int n_regs, const int *outputs, int n_out
   return 0;
 }
 
+// Training: the (in, out) rule lists the backward pass will read (scn_*_convolution_backward), built on the plan worker after every
+// plan, in the order the backward pass requests them.  Only ops whose output reaches a program output (the backward pass skips
+// the others); the gradient of the network input is assumed not wanted.  Nothing depends on the features, so a step prepared
+// ahead (scn_program_prepare_training) has its lists ready when its backward pass starts.  Only prepared steps get them: queued
+// behind an unprepared step's own plans they cost its forward more than they save its backward (DESIGN.md section 8).
+// SCN_TRAIN_LISTS_AHEAD (developer switch, read per call: tools/train_stream_bench.py alternates it in one process): 0 = built on
+// demand only, 1 (default) = for prepared steps, 2 = for every replayed training step.
+static bool lists_ahead(bool prepared) {
+  const char *env = getenv("SCN_TRAIN_LISTS_AHEAD");
+  const int mode = env ? atoi(env) : 1;
+  return mode >= 2 || (mode == 1 && prepared);
+}
+static void rule_list_hints(const scn_program *p, std::vector<long> &hints) {
+  std::vector<char> live(p->nRegs, 0);
+  for (int r = 0; r < p->nRegs; r++) live[r] = p->isOutput[r];
+  for (int i = (int)p->ops.size() - 1; i >= 0; i--) {
+    const Op &o = p->ops[i];
+    if (o.kind == K_INPUT) continue;
+    if (o.kind == K_ADD) { if (live[o.a[2]]) live[o.a[0]] = live[o.a[1]] = 1; continue; }
+    if (!live[o.a[1]]) continue;
+    live[o.a[0]] = 1;
+    if (o.kind == K_BN) continue;
+    if (o.a[22] >= 0) live[o.a[22]] = 1;
+    if (o.a[18] >= 0) live[o.a[18]] = 1;
+    bool fromInput = false;
+    for (const Op &q : p->ops) if (q.kind == K_INPUT && q.a[0] == o.a[0]) fromInput = true;
+    const long *f = o.kind == K_SUBM ? o.a + 5 : o.a + 8, *st = o.kind == K_SUBM ? o.a + 5 : o.a + 11;
+    const int Cin = (int)(o.kind == K_SUBM ? o.a[10] : o.a[16]), Cout = (int)(o.kind == K_SUBM ? o.a[11] : o.a[17]);
+    if (!scn::backward_reads_lists(o.kind, f, st, Cin, Cout, !(fromInput && o.kind == K_SUBM))) continue;
+    long h[13] = {0};
+    if (o.kind == K_SUBM) { h[0] = 4; for (int d = 0; d < 3; d++) { h[1 + d] = o.a[2 + d]; h[7 + d] = o.a[5 + d]; } }
+    else { // the deconvolution's backward reads the lists of the convolution fine -> coarse
+      h[0] = 5;
+      for (int d = 0; d < 3; d++) {
+        h[1 + d] = o.kind == K_CONV ? o.a[2 + d] : o.a[5 + d];
+        h[4 + d] = o.kind == K_CONV ? o.a[5 + d] : o.a[2 + d];
+        h[7 + d] = o.a[8 + d];
+        h[10 + d] = o.a[11 + d];
+      }
+    }
+    bool seen = false; // (layers of one level share a rulebook)
+    for (size_t j = 0; j < hints.size() && !seen; j += 13) seen = std::equal(h, h + 13, hints.begin() + j);
+    if (!seen) hints.insert(hints.end(), h, h + 13);
+  }
+}
 // The build half of a run: input layer (active sites of the finest grid) and, on the worker threads, every rulebook /
 // plan the program will request.  scn_program_run calls it when the Metadata comes unprepared; a caller that streams
 // buildings through the network calls it for building i+1 right after it has queued building i
@@ -318,7 +379,8 @@ int scn_program_throttle(scn_program *p) {
   if (p->nRuns >= 2 && p->evEnd[p->nRuns & 1]) SCN_CUDA(cudaEventSynchronize(p->evEnd[p->nRuns & 1]));
   return 0;
 }
-int scn_program_prepare(scn_program *p, scn_metadata *m, const long *coords, int coords_on_device, long nrows, int ncols) {
+// prepared: a training step prepared ahead (scn_program_prepare_training), which also gets the rule lists of its backward pass
+static int prepare_build(scn_program *p, scn_metadata *m, const long *coords, int coords_on_device, long nrows, int ncols, bool prepared) {
   SCN_CHECK(p && m && p->nRegs > 0, "program not finished");
   SCN_TRY(scn_program_throttle(p));
   for (const Op &op : p->ops) {
@@ -335,11 +397,101 @@ int scn_program_prepare(scn_program *p, scn_metadata *m, const long *coords, int
       else continue;
       hints.insert(hints.end(), h, h + 13);
     }
+    if (p->train && lists_ahead(prepared)) rule_list_hints(p, hints);
     if (!hints.empty()) SCN_TRY(scn_metadata_prefetch(m, (int)(hints.size() / 13), hints.data()));
     return 0;
   }
   scn::set_error("program has no input layer");
   return -2;
+}
+int scn_program_prepare(scn_program *p, scn_metadata *m, const long *coords, int coords_on_device, long nrows, int ncols) {
+  return prepare_build(p, m, coords, coords_on_device, nrows, ncols, false);
+}
+
+static const Op *input_op(const scn_program *p) {
+  for (const Op &o : p->ops) if (o.kind == K_INPUT) return &o;
+  return nullptr;
+}
+// Whether a run on an unprepared Metadata numbers its rows internally (see scn_program_run).  Training runs do too, so that every
+// gather of the forward AND backward pass stays local; SCN_TRAIN_INTERNAL=0 keeps them on the caller's Metadata.
+static bool uses_internal_numbering(const scn_program *p, const Op *inOp) {
+  static const int internalOn = getenv("SCN_INTERNAL_IDS") ? atoi(getenv("SCN_INTERNAL_IDS")) : 1;
+  static const int trainInternal = getenv("SCN_TRAIN_INTERNAL") ? atoi(getenv("SCN_TRAIN_INTERNAL")) : 1;
+  return (!p->train || trainInternal) && internalOn && inOp && inOp->a[4] != 0;
+}
+// The internally numbered Metadata of a run on `m` (see scn_program_run): input layer and plan hints (prepare_build), and
+// the reference-numbered twin started on `m`.  *out = nullptr when the input has several batch items: `m` then does everything.
+static int start_internal(scn_program *p, scn_metadata *m, const Op *inOp, const long *coords, int coords_on_device, long nrows, int ncols,
+                          void *stream, bool prepared, scn_metadata **out) {
+  scn_metadata *ms = nullptr;
+  SCN_TRY(scn_metadata_create(&ms, stream));
+  int rc = scn_metadata_set_internal_numbering(ms, 1);
+  if (rc == 0) rc = prepare_build(p, ms, coords, coords_on_device, nrows, ncols, prepared);
+  int batch = 0;
+  if (rc == 0) rc = scn_get_batch_size(ms, inOp->a + 1, &batch);
+  if (rc || batch != 1) { // several batch items: the caller's Metadata does everything (reference numbering throughout)
+    scn_metadata_destroy(ms);
+    *out = nullptr;
+    return rc;
+  }
+  // the strided convolutions whose output grid an output register lives on, or that lead there
+  std::vector<std::array<long, 3>> need;
+  for (int r = 0; r < p->nRegs; r++) if (p->isOutput[r]) need.push_back(p->outSize[r]);
+  std::vector<long> hints;
+  for (bool grew = true; grew;) {
+    grew = false;
+    for (const Op &o : p->ops) {
+      if (o.kind != K_CONV) continue;
+      const std::array<long, 3> in{o.a[2], o.a[3], o.a[4]}, out{o.a[5], o.a[6], o.a[7]};
+      if (std::find(need.begin(), need.end(), out) != need.end() && std::find(need.begin(), need.end(), in) == need.end()) { need.push_back(in); grew = true; }
+    }
+  }
+  for (const Op &o : p->ops) {
+    if (o.kind != K_CONV) continue;
+    const std::array<long, 3> out{o.a[5], o.a[6], o.a[7]};
+    if (std::find(need.begin(), need.end(), out) == need.end()) continue;
+    long h[13] = {0};
+    h[0] = 2;
+    for (int d = 0; d < 12; d++) h[1 + d] = o.a[2 + d];
+    hints.insert(hints.end(), h, h + 13);
+  }
+  static const bool skipTwin = getenv("SCN_SKIP_TWIN") && atoi(getenv("SCN_SKIP_TWIN")); // developer timing experiment only: outputs stay in internal row order
+  if (!skipTwin) rc = scn_metadata_build_reference_grids(m, ms, inOp->a + 1, (int)(hints.size() / 13), hints.data());
+  if (rc) { scn_metadata_destroy(ms); ms = nullptr; }
+  *out = ms;
+  return rc;
+}
+
+// Training step i+1 prepared while step i still runs: what scn_program_run does before the first layer of an unprepared training
+// step (the internally numbered Metadata with its input layer and plan hints, the reference-numbered twin on `m`), or -- where
+// that step runs on `m` itself (several batch items, SCN_TRAIN_INTERNAL=0, input modes the internal numbering does not cover) --
+// scn_program_prepare on `m`; either way with the rule lists of its backward pass.  Nothing here waits for the GPU work queued
+// before: the builds run on the Metadata's build streams.  At most two steps are kept; a third drops the oldest (its `m` is then
+// an ordinary reference-numbered Metadata, see drop_prepared).
+int scn_program_prepare_training(scn_program *p, scn_metadata *m, const long *coords, int coords_on_device, long nrows, int ncols) {
+  SCN_CHECK(p && m && p->nRegs > 0 && p->train, "scn_program_prepare_training needs a finished program in training mode");
+  for (const auto &e : p->prepared) SCN_CHECK(e.first != m, "scn_program_prepare_training: this Metadata is prepared already");
+  // (an empty Metadata is never one a pending backward pass reads: a run leaves its input layer built; the internal one is new)
+  SCN_CHECK(!scn_input_layer_built(m, nullptr, nullptr), "scn_program_prepare_training needs an empty Metadata");
+  const Op *inOp = input_op(p);
+  SCN_CHECK(inOp, "program has no input layer");
+  scn_metadata *ms = nullptr;
+  if (uses_internal_numbering(p, inOp))
+    SCN_TRY(start_internal(p, m, inOp, coords, coords_on_device, nrows, ncols, scn::metadata_stream(m), true, &ms));
+  if (!ms) SCN_TRY(prepare_build(p, m, coords, coords_on_device, nrows, ncols, true));
+  if (p->prepared.size() == 2) {
+    drop_prepared(p->prepared.front());
+    p->prepared.pop_front();
+  }
+  p->prepared.emplace_back(m, ms);
+  return 0;
+}
+
+int scn_program_drop_prepared(scn_program *p) {
+  SCN_CHECK(p, "null program");
+  for (const auto &e : p->prepared) drop_prepared(e);
+  p->prepared.clear();
+  return 0;
 }
 
 // params[i] / tags[i]: device pointers of the recorded parameter tensors (and their content tags, see
@@ -360,58 +512,31 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
   // block structure of the internal grids, scn_metadata_build_reference_grids) and the output rows are handed out in that
   // numbering (scn_program_output_copy).  The layers' rulebooks on `m` are built on first use.  A Metadata prepared ahead
   // (scn_program_prepare) or an input mode / batch the internal numbering does not cover uses `m` for everything, as before.
-  static int internalOn = -1;
-  if (internalOn < 0) internalOn = getenv("SCN_INTERNAL_IDS") ? atoi(getenv("SCN_INTERNAL_IDS")) : 1;
+  // A training step prepared ahead (scn_program_prepare_training) takes the pair built then.
   if (p->ms) { scn_metadata_destroy(p->ms); p->ms = nullptr; }
   p->internal = false;
-  const bool preparedAhead = scn_input_layer_built(m, nullptr, nullptr) != 0; // scn_program_prepare ran for `m` (streaming): its workers build everything
-  scn_metadata *M = m;
-  const Op *inOp = nullptr;
-  for (const Op &o : p->ops) if (o.kind == K_INPUT) { inOp = &o; break; }
+  const Op *inOp = input_op(p);
   const bool train = p->train;
+  bool preparedTrain = false;
+  for (auto it = p->prepared.begin(); train && it != p->prepared.end(); ++it)
+    if (it->first == m) {
+      p->ms = it->second;
+      p->prepared.erase(it);
+      preparedTrain = true;
+      ++scn::g_counters[scn::kCntTrainPrepared];
+      break;
+    }
+  // (a prepared pair's `m` is still being numbered by its twin job: its input layer is not read here)
+  const bool preparedAhead = preparedTrain || scn_input_layer_built(m, nullptr, nullptr) != 0; // its workers build everything
+  scn_metadata *M = m;
   p->lastMd = train ? m : nullptr;
   p->lastRef = train ? m : nullptr;
   if (train) p->bnSave.assign(p->ops.size(), nullptr);
-  static int trainInternal = -1; // training runs on the internally numbered Metadata too (rows in spatial order: every gather of the
-  if (trainInternal < 0) trainInternal = getenv("SCN_TRAIN_INTERNAL") ? atoi(getenv("SCN_TRAIN_INTERNAL")) : 1; // forward AND backward pass stays local)
-  if ((!train || trainInternal) && internalOn && inOp && inOp->a[4] != 0 && !scn_input_layer_built(m, nullptr, nullptr)) {
-    SCN_TRY(scn_metadata_create(&p->ms, stream));
-    SCN_TRY(scn_metadata_set_internal_numbering(p->ms, 1));
-    SCN_TRY(scn_program_prepare(p, p->ms, coords, coords_on_device, nrows, ncols));
-    int batch = 0;
-    SCN_TRY(scn_get_batch_size(p->ms, inOp->a + 1, &batch));
-    // the strided convolutions whose output grid an output register lives on, or that lead there
-    std::vector<std::array<long, 3>> need;
-    for (int r = 0; r < p->nRegs; r++) if (p->isOutput[r]) need.push_back(p->outSize[r]);
-    std::vector<long> hints;
-    for (bool grew = true; grew;) {
-      grew = false;
-      for (const Op &o : p->ops) {
-        if (o.kind != K_CONV) continue;
-        const std::array<long, 3> in{o.a[2], o.a[3], o.a[4]}, out{o.a[5], o.a[6], o.a[7]};
-        if (std::find(need.begin(), need.end(), out) != need.end() && std::find(need.begin(), need.end(), in) == need.end()) { need.push_back(in); grew = true; }
-      }
-    }
-    for (const Op &o : p->ops) {
-      if (o.kind != K_CONV) continue;
-      const std::array<long, 3> out{o.a[5], o.a[6], o.a[7]};
-      if (std::find(need.begin(), need.end(), out) == need.end()) continue;
-      long h[13] = {0};
-      h[0] = 2;
-      for (int d = 0; d < 12; d++) h[1 + d] = o.a[2 + d];
-      hints.insert(hints.end(), h, h + 13);
-    }
-    static const bool skipTwin = getenv("SCN_SKIP_TWIN") && atoi(getenv("SCN_SKIP_TWIN")); // developer timing experiment only: outputs stay in internal row order
-    if (batch == 1 && !skipTwin)
-    SCN_TRY(scn_metadata_build_reference_grids(m, p->ms, inOp->a + 1, (int)(hints.size() / 13), hints.data()));
-    if (batch == 1) {
-      M = p->ms;
-      p->internal = true;
-      if (train) p->lastMd = p->ms;
-    } else { // several batch items: the caller's Metadata does everything (reference numbering throughout)
-      scn_metadata_destroy(p->ms);
-      p->ms = nullptr;
-    }
+  if (!preparedAhead && uses_internal_numbering(p, inOp)) SCN_TRY(start_internal(p, m, inOp, coords, coords_on_device, nrows, ncols, stream, false, &p->ms));
+  if (p->ms) {
+    M = p->ms;
+    p->internal = true;
+    if (train) p->lastMd = p->ms;
   }
   if (!p->bnScratch) SCN_CUDA(cudaMalloc((void **)&p->bnScratch, 2 * scn::kBnMaxC * sizeof(float)));
   auto P = [&](long i) -> const float * { return (i < 0 || i >= n_params) ? nullptr : static_cast<const float *>(params[i]); };

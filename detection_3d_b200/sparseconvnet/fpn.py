@@ -147,7 +147,7 @@ class FPN_Net(nn.Module):
             mode = native.math_mode()
             prog = self.__dict__.get("_program_train")
             if prog is not None and prog.usable(coords, feats, mode):
-                md = L.Metadata(self.dimension)
+                md = self._take_prefetched("_prefetched_train", coords) or L.Metadata(self.dimension)
                 import detection_3d_b200.sparseconvnet as pkg
                 uniq = program.TrainFunction.apply(prog, md, coords, feats, *prog.params)
                 pkg.forward_pass_multiplyAdd_count += prog.last_macs
@@ -169,15 +169,33 @@ class FPN_Net(nn.Module):
     def _has_prefetched(self, coords):
         return any(pre[0] is coords and pre[1] == coords._version for pre in self.__dict__.get("_prefetched", ()))
 
+    def _take_prefetched(self, queue, coords):
+        """The Metadata of the oldest entry of `queue` made for this very coordinate tensor, unmodified since (or None)."""
+        q = self.__dict__.get(queue)
+        for i, pre in enumerate(q or ()):
+            if pre[0] is coords and pre[1] == coords._version:
+                del q[i]
+                return pre[2]
+        return None
+
     def prefetch(self, coords):
-        """Streaming inference: start building the Metadata (active-site grids, rulebooks) of the NEXT input now, on the
-        library's build streams, while the GPU still computes the forwards queued before.  May be called for several inputs
-        (first in, first out); a `forward` whose coordinate tensor is one of these objects uses its Metadata, any other
-        input simply ignores them.  Calling it TWO buildings ahead hides the whole build behind the computation.  Results are identical with or
-        without the call.  Device coordinates must be complete (not still being written by another stream).
-        No-op until a program has been recorded (i.e. before the second inference forward)."""
-        prog = self.__dict__.get("_program")
-        if prog is None or self.training or not isinstance(coords, torch.Tensor) or coords.dtype != torch.int64 or coords.dim() != 2:
+        """Start building the Metadata (active-site grids, rulebooks) of the NEXT input now, on the library's build streams,
+        while the GPU still computes the work queued before.  A `forward` whose coordinate tensor is this very object, unmodified
+        since, uses that Metadata; any other input ignores it.  Results are identical with or without the call.  Device
+        coordinates must be complete (not still being written by another stream).  Returns False (and does nothing) until a
+        program has been recorded in the current mode -- the second inference forward, the second training step -- or when the
+        math mode has changed since.
+
+        Inference (eval mode): may be called for several inputs (first in, first out); calling it TWO buildings ahead hides the
+        whole build behind the computation.
+
+        Training (train mode): prepares the next training step (scn_program_prepare_training): its grids, plans and the rule lists
+        its backward pass reads are built while the current step runs.  Call it with the next batch's coordinates before the
+        current step's forward or backward; at most two steps stay prepared.  Inference and training entries are kept apart:
+        neither is used by the other mode, and switching to eval drops the training entries."""
+        key = "_program_train" if self.training else "_program"
+        prog = self.__dict__.get(key)
+        if prog is None or not isinstance(coords, torch.Tensor) or coords.dtype != torch.int64 or coords.dim() != 2:
             return False
         if native.math_mode() != prog.math_mode:
             return False
@@ -185,25 +203,36 @@ class FPN_Net(nn.Module):
         native.lib().scn_set_pool_growth(1)  # built ahead: do not queue behind a running forward for memory
         try:
             md = L.Metadata(self.dimension)
-            prog.prepare(md, coords)
+            if self.training:
+                prog.prepare_training(md, coords)
+            else:
+                prog.prepare(md, coords)
         finally:
             native.lib().scn_set_pool_growth(0)
-        q = self.__dict__.setdefault("_prefetched", [])
+        q = self.__dict__.setdefault("_prefetched_train" if self.training else "_prefetched", [])
         q.append((coords, coords._version, md))
-        del q[:-4]  # at most a few buildings ahead
+        del q[:-2 if self.training else -4]  # at most a few buildings ahead (training: as many as the program keeps prepared)
         return True
+
+    def train(self, mode=True):
+        if not mode:  # evaluation: the training steps prepared ahead are dropped and release their memory
+            self.__dict__.pop("_prefetched_train", None)
+            if self.__dict__.get("_program_train") is not None:
+                self.__dict__["_program_train"].drop_prepared()
+        return nn.Module.train(self, mode)
 
     def reset_program(self):
         """Forget the recorded program (call after changing the module tree)."""
         self.__dict__.pop("_program", None)
         self.__dict__.pop("_program_error", None)
         self.__dict__.pop("_prefetched", None)
-        for k in ("_program_train", "_program_train_error", "_program_train_n_rpn"):
+        for k in ("_program_train", "_program_train_error", "_program_train_n_rpn", "_prefetched_train"):
             self.__dict__.pop(k, None)
 
     # The recorded program and the Metadata objects built ahead are handles into the native library (ctypes pointers):
     # a copy / pickle of the network (EMA copies, torch.save(model), as with the reference) drops them and records again.
-    _RUNTIME_STATE = ("_program", "_program_error", "_program_n_rpn", "_prefetched", "_program_train", "_program_train_error", "_program_train_n_rpn")
+    _RUNTIME_STATE = ("_program", "_program_error", "_program_n_rpn", "_prefetched", "_program_train", "_program_train_error", "_program_train_n_rpn",
+                      "_prefetched_train")
 
     def __getstate__(self):
         state = self.__dict__.copy()
@@ -230,16 +259,7 @@ class FPN_Net(nn.Module):
 
     def _run_program(self, prog, coords, feats):
         import detection_3d_b200.sparseconvnet as pkg
-        md = None
-        q = self.__dict__.get("_prefetched")
-        if q:  # built ahead by prefetch(): the oldest entry made for this very tensor
-            for i, pre in enumerate(q):
-                if pre[0] is coords and pre[1] == coords._version:
-                    md = pre[2]
-                    del q[i]
-                    break
-        if md is None:
-            md = L.Metadata(self.dimension)
+        md = self._take_prefetched("_prefetched", coords) or L.Metadata(self.dimension)  # built ahead by prefetch()
         outs, macs = prog.run(md, coords, feats)
         pkg.forward_pass_multiplyAdd_count += macs
         maps = [SparseConvNetTensor(features=f, metadata=md, spatial_size=s.clone()) for f, s in zip(outs, prog.out_sizes)]

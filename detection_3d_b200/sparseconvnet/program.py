@@ -128,6 +128,7 @@ class Program(object):
         uniq = sorted(set(self.out_regs))
         check(lib().scn_program_finish(self._h, len(trace.regs), (C.c_int * len(uniq))(*uniq), len(uniq)))
         self.n_ops = len(trace.ops)
+        self._prepared = []  # Metadata of training steps prepared ahead: the native program reads them until they run or are dropped
         if self.training:
             check(lib().scn_program_set_training(self._h, 1))
 
@@ -157,9 +158,25 @@ class Program(object):
         metadata._keep.append(coords)
         check(lib().scn_program_prepare(self._h, metadata._h, C.c_void_p(coords.data_ptr()), 2 if coords.is_cuda else 0, coords.size(0), coords.size(1)))
 
+    def prepare_training(self, metadata, coords):
+        """Training program: build ahead, for a later training step on `metadata`, what that step would build before its first
+        layer (scn_program_prepare_training).  At most two steps stay prepared; a third drops the oldest."""
+        coords = coords.contiguous()
+        metadata._keep.append(coords)
+        check(lib().scn_program_prepare_training(self._h, metadata._h, C.c_void_p(coords.data_ptr()), 2 if coords.is_cuda else 0,
+                                                 coords.size(0), coords.size(1)))
+        self._prepared.append(metadata)
+        del self._prepared[:-2]
+
+    def drop_prepared(self):
+        """Forget every training step prepared ahead (scn_program_drop_prepared): their memory is released."""
+        check(lib().scn_program_drop_prepared(self._h))
+        self._prepared = []
+
     def run(self, metadata, coords, feats):
         """-> (list of output feature tensors, multiply-add count)."""
         from . import native
+        self._prepared = [m for m in self._prepared if m is not metadata]  # (the run takes it out of the native program's list)
         coords = coords.contiguous()
         feats = feats.contiguous()
         metadata._keep.append(coords)

@@ -73,7 +73,9 @@ int scn_submanifold_prepare(scn_metadata *m, const long spatial_size[3], const l
  * calling thread, Metadata.cpp:429-510): build these rulebooks ahead on a worker thread + the build
  * stream while the caller keeps submitting feature kernels.  ops = n_ops x 13 longs: kind (1 submanifold,
  * 2 convolution, 3 deconvolution), a[3], b[3], filter[3], stride[3] with (a, b) = (size, -) / (in, out) /
- * (in, out) exactly as the corresponding *_forward call receives them.  Results are unaffected. */
+ * (in, out) exactly as the corresponding *_forward call receives them.  Kinds 4 (submanifold, a = size) and
+ * 5 (convolution, a = in, b = out) build the (in, out) rule lists a backward entry reads, after every
+ * rulebook of kinds 1-3, in the order given.  Results are unaffected. */
 int scn_metadata_prefetch(scn_metadata *m, int n_ops, const long *ops);
 /* Metadata::getRuleBook (Metadata.cpp:484-510): builds (once) the strided rulebook AND the output
  * grid; reports the output grid's active count and the number of rules. */
@@ -225,6 +227,20 @@ int scn_rows_from_reference_order(scn_metadata *ref, scn_metadata *internal, con
  * program requests.  coords_on_device: 0 host, 1 device (ordered after the caller's stream), 2 device and complete.
  * scn_program_run on a Metadata prepared this way skips its own build. */
 int scn_program_prepare(scn_program *p, scn_metadata *m, const long *coords, int coords_on_device, long nrows, int ncols);
+/* Training step i+1 prepared while step i still runs (program in training mode): builds ahead what scn_program_run would build
+ * before the first layer of a training step on the empty Metadata m -- the internally numbered Metadata with its input layer and
+ * plan hints, and the reference-numbered twin on m -- or, where that step runs on m itself (several batch items,
+ * SCN_TRAIN_INTERNAL=0, input modes 0), scn_program_prepare on m.  The rule lists the backward pass will read are hinted after the
+ * plans (scn_metadata_prefetch kinds 4 / 5; an unprepared step builds them on demand).  Does not wait for the GPU work queued before
+ * (call scn_program_throttle and scn_set_pool_growth(1) around creating m, as for scn_program_prepare).  The program keeps at most two
+ * prepared steps: a third drops the oldest, whose m then remains an ordinary Metadata; dropping waits on the host for that step's
+ * reference numbering to finish, which waits on the GPU only when the Metadata memory pool has grown past its bound.  A
+ * scn_program_run of this program on m computes exactly what it computes on an unprepared Metadata.  m must stay alive until that
+ * run, until it is dropped, or until the program is destroyed. */
+int scn_program_prepare_training(scn_program *p, scn_metadata *m, const long *coords, int coords_on_device, long nrows, int ncols);
+/* Drops every step prepared by scn_program_prepare_training (with its internally numbered Metadata); their Metadata m remain ordinary
+ * Metadata.  For a caller that stops training for a while (evaluation), so that the prepared steps do not hold their memory. */
+int scn_program_drop_prepared(scn_program *p);
 /* Blocks until at most one forward of this program is still running on the GPU (call before scn_metadata_create of the
  * Metadata to prepare: it then reuses the memory of the forward that just finished). */
 int scn_program_throttle(scn_program *p);
@@ -335,7 +351,9 @@ long scn_kernel_launch_count(void);
  * weight-gradient kernel took from its caller (forward shadow / shared d_out copy) instead of converting again, 13 = weight-gradient
  * launches driven by the output-stationary plan, 14 = float-atomic launches: launches whose float result depends on the order in
  * which atomics land (0 in deterministic mode except for scn_roi_align_rotated_3d_backward), 17 = host -> device copies of
- * input-layer coordinates, 18 = tensor-core launches with fp16 operands (convolutions and weight gradients, math mode 5). */
+ * input-layer coordinates, 18 = tensor-core launches with fp16 operands (convolutions and weight gradients, math mode 5), 19 = rule
+ * lists a convolution's backward entry found already built (hinted ahead by a training run), 20 = training runs that took a Metadata
+ * prepared by scn_program_prepare_training. */
 long scn_debug_counter(int which);
 /* Hands the library's idle device memory back to the driver: Metadata chunks not owned by a live Metadata, cached weight operand
  * images, per-stream scratch buffers (the library recycles these itself instead of returning them; torch.cuda.empty_cache() cannot
