@@ -1,6 +1,7 @@
 // extern "C" boundary (include/scn_b200.h).  No torch types: raw device pointers, sizes, a stream.
 #include "../../include/scn_b200.h"
 #include "metadata.cuh"
+#include "conv.cuh"
 #include <algorithm>
 #include <atomic>
 #include <mutex>
@@ -15,10 +16,6 @@
 namespace scn {
 std::atomic<long> g_launches{0};
 std::atomic<long> g_counters[kCntCounters];
-void epilogue_stats_arm(double *sums);
-bool epilogue_stats_take();
-void lateral_arm(const float *in, const void *in16, const float *w, long long tag, int Cin, long rows);
-bool lateral_take();
 namespace {
 struct TlEv { const char *who; int kind; long a, b; double t; };
 std::vector<TlEv> g_tl;
@@ -45,41 +42,6 @@ void timeline_dump() {
   for (const TlEv &e : g_tl) fprintf(stderr, "[tl] %8.1f us %-8s kind %d  %ld %ld\n", e.t - t0, e.who, e.kind, e.a, e.b);
   g_tl.clear();
 }
-const char *last_error();
-void set_prefetch_worker_thread(bool on, int ctx);
-int launch_conv_plan_simt(const float *in, float *out, const float *W, const int *nbr, const int *outRow, int nOut, int K, int Cin, int Cout,
-                          const float *bias, cudaStream_t s);
-int launch_conv_list_simt(const float *in, float *out, const float *W, const int2 *pairs, const int *d_off, const int *offHost, int K, int Cin,
-                          int Cout, int srcIsY, int singlePass, cudaStream_t s);
-int bn_forward(const float *x, float *y, long n, int C, float *saveMean, float *saveInvStd, float *runningMean, float *runningVar,
-               const float *weight, const float *bias, float eps, float momentum, int mode, float leak, void *workspace, cudaStream_t s, void *y16);
-int bn_backward(const float *x, float *dx, const float *y, float *dy, long n, int C, const float *saveMean, const float *saveInvStd,
-                const float *weight, float *dWeight, float *dBias, float leak, void *workspace, cudaStream_t s, const void *y16 = nullptr);
-int input_forward(const float *in, float *out, int nOut, int maxActive, int C, const int *tab, int average, cudaStream_t s);
-int input_forward_pad16(const float *in, float *out, void *out16, int nOut, int maxActive, int C, int Cp, const int *tab, int average, cudaStream_t s);
-int input_backward(float *din, const float *dout, long nIn, int nOut, int maxActive, int C, const int *tab, int average, cudaStream_t s);
-int add_rows(const float *a, const float *b, float *o, long n, cudaStream_t s, void *o16);
-int conv_backward_simt(const float *in, float *d_in, const float *d_out, const float *W, float *dW, float *d_bias, const int2 *pairs,
-                       const int *d_off, const int *offHost, int K, long nInRows, long nOutRows, int Cin, int Cout, int srcIsY, cudaStream_t s, int skipDIn = 0, int mathMode = 0,
-                       const void *in16 = nullptr, const void *dout16 = nullptr, const int *planNbr = nullptr, const int *planOutRow = nullptr,
-                       const unsigned long long *planMask = nullptr, int planPos = 0);
-int dout16_copy(const float *d_out, long n, cudaStream_t s, const void **out);
-bool dw_plan_ok(int Cin, int Cout, int K, int mathMode);
-void bwd_in16_arm(const void *in16);
-const void *bwd_in16_take();
-int transpose_weights(const float *W, float *Wt, int K, int Cin, int Cout, int reverse, cudaStream_t s);
-int tc_available();
-void set_pool_growth(int on);
-long debug_chunk_mallocs();
-long debug_chunk_waits();
-long debug_chunk_total_mb();
-long release_idle_chunks();
-long release_conv_caches();
-int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
-                        int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, const int *tileW, int nWeights,
-                        long nInRows, const void *in16, long long wTag, const float *addend, void *out16, long nOutRows, int CinW = 0, int wT = 0);
-int to_16(const float *x, void *y, long n, cudaStream_t s);
-int dense_rows_dw(const float *in, const float *d_out, float *dW, float *d_bias, long n, int Cin, int Cout, cudaStream_t s);
 static int g_math_mode = 0;
 int math_mode() { return g_math_mode; }
 static std::atomic<int> g_deterministic{0};
@@ -105,7 +67,6 @@ struct scn_metadata {
 using scn::Metadata;
 namespace scn {
 Metadata *metadata_of(scn_metadata *m) { return &m->md; }
-int build_subm_on_caller(Metadata &md, const long *sz, const long *f);
 int build_subm_on_caller(scn_metadata *m, const long *sz, const long *f) { return m ? build_subm_on_caller(m->md, sz, f) : -3; }
 } // for the translation units that only see the opaque handle
 
@@ -115,6 +76,18 @@ int build_subm_on_caller(scn_metadata *m, const long *sz, const long *f) { retur
     return -3;                                     \
   }
 
+// The fusion request of scn_fuse_next_lateral / scn_fuse_next_stats: pending until the next of the three convolution forward entries
+// takes it, and the result of the last such call for scn_fuse_result.
+namespace {
+struct AbiFusion { scn::ConvFusion pending; scn::ConvFused result; };
+thread_local AbiFusion tl_fusion;
+// taken by a forward entry when it is entered, whether or not the call can honour it
+scn::ConvFusion take_fusion_request() {
+  const scn::ConvFusion f = tl_fusion.pending;
+  tl_fusion = AbiFusion();
+  return f;
+}
+} // namespace
 
 extern "C" {
 
@@ -133,18 +106,20 @@ long scn_release_cached_memory(void) {
 }
 int scn_fuse_next_lateral(const float *lat_in, const void *lat_in_bf16, const float *lat_weight, long long weight_tag, int n_in, long rows) {
   SCN_CHECK(lat_in && lat_weight && n_in > 0 && rows >= 0, "lateral request");
-  scn::lateral_arm(lat_in, lat_in_bf16, lat_weight, weight_tag, n_in, rows);
+  tl_fusion.pending.lat = scn::Lateral{lat_in, lat_in_bf16, lat_weight, weight_tag, n_in, rows};
+  tl_fusion.result.lateral = false;
   return 0;
 }
 int scn_fuse_next_stats(double *sums) {
   SCN_CHECK(sums, "statistics buffer");
-  scn::epilogue_stats_arm(sums);
+  tl_fusion.pending.stats = sums;
+  tl_fusion.result.stats = false;
   return 0;
 }
 int scn_fuse_result(int *lateral_taken, int *stats_taken) {
-  const bool l = scn::lateral_take(), st = scn::epilogue_stats_take();
-  if (lateral_taken) *lateral_taken = l ? 1 : 0;
-  if (stats_taken) *stats_taken = st ? 1 : 0;
+  if (lateral_taken) *lateral_taken = tl_fusion.result.lateral ? 1 : 0;
+  if (stats_taken) *stats_taken = tl_fusion.result.stats ? 1 : 0;
+  tl_fusion = AbiFusion();
   return 0;
 }
 int scn_set_math_mode(int mode) {
@@ -709,68 +684,9 @@ static int plain_epilogue(float *out, const float *addend, void *out16, long row
   if (out16) return scn::to_16(out, out16, rows * C, s);
   return 0;
 }
-static int run_plan(Metadata &M, const scn::NbrPlan &plan, const float *in, float *out, const float *w, const float *bias, int Cin, int Cout,
-                    long nInRows, const void *in16, long long wTag, const float *addend, void *out16) {
-  if (tc_ok(Cin, Cout, plan.K))
-    return scn::launch_conv_plan_tc(in, out, w, plan.nbr, plan.outRow, plan.tileMask, plan.nOut, plan.K, Cin, Cout, bias, scn::g_math_mode, M.cstream,
-                                    nullptr, plan.K, nInRows, in16, wTag, addend, out16, plan.nOut);
-  SCN_CHECK(in && out, "CUDA-core path needs the fp32 rows");
-  SCN_TRY(scn::launch_conv_plan_simt(in, out, w, plan.nbr, plan.outRow, plan.nOut, plan.K, Cin, Cout, bias, M.cstream));
-  return plain_epilogue(out, addend, out16, plan.nOut, Cout, M.cstream);
-}
-
-int scn_submanifold_convolution_forward(scn_metadata *m, const long sz[3], const long f[3], const float *in, float *out, const float *w,
-                                        const float *bias, int Cin, int Cout, double *macs, const void *in_bf16, long long weight_tag,
-                                        const float *add_in, void *out_bf16) {
-  M_OR_FAIL(m);
-  scn::SubmEntry *e;
-  SCN_TRY(m->md.get_submanifold(sz, f, &e));
-  if (macs) *macs = (double)e->rb.total * Cin * Cout;
-  SCN_TRY(m->md.wait_ready(e->rdy));
-  return run_plan(m->md, e->plan, in, out, w, bias, Cin, Cout, m->md.find_grid(sz)->n, in_bf16, weight_tag, add_in, out_bf16);
-}
-int scn_convolution_forward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in,
-                            float *out, const float *w, const float *bias, int Cin, int Cout, double *macs, const void *in_bf16, long long weight_tag,
-                              const float *add_in, void *out_bf16) {
-  M_OR_FAIL(m);
-  scn::ConvEntry *e;
-  SCN_TRY(m->md.get_conv(inS, outS, f, st, &e));
-  if (macs) *macs = (double)e->rb.total * Cin * Cout;
-  SCN_TRY(m->md.wait_ready(e->rdy));
-  return run_plan(m->md, e->plan, in, out, w, bias, Cin, Cout, m->md.find_grid(inS)->n, in_bf16, weight_tag, add_in, out_bf16);
-}
 __global__ void k_fill_rows_bias(float *out, long n, int C, const float *bias) {
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n * C; i += (long)gridDim.x * blockDim.x) out[i] = bias ? bias[i % C] : 0.f;
 }
-int scn_deconvolution_forward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in,
-                              float *out, const float *w, const float *bias, int Cin, int Cout, double *macs, const void *in_bf16, long long weight_tag,
-                              const float *add_in, void *out_bf16) {
-  M_OR_FAIL(m);
-  // CPU/Deconvolution.cpp:15-16: the rulebook of the convolution outS -> inS
-  scn::ConvEntry *e;
-  SCN_TRY(m->md.get_conv(outS, inS, f, st, &e));
-  if (macs) *macs = (double)e->rb.total * Cin * Cout;
-  scn::Grid *gf = m->md.find_grid(outS);
-  SCN_CHECK(gf, "output grid");
-  cudaStream_t s = m->md.cstream;
-  // every fine row with a parent is written exactly once when each input site has one output cell
-  bool single = e->rb.total == gf->n && !bias;
-  if (single && e->geom.M == 1 && tc_ok(Cin, Cout, 1) && gf->n > 0) {
-    SCN_TRY(m->md.get_deconv_plan(*e));
-    SCN_TRY(m->md.wait_ready(e->deconvRdy));
-    const scn::DeconvPlan &d = e->deconv;
-    return scn::launch_conv_plan_tc(in, out, w, d.nbr, d.outRow, d.tileMask, d.nTiles * 128, 1, Cin, Cout, nullptr, scn::g_math_mode, s, d.tileW,
-                                    e->rb.nLists, m->md.find_grid(inS)->n, in_bf16, weight_tag, add_in, out_bf16, gf->n);
-  }
-  SCN_CHECK(in && out, "CUDA-core deconvolution needs the fp32 rows");
-  SCN_TRY(m->md.ensure_conv_rules(*e));
-  SCN_TRY(m->md.wait_ready(e->rdy));
-  SCN_TRY(m->md.wait_ready(e->rulesRdy));
-  if (!single && gf->n) k_fill_rows_bias<<<scn::stream_grid((long)gf->n * Cout, 256), 256, 0, scn::LS(s)>>>(out, gf->n, Cout, bias);
-  SCN_TRY(scn::launch_conv_list_simt(in, out, w, e->rb.pairs, e->rb.d_off, e->rb.off.data(), e->rb.nLists, Cin, Cout, /*srcIsY=*/1, single ? 1 : 0, s));
-  return plain_epilogue(out, add_in, out_bf16, gf->n, Cout, s);
-}
-
 // Whether a convolution's backward entry reads the (in, out) rule lists: the CUDA-core weight-gradient kernel does; the
 // tensor-core one reads the execution plan, where the input gradient runs on the tensor cores too (or is not wanted).
 static bool reads_lists(int Cin, int Cout, int K, bool tcInOrNone) { return !(tcInOrNone && scn::dw_plan_ok(Cin, Cout, K, scn::g_math_mode)); }
@@ -779,8 +695,101 @@ static void count_lists_ahead(Metadata &md, const scn::Ready &r) {
   std::lock_guard<std::mutex> lk(md.mapMu);
   if (r.ready && r.ahead) ++scn::g_counters[scn::kCntRulesAhead];
 }
+// d_in = forward tensor-core convolution of d_out with transposed weights (conv_bwd.cu header).  W: [K][Cin][Cout] of the
+// FORWARD layer; d_out rows have Cout channels (nSrcRows of them), d_in rows Cin channels (nDstRows, all written by the plan).
+static int dIn_tensor_core(Metadata &M, const float *d_out, float *d_in, const float *W, int K, int Cin, int Cout, int reverse, const int *nbr,
+                           const int *outRow, const unsigned long long *tileMask, int nOutPlan, const int *tileW, long nSrcRows, long nDstRows,
+                           const void *dout16) {
+  scn::TcConv c;
+  c.in = d_out; c.in16 = dout16; c.nInRows = nSrcRows;
+  // the transposed (and, for the symmetric submanifold plan, offset-reversed) weights are read in place by the operand-image kernel
+  c.W = W; c.nWeights = K; c.wT = reverse ? 2 : 1;
+  c.nbr = nbr; c.outRow = outRow; c.tileMask = tileMask; c.tileW = tileW; c.nOut = nOutPlan; c.K = tileW ? 1 : K;
+  c.Cin = Cout; c.Cout = Cin;
+  c.out = d_in; c.nOutRows = nDstRows;
+  c.mathMode = scn::g_math_mode;
+  return scn::launch_conv_plan_tc(c, M.cstream);
+}
+// bf16 / fp16 mode: one 16-bit copy of d_out serves both gradient kernels of a backward call (each used to make its own)
+static int shared_dout16(cudaStream_t s, const float *d_out, long rows, int Cin, int Cout, const void **out) {
+  *out = nullptr;
+  if (!scn::half_mode(scn::g_math_mode) || !scn::tc_available() || rows == 0 || Cout % 32 != 0 || !tc_ok(Cout, Cin, 1)) return 0;
+  return scn::dout16_copy(d_out, rows * Cout, s, out);
+}
 extern "C++" {
 namespace scn {
+static int run_plan(Metadata &M, const NbrPlan &plan, const float *in, float *out, const float *w, const float *bias, int Cin, int Cout, long nInRows,
+                    const void *in16, long long wTag, const float *addend, void *out16, const ConvFusion &fuse, ConvFused *fused) {
+  if (tc_ok(Cin, Cout, plan.K)) {
+    TcConv c;
+    c.in = in; c.in16 = in16; c.nInRows = nInRows;
+    c.W = w; c.wTag = wTag; c.nWeights = plan.K;
+    c.nbr = plan.nbr; c.outRow = plan.outRow; c.tileMask = plan.tileMask; c.nOut = plan.nOut; c.K = plan.K;
+    c.Cin = Cin; c.Cout = Cout; c.bias = bias; c.addend = addend;
+    c.out = out; c.out16 = out16; c.nOutRows = plan.nOut;
+    c.mathMode = g_math_mode; c.fuse = fuse; c.fused = fused;
+    return launch_conv_plan_tc(c, M.cstream);
+  }
+  SCN_CHECK(in && out, "CUDA-core path needs the fp32 rows");
+  SCN_TRY(launch_conv_plan_simt(in, out, w, plan.nbr, plan.outRow, plan.nOut, plan.K, Cin, Cout, bias, M.cstream));
+  return plain_epilogue(out, addend, out16, plan.nOut, Cout, M.cstream);
+}
+
+int submanifold_forward(scn_metadata *m, const long sz[3], const long f[3], const float *in, float *out, const float *w, const float *bias, int Cin,
+                        int Cout, double *macs, const void *in_bf16, long long weight_tag, const float *add_in, void *out_bf16, const ConvFusion &fuse,
+                        ConvFused *fused) {
+  M_OR_FAIL(m);
+  SubmEntry *e;
+  SCN_TRY(m->md.get_submanifold(sz, f, &e));
+  if (macs) *macs = (double)e->rb.total * Cin * Cout;
+  SCN_TRY(m->md.wait_ready(e->rdy));
+  return run_plan(m->md, e->plan, in, out, w, bias, Cin, Cout, m->md.find_grid(sz)->n, in_bf16, weight_tag, add_in, out_bf16, fuse, fused);
+}
+int convolution_forward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in, float *out,
+                        const float *w, const float *bias, int Cin, int Cout, double *macs, const void *in_bf16, long long weight_tag, const float *add_in,
+                        void *out_bf16, const ConvFusion &fuse, ConvFused *fused) {
+  M_OR_FAIL(m);
+  ConvEntry *e;
+  SCN_TRY(m->md.get_conv(inS, outS, f, st, &e));
+  if (macs) *macs = (double)e->rb.total * Cin * Cout;
+  SCN_TRY(m->md.wait_ready(e->rdy));
+  return run_plan(m->md, e->plan, in, out, w, bias, Cin, Cout, m->md.find_grid(inS)->n, in_bf16, weight_tag, add_in, out_bf16, fuse, fused);
+}
+int deconvolution_forward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in, float *out,
+                          const float *w, const float *bias, int Cin, int Cout, double *macs, const void *in_bf16, long long weight_tag, const float *add_in,
+                          void *out_bf16, const ConvFusion &fuse, ConvFused *fused) {
+  M_OR_FAIL(m);
+  // CPU/Deconvolution.cpp:15-16: the rulebook of the convolution outS -> inS
+  ConvEntry *e;
+  SCN_TRY(m->md.get_conv(outS, inS, f, st, &e));
+  if (macs) *macs = (double)e->rb.total * Cin * Cout;
+  Grid *gf = m->md.find_grid(outS);
+  SCN_CHECK(gf, "output grid");
+  cudaStream_t s = m->md.cstream;
+  // every fine row with a parent is written exactly once when each input site has one output cell
+  bool single = e->rb.total == gf->n && !bias;
+  if (single && e->geom.M == 1 && tc_ok(Cin, Cout, 1) && gf->n > 0) {
+    SCN_TRY(m->md.get_deconv_plan(*e));
+    SCN_TRY(m->md.wait_ready(e->deconvRdy));
+    const DeconvPlan &d = e->deconv;
+    TcConv c;
+    c.in = in; c.in16 = in_bf16; c.nInRows = m->md.find_grid(inS)->n;
+    c.W = w; c.wTag = weight_tag; c.nWeights = e->rb.nLists;
+    c.nbr = d.nbr; c.outRow = d.outRow; c.tileMask = d.tileMask; c.tileW = d.tileW; c.nOut = d.nTiles * 128; c.K = 1;
+    c.Cin = Cin; c.Cout = Cout; c.addend = add_in;
+    c.out = out; c.out16 = out_bf16; c.nOutRows = gf->n;
+    c.mathMode = g_math_mode; c.fuse = fuse; c.fused = fused;
+    return launch_conv_plan_tc(c, s);
+  }
+  SCN_CHECK(in && out, "CUDA-core deconvolution needs the fp32 rows");
+  SCN_TRY(m->md.ensure_conv_rules(*e));
+  SCN_TRY(m->md.wait_ready(e->rdy));
+  SCN_TRY(m->md.wait_ready(e->rulesRdy));
+  if (!single && gf->n) k_fill_rows_bias<<<stream_grid((long)gf->n * Cout, 256), 256, 0, LS(s)>>>(out, gf->n, Cout, bias);
+  SCN_TRY(launch_conv_list_simt(in, out, w, e->rb.pairs, e->rb.d_off, e->rb.off.data(), e->rb.nLists, Cin, Cout, /*srcIsY=*/1, single ? 1 : 0, s));
+  return plain_epilogue(out, add_in, out_bf16, gf->n, Cout, s);
+}
+
 // The rule lists the backward entry of a recorded convolution (kind 1 submanifold, 2 strided, 3 deconvolution) will read for a
 // non-empty level, decided from its shape as the entries below decide it from the built rulebook.  A strided convolution's
 // rulebook gives every input site exactly one parent when filter == stride; wantDIn: the input gradient is computed.
@@ -793,32 +802,14 @@ bool backward_reads_lists(int kind, const long *f, const long *st, int Cin, int 
   return reads_lists(Cin, Cout, K, tcIn);
 }
 cudaStream_t metadata_stream(scn_metadata *m) { return m->md.cstream; }
-} // namespace scn
-} // extern "C++"
 
-// d_in = forward tensor-core convolution of d_out with transposed weights (conv_bwd.cu header).  W: [K][Cin][Cout] of the
-// FORWARD layer; d_out rows have Cout channels (nSrcRows of them), d_in rows Cin channels (nDstRows, all written by the plan).
-static int dIn_tensor_core(Metadata &M, const float *d_out, float *d_in, const float *W, int K, int Cin, int Cout, int reverse, const int *nbr,
-                           const int *outRow, const unsigned long long *tileMask, int nOutPlan, const int *tileW, long nSrcRows, long nDstRows,
-                           const void *dout16 = nullptr) {
-  cudaStream_t s = M.cstream;
-  // the transposed (and, for the symmetric submanifold plan, offset-reversed) weights are read in place by the operand-image kernel
-  return scn::launch_conv_plan_tc(d_out, d_in, W, nbr, outRow, tileMask, nOutPlan, tileW ? 1 : K, /*Cin=*/Cout, /*Cout=*/Cin, nullptr, scn::g_math_mode, s, tileW, K,
-                                  nSrcRows, dout16, 0, nullptr, nullptr, nDstRows, 0, reverse ? 2 : 1);
-}
-// bf16 / fp16 mode: one 16-bit copy of d_out serves both gradient kernels of a backward call (each used to make its own)
-static int shared_dout16(cudaStream_t s, const float *d_out, long rows, int Cin, int Cout, const void **out) {
-  *out = nullptr;
-  if (!scn::half_mode(scn::g_math_mode) || !scn::tc_available() || rows == 0 || Cout % 32 != 0 || !tc_ok(Cout, Cin, 1)) return 0;
-  return scn::dout16_copy(d_out, rows * Cout, s, out);
-}
-int scn_submanifold_convolution_backward(scn_metadata *m, const long sz[3], const long f[3], const float *in, float *d_in, const float *d_out,
-                                         const float *w, float *dw, float *d_bias, int Cin, int Cout) {
-  const void *in16 = scn::bwd_in16_take(), *dout16 = nullptr;
+int submanifold_backward(scn_metadata *m, const long sz[3], const long f[3], const float *in, float *d_in, const float *d_out, const float *w,
+                         float *dw, float *d_bias, int Cin, int Cout, const void *in16) {
+  const void *dout16 = nullptr;
   M_OR_FAIL(m);
-  scn::SubmEntry *e;
+  SubmEntry *e;
   SCN_TRY(m->md.get_submanifold(sz, f, &e));
-  scn::Grid *g = m->md.find_grid(sz);
+  Grid *g = m->md.find_grid(sz);
   // d_in on the tensor cores: the plan of an odd filter is symmetric, d_in[q] = sum_j d_out[nbr[q][j]] @ W[K-1-j]^T
   const bool tcIn = d_in && tc_ok(Cout, Cin, e->plan.K) && f[0] % 2 == 1 && f[1] % 2 == 1 && f[2] % 2 == 1 && g->n > 0;
   // the per-offset rule lists (reference order) are only materialised when a CUDA-core kernel needs them: both tensor-core
@@ -829,17 +820,17 @@ int scn_submanifold_convolution_backward(scn_metadata *m, const long sz[3], cons
   if (lists) SCN_TRY(m->md.wait_ready(e->rulesRdy));
   SCN_TRY(shared_dout16(m->md.cstream, d_out, g->n, Cin, Cout, &dout16));
   if (tcIn) SCN_TRY(dIn_tensor_core(m->md, d_out, d_in, w, e->plan.K, Cin, Cout, /*reverse=*/1, e->plan.nbr, e->plan.outRow, e->plan.tileMask, e->plan.nOut, nullptr, g->n, g->n, dout16));
-  return scn::conv_backward_simt(in, d_in, d_out, w, dw, d_bias, lists ? e->rb.pairs : nullptr, e->rb.d_off, lists ? e->rb.off.data() : nullptr, e->plan.K, g->n, g->n, Cin, Cout, 0, m->md.cstream, tcIn || !d_in, scn::g_math_mode, in16, dout16,
-                                 e->plan.nbr, e->plan.outRow, e->plan.tileMask, e->plan.nOut); // d_in == NULL: input gradient not wanted
+  return conv_backward_simt(in, d_in, d_out, w, dw, d_bias, lists ? e->rb.pairs : nullptr, e->rb.d_off, lists ? e->rb.off.data() : nullptr, e->plan.K, g->n, g->n, Cin, Cout, 0, m->md.cstream, tcIn || !d_in, g_math_mode, in16, dout16,
+                            e->plan.nbr, e->plan.outRow, e->plan.tileMask, e->plan.nOut); // d_in == NULL: input gradient not wanted
 }
-int scn_convolution_backward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in,
-                             float *d_in, const float *d_out, const float *w, float *dw, float *d_bias, int Cin, int Cout) {
-  const void *in16 = scn::bwd_in16_take(), *dout16 = nullptr;
+int convolution_backward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in, float *d_in,
+                         const float *d_out, const float *w, float *dw, float *d_bias, int Cin, int Cout, const void *in16) {
+  const void *dout16 = nullptr;
   M_OR_FAIL(m);
-  scn::ConvEntry *e;
+  ConvEntry *e;
   SCN_TRY(m->md.get_conv(inS, outS, f, st, &e));
   // d_in (fine rows) on the tensor cores: a deconvolution of d_out with W^T over the single-parent plan
-  scn::Grid *gf = m->md.find_grid(inS), *gc = m->md.find_grid(outS);
+  Grid *gf = m->md.find_grid(inS), *gc = m->md.find_grid(outS);
   const bool tcIn = tc_ok(Cout, Cin, 1) && e->geom.M == 1 && e->rb.total == gf->n && gf->n > 0;
   const bool lists = reads_lists(Cin, Cout, e->plan.K, tcIn);
   if (lists) { count_lists_ahead(m->md, e->rulesRdy); SCN_TRY(m->md.ensure_conv_rules(*e)); }
@@ -849,20 +840,20 @@ int scn_convolution_backward(scn_metadata *m, const long inS[3], const long outS
   if (tcIn) {
     SCN_TRY(m->md.get_deconv_plan(*e));
     SCN_TRY(m->md.wait_ready(e->deconvRdy));
-    const scn::DeconvPlan &d = e->deconv;
+    const DeconvPlan &d = e->deconv;
     SCN_TRY(dIn_tensor_core(m->md, d_out, d_in, w, e->rb.nLists, Cin, Cout, /*reverse=*/0, d.nbr, d.outRow, d.tileMask, d.nTiles * 128, d.tileW, gc->n, gf->n, dout16));
   }
-  return scn::conv_backward_simt(in, d_in, d_out, w, dw, d_bias, lists ? e->rb.pairs : nullptr, e->rb.d_off, lists ? e->rb.off.data() : nullptr, e->plan.K, gf->n, gc->n, Cin, Cout, 0, m->md.cstream, tcIn, scn::g_math_mode, in16, dout16,
-                                 e->plan.nbr, e->plan.outRow, e->plan.tileMask, e->plan.nOut);
+  return conv_backward_simt(in, d_in, d_out, w, dw, d_bias, lists ? e->rb.pairs : nullptr, e->rb.d_off, lists ? e->rb.off.data() : nullptr, e->plan.K, gf->n, gc->n, Cin, Cout, 0, m->md.cstream, tcIn, g_math_mode, in16, dout16,
+                            e->plan.nbr, e->plan.outRow, e->plan.tileMask, e->plan.nOut);
 }
-int scn_deconvolution_backward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in,
-                               float *d_in, const float *d_out, const float *w, float *dw, float *d_bias, int Cin, int Cout) {
-  const void *in16 = scn::bwd_in16_take(), *dout16 = nullptr;
+int deconvolution_backward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in, float *d_in,
+                           const float *d_out, const float *w, float *dw, float *d_bias, int Cin, int Cout, const void *in16) {
+  const void *dout16 = nullptr;
   M_OR_FAIL(m);
-  scn::ConvEntry *e;
+  ConvEntry *e;
   SCN_TRY(m->md.get_conv(outS, inS, f, st, &e));
   // d_in (coarse rows) on the tensor cores: the strided convolution fine -> coarse of d_out with W^T
-  scn::Grid *gc = m->md.find_grid(inS), *gf = m->md.find_grid(outS);
+  Grid *gc = m->md.find_grid(inS), *gf = m->md.find_grid(outS);
   const bool tcIn = tc_ok(Cout, Cin, e->plan.K) && gc->n > 0;
   const bool lists = reads_lists(Cin, Cout, e->plan.K, tcIn);
   if (lists) { count_lists_ahead(m->md, e->rulesRdy); SCN_TRY(m->md.ensure_conv_rules(*e)); }
@@ -870,16 +861,63 @@ int scn_deconvolution_backward(scn_metadata *m, const long inS[3], const long ou
   if (lists) SCN_TRY(m->md.wait_ready(e->rulesRdy));
   SCN_TRY(shared_dout16(m->md.cstream, d_out, gf->n, Cin, Cout, &dout16));
   if (tcIn) SCN_TRY(dIn_tensor_core(m->md, d_out, d_in, w, e->plan.K, Cin, Cout, /*reverse=*/0, e->plan.nbr, e->plan.outRow, e->plan.tileMask, e->plan.nOut, nullptr, gf->n, gc->n, dout16));
-  return scn::conv_backward_simt(in, d_in, d_out, w, dw, d_bias, lists ? e->rb.pairs : nullptr, e->rb.d_off, lists ? e->rb.off.data() : nullptr, e->plan.K, gc->n, gf->n, Cin, Cout, 1, m->md.cstream, tcIn, scn::g_math_mode, in16, dout16,
-                                 e->plan.nbr, e->plan.outRow, e->plan.tileMask, e->plan.nOut);
+  return conv_backward_simt(in, d_in, d_out, w, dw, d_bias, lists ? e->rb.pairs : nullptr, e->rb.d_off, lists ? e->rb.off.data() : nullptr, e->plan.K, gc->n, gf->n, Cin, Cout, 1, m->md.cstream, tcIn, g_math_mode, in16, dout16,
+                            e->plan.nbr, e->plan.outRow, e->plan.tileMask, e->plan.nOut);
+}
+// (out may be NULL when out_bf16 is given: only the sign of the output is read)
+int batchnorm_backward_y16(const float *in, float *d_in, const float *out, const void *out_bf16, float *d_out, long n, int C, const float *save_mean,
+                           const float *save_invstd, const float *weight, float *d_weight, float *d_bias, float leak, cudaStream_t s) {
+  void *ws = nullptr;
+  SCN_CUDA(cudaMallocAsync(&ws, (size_t)C * 24 + 64, s));
+  int r = bn_backward(in, d_in, out, d_out, n, C, save_mean, save_invstd, weight, d_weight, d_bias, leak, ws, s, out_bf16);
+  cudaFreeAsync(ws, s);
+  return r;
+}
+} // namespace scn
+} // extern "C++"
+
+int scn_submanifold_convolution_forward(scn_metadata *m, const long sz[3], const long f[3], const float *in, float *out, const float *w,
+                                        const float *bias, int Cin, int Cout, double *macs, const void *in_bf16, long long weight_tag,
+                                        const float *add_in, void *out_bf16) {
+  return scn::submanifold_forward(m, sz, f, in, out, w, bias, Cin, Cout, macs, in_bf16, weight_tag, add_in, out_bf16, take_fusion_request(), &tl_fusion.result);
+}
+int scn_convolution_forward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in,
+                            float *out, const float *w, const float *bias, int Cin, int Cout, double *macs, const void *in_bf16, long long weight_tag,
+                            const float *add_in, void *out_bf16) {
+  return scn::convolution_forward(m, inS, outS, f, st, in, out, w, bias, Cin, Cout, macs, in_bf16, weight_tag, add_in, out_bf16, take_fusion_request(), &tl_fusion.result);
+}
+int scn_deconvolution_forward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in,
+                              float *out, const float *w, const float *bias, int Cin, int Cout, double *macs, const void *in_bf16, long long weight_tag,
+                              const float *add_in, void *out_bf16) {
+  return scn::deconvolution_forward(m, inS, outS, f, st, in, out, w, bias, Cin, Cout, macs, in_bf16, weight_tag, add_in, out_bf16, take_fusion_request(), &tl_fusion.result);
+}
+int scn_submanifold_convolution_backward(scn_metadata *m, const long sz[3], const long f[3], const float *in, float *d_in, const float *d_out,
+                                         const float *w, float *dw, float *d_bias, int Cin, int Cout) {
+  return scn::submanifold_backward(m, sz, f, in, d_in, d_out, w, dw, d_bias, Cin, Cout, nullptr);
+}
+int scn_convolution_backward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in,
+                             float *d_in, const float *d_out, const float *w, float *dw, float *d_bias, int Cin, int Cout) {
+  return scn::convolution_backward(m, inS, outS, f, st, in, d_in, d_out, w, dw, d_bias, Cin, Cout, nullptr);
+}
+int scn_deconvolution_backward(scn_metadata *m, const long inS[3], const long outS[3], const long f[3], const long st[3], const float *in,
+                               float *d_in, const float *d_out, const float *w, float *dw, float *d_bias, int Cin, int Cout) {
+  return scn::deconvolution_backward(m, inS, outS, f, st, in, d_in, d_out, w, dw, d_bias, Cin, Cout, nullptr);
 }
 
 // ---- NetworkInNetwork: a 1x1 "convolution" = dense GEMM over the feature rows, no Metadata involved
 static int dense_rows_gemm(const float *in, float *out, const float *w, const float *bias, long n, int Cin, int Cout, cudaStream_t s, const void *in16, long long tag) {
   if (n == 0) return 0;
   SCN_CHECK(n < (1l << 31) - 256, "too many rows");
-  if (tc_ok(Cin, Cout, 1)) // the tensor-core gather-GEMM with the identity plan (site p reads row p, writes row p)
-    return scn::launch_conv_plan_tc(in, out, w, nullptr, nullptr, nullptr, (int)n, 1, Cin, Cout, bias, scn::g_math_mode, s, nullptr, 1, n, in16, tag, nullptr, nullptr, n);
+  if (tc_ok(Cin, Cout, 1)) { // the tensor-core gather-GEMM with the identity plan (site p reads row p, writes row p)
+    scn::TcConv c;
+    c.in = in; c.in16 = in16; c.nInRows = n;
+    c.W = w; c.wTag = tag; c.nWeights = 1;
+    c.nOut = (int)n; c.K = 1;
+    c.Cin = Cin; c.Cout = Cout; c.bias = bias;
+    c.out = out; c.nOutRows = n;
+    c.mathMode = scn::g_math_mode;
+    return scn::launch_conv_plan_tc(c, s);
+  }
   return scn::launch_conv_plan_simt(in, out, w, nullptr, nullptr, (int)n, 1, Cin, Cout, bias, s);
 }
 int scn_network_in_network_forward(const float *in, float *out, const float *weight, const float *bias, long n_rows, int n_in, int n_out, double *macs,
@@ -929,19 +967,6 @@ int scn_batchnorm_forward(const float *in, float *out, long n, int C, float *sav
   }
   return scn::bn_forward(in, out, n, C, save_mean, save_invstd, running_mean, running_var, weight, bias, eps, momentum, mode, leak, ws, s, out_bf16);
 }
-extern "C++" {
-namespace scn {
-// (out may be NULL when out_bf16 is given: only the sign of the output is read)
-int batchnorm_backward_y16(const float *in, float *d_in, const float *out, const void *out_bf16, float *d_out, long n, int C, const float *save_mean,
-                           const float *save_invstd, const float *weight, float *d_weight, float *d_bias, float leak, cudaStream_t s) {
-  void *ws = nullptr;
-  SCN_CUDA(cudaMallocAsync(&ws, (size_t)C * 24 + 64, s));
-  int r = bn_backward(in, d_in, out, d_out, n, C, save_mean, save_invstd, weight, d_weight, d_bias, leak, ws, s, out_bf16);
-  cudaFreeAsync(ws, s);
-  return r;
-}
-} // namespace scn
-} // extern "C++"
 int scn_batchnorm_backward(const float *in, float *d_in, const float *out, float *d_out, long n, int C, const float *save_mean,
                            const float *save_invstd, const float *weight, float *d_weight, float *d_bias, float leak, void *stream) {
   return scn::batchnorm_backward_y16(in, d_in, out, nullptr, d_out, n, C, save_mean, save_invstd, weight, d_weight, d_bias, leak, static_cast<cudaStream_t>(stream));

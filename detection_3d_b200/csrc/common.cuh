@@ -10,6 +10,7 @@ namespace scn {
 
 // ---------------------------------------------------------------- errors
 void set_error(const std::string &msg);
+const char *last_error(); // this thread's last message
 #define SCN_CUDA(call)                                                                   \
   do {                                                                                   \
     cudaError_t e__ = (call);                                                            \

@@ -8,14 +8,9 @@
 //          atomics into dW (replaces dConvolution_KMxKN_backward_dW_A/B, SCN/CUDA/Convolution.cu:249-410); in deterministic mode
 //          each chunk stores its partial dW[k] into its own slot and ordered_sum adds the chunks in chunk order.
 // Reference semantics: SCN/CPU/Convolution.cpp:81-115,152-185, SCN/CPU/Deconvolution.cpp:43-77.
-#include "common.cuh"
+#include "conv.cuh"
 
 namespace scn {
-int launch_conv_list_simt(const float *in, float *out, const float *W, const int2 *pairs, const int *d_off, const int *offHost, int K, int Cin,
-                          int Cout, int srcIsY, int singlePass, cudaStream_t s);
-int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2 *pairs, const int *d_off, const int *offHost, int K, long nInRows,
-                      long nOutRows, int Cin, int Cout, int srcIsY, int mathMode, cudaStream_t s, const void *in16, const void *dout16,
-                      const int *planNbr, const int *planOutRow, const unsigned long long *planMask, int planPos);
 
 // Wt[k'][co][ci] = W[k][ci][co], k' = k or (reverse) K - 1 - k
 __global__ void k_transpose_w(const float *__restrict__ W, float *__restrict__ Wt, int K, int Cin, int Cout, int reverse) {

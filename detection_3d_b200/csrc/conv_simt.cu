@@ -8,7 +8,7 @@
 //    SCN/CUDA/Convolution.cu:57-203, RuleBookIterator.h:15-32).
 //  * conv_list_simt : rule-list driven (gather rows by pairs[i].src, write rows pairs[i].dst) for
 //    deconvolution, where every fine row has one parent (SCN/CUDA/Deconvolution.cu).
-#include "common.cuh"
+#include "conv.cuh"
 
 namespace scn {
 

@@ -23,7 +23,7 @@
 //
 // Replaces dConvolution_KMxKN_forwardA/B (SCN/CUDA/Convolution.cu:57-203: SIMT tiles, fp64
 // accumulators, one launch + one blocking H2D rule copy per filter offset).
-#include "common.cuh"
+#include "conv.cuh"
 #include <cuda_bf16.h>
 #include <stdlib.h>
 #include <algorithm>
@@ -949,11 +949,6 @@ int dout16_copy(const float *d_out, long n, cudaStream_t s, const void **out) {
   *out = p;
   return 0;
 }
-// Side channel of the program executor's backward pass: a bf16 copy of the NEXT scn_*_convolution_backward call's `in` rows
-// (the forward pass wrote it: the bf16 shadow of the register) -- taken (and cleared) by that call.
-static thread_local const void *tl_bwd_in16 = nullptr;
-void bwd_in16_arm(const void *in16) { tl_bwd_in16 = in16; }
-const void *bwd_in16_take() { const void *p = tl_bwd_in16; tl_bwd_in16 = nullptr; return p; }
 // Grow-only scratch per (device, stream, slot) for the operand copies a call may need (slot 0: zero-padded rows of a
 // narrow input; slot 1: bf16 copy of an input that arrived without one -- one launch can need both, the second derived
 // from the first, so they must not share a buffer; slot 2: the operand pair of the weight-gradient kernel).  Uses of a
@@ -993,106 +988,80 @@ static int sched_counters(cudaStream_t s, unsigned **out) {
   *out = e;
   return 0;
 }
-// Side channel used by the program executor (program.cu): the next tensor-core convolution launched by THIS thread
-// also accumulates the per-channel sum / sum of squares of its output into `sums` (zeroed by the caller) when its
-// configuration allows it; epilogue_stats_take() says whether it did and disarms the request.
-static thread_local double *tl_stats = nullptr;
-static thread_local bool tl_stats_done = false;
-void epilogue_stats_arm(double *sums) { tl_stats = sums; tl_stats_done = false; }
-// A bf16 copy of the next convolution's input rows that is already zero-padded to `Cp` channels (written by the input layer).
-static thread_local const void *tl_prepad = nullptr;
-static thread_local int tl_prepad_c = 0;
-void prepadded_arm(const void *rows16, int Cp) { tl_prepad = rows16; tl_prepad_c = Cp; }
-void prepadded_disarm() { tl_prepad = nullptr; tl_prepad_c = 0; }
-// Same for a lateral 1x1x1 convolution folded into the next convolution: out = conv(in) [+ addend] + lat_in[row] @ lat_w.
-// lat_in: fp32 rows; lat_in16: their bf16 copy (may be null); taken when the launch is a whole-atom (unpacked) tensor-core launch.
-struct Lateral { const float *in; const void *in16; const float *w; long long tag; int Cin; long rows; };
-static thread_local Lateral tl_lat = {nullptr, nullptr, nullptr, 0, 0, 0};
-static thread_local bool tl_lat_done = false;
-void lateral_arm(const float *in, const void *in16, const float *w, long long tag, int Cin, long rows) { tl_lat = Lateral{in, in16, w, tag, Cin, rows}; tl_lat_done = false; }
-bool lateral_take() { bool d = tl_lat_done; tl_lat.in = nullptr; tl_lat_done = false; return d; }
-bool epilogue_stats_take() { bool d = tl_stats_done; tl_stats = nullptr; tl_stats_done = false; return d; }
-template <bool DET>
-static int set_plan_attributes() {
-  const int half = (233472 - kBuildRoom) / 2 - 1024;
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpTF32, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpTF32, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 4, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 4, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpTF32, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpBF16, 8, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpTF32X3, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 8, 1, 1, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 4, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 4, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 4, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 8, 1, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 8, 2, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
-  SCN_CUDA(cudaFuncSetAttribute(conv_plan_tc<kOpF16, 8, 4, 2, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, half));
+// A plan of more than 64 filter offsets (chunk-major, common.cuh) runs as one launch per chunk of <= 63 offsets.  Chunk c is an
+// ordinary plan -- its own block of neighbour ids and mask array, the weights of its offsets -- and takes the running sum of the
+// chunks before it as its fused addend.  Bias and the caller's addend go into chunk 0; the lateral stage, the epilogue statistics
+// and the bf16 copy into the last chunk, the only one that sees finished rows.  The running sums alternate between two scratch
+// buffers, so no launch reads rows it writes (an offset-split launch zeroes its output first).  Each chunk boundary adds one fp32
+// rounding of the partial sum (DESIGN.md section 7).
+static int launch_conv_plan_tc_chunked(const TcConv &c, cudaStream_t s) {
+  const int K = c.K, CinW = c.CinW ? c.CinW : c.Cin, nC = plan_chunks(K);
+  const long nPad = plan_padded(c.nOut);
+  float *run = nullptr;
+  SCN_TRY(stream_scratch(s, kScratchChunk, (size_t)std::min(nC - 1, 2) * c.nOutRows * c.Cout * 4 + 16, (void **)&run));
+  const float *prev = c.addend;
+  for (int i = 0; i < nC; i++) {
+    const int k0 = i * kChunkOffsets, Kc = std::min(kChunkOffsets, K - k0);
+    const bool last = i == nC - 1;
+    TcConv ch = c;
+    ch.out = last ? c.out : run + (size_t)(i & 1) * c.nOutRows * c.Cout;
+    // W: [K][CinW][Cout] (or [K][Cout][CinW] transposed): CinW x Cout floats per offset.  Offset-reversed operands (wT = 2): offset j
+    // of this chunk is W[K - 1 - k0 - j], i.e. the reversal of the block W[K - k0 - Kc, K - k0)
+    ch.W = c.W + (size_t)(c.wT == 2 ? K - k0 - Kc : k0) * CinW * c.Cout;
+    ch.nbr = c.nbr + (size_t)k0 * nPad;
+    ch.tileMask = c.tileMask + (size_t)i * (nPad / 128);
+    ch.K = ch.nWeights = Kc;
+    ch.bias = i == 0 ? c.bias : nullptr; ch.addend = prev;
+    if (!last) { ch.out16 = nullptr; ch.fuse.lat.in = nullptr; ch.fuse.stats = nullptr; } // (the padded input rows go to every chunk)
+    ++g_counters[kCntChunkedLaunch];
+    SCN_TRY(launch_conv_plan_tc(ch, s));
+    prev = ch.out;
+  }
   return 0;
 }
-// H = the 16-bit operand type (kOpBF16 or kOpF16) of a launch with P.bf16 set
-template <bool DET, int H>
-static cudaError_t launch_plan_variant16(const TcParams &P, int packG, bool pw8, int ctas, int grid, int th2, size_t smem, cudaStream_t s) {
-  if (packG == 2) return pw8 ? launch_pdl(conv_plan_tc<H, 8, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<H, 4, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
-  if (packG == 4) return pw8 ? launch_pdl(conv_plan_tc<H, 8, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<H, 4, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
-  if (ctas == 2) return pw8 ? launch_pdl(conv_plan_tc<H, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<H, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
-  return launch_pdl(conv_plan_tc<H, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
-}
-template <bool DET>
-static cudaError_t launch_plan_variant(const TcParams &P, int packG, bool pw8, int ctas, int grid, int th2, size_t smem, cudaStream_t s, bool x3, bool f16) {
-  if (f16 && P.bf16) return launch_plan_variant16<DET, kOpF16>(P, packG, pw8, ctas, grid, th2, smem, s);
-  if (x3) return launch_pdl(conv_plan_tc<kOpTF32X3, 8, 1, 1, DET>, dim3(grid), dim3(32 * (14 + kSplitWarps)), smem, LS(s), P);
-  if (packG == 2) return pw8 ? launch_pdl(conv_plan_tc<kOpBF16, 8, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpBF16, 4, 2, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
-  if (packG == 4) return pw8 ? launch_pdl(conv_plan_tc<kOpBF16, 8, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpBF16, 4, 4, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
-  if (ctas == 2) {
-    if (P.bf16) return pw8 ? launch_pdl(conv_plan_tc<kOpBF16, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpBF16, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
-    return pw8 ? launch_pdl(conv_plan_tc<kOpTF32, 8, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P) : launch_pdl(conv_plan_tc<kOpTF32, 4, 1, 2, DET>, dim3(grid), dim3(th2), smem, LS(s), P);
-  }
-  if (P.bf16) return launch_pdl(conv_plan_tc<kOpBF16, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
-  return launch_pdl(conv_plan_tc<kOpTF32, 8, 1, 1, DET>, dim3(grid), dim3(32 * 14), smem, LS(s), P);
-}
-static int launch_conv_plan_tc_chunked(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
-                                       int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, long nInRows, const void *in16,
-                                       long long wTag, const float *addend, void *out16, long nOutRows, int CinW, int wT);
-// in16: optional 16-bit copy of `in` (same layout, the mode's format); used in math modes 2 / 5 when Cin is a multiple of 64.
-// mathMode 1 = TF32 operands, 2 = BF16 where the channel counts allow (TF32 elsewhere), 3 = TF32X3 (the fp32 rows as hi / lo TF32 pairs),
-// 5 = F16 where mode 2 has BF16 (TF32 elsewhere).  out16 (optional) receives the result in the mode's 16-bit format.
-int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
-                        int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, const int *tileW, int nWeights,
-                        long nInRows, const void *in16, long long wTag, const float *addend, void *out16, long nOutRows, int CinW = 0, int wT = 0) {
+// Every conv_plan_tc instantiation the launcher uses: operand type, producer warps, filter offsets per packed atom (G), CTAs per
+// SM, deterministic mode.
+struct PlanKernel { int op, pw, G, ctas; bool det; void (*fn)(TcParams); };
+#define SCN_PLAN(OP, PW, G, CTAS) {OP, PW, G, CTAS, false, conv_plan_tc<OP, PW, G, CTAS, false>}, {OP, PW, G, CTAS, true, conv_plan_tc<OP, PW, G, CTAS, true>}
+static const PlanKernel kPlanKernels[] = {
+    SCN_PLAN(kOpTF32, 8, 1, 1),   SCN_PLAN(kOpTF32, 4, 1, 2), SCN_PLAN(kOpTF32, 8, 1, 2), SCN_PLAN(kOpTF32X3, 8, 1, 1),
+    SCN_PLAN(kOpBF16, 8, 1, 1),   SCN_PLAN(kOpBF16, 4, 1, 2), SCN_PLAN(kOpBF16, 4, 2, 2), SCN_PLAN(kOpBF16, 4, 4, 2),
+    SCN_PLAN(kOpBF16, 8, 1, 2),   SCN_PLAN(kOpBF16, 8, 2, 2), SCN_PLAN(kOpBF16, 8, 4, 2),
+    SCN_PLAN(kOpF16, 8, 1, 1),    SCN_PLAN(kOpF16, 4, 1, 2),  SCN_PLAN(kOpF16, 4, 2, 2),  SCN_PLAN(kOpF16, 4, 4, 2),
+    SCN_PLAN(kOpF16, 8, 1, 2),    SCN_PLAN(kOpF16, 8, 2, 2),  SCN_PLAN(kOpF16, 8, 4, 2)};
+#undef SCN_PLAN
+int launch_conv_plan_tc(const TcConv &c, cudaStream_t s) {
+  const int nOut = c.nOut, K = c.K, Cin = c.Cin, Cout = c.Cout, CinW = c.CinW ? c.CinW : c.Cin;
   if (nOut == 0) return 0;
-  if (CinW == 0) CinW = Cin;
-  if (K > 64 && !tileW) {
-    SCN_CHECK(nbr && tileMask && nWeights == K && K <= kMaxFilterVolume, "tcgen05 path: wide plan");
-    return launch_conv_plan_tc_chunked(in, out, W, nbr, outRow, tileMask, nOut, K, Cin, Cout, bias, mathMode, s, nInRows, in16, wTag, addend, out16, nOutRows, CinW, wT);
+  if (K > 64 && !c.tileW) {
+    SCN_CHECK(c.nbr && c.tileMask && c.nWeights == K && K <= kMaxFilterVolume, "tcgen05 path: wide plan");
+    return launch_conv_plan_tc_chunked(c, s);
   }
-  const bool f16 = mathMode == kModeF16; // 16-bit operands and copies are fp16 (else bf16)
-  const bool canPack = half_mode(mathMode) && !tileW && Cout <= 128; // packed narrow rows: two-CTA configuration only
+  const bool f16 = c.mathMode == kModeF16; // 16-bit operands and copies are fp16 (else bf16)
+  const bool canPack = half_mode(c.mathMode) && !c.tileW && Cout <= 128; // packed narrow rows: two-CTA configuration only
   if (canPack && CinW == Cin && Cin != 16 && Cin % 32 != 0) {
     // bf16 / fp16 mode, odd channel counts (e.g. the 9-channel network input): 16-bit rows zero-padded to 16 channels (packed, G = 4),
     // 32 channels (G = 2) or a multiple of 64 (whole atoms), written by one pass; the weight image pads itself
     const int Cp = Cin < 16 ? 16 : (Cin < 32 ? 32 : (Cin + 63) / 64 * 64);
+    TcConv p = c;
     void *xp = nullptr;
-    if (tl_prepad && tl_prepad_c == Cp) {
-      xp = const_cast<void *>(tl_prepad); // the producer already wrote the padded copy
+    if (c.fuse.pad16 && c.fuse.padC == Cp) {
+      xp = const_cast<void *>(c.fuse.pad16); // the producer already wrote the padded copy
     } else {
-      SCN_TRY(stream_scratch(s, kScratchBf16, (size_t)nInRows * Cp * 2 + 16, &xp));
-      launch_pad_rows16(in, xp, nInRows, Cin, Cp, f16, s);
+      SCN_TRY(stream_scratch(s, kScratchBf16, (size_t)c.nInRows * Cp * 2 + 16, &xp));
+      launch_pad_rows16(c.in, xp, c.nInRows, Cin, Cp, f16, s);
     }
-    tl_prepad = nullptr;
-    return launch_conv_plan_tc(in, out, W, nbr, outRow, tileMask, nOut, K, Cp, Cout, bias, mathMode, s, tileW, nWeights, nInRows, xp, wTag, addend, out16, nOutRows, Cin, wT);
+    p.in16 = xp; p.Cin = Cp; p.CinW = Cin;
+    return launch_conv_plan_tc(p, s);
   }
   if (Cin % 32 != 0 && !(canPack && Cin == 16)) { // rows zero-padded to a multiple of 32 channels (the weight image pads itself)
     const int Cp = (Cin + 31) / 32 * 32;
     float *xp = nullptr;
-    SCN_TRY(stream_scratch(s, kScratchPad, (size_t)nInRows * Cp * 4 + 16, (void **)&xp));
-    k_pad_rows<<<stream_grid(nInRows * Cp, 256), 256, 0, LS(s)>>>(in, xp, nInRows, Cin, Cp);
-    return launch_conv_plan_tc(xp, out, W, nbr, outRow, tileMask, nOut, K, Cp, Cout, bias, mathMode, s, tileW, nWeights, nInRows, nullptr, wTag, addend, out16, nOutRows, Cin, wT);
+    SCN_TRY(stream_scratch(s, kScratchPad, (size_t)c.nInRows * Cp * 4 + 16, (void **)&xp));
+    k_pad_rows<<<stream_grid(c.nInRows * Cp, 256), 256, 0, LS(s)>>>(c.in, xp, c.nInRows, Cin, Cp);
+    TcConv p = c;
+    p.in = xp; p.in16 = nullptr; p.Cin = Cp; p.CinW = Cin;
+    return launch_conv_plan_tc(p, s);
   }
   SCN_CHECK(Cout % 16 == 0 && Cout >= 16 && Cout <= 256 && K <= 64, "tcgen05 path: unsupported channel counts");
   static int envT = -1, envS = -1, envDbg = 0, envProf = 0, envCtas = 0;
@@ -1104,19 +1073,22 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
     envProf = getenv("SCN_TC_PROF") ? atoi(getenv("SCN_TC_PROF")) : 0;
   }
   TcParams P;
-  P.in = reinterpret_cast<const unsigned char *>(in); P.out = out; P.bias = bias; P.addend = addend; P.out16 = out16; P.nbr = nbr; P.outRow = outRow; P.tileMask = tileMask; P.tileW = tileW;
+  P.in = reinterpret_cast<const unsigned char *>(c.in); P.out = c.out; P.bias = c.bias; P.addend = c.addend; P.out16 = c.out16; P.nbr = c.nbr; P.outRow = c.outRow; P.tileMask = c.tileMask; P.tileW = c.tileW;
   P.nOut = nOut; P.K = K; P.Cout = Cout;
   // bf16 / fp16 mode: rows of >= 64 channels are whole 128-byte atoms; 32- and 16-channel rows (64 / 32 bytes) are PACKED, G = 2 / 4
   // filter offsets side by side in one atom: half / a quarter of the stages, gather bytes and MMAs of the 128-byte-row layout
   const int packG = (canPack && (Cin == 32 || Cin == 16)) ? 64 / Cin : 1;
-  P.bf16 = (half_mode(mathMode) && (Cin % 64 == 0 || packG > 1)) ? 1 : 0; // 16-bit operands (fp16 in mode 5); other narrow layers keep TF32 operands
+  P.bf16 = (half_mode(c.mathMode) && (Cin % 64 == 0 || packG > 1)) ? 1 : 0; // 16-bit operands (fp16 in mode 5); other narrow layers keep TF32 operands
   P.f16 = f16 && !P.bf16; // (a TF32-operand launch in fp16 mode writes its 16-bit copy as fp16)
-  const bool x3 = mathMode == 3 && !P.bf16; // TF32X3: the fp32 rows split into two TF32 operands (one-CTA configuration, stages twice as large)
+  // TF32X3: the fp32 rows split into two TF32 operands (one-CTA configuration, stages twice as large)
+  const int op = P.bf16 ? (f16 ? kOpF16 : kOpBF16) : (c.mathMode == 3 ? kOpTF32X3 : kOpTF32);
+  const bool x3 = op == kOpTF32X3;
   void *tmp16 = nullptr;
   if (P.bf16) {
+    const void *in16 = c.in16;
     if (!in16) {
-      SCN_TRY(stream_scratch(s, kScratchBf16, (size_t)nInRows * Cin * 2 + 16, &tmp16));
-      if (nInRows) SCN_CUDA(launch_to_16(in, tmp16, nInRows * Cin / 4, f16, s));
+      SCN_TRY(stream_scratch(s, kScratchBf16, (size_t)c.nInRows * Cin * 2 + 16, &tmp16));
+      if (c.nInRows) SCN_CUDA(launch_to_16(c.in, tmp16, c.nInRows * Cin / 4, f16, s));
       in16 = tmp16;
     }
     P.in = static_cast<const unsigned char *>(in16);
@@ -1150,8 +1122,8 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   if (ctas == 1) while (T > 2 && ring(T) < 3) T--; // a 2-slot ring exposes the gather latency (measured: T=3/S=3 beats T=4/S=2 by 12 %)
   while (T > 1 && ring(T) < 2) T--;
   while (T > 1 && cdiv(P.nTiles, T) < 2 * kSMs * ctas) T--;
-  if (tileW) T = 1;
-  if (envT > 0 && envT <= Tcap && !tileW && ring(envT) >= 2) T = envT; // (a forced T must leave room for a 2-stage ring)
+  if (c.tileW) T = 1;
+  if (envT > 0 && envT <= Tcap && !c.tileW && ring(envT) >= 2) T = envT; // (a forced T must leave room for a 2-stage ring)
   P.T = T;
   P.nAcc = 2 * T * Cout <= P.tmemCols ? 2 : 1;
   P.nSuper = cdiv(P.nTiles, P.T);
@@ -1161,13 +1133,12 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   // items on, one CTA per item doing all offsets is as fast and needs one launch instead of three.
   static int kSplitMaxItems = -1;
   if (kSplitMaxItems < 0) kSplitMaxItems = getenv("SCN_TC_SPLIT_MAX") ? atoi(getenv("SCN_TC_SPLIT_MAX")) : 40;
-  if (P.nSuper <= kSplitMaxItems && !tileW) P.kSplit = std::max(1, std::min(packG > 1 ? P.KG : K, kSMs * ctas / P.nSuper));
+  if (P.nSuper <= kSplitMaxItems && !c.tileW) P.kSplit = std::max(1, std::min(packG > 1 ? P.KG : K, kSMs * ctas / P.nSuper));
   P.stats = nullptr;
   P.statsPart = nullptr;
   P.part = nullptr;
   const bool det = deterministic();
-  if (tl_stats && P.kSplit == 1 && Cout <= kFusedStatsC && Cout % 32 == 0) { P.stats = tl_stats; tl_stats_done = true; ++g_counters[kCntEpilogueStats]; }
-  tl_stats = nullptr;
+  if (c.fuse.stats && P.kSplit == 1 && Cout <= kFusedStatsC && Cout % 32 == 0) { P.stats = c.fuse.stats; if (c.fused) c.fused->stats = true; ++g_counters[kCntEpilogueStats]; }
   if (P.stats) { // deterministic mode: per-(item, epilogue warp) sums, added in item order after the launch
     if (det) SCN_TRY(det_scratch(s, (size_t)P.nSuper * 4 * 2 * Cout * sizeof(double), (void **)&P.statsPart));
     else ++g_counters[kCntFloatAtomic];
@@ -1180,39 +1151,39 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   P.lag = std::max(0, std::min(3, envLag >= 0 ? envLag : P.S - 2));
   if (P.lag > P.S - 2) P.lag = std::max(0, P.S - 2);
   const size_t smem = (size_t)P.S * stageBytes + fixed;
-  SCN_CHECK(out || (P.kSplit == 1 && out16), "tcgen05 path: fp32 output dropped on a launch that needs it");
+  SCN_CHECK(c.out || (P.kSplit == 1 && c.out16), "tcgen05 path: fp32 output dropped on a launch that needs it");
   ++g_counters[kCntTcLaunch];
   if (x3) ++g_counters[kCntTf32x3Launch];
-  if (f16 && P.bf16) ++g_counters[kCntF16Launch];
+  if (op == kOpF16) ++g_counters[kCntF16Launch];
   if (P.kSplit > 1) ++g_counters[kCntSplitLaunch];
   if (P.kSplit > 1 && det) SCN_TRY(det_scratch(s, (size_t)P.kSplit * nOut * Cout * 4, (void **)&P.part)); // (k_split_sum writes every output row)
-  else if (P.kSplit > 1) { ++g_counters[kCntFloatAtomic]; SCN_CUDA(cudaMemsetAsync(out, 0, (size_t)nOut * Cout * 4, s)); }
+  else if (P.kSplit > 1) { ++g_counters[kCntFloatAtomic]; SCN_CUDA(cudaMemsetAsync(c.out, 0, (size_t)nOut * Cout * 4, s)); }
   unsigned char *wimg = nullptr;
   bool wimgOwned = false;
   const int el16 = f16 ? kWimgF16 : kWimgBF16; // element format of a 16-bit image
-  SCN_TRY(get_wimg(W, wTag, nWeights, Cin, CinW, Cout, packG > 1 ? el16 + 16 * packG : x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg, &wimgOwned, wT));
+  SCN_TRY(get_wimg(c.W, c.wTag, c.nWeights, Cin, CinW, Cout, packG > 1 ? el16 + 16 * packG : x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg, &wimgOwned, c.wT));
   P.wimg = wimg;
   P.in2 = nullptr; P.wimg2 = nullptr; P.rowBytes2 = 0; P.nAtoms2 = 0;
   unsigned char *wimg2 = nullptr;
   bool wimg2Owned = false;
-  if (tl_lat.in && packG == 1 && K < kLateralBit && tl_lat.rows > 0 && (!P.bf16 || tl_lat.in16)) {
-    const int esz = P.bf16 ? 2 : 4, per = 128 / esz, C2 = tl_lat.Cin; // per = channels of one K atom
+  const Lateral &lat = c.fuse.lat; // taken when the launch is a whole-atom (unpacked) tensor-core launch
+  if (lat.in && packG == 1 && K < kLateralBit && lat.rows > 0 && (!P.bf16 || lat.in16)) {
+    const int esz = P.bf16 ? 2 : 4, per = 128 / esz, C2 = lat.Cin; // per = channels of one K atom
     if ((C2 * esz) % 16 == 0) {
       const int C2p = (C2 + per - 1) / per * per;
-      SCN_TRY(get_wimg(tl_lat.w, tl_lat.tag, 1, C2p, C2, Cout, x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg2, &wimg2Owned));
-      P.in2 = static_cast<const unsigned char *>(P.bf16 ? tl_lat.in16 : static_cast<const void *>(tl_lat.in));
+      SCN_TRY(get_wimg(lat.w, lat.tag, 1, C2p, C2, Cout, x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg2, &wimg2Owned));
+      P.in2 = static_cast<const unsigned char *>(P.bf16 ? lat.in16 : static_cast<const void *>(lat.in));
       P.rowBytes2 = C2 * esz;
       P.nAtoms2 = C2p / per;
       P.wimg2 = wimg2;
-      tl_lat_done = true;
+      if (c.fused) c.fused->lateral = true;
       ++g_counters[kCntLateralFolded];
     }
   }
-  tl_lat.in = nullptr;
   static bool attr = false;
   if (!attr) {
-    SCN_TRY(set_plan_attributes<false>());
-    SCN_TRY(set_plan_attributes<true>());
+    const int half = (233472 - kBuildRoom) / 2 - 1024;
+    for (const PlanKernel &k : kPlanKernels) SCN_CUDA(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, k.ctas == 1 ? 227 * 1024 : half));
     attr = true;
   }
   static int envSms = -1;
@@ -1230,10 +1201,13 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
   // producer warps of the two-CTA configuration: 4 (96 registers) or 8 (72 registers); bit 0 = packed layers, bit 1 = whole-atom layers
   static int envPw8 = -1;
   if (envPw8 < 0) envPw8 = getenv("SCN_TC_PW8") ? atoi(getenv("SCN_TC_PW8")) : 0;
-  const bool pw8 = ctas == 2 && ((packG > 1 && (envPw8 & 1)) || (packG == 1 && (envPw8 & 2)));
-  const int th2 = 32 * (pw8 ? 14 : 10);
-  if (det) SCN_CUDA(launch_plan_variant<true>(P, packG, pw8, ctas, grid, th2, smem, s, x3, f16));
-  else SCN_CUDA(launch_plan_variant<false>(P, packG, pw8, ctas, grid, th2, smem, s, x3, f16));
+  const int pw = ctas == 1 || (packG > 1 && (envPw8 & 1)) || (packG == 1 && (envPw8 & 2)) ? 8 : 4;
+  const PlanKernel *kern = nullptr;
+  for (const PlanKernel &k : kPlanKernels)
+    if (k.op == op && k.pw == pw && k.G == packG && k.ctas == ctas && k.det == det) kern = &k;
+  SCN_CHECK(kern, "tcgen05 path: no kernel instantiated for this configuration");
+  // warps: 4 epilogue, the producers, the MMA issuer, the weight loader (and the TF32X3 splitters)
+  SCN_CUDA(launch_pdl(kern->fn, dim3(grid), dim3(32 * (4 + pw + 2 + (x3 ? kSplitWarps : 0))), smem, LS(s), P));
   SCN_CUDA(cudaGetLastError());
   if (envProf) { // developer aid: mean stall cycles per role over the CTAs of this launch
     static long long h[2 * kSMs * 32];
@@ -1242,57 +1216,18 @@ int launch_conv_plan_tc(const float *in, float *out, const float *W, const int *
     double m[32] = {0};
     for (int b = 0; b < grid; b++) for (int i = 0; i < 32; i++) m[i] += (double)h[b * 32 + i] / grid;
     fprintf(stderr, "[tcprof] ctas=%d pw=%d grid=%d T=%d K=%d Cin=%d Cout=%d S=%d lag=%d nAcc=%d kSplit=%d | epi total %.0f waitAcc %.0f | prod total %.0f empty %.0f cpwait %.0f stages %.0f | mma total %.0f accEmpty %.0f full %.0f stages %.0f issue %.0f commit %.0f | bld total %.0f empty %.0f\n",
-            ctas, x3 || ctas == 1 || pw8 ? 8 : 4, grid, P.T, K, Cin, Cout, P.S, P.lag, P.nAcc, P.kSplit, m[0], m[1], m[4], m[5], m[6], m[7], m[10], m[11], m[12], m[13], m[14], m[15], m[16], m[17]);
+            ctas, pw, grid, P.T, K, Cin, Cout, P.S, P.lag, P.nAcc, P.kSplit, m[0], m[1], m[4], m[5], m[6], m[7], m[10], m[11], m[12], m[13], m[14], m[15], m[16], m[17]);
     cudaFreeAsync(P.prof, s);
   }
   if (P.statsPart) SCN_TRY(ordered_sum(P.statsPart, P.nSuper * 4, 2l * Cout, P.stats, s, Cout, kFusedStatsC)); // into replica 0
   if (P.part) // the split partials in split order, and the 16-bit copy from the same registers
     SCN_CUDA(launch_pdl(f16 ? k_split_sum<true> : k_split_sum<false>, dim3(stream_grid((long)nOut * Cout / 4, 256)), dim3(256), 0, LS(s),
-                        reinterpret_cast<const float4 *>(P.part), P.kSplit, (long)nOut * Cout / 4, reinterpret_cast<float4 *>(out), static_cast<uint2 *>(out16)));
-  else if (out16 && P.kSplit > 1 && nOutRows > 0) // partial sums were accumulated atomically: the 16-bit copy needs the finished rows
-    SCN_CUDA(launch_to_16(out, out16, nOutRows * Cout / 4, f16, s));
+                        reinterpret_cast<const float4 *>(P.part), P.kSplit, (long)nOut * Cout / 4, reinterpret_cast<float4 *>(c.out), static_cast<uint2 *>(c.out16)));
+  else if (c.out16 && P.kSplit > 1 && c.nOutRows > 0) // partial sums were accumulated atomically: the 16-bit copy needs the finished rows
+    SCN_CUDA(launch_to_16(c.out, c.out16, c.nOutRows * Cout / 4, f16, s));
   if (wimgOwned) cudaFreeAsync(wimg, s);
   if (wimg2Owned) cudaFreeAsync(wimg2, s);
 
-  return 0;
-}
-
-// A plan of more than 64 filter offsets (chunk-major, common.cuh) runs as one launch per chunk of <= 63 offsets.  Chunk c is an
-// ordinary plan -- its own block of neighbour ids and mask array, the weights of its offsets -- and takes the running sum of the
-// chunks before it as its fused addend.  Bias and the caller's addend go into chunk 0; the lateral stage, the epilogue statistics
-// and the bf16 copy into the last chunk, the only one that sees finished rows.  The running sums alternate between two scratch
-// buffers, so no launch reads rows it writes (an offset-split launch zeroes its output first).  Each chunk boundary adds one fp32
-// rounding of the partial sum (DESIGN.md section 7).
-static int launch_conv_plan_tc_chunked(const float *in, float *out, const float *W, const int *nbr, const int *outRow, const unsigned long long *tileMask,
-                                       int nOut, int K, int Cin, int Cout, const float *bias, int mathMode, cudaStream_t s, long nInRows, const void *in16,
-                                       long long wTag, const float *addend, void *out16, long nOutRows, int CinW, int wT) {
-  const int nC = plan_chunks(K);
-  const long nPad = plan_padded(nOut);
-  float *run = nullptr;
-  SCN_TRY(stream_scratch(s, kScratchChunk, (size_t)std::min(nC - 1, 2) * nOutRows * Cout * 4 + 16, (void **)&run));
-  // the side channels are consumed by the first launch that can take them: hold them back for the chunk they belong to
-  const Lateral lat = tl_lat;
-  double *const stats = tl_stats;
-  const void *const pre = tl_prepad;
-  const int preC = tl_prepad_c;
-  tl_lat.in = nullptr;
-  tl_stats = nullptr;
-  const float *prev = addend;
-  for (int c = 0; c < nC; c++) {
-    const int k0 = c * kChunkOffsets, Kc = std::min(kChunkOffsets, K - k0);
-    const bool last = c == nC - 1;
-    float *dst = last ? out : run + (size_t)(c & 1) * nOutRows * Cout;
-    // W: [K][CinW][Cout] (or [K][Cout][CinW] transposed): CinW x Cout floats per offset.  Offset-reversed operands (wT = 2): offset j
-    // of this chunk is W[K - 1 - k0 - j], i.e. the reversal of the block W[K - k0 - Kc, K - k0)
-    const float *Wc = W + (size_t)(wT == 2 ? K - k0 - Kc : k0) * CinW * Cout;
-    if (last) { tl_lat = lat; tl_stats = stats; }
-    tl_prepad = pre;
-    tl_prepad_c = preC;
-    ++g_counters[kCntChunkedLaunch];
-    SCN_TRY(launch_conv_plan_tc(in, dst, Wc, nbr + (size_t)k0 * nPad, outRow, tileMask + (size_t)c * (nPad / 128), nOut, Kc, Cin, Cout, c == 0 ? bias : nullptr,
-                                mathMode, s, nullptr, Kc, nInRows, in16, wTag, prev, last ? out16 : nullptr, nOutRows, CinW, wT));
-    prev = dst;
-  }
   return 0;
 }
 

@@ -10,7 +10,6 @@
 
 struct scn_metadata; // capi.cu
 namespace scn {
-Metadata *metadata_of(scn_metadata *m);
 namespace {
 template <bool BACKWARD>
 __global__ void __launch_bounds__(256) k_sparse_dense(const int *__restrict__ id2pOrP2id, const int4 *__restrict__ coords, int n, int C, long vol, int sy, int sz,

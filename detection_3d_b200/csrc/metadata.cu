@@ -38,7 +38,6 @@ std::atomic<int> g_pool_growth{0};
 void set_pool_growth(int on) { g_pool_growth.store(on); }
 long debug_chunk_mallocs() { return g_chunk_mallocs; }
 long debug_chunk_waits() { return g_chunk_waits; }
-long debug_chunk_total_mb() ;
 static size_t g_chunk_bytes_total = 0; // every chunk ever taken from the driver and not returned
 constexpr size_t kChunkKeep = 32ull << 30; // beyond this much idle memory, chunks go back to the driver
 long debug_chunk_total_mb() { return (long)(g_chunk_bytes_total >> 20); }

@@ -13,6 +13,8 @@
 #include <atomic>
 #include <thread>
 
+struct scn_metadata;
+
 namespace scn {
 
 typedef std::array<long, 3> P3;
@@ -200,6 +202,15 @@ struct Metadata {
   int build_tile_masks(NbrPlan &plan);
   int get_deconv_plan(ConvEntry &e);
 };
+int build_subm_on_caller(Metadata &md, const long *sz, const long *f);
+void set_prefetch_worker_thread(bool on, int ctx);
+// the process-wide chunk pool (scn_set_pool_growth, scn_debug_counter(0..2), scn_release_cached_memory)
+void set_pool_growth(int on);
+long debug_chunk_mallocs();
+long debug_chunk_waits();
+long debug_chunk_total_mb();
+long release_idle_chunks();
+Metadata *metadata_of(scn_metadata *m); // (capi.cu)
 
 // ------------------------------------------------------------------ device helpers
 __host__ __device__ __forceinline__ uint32_t point_hash(int x, int y, int z) {

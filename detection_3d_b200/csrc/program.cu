@@ -6,32 +6,13 @@
 // same results; feature tensors live in registers whose buffers the executor allocates on the
 // caller's stream and frees after their last use.
 #include "../../include/scn_b200.h"
-#include "common.cuh"
+#include "conv.cuh"
 #include <algorithm>
 #include <stdlib.h>
 #include <array>
 #include <deque>
 #include <utility>
 #include <vector>
-
-namespace scn {
-void epilogue_stats_arm(double *sums);
-bool epilogue_stats_take();
-void lateral_arm(const float *in, const void *in16, const float *w, long long tag, int Cin, long rows);
-bool lateral_take();
-void prepadded_arm(const void *rows16, int Cp);
-void bwd_in16_arm(const void *in16);
-bool dw_tc_ok(int Cin, int Cout, int K, int mathMode);
-int from_16(const void *x, float *y, long n, cudaStream_t s);
-int batchnorm_backward_y16(const float *in, float *d_in, const float *out, const void *out_bf16, float *d_out, long n, int C, const float *save_mean,
-                           const float *save_invstd, const float *weight, float *d_weight, float *d_bias, float leak, cudaStream_t s);
-void prepadded_disarm();
-int build_subm_on_caller(scn_metadata *m, const long *sz, const long *f);
-int bn_forward_from_sums(const float *x, float *y, long n, int C, const double *sums, float *saveMean, float *saveInvStd, float *runningMean,
-                         float *runningVar, const float *weight, const float *bias, float eps, float momentum, int mode, float leak, cudaStream_t s, void *y16);
-bool backward_reads_lists(int kind, const long *f, const long *st, int Cin, int Cout, bool wantDIn);
-cudaStream_t metadata_stream(scn_metadata *m);
-} // namespace scn
 
 namespace {
 
@@ -563,16 +544,22 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
     SCN_CUDA(cudaMemsetAsync(p->stats, 0, p->nStats * statsStride * sizeof(double), s));
     p->statsDone.assign(p->nStats, 0);
   }
-  auto arm = [&](const Op &op) { if (op.a[21] >= 0) scn::epilogue_stats_arm(p->stats + op.a[21] * statsStride); };
-  auto took = [&](const Op &op) { const bool d = scn::epilogue_stats_take(); if (op.a[21] >= 0) p->statsDone[op.a[21]] = d; };
-  auto arm_lateral = [&](const Op &op) {
-    if (op.a[18] < 0) return;
-    const Reg &Y = p->regs[op.a[18]];
-    scn::lateral_arm(Y.p, Y.pad16 ? nullptr : Y.p16, P(op.a[19]), T(op.a[19]), (int)op.a[20], Y.rows);
+  // what a convolution op asks its launch to fold in: the lateral (a[18..20]), the statistics of the BatchNorm that reads its output
+  // (a[21]) and, for a submanifold convolution of the network input, the input layer's zero-padded 16-bit rows
+  auto fusion_of = [&](const Op &op) {
+    scn::ConvFusion f;
+    if (op.a[21] >= 0) f.stats = p->stats + op.a[21] * statsStride;
+    if (op.a[18] >= 0) {
+      const Reg &Y = p->regs[op.a[18]];
+      f.lat = scn::Lateral{Y.p, Y.pad16 ? nullptr : Y.p16, P(op.a[19]), T(op.a[19]), (int)op.a[20], Y.rows};
+    }
+    const Reg &I = p->regs[op.a[0]];
+    if (op.kind == K_SUBM && I.pad16) { f.pad16 = I.p16; f.padC = I.pad16; }
+    return f;
   };
   // the convolution did not take the lateral (e.g. it ran on the CUDA-core path): run the 1x1x1 convolution on its own and add it
-  auto lateral_fallback = [&](const Op &op, scn_metadata *md, const long *sz, Reg &out, int Cout) -> int {
-    const bool done = scn::lateral_take();
+  auto lateral_fallback = [&](const Op &op, const scn::ConvFused &fused, scn_metadata *md, const long *sz, Reg &out, int Cout) -> int {
+    const bool done = fused.lateral;
     if (op.a[18] < 0) return 0;
     const Reg &Y = p->regs[op.a[18]];
     macs += (double)Y.rows * (double)op.a[20] * Cout;
@@ -583,7 +570,8 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
     if (!tmp) return -1;
     const long one[3] = {1, 1, 1};
     double mk2 = 0;
-    int r = scn_submanifold_convolution_forward(md, sz, one, Y.p, tmp, P(op.a[19]), nullptr, (int)op.a[20], Cout, &mk2, Y.pad16 ? nullptr : Y.p16, T(op.a[19]), nullptr, nullptr);
+    int r = scn::submanifold_forward(md, sz, one, Y.p, tmp, P(op.a[19]), nullptr, (int)op.a[20], Cout, &mk2, Y.pad16 ? nullptr : Y.p16, T(op.a[19]), nullptr, nullptr,
+                                     scn::ConvFusion(), nullptr);
     if (r == 0) r = scn_add_features(out.p, tmp, out.p, out.rows * Cout, s, out.p16);
     slot_put(p, tmp);
     return r;
@@ -616,55 +604,30 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
         } else if (rc == 0 && nActive) rc = scn_input_layer_forward(M, feats, p->regs[a[0]].p, (int)a[6]);
         break;
       }
-      case K_SUBM: { // in, out, size[3], filter[3], w, bias, Cin, Cout
+      case K_SUBM: case K_CONV: case K_DECONV: { // in, out, then subm: size[3], filter[3], w, bias, Cin, Cout; (de)conv: inS[3], outS[3], f[3], s[3], w, bias, Cin, Cout
+        const bool subm = op.kind == K_SUBM;
         long n = 0;
-        if (firstPlanHere && !firstPlanDone) { // the first plan of an unprepared forward: built here, now (see build_subm_on_caller)
+        if (subm && firstPlanHere && !firstPlanDone) { // the first plan of an unprepared forward: built here, now (see build_subm_on_caller)
           firstPlanDone = true;
           rc = scn::build_subm_on_caller(M, a + 2, a + 5);
           if (rc) break;
         }
-        rc = scn_get_nactive(M, a + 2, &n);
+        if (op.kind == K_CONV) rc = scn_convolution_prepare(M, a + 2, a + 5, a + 8, a + 11, &n, nullptr);
+        else rc = scn_get_nactive(M, subm ? a + 2 : a + 5, &n);
+        const int Cout = (int)(subm ? a[11] : a[17]);
         const bool half = !train && a[23] == 1 && scn::half_mode(mode) && n >= kHalfOnlyRows && scn_tensor_core_path_available();
-        if (rc == 0) rc = alloc_reg(a[1], n, (int)a[11], half || a[22] >= 0 || a[18] >= 0, half);
-        const Reg &I = p->regs[a[0]];
-        if (rc == 0) { arm(op); arm_lateral(op); }
-        if (rc == 0 && I.pad16) scn::prepadded_arm(I.p16, I.pad16);
-        if (rc == 0)
-          rc = scn_submanifold_convolution_forward(M, a + 2, a + 5, I.p, p->regs[a[1]].p, P(a[8]), P(a[9]), (int)a[10], (int)a[11], &mk, I.pad16 ? nullptr : I.p16, T(a[8]),
-                                                   a[22] >= 0 ? p->regs[a[22]].p : nullptr, p->regs[a[1]].p16);
-        took(op);
-        scn::prepadded_disarm();
-        if (rc == 0) rc = lateral_fallback(op, M, a + 2, p->regs[a[1]], (int)a[11]);
-        macs += mk;
-        break;
-      }
-      case K_CONV: { // in, out, inS[3], outS[3], f[3], s[3], w, bias, Cin, Cout
-        long n = 0, nr = 0;
-        rc = scn_convolution_prepare(M, a + 2, a + 5, a + 8, a + 11, &n, &nr);
-        const bool half = !train && a[23] == 1 && scn::half_mode(mode) && n >= kHalfOnlyRows && scn_tensor_core_path_available();
-        if (rc == 0) rc = alloc_reg(a[1], n, (int)a[17], half || a[22] >= 0 || a[18] >= 0, half);
-        const Reg &I = p->regs[a[0]];
-        if (rc == 0) { arm(op); arm_lateral(op); }
-        if (rc == 0)
-          rc = scn_convolution_forward(M, a + 2, a + 5, a + 8, a + 11, I.p, p->regs[a[1]].p, P(a[14]), P(a[15]), (int)a[16], (int)a[17], &mk, I.pad16 ? nullptr : I.p16, T(a[14]),
-                                       a[22] >= 0 ? p->regs[a[22]].p : nullptr, p->regs[a[1]].p16);
-        took(op);
-        if (rc == 0) rc = lateral_fallback(op, M, a + 5, p->regs[a[1]], (int)a[17]);
-        macs += mk;
-        break;
-      }
-      case K_DECONV: {
-        long n = 0;
-        rc = scn_get_nactive(M, a + 5, &n);
-        const bool half = !train && a[23] == 1 && scn::half_mode(mode) && n >= kHalfOnlyRows && scn_tensor_core_path_available();
-        if (rc == 0) rc = alloc_reg(a[1], n, (int)a[17], half || a[22] >= 0 || a[18] >= 0, half);
-        const Reg &I = p->regs[a[0]];
-        if (rc == 0) { arm(op); arm_lateral(op); }
-        if (rc == 0)
-          rc = scn_deconvolution_forward(M, a + 2, a + 5, a + 8, a + 11, I.p, p->regs[a[1]].p, P(a[14]), P(a[15]), (int)a[16], (int)a[17], &mk, I.pad16 ? nullptr : I.p16, T(a[14]),
-                                         a[22] >= 0 ? p->regs[a[22]].p : nullptr, p->regs[a[1]].p16);
-        took(op);
-        if (rc == 0) rc = lateral_fallback(op, M, a + 5, p->regs[a[1]], (int)a[17]);
+        if (rc == 0) rc = alloc_reg(a[1], n, Cout, half || a[22] >= 0 || a[18] >= 0, half);
+        const Reg &I = p->regs[a[0]], &O = p->regs[a[1]];
+        const void *in16 = I.pad16 ? nullptr : I.p16;
+        const float *add = a[22] >= 0 ? p->regs[a[22]].p : nullptr;
+        scn::ConvFused fused;
+        if (rc == 0 && subm)
+          rc = scn::submanifold_forward(M, a + 2, a + 5, I.p, O.p, P(a[8]), P(a[9]), (int)a[10], Cout, &mk, in16, T(a[8]), add, O.p16, fusion_of(op), &fused);
+        else if (rc == 0)
+          rc = (op.kind == K_CONV ? scn::convolution_forward : scn::deconvolution_forward)(M, a + 2, a + 5, a + 8, a + 11, I.p, O.p, P(a[14]), P(a[15]), (int)a[16], Cout,
+                                                                                            &mk, in16, T(a[14]), add, O.p16, fusion_of(op), &fused);
+        if (a[21] >= 0) p->statsDone[a[21]] = fused.stats;
+        if (rc == 0) rc = lateral_fallback(op, fused, M, subm ? a + 2 : a + 5, p->regs[a[1]], Cout);
         macs += mk;
         break;
       }
@@ -713,10 +676,7 @@ int scn_program_run(scn_program *p, scn_metadata *m, const long *coords, int coo
         if (R.p16) { slot_put(p, R.p16); R.p16 = nullptr; }
       }
   }
-  if (rc) { // no fusion request may stay armed for the next convolution this thread makes
-    scn::lateral_take();
-    scn::epilogue_stats_take();
-    scn::prepadded_disarm();
+  if (rc) {
     release_regs(p, true);
     if (p->internal) scn_metadata_wait_jobs(m); // the twin reads p->ms, which the next run destroys
     return rc;
@@ -853,7 +813,7 @@ int scn_program_backward(scn_program *p, int n_out, const int *out_regs, const f
         }
         // bf16 mode: the forward pass left a bf16 copy of the input rows (same layout: whole rows, no padding) -- the
         // weight-gradient kernel gathers from it instead of converting the fp32 rows again
-        if (I.p16 && !I.pad16 && Cin % 32 == 0 && scn::half_mode(scn_get_math_mode())) scn::bwd_in16_arm(I.p16);
+        const void *in16 = I.p16 && !I.pad16 && Cin % 32 == 0 && scn::half_mode(scn_get_math_mode()) ? I.p16 : nullptr;
         const float *inRows = I.p;
         float *inTmp = nullptr;
         if (!inRows) { // the forward pass kept only the bf16 copy of these rows (a BatchNorm output read by tensor-core convolutions alone)
@@ -866,9 +826,8 @@ int scn_program_backward(scn_program *p, int n_out, const int *out_regs, const f
             inRows = inTmp;
           }
         }
-        if (op.kind == K_SUBM) rc = scn_submanifold_convolution_backward(m, a + 2, a + 5, inRows, din, dy, P(wi), dw, G(bi), Cin, Cout);
-        else if (op.kind == K_CONV) rc = scn_convolution_backward(m, a + 2, a + 5, a + 8, a + 11, inRows, din, dy, P(wi), dw, G(bi), Cin, Cout);
-        else rc = scn_deconvolution_backward(m, a + 2, a + 5, a + 8, a + 11, inRows, din, dy, P(wi), dw, G(bi), Cin, Cout);
+        if (op.kind == K_SUBM) rc = scn::submanifold_backward(m, a + 2, a + 5, inRows, din, dy, P(wi), dw, G(bi), Cin, Cout, in16);
+        else rc = (op.kind == K_CONV ? scn::convolution_backward : scn::deconvolution_backward)(m, a + 2, a + 5, a + 8, a + 11, inRows, din, dy, P(wi), dw, G(bi), Cin, Cout, in16);
         if (dwTmp) slot_put(p, dwTmp);
         if (inTmp) slot_put(p, inTmp);
         done(wi); done(bi);

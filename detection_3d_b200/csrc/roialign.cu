@@ -17,7 +17,6 @@
 
 struct scn_metadata;
 namespace scn {
-Metadata *metadata_of(scn_metadata *m);
 namespace {
 struct RoiGeom {
   float cw, ch, cz, w, h, z, cosT, sinT, binH, binW, binZ, startH, startW, startZ;

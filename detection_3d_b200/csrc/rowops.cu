@@ -4,7 +4,7 @@
 //
 // Replaces BatchNormalization_f_train/f_test/b (SCN/CUDA/BatchNormalization.cu:14-198, which run
 // on <= 16 CTAs) and InputLayer_fp_/bp_ (SCN/CUDA/IOLayers.cu:14-58).
-#include "common.cuh"
+#include "conv.cuh"
 #include <cuda_bf16.h>
 
 namespace scn {

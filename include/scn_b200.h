@@ -361,8 +361,10 @@ long scn_debug_counter(int which);
  * recorded programs keep their memory (destroy them first). */
 long scn_release_cached_memory(void);
 
-/* Fusion requests for the NEXT convolution forward call made by this thread (what the program executor uses to fold the
- * FPN's lateral 1x1x1 convolution and the statistics of a following BatchNorm into a convolution; no reference counterpart:
+/* Fusion requests for the next call this thread makes to scn_submanifold_convolution_forward, scn_convolution_forward or
+ * scn_deconvolution_forward, and to no other entry: that call takes the pending requests when it is entered, whether or not it
+ * can honour them (the fusions of a recorded program: the FPN's lateral 1x1x1 convolution and the statistics of a following
+ * BatchNorm folded into a convolution; no reference counterpart:
  * the reference runs NetworkInNetwork / SubmanifoldConvolution(1), AddTable and BatchNormalization as separate passes,
  * fpn_net.py:166-176, CPU/BatchNormalization.cpp:12-62).
  *  lateral: out = conv(in) [+ add_in] + lat_in[row] @ lat_weight ([n_in][n_out], one filter offset), lat_in_bf16 = 16-bit
@@ -370,8 +372,8 @@ long scn_release_cached_memory(void);
  *  stats:   sums = [8 replicas][2][128] doubles, zeroed by the caller; the launch adds per-channel sum (first 128) and sum
  *           of squares (second 128) of the rows it stores, spread over the replicas (deterministic mode: written into replica
  *           0 after the launch, in a fixed order).
- * A launch that cannot honour a request (CUDA-core path, packed rows, split offsets, > 128 channels) ignores it;
- * scn_fuse_result reports what the last call did and disarms both requests. */
+ * A call that cannot honour a request (CUDA-core path, packed rows, split offsets, > 128 channels) drops it;
+ * scn_fuse_result reports what the last of those three calls took and disarms both requests. */
 int scn_fuse_next_lateral(const float *lat_in, const void *lat_in_bf16, const float *lat_weight, long long weight_tag, int n_in, long rows);
 int scn_fuse_next_stats(double *sums);
 int scn_fuse_result(int *lateral_taken, int *stats_taken);
