@@ -674,8 +674,9 @@ int scn_iteration_order(scn_metadata *m, const long sz[3], int *dst) {
   return 0;
 }
 
+// (more than 256 output channels: column slabs of <= 256, launch_conv_plan_tc)
 static bool tc_ok(int Cin, int Cout, int K) {
-  return scn::g_math_mode != 0 && scn::tc_available() && Cout % 32 == 0 && Cout >= 32 && Cout <= 256 && K <= scn::kMaxFilterVolume && Cin >= 4 && Cin <= 1024;
+  return scn::g_math_mode != 0 && scn::tc_available() && Cout % 32 == 0 && Cout >= 32 && Cout <= 1024 && K <= scn::kMaxFilterVolume && Cin >= 4 && Cin <= 1024;
 }
 // out += addend (optional) and the 16-bit copy of out (optional), for the paths whose kernels do not fuse them
 static int plain_epilogue(float *out, const float *addend, void *out16, long rows, int C, cudaStream_t s) {

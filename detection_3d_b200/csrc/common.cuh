@@ -64,7 +64,8 @@ enum DebugCounter {
   kCntF16Launch = 18,      // tensor-core launches with fp16 operands (math mode 5): conv_plan_tc and the weight-gradient kernels
   kCntRulesAhead = 19,     // rule lists a backward entry found already built (hinted ahead by a training run, program.cu)
   kCntTrainPrepared = 20,  // training runs that took a Metadata prepared by scn_program_prepare_training
-  kCntCounters = 21
+  kCntSimtDwLaunch = 21,   // CUDA-core weight-gradient launches of the sparse convolutions (k_dw, one per rule list)
+  kCntCounters = 22
 };
 extern std::atomic<long> g_counters[kCntCounters];
 

@@ -37,6 +37,9 @@ struct TcConv {
   void *out16 = nullptr;      // optional: the result in the mode's 16-bit format
   long nOutRows = 0;
   int mathMode = 0;           // scn_set_math_mode: 1 = TF32, 2 = BF16, 3 = TF32X3, 5 = F16 operands (narrow layers keep TF32 in modes 2 and 5)
+  // column slab of a layer wider than 256 output channels (launch_conv_plan_tc_slabs): this launch computes output columns
+  // [col0, col0 + Cout) of rows ldOut wide -- out, addend, out16 and bias are full-width, W is [..][ldOut] (0: Cout, no slab)
+  int col0 = 0, ldOut = 0;
   ConvFusion fuse;
   ConvFused *fused = nullptr; // optional: set where the launch took a part of `fuse`
 };

@@ -163,6 +163,7 @@ int conv_backward_simt(const float *in, float *d_in, const float *d_out, const f
   for (int L_ = 0; L_ < K; L_++) {
     int len = offHost[L_ + 1] - offHost[L_];
     if (!len) continue;
+    ++g_counters[kCntSimtDwLaunch];
     SCN_TRY(dw_chunks(in, d_out, dW + (long)L_ * Cin * Cout, pairs, offHost[L_], len, Cin, Cout, srcIsY, s));
   }
   SCN_CUDA(cudaGetLastError());

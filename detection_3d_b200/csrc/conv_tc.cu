@@ -30,6 +30,7 @@
 #include <map>
 #include <mutex>
 #include <tuple>
+#include <vector>
 
 namespace scn {
 
@@ -67,7 +68,8 @@ struct TcParams {
   int rowBytes2, nAtoms2;
   double *stats;    // optional [kBnReplicas][2][kFusedStatsC]: per-channel sum / sum of squares of `out` (statistics of a following BatchNorm)
   long long *prof;  // developer: per-CTA stall counters (SCN_TC_PROF)
-  int nOut, K, Cout, nTiles, T, nSuper, S, nAcc, lag;
+  int nOut, K, Cout, ldo, nTiles, // ldo: row stride (elements) of out, addend and out16 -- Cout, or the full width of a column slab's rows
+      T, nSuper, S, nAcc, lag;
   int rowBytes, nAtoms, bf16, tmemCols;
   int KG;     // packed layers (template G > 1): number of offset groups = ceil(K / G)
   int dbg;    // developer switches (SCN_TC_DBG): 1 = skip A gathers, 2 = skip B copies, 4 = skip MMAs
@@ -392,7 +394,7 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
               float4 ad[4];
 #pragma unroll
               for (int i = 0; i < 4; i++)
-                ad[i] = rows[h + i] >= 0 ? __ldg(reinterpret_cast<const float4 *>(P.addend + (size_t)rows[h + i] * P.Cout + c0 + cc)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                ad[i] = rows[h + i] >= 0 ? __ldg(reinterpret_cast<const float4 *>(P.addend + (size_t)rows[h + i] * P.ldo + c0 + cc)) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
               for (int i = 0; i < 4; i++) { o[h + i].x += ad[i].x; o[h + i].y += ad[i].y; o[h + i].z += ad[i].z; o[h + i].w += ad[i].w; }
             }
@@ -421,9 +423,9 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
 #pragma unroll
             for (int i = 0; i < NI; i++)
               if (rows[i] >= 0) {
-                if (P.out) *reinterpret_cast<float4 *>(P.out + (size_t)rows[i] * P.Cout + c0 + cc) = o[i]; // null: only the bf16 copy is consumed
+                if (P.out) *reinterpret_cast<float4 *>(P.out + (size_t)rows[i] * P.ldo + c0 + cc) = o[i]; // null: only the bf16 copy is consumed
                 if (P.out16) {
-                  uint2 *dst16 = reinterpret_cast<uint2 *>(static_cast<unsigned char *>(P.out16) + ((size_t)rows[i] * P.Cout + c0 + cc) * 2);
+                  uint2 *dst16 = reinterpret_cast<uint2 *>(static_cast<unsigned char *>(P.out16) + ((size_t)rows[i] * P.ldo + c0 + cc) * 2);
                   if (OP == kOpF16 || (OP == kOpTF32 && P.f16)) *dst16 = pack16x4<true>(o[i]);
                   else *dst16 = pack16x4<false>(o[i]);
                 }
@@ -436,7 +438,7 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
 #pragma unroll
             for (int i = 0; i < NI; i++)
               if (rows[i] >= 0) {
-                float *dst = P.out + (size_t)rows[i] * P.Cout + c0 + cc;
+                float *dst = P.out + (size_t)rows[i] * P.ldo + c0 + cc;
                 atomicAdd(dst, o[i].x); atomicAdd(dst + 1, o[i].y); atomicAdd(dst + 2, o[i].z); atomicAdd(dst + 3, o[i].w);
               }
           }
@@ -739,7 +741,8 @@ __global__ void __launch_bounds__(CTAS == 1 ? 576 : (PW == 8 ? 448 : (SCN_EPI_CO
 // wT: 0 = W is [K][CinW][Cout]; 1 / 2 = the operand is the TRANSPOSE of a forward weight tensor stored as [K][Cout][CinW] (the input-gradient
 // convolutions: Wt[k'][co][ci] = W[k][ci][co]), 2 = with the filter offsets reversed as well (k' = K - 1 - k) -- read in place, no transposed copy.
 // el = element format: 0 = tf32, kWimgBF16, kWimgF16.
-__global__ void k_prep_wimg(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int Cin, int CinW, int Cout, int el, int wT) {
+// co0, ldW: the image holds output channels [co0, co0 + Cout) of a W whose output dimension is ldW wide (a column slab; 0, Cout otherwise).
+__global__ void k_prep_wimg(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int Cin, int CinW, int Cout, int el, int wT, int co0, int ldW) {
   const bool bf16 = el != 0; // (2-byte elements)
   const long n = (long)K * Cin * Cout;
   const int per = bf16 ? 64 : 32, nAtoms = Cin / per;
@@ -751,7 +754,7 @@ __global__ void k_prep_wimg(const float *__restrict__ W, unsigned char *__restri
     const int byte = j * (bf16 ? 2 : 4), chunk = byte >> 4, within = byte & 15;
     unsigned char *dst = img + ((long)k * nAtoms + c) * Cout * 128 + (long)co * 128 + ((chunk ^ (co & 7)) << 4) + within;
     const int ks = wT == 2 ? K - 1 - k : k;
-    const float w = ci < CinW ? (wT ? W[((long)ks * Cout + co) * CinW + ci] : W[((long)k * CinW + ci) * Cout + co]) : 0.f;
+    const float w = ci < CinW ? (wT ? W[((long)ks * ldW + co0 + co) * CinW + ci] : W[((long)k * CinW + ci) * ldW + co0 + co]) : 0.f;
     if (el == 3) { // (kWimgF16)
       *reinterpret_cast<unsigned short *>(dst) = to16<true>(w);
     } else if (bf16) {
@@ -766,7 +769,7 @@ __global__ void k_prep_wimg(const float *__restrict__ W, unsigned char *__restri
 
 // TF32X3 operands: the same image twice per (k, K atom), [W_hi atom][W_lo atom] side by side (one bulk copy per stage),
 // W_hi = tf32(w) and W_lo = tf32(w - W_hi), both exact TF32 values.  Same arguments as k_prep_wimg.
-__global__ void k_prep_wimg_split(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int Cin, int CinW, int Cout, int wT) {
+__global__ void k_prep_wimg_split(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int Cin, int CinW, int Cout, int wT, int co0, int ldW) {
   const long n = (long)K * Cin * Cout;
   const int nAtoms = Cin / 32;
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
@@ -777,7 +780,7 @@ __global__ void k_prep_wimg_split(const float *__restrict__ W, unsigned char *__
     const int byte = j * 4, chunk = byte >> 4, within = byte & 15;
     unsigned char *dst = img + ((long)k * nAtoms + c) * 2 * Cout * 128 + (long)co * 128 + ((chunk ^ (co & 7)) << 4) + within;
     const int ks = wT == 2 ? K - 1 - k : k;
-    const float w = ci < CinW ? (wT ? W[((long)ks * Cout + co) * CinW + ci] : W[((long)k * CinW + ci) * Cout + co]) : 0.f;
+    const float w = ci < CinW ? (wT ? W[((long)ks * ldW + co0 + co) * CinW + ci] : W[((long)k * CinW + ci) * ldW + co0 + co]) : 0.f;
     float hi, lo;
     tf32_split(w, hi, lo);
     *reinterpret_cast<float *>(dst) = hi;
@@ -788,7 +791,8 @@ __global__ void k_prep_wimg_split(const float *__restrict__ W, unsigned char *__
 // Packed layers (16-bit rows of 128 / G bytes, G = 2 or 4; fp16 elements with f16, else bf16): the K atom of offset group kg holds, for output channel co,
 // [offset kg G | offset kg G + 1 | ...] x Cin input channels -- the same order in which the producers lay the G
 // gathered neighbour rows side by side.  Offsets beyond K and channels beyond CinW are zero.
-__global__ void k_prep_wimg_packed(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int G, int Cin, int CinW, int Cout, int wT, int f16) {
+__global__ void k_prep_wimg_packed(const float *__restrict__ W, unsigned char *__restrict__ img, int K, int G, int Cin, int CinW, int Cout, int wT, int f16, int co0,
+                                   int ldW) {
   const int KG = (K + G - 1) / G;
   const long n = (long)KG * G * Cin * Cout;
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
@@ -799,7 +803,7 @@ __global__ void k_prep_wimg_packed(const float *__restrict__ W, unsigned char *_
     const int byte = (g * Cin + ci) * 2, chunk = byte >> 4, within = byte & 15;
     unsigned char *dst = img + (long)kg * Cout * 128 + (long)co * 128 + ((chunk ^ (co & 7)) << 4) + within;
     const int ks = wT == 2 ? K - 1 - k : k;
-    const float w = (k < K && ci < CinW) ? (wT ? W[((long)ks * Cout + co) * CinW + ci] : W[((long)k * CinW + ci) * Cout + co]) : 0.f;
+    const float w = (k < K && ci < CinW) ? (wT ? W[((long)ks * ldW + co0 + co) * CinW + ci] : W[((long)k * CinW + ci) * ldW + co0 + co]) : 0.f;
     *reinterpret_cast<unsigned short *>(dst) = f16 ? to16<true>(w) : to16<false>(w);
   }
 }
@@ -809,8 +813,9 @@ __global__ void k_prep_wimg_packed(const float *__restrict__ W, unsigned char *_
 // passes a per-Parameter token combined with the tensor's in-place version counter); tag 0 = no caching.
 struct WimgKey {
   const void *w; long long tag; int K, Cin, CinW, Cout, fmt, dev; // fmt: element format and packing of the image (launch_prep_wimg)
+  int co0, ldW;                                                   // the output columns of a slab (k_prep_wimg): one image per slab
   bool operator<(const WimgKey &o) const {
-    return std::tie(w, tag, K, Cin, CinW, Cout, fmt, dev) < std::tie(o.w, o.tag, o.K, o.Cin, o.CinW, o.Cout, o.fmt, o.dev);
+    return std::tie(w, tag, K, Cin, CinW, Cout, fmt, dev, co0, ldW) < std::tie(o.w, o.tag, o.K, o.Cin, o.CinW, o.Cout, o.fmt, o.dev, o.co0, o.ldW);
   }
 };
 struct WimgVal { unsigned char *img; size_t bytes; cudaEvent_t ready; cudaStream_t stream; unsigned long long lastUse; };
@@ -824,13 +829,16 @@ constexpr size_t kWimgBudget = 768u << 20;
 // offsets per atom).  The format is part of the cache key: the images of one weight tensor in different modes -- bf16 and fp16
 // included -- are separate entries, so a mode switch never hands a kernel an image in the other format.
 constexpr int kWimgBF16 = 1, kWimgSplit = 2, kWimgF16 = 3;
-static void launch_prep_wimg(const float *W, unsigned char *img, int K, int Cin, int CinW, int Cout, int fmt, cudaStream_t s, int wT) {
+static void launch_prep_wimg(const float *W, unsigned char *img, int K, int Cin, int CinW, int Cout, int fmt, cudaStream_t s, int wT, int co0, int ldW) {
   const int G = fmt >> 4;
-  if (G > 1) k_prep_wimg_packed<<<stream_grid((long)((K + G - 1) / G) * G * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, G, Cin, CinW, Cout, wT, (fmt & 15) == kWimgF16);
-  else if (fmt == kWimgSplit) k_prep_wimg_split<<<stream_grid((long)K * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, Cin, CinW, Cout, wT);
-  else k_prep_wimg<<<stream_grid((long)K * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, Cin, CinW, Cout, fmt & 15, wT);
+  if (G > 1) k_prep_wimg_packed<<<stream_grid((long)((K + G - 1) / G) * G * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, G, Cin, CinW, Cout, wT, (fmt & 15) == kWimgF16, co0, ldW);
+  else if (fmt == kWimgSplit) k_prep_wimg_split<<<stream_grid((long)K * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, Cin, CinW, Cout, wT, co0, ldW);
+  else k_prep_wimg<<<stream_grid((long)K * Cin * Cout, 256), 256, 0, LS(s)>>>(W, img, K, Cin, CinW, Cout, fmt & 15, wT, co0, ldW);
 }
-static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int Cout, int fmt, cudaStream_t s, unsigned char **img, bool *owned, int wT = 0) {
+// co0, ldW: output columns [co0, co0 + Cout) of a W ldW wide (a column slab); ldW = 0: Cout
+static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int Cout, int fmt, cudaStream_t s, unsigned char **img, bool *owned, int wT = 0,
+                    int co0 = 0, int ldW = 0) {
+  if (!ldW) ldW = Cout;
   if (wT) tag = 0; // (transposed operands belong to the backward pass of a training step: the weights change every step, nothing to cache)
   const int packG = fmt >> 4;
   const size_t bytes = packG > 1 ? (size_t)((K + packG - 1) / packG) * Cout * 128 : (size_t)K * Cin * Cout * (fmt == kWimgSplit ? 8 : fmt ? 2 : 4);
@@ -839,7 +847,7 @@ static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int
     int dev = 0;
     SCN_CUDA(cudaGetDevice(&dev));
     std::lock_guard<std::mutex> lk(g_wimg_mu);
-    WimgKey key{W, tag, K, Cin, CinW, Cout, fmt, dev};
+    WimgKey key{W, tag, K, Cin, CinW, Cout, fmt, dev, co0, ldW};
     auto it = g_wimg.find(key);
     if (it != g_wimg.end()) {
       it->second.lastUse = ++g_wimg_clock;
@@ -860,7 +868,7 @@ static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int
     WimgVal v;
     SCN_CUDA(cudaMalloc((void **)&v.img, bytes));
     SCN_CUDA(cudaEventCreateWithFlags(&v.ready, cudaEventDisableTiming));
-    launch_prep_wimg(W, v.img, K, Cin, CinW, Cout, fmt, s, 0);
+    launch_prep_wimg(W, v.img, K, Cin, CinW, Cout, fmt, s, 0, co0, ldW);
     SCN_CUDA(cudaEventRecord(v.ready, s));
     v.bytes = bytes; v.stream = s; v.lastUse = ++g_wimg_clock;
     g_wimg[key] = v;
@@ -869,7 +877,7 @@ static int get_wimg(const float *W, long long tag, int K, int Cin, int CinW, int
     return 0;
   }
   SCN_CUDA(cudaMallocAsync((void **)img, bytes, s));
-  launch_prep_wimg(W, *img, K, Cin, CinW, Cout, fmt, s, wT);
+  launch_prep_wimg(W, *img, K, Cin, CinW, Cout, fmt, s, wT, co0, ldW);
   *owned = true;
   return 0;
 }
@@ -925,19 +933,24 @@ int to_16(const float *x, void *y, long n, cudaStream_t s) {
   return 0;
 }
 // deterministic mode, split filter offsets: out = partial of split 0 + split 1 + ... in that order (bias and addend are in split 0's),
-// with the 16-bit copy of the finished rows (what the memset + atomic epilogue + k_to_16 do otherwise)
+// with the 16-bit copy of the finished rows (what the memset + atomic epilogue + k_to_16 do otherwise).  The n4 / cols4 rows of cols4
+// float4s lie pld4 (part) and ld4 (out, out16) apart -- a column slab of wider rows; part slice k starts at k n4 / cols4 pld4.  With
+// part == out and kSplit == 1 (out == null): the 16-bit copy of a slab's finished columns.
 template <bool F16>
-__global__ void __launch_bounds__(256) k_split_sum(const float4 *__restrict__ part, int kSplit, long n4, float4 *__restrict__ out, uint2 *__restrict__ out16) {
+__global__ void __launch_bounds__(256) k_split_sum(const float4 *__restrict__ part, int kSplit, long n4, int cols4, int pld4, int ld4, float4 *__restrict__ out,
+                                                   uint2 *__restrict__ out16) {
   pdl_launch_dependents();
   pdl_wait();
+  const long slice = n4 / cols4 * pld4;
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
-    float4 a = part[i];
+    const long r = i / cols4, j = i - r * cols4, ip = r * pld4 + j, io = r * ld4 + j;
+    float4 a = part[ip];
     for (int k = 1; k < kSplit; k++) {
-      const float4 b = part[(long)k * n4 + i];
+      const float4 b = part[(long)k * slice + ip];
       a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
     }
-    out[i] = a;
-    if (out16) out16[i] = pack16x4<F16>(a);
+    if (out) out[io] = a;
+    if (out16) out16[io] = pack16x4<F16>(a);
   }
 }
 static int stream_scratch(cudaStream_t s, int slot, size_t bytes, void **out);
@@ -1019,6 +1032,33 @@ static int launch_conv_plan_tc_chunked(const TcConv &c, cudaStream_t s) {
   }
   return 0;
 }
+// A layer of more than 256 output channels (the N of one tcgen05.mma, and half the TMEM columns of an SM) runs as ceil(Cout / 256)
+// launches over column slabs of balanced widths, multiples of 32 (320 = 160 + 160, 288 = 160 + 128, 1024 = 4 x 256).  Each slab is
+// an ordinary launch of <= 256 columns that writes its columns of the full-width rows (TcParams::ldo), with its own weight image
+// (the slab's output columns only), its columns of the bias, of the caller's addend, of the 16-bit copy and of the lateral weight.
+// The epilogue BatchNorm statistics (<= kFusedStatsC channels) are not taken.  A chunked plan (K > 64) splits into chunks first,
+// and each chunk into slabs.
+static int launch_conv_plan_tc_slabs(const TcConv &c, cudaStream_t s) {
+  SCN_CHECK(c.Cout % 32 == 0 && c.Cout <= 1024 && c.ldOut == 0, "tcgen05 path: more than 256 output channels need a multiple of 32, at most 1024");
+  TcConv b = c;
+  b.ldOut = c.Cout;
+  b.fuse.stats = nullptr;
+  if (half_mode(c.mathMode) && c.Cin % 64 == 0 && !c.in16 && c.nInRows) { // 16-bit operands: one copy of the input rows for all slabs
+    void *p = nullptr;
+    SCN_TRY(stream_scratch(s, kScratchBf16, (size_t)c.nInRows * c.Cin * 2 + 16, &p));
+    SCN_CUDA(launch_to_16(c.in, p, c.nInRows * c.Cin / 4, c.mathMode == kModeF16, s));
+    b.in16 = p;
+  }
+  const int units = c.Cout / 32, n = cdiv(c.Cout, 256);
+  for (int i = 0, col = 0; i < n; i++) {
+    TcConv sl = b;
+    sl.col0 = col;
+    sl.Cout = 32 * (units / n + (i < units % n ? 1 : 0));
+    SCN_TRY(launch_conv_plan_tc(sl, s));
+    col += sl.Cout;
+  }
+  return 0;
+}
 // Every conv_plan_tc instantiation the launcher uses: operand type, producer warps, filter offsets per packed atom (G), CTAs per
 // SM, deterministic mode.
 struct PlanKernel { int op, pw, G, ctas; bool det; void (*fn)(TcParams); };
@@ -1038,7 +1078,7 @@ int launch_conv_plan_tc(const TcConv &c, cudaStream_t s) {
     return launch_conv_plan_tc_chunked(c, s);
   }
   const bool f16 = c.mathMode == kModeF16; // 16-bit operands and copies are fp16 (else bf16)
-  const bool canPack = half_mode(c.mathMode) && !c.tileW && Cout <= 128; // packed narrow rows: two-CTA configuration only
+  const bool canPack = half_mode(c.mathMode) && !c.tileW && Cout <= 128 && !c.ldOut; // packed narrow rows: two-CTA configuration only, no column slabs
   if (canPack && CinW == Cin && Cin != 16 && Cin % 32 != 0) {
     // bf16 / fp16 mode, odd channel counts (e.g. the 9-channel network input): 16-bit rows zero-padded to 16 channels (packed, G = 4),
     // 32 channels (G = 2) or a multiple of 64 (whole atoms), written by one pass; the weight image pads itself
@@ -1063,7 +1103,9 @@ int launch_conv_plan_tc(const TcConv &c, cudaStream_t s) {
     p.in = xp; p.in16 = nullptr; p.Cin = Cp; p.CinW = Cin;
     return launch_conv_plan_tc(p, s);
   }
+  if (Cout > 256) return launch_conv_plan_tc_slabs(c, s);
   SCN_CHECK(Cout % 16 == 0 && Cout >= 16 && Cout <= 256 && K <= 64, "tcgen05 path: unsupported channel counts");
+  const int ldo = c.ldOut ? c.ldOut : Cout, col0 = c.col0; // (a column slab: columns [col0, col0 + Cout) of rows ldo wide)
   static int envT = -1, envS = -1, envDbg = 0, envProf = 0, envCtas = 0;
   if (envT < 0) {
     envCtas = getenv("SCN_TC_CTAS") ? atoi(getenv("SCN_TC_CTAS")) : 0;
@@ -1073,8 +1115,10 @@ int launch_conv_plan_tc(const TcConv &c, cudaStream_t s) {
     envProf = getenv("SCN_TC_PROF") ? atoi(getenv("SCN_TC_PROF")) : 0;
   }
   TcParams P;
-  P.in = reinterpret_cast<const unsigned char *>(c.in); P.out = c.out; P.bias = c.bias; P.addend = c.addend; P.out16 = c.out16; P.nbr = c.nbr; P.outRow = c.outRow; P.tileMask = c.tileMask; P.tileW = c.tileW;
-  P.nOut = nOut; P.K = K; P.Cout = Cout;
+  P.in = reinterpret_cast<const unsigned char *>(c.in); P.nbr = c.nbr; P.outRow = c.outRow; P.tileMask = c.tileMask; P.tileW = c.tileW;
+  P.out = c.out ? c.out + col0 : nullptr; P.bias = c.bias ? c.bias + col0 : nullptr; P.addend = c.addend ? c.addend + col0 : nullptr;
+  P.out16 = c.out16 ? static_cast<unsigned char *>(c.out16) + (size_t)col0 * 2 : nullptr;
+  P.nOut = nOut; P.K = K; P.Cout = Cout; P.ldo = ldo;
   // bf16 / fp16 mode: rows of >= 64 channels are whole 128-byte atoms; 32- and 16-channel rows (64 / 32 bytes) are PACKED, G = 2 / 4
   // filter offsets side by side in one atom: half / a quarter of the stages, gather bytes and MMAs of the 128-byte-row layout
   const int packG = (canPack && (Cin == 32 || Cin == 16)) ? 64 / Cin : 1;
@@ -1157,11 +1201,12 @@ int launch_conv_plan_tc(const TcConv &c, cudaStream_t s) {
   if (op == kOpF16) ++g_counters[kCntF16Launch];
   if (P.kSplit > 1) ++g_counters[kCntSplitLaunch];
   if (P.kSplit > 1 && det) SCN_TRY(det_scratch(s, (size_t)P.kSplit * nOut * Cout * 4, (void **)&P.part)); // (k_split_sum writes every output row)
-  else if (P.kSplit > 1) { ++g_counters[kCntFloatAtomic]; SCN_CUDA(cudaMemsetAsync(c.out, 0, (size_t)nOut * Cout * 4, s)); }
+  else if (P.kSplit > 1 && ldo == Cout) { ++g_counters[kCntFloatAtomic]; SCN_CUDA(cudaMemsetAsync(c.out, 0, (size_t)nOut * Cout * 4, s)); }
+  else if (P.kSplit > 1) { ++g_counters[kCntFloatAtomic]; SCN_CUDA(cudaMemset2DAsync(P.out, (size_t)ldo * 4, 0, (size_t)Cout * 4, nOut, s)); } // (the slab's columns only)
   unsigned char *wimg = nullptr;
   bool wimgOwned = false;
   const int el16 = f16 ? kWimgF16 : kWimgBF16; // element format of a 16-bit image
-  SCN_TRY(get_wimg(c.W, c.wTag, c.nWeights, Cin, CinW, Cout, packG > 1 ? el16 + 16 * packG : x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg, &wimgOwned, c.wT));
+  SCN_TRY(get_wimg(c.W, c.wTag, c.nWeights, Cin, CinW, Cout, packG > 1 ? el16 + 16 * packG : x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg, &wimgOwned, c.wT, col0, ldo));
   P.wimg = wimg;
   P.in2 = nullptr; P.wimg2 = nullptr; P.rowBytes2 = 0; P.nAtoms2 = 0;
   unsigned char *wimg2 = nullptr;
@@ -1171,7 +1216,7 @@ int launch_conv_plan_tc(const TcConv &c, cudaStream_t s) {
     const int esz = P.bf16 ? 2 : 4, per = 128 / esz, C2 = lat.Cin; // per = channels of one K atom
     if ((C2 * esz) % 16 == 0) {
       const int C2p = (C2 + per - 1) / per * per;
-      SCN_TRY(get_wimg(lat.w, lat.tag, 1, C2p, C2, Cout, x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg2, &wimg2Owned));
+      SCN_TRY(get_wimg(lat.w, lat.tag, 1, C2p, C2, Cout, x3 ? kWimgSplit : P.bf16 ? el16 : 0, s, &wimg2, &wimg2Owned, 0, col0, ldo));
       P.in2 = static_cast<const unsigned char *>(P.bf16 ? lat.in16 : static_cast<const void *>(lat.in));
       P.rowBytes2 = C2 * esz;
       P.nAtoms2 = C2p / per;
@@ -1222,9 +1267,14 @@ int launch_conv_plan_tc(const TcConv &c, cudaStream_t s) {
   if (P.statsPart) SCN_TRY(ordered_sum(P.statsPart, P.nSuper * 4, 2l * Cout, P.stats, s, Cout, kFusedStatsC)); // into replica 0
   if (P.part) // the split partials in split order, and the 16-bit copy from the same registers
     SCN_CUDA(launch_pdl(f16 ? k_split_sum<true> : k_split_sum<false>, dim3(stream_grid((long)nOut * Cout / 4, 256)), dim3(256), 0, LS(s),
-                        reinterpret_cast<const float4 *>(P.part), P.kSplit, (long)nOut * Cout / 4, reinterpret_cast<float4 *>(c.out), static_cast<uint2 *>(c.out16)));
-  else if (c.out16 && P.kSplit > 1 && c.nOutRows > 0) // partial sums were accumulated atomically: the 16-bit copy needs the finished rows
+                        reinterpret_cast<const float4 *>(P.part), P.kSplit, (long)nOut * Cout / 4, Cout / 4, Cout / 4, ldo / 4, reinterpret_cast<float4 *>(P.out),
+                        static_cast<uint2 *>(P.out16)));
+  else if (c.out16 && P.kSplit > 1 && c.nOutRows > 0 && ldo == Cout) // partial sums were accumulated atomically: the 16-bit copy needs the finished rows
     SCN_CUDA(launch_to_16(c.out, c.out16, c.nOutRows * Cout / 4, f16, s));
+  else if (c.out16 && P.kSplit > 1 && c.nOutRows > 0) // (the same for the columns of a slab)
+    SCN_CUDA(launch_pdl(f16 ? k_split_sum<true> : k_split_sum<false>, dim3(stream_grid(c.nOutRows * Cout / 4, 256)), dim3(256), 0, LS(s),
+                        reinterpret_cast<const float4 *>(P.out), 1, c.nOutRows * Cout / 4, Cout / 4, ldo / 4, ldo / 4, static_cast<float4 *>(nullptr),
+                        static_cast<uint2 *>(P.out16)));
   if (wimgOwned) cudaFreeAsync(wimg, s);
   if (wimg2Owned) cudaFreeAsync(wimg2, s);
 
@@ -1257,9 +1307,10 @@ __device__ __forceinline__ DwLane dw_lane(int rowBytesA, int rowBytesB, int lane
   }
   return L;
 }
-// one operand of a stage: the RW rows of this warp, ids in lanes 0..RW-1 (replicated every RW lanes)
+// one operand of a stage: the RW rows of this warp, ids in lanes 0..RW-1 (replicated every RW lanes); rows of rowBytes, ld bytes apart
+// (ld > rowBytes: a channel block of wider rows)
 template <int RW>
-__device__ __forceinline__ void dw_fill_operand(const unsigned char *base, int rowBytes, int nB, uint32_t mask, uint32_t chunkOff, int ids, uint32_t sOp,
+__device__ __forceinline__ void dw_fill_operand(const unsigned char *base, int rowBytes, int ld, int nB, uint32_t mask, uint32_t chunkOff, int ids, uint32_t sOp,
                                                 uint32_t blockBytes, int pw, int lane) {
   if (rowBytes <= 64) {
     // Narrow rows (64 / 32 bytes = 32 / 16 bf16 channels): 4 / 2 lanes per row, 8 / 16 rows per instruction instead of 4 -- only the
@@ -1272,7 +1323,7 @@ __device__ __forceinline__ void dw_fill_operand(const unsigned char *base, int r
       const bool mine = rl < RW;
       const int id = __shfl_sync(0xffffffffu, ids, mine ? rl : 0);
       const int row = pw * RW + rl;
-      if (mine) cp_async16(sOp + (uint32_t)row * 128u + ((uint32_t)(ch ^ (row & 7)) << 4), base + (size_t)max(id, 0) * rowBytes + ch * 16, id >= 0 ? 16u : 0u);
+      if (mine) cp_async16(sOp + (uint32_t)row * 128u + ((uint32_t)(ch ^ (row & 7)) << 4), base + (size_t)max(id, 0) * ld + ch * 16, id >= 0 ? 16u : 0u);
     }
     return;
   }
@@ -1283,7 +1334,7 @@ __device__ __forceinline__ void dw_fill_operand(const unsigned char *base, int r
     const int id = __shfl_sync(0xffffffffu, ids, rl);
     const int row = pw * RW + rl;
     const uint32_t dst = sOp + (uint32_t)row * 128u + ((uint32_t)(chunk ^ (row & 7)) << 4);
-    const unsigned char *pr = base + (size_t)max(id, 0) * rowBytes;
+    const unsigned char *pr = base + (size_t)max(id, 0) * ld;
     const uint32_t ok = id >= 0 ? 16u : 0u;
 #pragma unroll 1
     for (int b = 0; b < nB; b++) {
@@ -1293,13 +1344,13 @@ __device__ __forceinline__ void dw_fill_operand(const unsigned char *base, int r
   }
 }
 template <int RW>
-__device__ __forceinline__ void dw_fill_stage(const DwLane &L, const unsigned char *A, const unsigned char *B, int rowBytesA, int rowBytesB, int srcId, int dstId,
-                                              uint32_t sbase, uint32_t blockBytes, int nBa, int pw, int lane) {
+__device__ __forceinline__ void dw_fill_stage(const DwLane &L, const unsigned char *A, const unsigned char *B, int rowBytesA, int rowBytesB, int ldA, int ldB, int srcId,
+                                              int dstId, uint32_t sbase, uint32_t blockBytes, int nBa, int pw, int lane) {
   static_assert(RW >= 4 && RW % 4 == 0, "a producer warp requests 4 rows per instruction");
   // Rolled loops with everything loop-invariant hoisted: ~10 instructions per copy.  (Fully unrolled with per-copy predicates the
   // compiler produced ~40 instructions per copy, ~800 per warp and stage, and the producer warps' issue rate set the pace.)
-  dw_fill_operand<RW>(A, rowBytesA, L.nBaReal, L.maskA, L.chunkOff, srcId, sbase, blockBytes, pw, lane);
-  dw_fill_operand<RW>(B, rowBytesB, L.nBb, L.maskB, L.chunkOff, dstId, sbase + (uint32_t)nBa * blockBytes, blockBytes, pw, lane);
+  dw_fill_operand<RW>(A, rowBytesA, ldA, L.nBaReal, L.maskA, L.chunkOff, srcId, sbase, blockBytes, pw, lane);
+  dw_fill_operand<RW>(B, rowBytesB, ldB, L.nBb, L.maskB, L.chunkOff, dstId, sbase + (uint32_t)nBa * blockBytes, blockBytes, pw, lane);
 }
 // Zero the whole stage ring once per launch: the blocks that hold the channel padding of A (rows narrower than 256 bytes) and the
 // chunks of a 128-byte row beyond a narrow row's end are never written by the producers and read (as zeros) by every MMA.
@@ -1327,12 +1378,16 @@ constexpr int kDwProd = 16; // producer warps of the weight-gradient kernels (th
 // One CTA per SM: 4 epilogue warps (TMEM -> red.global.add), 8 producer warps, 1 MMA warp; a work item is a chunk of
 // one offset's rule list, its partial dW[k] is accumulated in TMEM and added to global memory once.
 struct DwParams {
-  const unsigned char *a, *b; // operand-typed rows: `in` (rowBytesA per row) and `d_out` (rowBytesB)
+  const unsigned char *a, *b; // operand-typed rows: `in` (rowBytesA per row, ldA apart) and `d_out` (rowBytesB, ldB apart)
   const int2 *pairs;
   const int *d_off;           // K + 1 list offsets
   float *dW;
   float *part;                // deterministic mode: [item][Cin][Cout], item w's partial dW[w % K] (plain stores), summed in part order afterwards
   int K, Cin, Cout, nC, srcIsY, rowBytesA, rowBytesB, R, S, nAcc; // nC: parts per rule list
+  // a channel block of a wider layer (launch_conv_dw_tc): rows ldA / ldB bytes apart, and dW / part rows ldW floats apart, offsets
+  // (and work-item slots) wStride floats apart; Cin x Cout, rowBytes and wStride = Cin Cout otherwise
+  int ldA, ldB, ldW;
+  long wStride;
 };
 __device__ __forceinline__ uint64_t smem_desc_mn_sw128(uint32_t addr, uint32_t lboBytes) {
   return (uint64_t)((addr >> 4) & 0x3fffu) | ((uint64_t)((lboBytes >> 4) & 0x3fffu) << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
@@ -1386,7 +1441,7 @@ __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwPara
       item(w, k, r0, cnt);
       if (cnt <= 0) {
         if (P.part) // (an empty part still owns a slot of the ordered sum)
-          for (long i = tid; i < (long)P.Cin * P.Cout; i += 128) P.part[(size_t)w * P.Cin * P.Cout + i] = 0.f;
+          for (long i = tid; i < (long)P.Cin * P.Cout; i += 128) P.part[(size_t)w * P.wStride + i / P.Cout * P.ldW + i % P.Cout] = 0.f;
         continue;
       }
       const int it = itN++;
@@ -1395,7 +1450,7 @@ __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwPara
       tc_fence_after();
       for (int mh = 0; mh < nMh; mh++) {
         const int ci = mh * 128 + warp * 32 + lane;
-        float *dst = P.part ? P.part + ((size_t)w * P.Cin + ci) * P.Cout : P.dW + ((size_t)k * P.Cin + ci) * P.Cout;
+        float *dst = (P.part ? P.part + (size_t)w * P.wStride : P.dW + (size_t)k * P.wStride) + (size_t)ci * P.ldW;
         if (mh * 128 + warp * 32 >= P.Cin) continue; // rows of the channel padding (warp-uniform)
         for (int c0 = 0; c0 < P.Cout; c0 += 32) {
           uint32_t v[32];
@@ -1437,8 +1492,8 @@ __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwPara
         const int srcId = P.srcIsY ? pr.y : pr.x, dstId = P.srcIsY ? pr.x : pr.y;
         mbar_wait(smem_u32(empty + slot), (round & 1u) ^ 1u);
         const uint32_t sbase = smem_u32(sStage) + slot * stageBytes;
-        if (R == 128) dw_fill_stage<128 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
-        else dw_fill_stage<64 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
+        if (R == 128) dw_fill_stage<128 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, P.ldA, P.ldB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
+        else dw_fill_stage<64 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, P.ldA, P.ldB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
         cp_async_mbar_arrive_noinc(smem_u32(full + slot));
         if (++slot == (uint32_t)P.S) { slot = 0; round++; }
       }
@@ -1641,8 +1696,8 @@ __global__ void __launch_bounds__(32 * (6 + kDwProd), 1) conv_dw_plan_tc(const D
         const int srcId = P.swap ? ido : idn, dstId = P.swap ? idn : ido;
         { const long long c0 = P.prof ? clock64() : 0; mbar_wait(smem_u32(empty + slot), (round & 1u) ^ 1u); if (P.prof) { pwait += clock64() - c0; pstages++; } }
         const uint32_t sbase = smem_u32(sStage) + slot * stageBytes;
-        if (R == 128) dw_fill_stage<128 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
-        else dw_fill_stage<64 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
+        if (R == 128) dw_fill_stage<128 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, P.rowBytesA, P.rowBytesB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
+        else dw_fill_stage<64 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, P.rowBytesA, P.rowBytesB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
         cp_async_mbar_arrive_noinc(smem_u32(full + slot));
         if (++slot == (uint32_t)P.S) { slot = 0; round++; }
         t = tB; h = hB;
@@ -1710,10 +1765,20 @@ __global__ void __launch_bounds__(32 * (6 + kDwProd), 1) conv_dw_plan_tc(const D
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmemBase), "r"(512u) : "memory");
   }
 }
+// the shapes one weight-gradient launch takes: M = Cin in one or two halves of 128 rows, N = Cout, nMh x Cout TMEM columns
+static bool dw_block_ok(int Cin, int Cout, int K) {
+  return !((Cin % 32 != 0 && Cin > 32) || Cin > 256 || (Cin > 128 && Cin % 128 != 0) || Cout % 32 != 0 || Cout > 256 || ((Cin + 127) / 128) * Cout > 512 || K > 64);
+}
+// Layers wider than 256 channels on either side run as channel blocks of such shapes (launch_conv_dw_tc), from the rule lists,
+// which have no filter-offset limit.
+static bool dw_shape_ok(int Cin, int Cout, int K) {
+  if (Cin <= 256 && Cout <= 256) return dw_block_ok(Cin, Cout, K);
+  return Cin % 32 == 0 && Cout % 32 == 0 && Cin <= 1024 && Cout <= 1024 && K <= kMaxFilterVolume;
+}
 // whether launch_conv_dw_tc takes this shape at all (else the caller falls back to the CUDA-core kernel, which needs the fp32 rows)
 bool dw_tc_ok(int Cin, int Cout, int K, int mathMode) {
   if (!half_mode(mathMode) || !tc_available()) return false;
-  return !((Cin % 32 != 0 && Cin > 32) || Cin > 256 || (Cin > 128 && Cin % 128 != 0) || Cout % 32 != 0 || Cout > 256 || ((Cin + 127) / 128) * Cout > 512 || K > 64);
+  return dw_shape_ok(Cin, Cout, K);
 }
 template <bool F16>
 __global__ void __launch_bounds__(256) k_from_16(const uint2 *__restrict__ x, float4 *__restrict__ y, long n4) {
@@ -1740,7 +1805,7 @@ bool dw_plan_ok(int Cin, int Cout, int K, int mathMode) {
   static int planOn = -1;
   if (planOn < 0) planOn = getenv("SCN_DW_PLAN") ? atoi(getenv("SCN_DW_PLAN")) : 0;
   if (!planOn || !half_mode(mathMode) || !tc_available() || deterministic()) return false; // (its partial sums are not indexed by work item)
-  return !((Cin % 32 != 0 && Cin > 32) || Cin > 256 || (Cin > 128 && Cin % 128 != 0) || Cout % 32 != 0 || Cout > 256 || ((Cin + 127) / 128) * Cout > 512 || K > 64);
+  return dw_block_ok(Cin, Cout, K); // (channel blocks of wider layers run from the rule lists)
 }
 // dW must be zero on entry.  Returns 1 when the configuration is not supported (the caller then uses the CUDA-core kernel).
 // in16 / dout16: optional 16-bit copies (the mode's format) of `in` / `d_out` ([rows][Cin] / [rows][Cout], same layout) the caller already has.
@@ -1750,14 +1815,15 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
   // bf16 / fp16 mode only: with TF32 operands the MN-major product came out as zeros on B200 (unresolved; tf32 mode keeps the CUDA-core kernel)
   if (!half_mode(mathMode) || !tc_available()) return 1;
   const bool bf16 = true, f16 = mathMode == kModeF16;
-  if ((Cin % 32 != 0 && Cin > 32) || Cin > 256 || (Cin > 128 && Cin % 128 != 0) || Cout % 32 != 0 || Cout > 256 || ((Cin + 127) / 128) * Cout > 512 || K > 64) return 1;
+  if (!dw_shape_ok(Cin, Cout, K)) return 1;
+  const bool wide = Cin > 256 || Cout > 256;
   const int CinP = Cin % 32 == 0 ? Cin : (Cin <= 16 ? 16 : 32); // odd narrow inputs (the 9-channel network input): bf16 rows zero-padded to 16 / 32 channels
   static int planOn = -1;
   // Measured on B470 / 6c_fpn4321 (internal numbering, 16 producer warps): level-0 32 -> 32 layers 0.45 ms with the rule lists
   // (100 % row fill, equal work items) against 0.69 ms with the plan (row fill 89 %, items of unequal cost), all 39 launches of a
   // step 2.6 against 4.2 ms -- the list kernel is the default, SCN_DW_PLAN=1 selects the plan-driven one.
   if (planOn < 0) planOn = getenv("SCN_DW_PLAN") ? atoi(getenv("SCN_DW_PLAN")) : 0;
-  const bool usePlan = planOn && planNbr && planMask && planPos > 0 && !deterministic();
+  const bool usePlan = planOn && planNbr && planMask && planPos > 0 && !deterministic() && !wide;
   SCN_CHECK(usePlan || offHost, "weight gradient: neither a plan nor rule lists");
   const long total = usePlan ? 1 : offHost[K];
   if (total == 0) return 0;
@@ -1780,14 +1846,38 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
   } else {
     P.a = reinterpret_cast<const unsigned char *>(in); P.b = reinterpret_cast<const unsigned char *>(d_out);
   }
-  const int nBlocks = std::max(P.rowBytesA, 256) / 128 + (P.rowBytesB + 127) / 128;
+  P.ldA = P.rowBytesA; P.ldB = P.rowBytesB; P.ldW = Cout; P.wStride = (long)Cin * Cout;
+  // Channel blocks: Cin in blocks of 256 (two M halves), the rest in one block of <= 128 or 128 + the remainder; Cout in balanced
+  // blocks of <= 256 (multiples of 32).  Every block is a shape dw_block_ok takes: one launch each, gathering its channel slice
+  // of the same operand rows.  Layers of <= 256 x 256 are one block.
+  std::vector<std::pair<int, int>> bi, bo; // (first channel, channels)
+  for (int c = 0; c < Cin;) {
+    const int r = Cin - c, w = !wide || r >= 256 ? std::min(r, 256) : (r <= 128 ? r : 128);
+    bi.emplace_back(c, w);
+    c += w;
+  }
+  const int nOb = wide ? cdiv(Cout, 256) : 1, units = Cout / 32;
+  for (int i = 0, c = 0; i < nOb; i++) {
+    const int w = wide ? 32 * (units / nOb + (i < units % nOb ? 1 : 0)) : Cout;
+    bo.emplace_back(c, w);
+    c += w;
+  }
+  const unsigned char *baseA = P.a, *baseB = P.b;
   const size_t budget = 225 * 1024 - 1024; // (the kernel also has ~1 KB of static shared memory)
-  P.R = (size_t)nBlocks * 128 * 128 * 3 <= budget ? 128 : 64;
-  const size_t stageBytes = (size_t)nBlocks * P.R * 128;
-  P.S = (int)std::min<size_t>(4, budget / stageBytes);
+  // stage shape of a block: R rules per stage, S stages, one or two TMEM accumulators
+  auto shape = [&](DwParams &Q, int cinB, int coutB) {
+    Q.Cin = cinB; Q.Cout = coutB;
+    Q.rowBytesA = (cinB == Cin ? CinP : cinB) * 2;
+    Q.rowBytesB = coutB * 2;
+    const int nBlocks = std::max(Q.rowBytesA, 256) / 128 + (Q.rowBytesB + 127) / 128;
+    Q.R = (size_t)nBlocks * 128 * 128 * 3 <= budget ? 128 : 64;
+    const size_t stageBytes = (size_t)nBlocks * Q.R * 128;
+    Q.S = (int)std::min<size_t>(4, budget / stageBytes);
+    Q.nAcc = 2 * ((cinB + 127) / 128) * coutB <= 512 ? 2 : 1;
+    return stageBytes;
+  };
+  const size_t stageBytes = shape(P, bi[0].second, bo[0].second);
   if (P.S < 2) return 1;
-  const int accCols = ((Cin + 127) / 128) * Cout;
-  P.nAcc = 2 * accCols <= 512 ? 2 : 1;
   if (usePlan) { // plan order (spatially coherent gathers), see conv_dw_plan_tc
     DwPlanParams Q;
     Q.a = P.a; Q.b = P.b; Q.nbr = planNbr; Q.outRow = planOutRow; Q.tileMask = planMask; Q.dW = dW;
@@ -1842,12 +1932,13 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
     constexpr size_t kDetDwBytes = 256u << 20;
     const size_t perItem = (size_t)Cin * Cout * 4;
     P.nC = (int)std::max<size_t>(1, std::min<size_t>((size_t)P.nC, kDetDwBytes / (perItem * K)));
-    SCN_TRY(det_scratch(s, (size_t)K * P.nC * perItem, (void **)&P.part));
+    // (a wide layer with one part per list: item k is the only writer of dW[k] -- its plain stores go to dW, no workspace)
+    if (wide && P.nC == 1) P.part = dW;
+    else SCN_TRY(det_scratch(s, (size_t)K * P.nC * perItem, (void **)&P.part));
   } else {
-    ++g_counters[kCntFloatAtomic];
+    g_counters[kCntFloatAtomic] += (long)(bi.size() * bo.size()); // (one per launch)
   }
   const long nItems = (long)K * P.nC;
-  const size_t smemBytes = (size_t)P.S * stageBytes + 64 * 8 + 64;
   static bool attr = false;
   if (!attr) {
     SCN_CUDA(cudaFuncSetAttribute(conv_dw_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
@@ -1856,11 +1947,22 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
     attr = true;
   }
   const int grid = (int)std::min<long>(nItems, kSMs);
-  if (f16) { ++g_counters[kCntF16Launch]; conv_dw_tc<true, true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(P); }
-  else if (bf16) conv_dw_tc<true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(P);
-  else conv_dw_tc<false><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(P);
-  SCN_CUDA(cudaGetLastError());
-  if (P.part) SCN_TRY(ordered_sum(P.part, P.nC, (long)K * Cin * Cout, dW, s)); // item c K + k = part c of list k: rows [nC][K][Cin][Cout]
+  // every block with the same parts per list: in deterministic mode they all fill the one [nC][K][Cin][Cout] workspace
+  for (const auto &ib : bi)
+    for (const auto &ob : bo) {
+      DwParams Q = P;
+      const size_t sb = shape(Q, ib.second, ob.second);
+      SCN_CHECK(Q.S >= 2, "weight gradient: channel block does not fit in shared memory");
+      Q.a = baseA + (size_t)ib.first * 2; Q.b = baseB + (size_t)ob.first * 2;
+      Q.dW = dW + (size_t)ib.first * Cout + ob.first;
+      if (P.part) Q.part = P.part + (size_t)ib.first * Cout + ob.first;
+      const size_t smemBytes = (size_t)Q.S * sb + 64 * 8 + 64;
+      if (f16) { ++g_counters[kCntF16Launch]; conv_dw_tc<true, true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(Q); }
+      else if (bf16) conv_dw_tc<true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(Q);
+      else conv_dw_tc<false><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(Q);
+      SCN_CUDA(cudaGetLastError());
+    }
+  if (P.part && P.part != dW) SCN_TRY(ordered_sum(P.part, P.nC, (long)K * Cin * Cout, dW, s)); // item c K + k = part c of list k: rows [nC][K][Cin][Cout]
   return 0;
 }
 

@@ -245,7 +245,9 @@ int scn_program_finish(scn_program *p, int n_regs, const int *outputs, int n_out
       const long Cin = o.kind == K_SUBM ? o.a[10] : o.a[16], Cout = o.kind == K_SUBM ? o.a[11] : o.a[17];
       long K = 1;
       for (int d = 0; d < 3; d++) K *= o.kind == K_SUBM ? o.a[5 + d] : o.a[8 + d];
-      const bool tc = Cout % 32 == 0 && Cout >= 32 && Cout <= 256 && K <= 63 && (Cin % 64 == 0 || (Cin == 32 && Cout <= 128));
+      // (wider layers run as column slabs of <= 256 that all gather the 16-bit copy when Cin is a multiple of 64)
+      const bool tc = Cout % 32 == 0 && Cout >= 32 && K <= 63 &&
+                      (Cout <= 256 ? (Cin % 64 == 0 || (Cin == 32 && Cout <= 128)) : (Cout <= 1024 && Cin % 64 == 0 && Cin <= 1024));
       // a deconvolution takes the tensor-core path when every fine site has exactly one parent: guaranteed by filter == stride
       const bool deconvTc = o.kind == K_DECONV && Cin % 64 == 0 && o.a[8] == o.a[11] && o.a[9] == o.a[12] && o.a[10] == o.a[13];
       if (tc && (o.kind != K_DECONV || deconvTc)) good[o.a[0]] = 1; else bad[o.a[0]] = 1;

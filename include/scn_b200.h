@@ -326,8 +326,10 @@ int scn_voxelize(const float *xyz, const float *feats, long n, int n_feat, const
  * accumulator, fp32-class accuracy, 5 = tcgen05 FP16 inputs / fp32 accumulate wherever mode 2 has BF16 inputs
  * (everything else as in mode 2): 11 significant bits instead of 8, range +-65504 -- conversions round to nearest
  * even with IEEE overflow (a larger value becomes +-inf and propagates) and keep subnormals.  Code 4 is not a mode.
- * In modes 1 and 3 every convolution the tensor-core kernel cannot take, and every weight gradient, runs on the
- * exact fp32 CUDA-core kernels. */
+ * The tensor-core kernels take convolutions with up to 1024 input channels and, in multiples of 32, up to 1024 output
+ * channels (layers wider than 256 run as column slabs of <= 256).  In modes 1 and 3 every convolution the tensor-core kernel
+ * cannot take, and every weight gradient, runs on the exact fp32 CUDA-core kernels; in modes 2 and 5 the weight gradients of
+ * up to 1024 x 1024 channels (multiples of 32 beyond 256) run on the tensor cores too. */
 int scn_set_math_mode(int mode);
 int scn_get_math_mode(void);
 /* Deterministic mode for this process (0 = off, the default): with 1, every float result of the calls above except
@@ -353,7 +355,8 @@ long scn_kernel_launch_count(void);
  * which atomics land (0 in deterministic mode except for scn_roi_align_rotated_3d_backward), 17 = host -> device copies of
  * input-layer coordinates, 18 = tensor-core launches with fp16 operands (convolutions and weight gradients, math mode 5), 19 = rule
  * lists a convolution's backward entry found already built (hinted ahead by a training run), 20 = training runs that took a Metadata
- * prepared by scn_program_prepare_training. */
+ * prepared by scn_program_prepare_training, 21 = CUDA-core weight-gradient
+ * launches of the sparse convolutions (k_dw, one per non-empty rule list; NetworkInNetwork's dense weight gradient is not counted). */
 long scn_debug_counter(int which);
 /* Hands the library's idle device memory back to the driver: Metadata chunks not owned by a live Metadata, cached weight operand
  * images, per-stream scratch buffers (the library recycles these itself instead of returning them; torch.cuda.empty_cache() cannot
