@@ -65,7 +65,8 @@ enum DebugCounter {
   kCntRulesAhead = 19,     // rule lists a backward entry found already built (hinted ahead by a training run, program.cu)
   kCntTrainPrepared = 20,  // training runs that took a Metadata prepared by scn_program_prepare_training
   kCntSimtDwLaunch = 21,   // CUDA-core weight-gradient launches of the sparse convolutions (k_dw, one per rule list)
-  kCntCounters = 22
+  kCntDwX3Launch = 22,     // weight-gradient launches with three-way bf16 operand splits (conv_dw_tc, math mode 3)
+  kCntCounters = 23
 };
 extern std::atomic<long> g_counters[kCntCounters];
 
@@ -87,7 +88,7 @@ int ordered_sum(const T *part, int nPart, long width, T *out, cudaStream_t s, lo
 // and the packed 16- / 32-channel rows; the other layers keep TF32 operands.  Every 16-bit copy of a feature matrix -- the
 // "bf16" arguments of the C ABI, the shadows of a recorded program, the operand copies the launchers make -- is written and read
 // in the format of the current mode: fp16 in mode 5, bf16 in every other mode (as before mode 5 existed).
-constexpr int kModeBF16 = 2, kModeF16 = 5;
+constexpr int kModeBF16 = 2, kModeTF32X3 = 3, kModeF16 = 5;
 static inline bool half_mode(int mathMode) { return mathMode == kModeBF16 || mathMode == kModeF16; }
 int math_mode(); // the current mode (capi.cu)
 static inline bool f16_copies() { return math_mode() == kModeF16; }

@@ -1374,6 +1374,34 @@ __device__ __forceinline__ void dw_issue_stage(uint32_t sbase, uint32_t blockByt
     if (nMh > 1) tc_mma<BF16>(tmemD + (uint32_t)Cout, a0 + (uint64_t)(aBlkStride16 + j * kStep16), b0 + (uint64_t)(j * kStep16), idesc, (!first || j > 0) ? 1u : 0u);
   }
 }
+// The same for split operands (math mode 3): the stage holds the parts h, m, l of both operands, partBytes apart, and every
+// 16-rule step issues six bf16 products, the small ones first: h l, l h, m m, h m, m h into the correction accumulator tmemC,
+// then h h into tmemD; the epilogue adds the two.  (m l, l m and l l, each below 2^-24 |x y|, are left out.)  The tensor core
+// does not round the sum it adds to an accumulator to nearest: with all six products in one accumulator the small ones met the
+// full partial sum 6 x per step, and on 4096-rule parts of N(0, 1) rows the error grew to 16 x 2^-24 of the sum of |products|.
+// Blocks of split operands have Cin <= 128: one M half.
+template <int NJ>
+__device__ __forceinline__ void dw_issue_stage_x3(uint32_t sbase, uint32_t partBytes, uint32_t blockBytes, int nBa, uint32_t tmemD, uint32_t tmemC, uint32_t idesc,
+                                                  bool first) {
+  constexpr uint32_t kStep16 = 16u * 128u >> 4;
+  uint64_t a[3], b[3];
+#pragma unroll
+  for (int p = 0; p < 3; p++) {
+    a[p] = smem_desc_mn_sw128(sbase + (uint32_t)p * partBytes, blockBytes);
+    b[p] = smem_desc_mn_sw128(sbase + (uint32_t)p * partBytes + (uint32_t)nBa * blockBytes, blockBytes);
+  }
+#pragma unroll
+  for (int j = 0; j < NJ; j++) {
+    const uint64_t o = (uint64_t)(j * kStep16);
+    const uint32_t acc = (!first || j > 0) ? 1u : 0u;
+    tc_mma<true>(tmemC, a[0] + o, b[2] + o, idesc, acc);
+    tc_mma<true>(tmemC, a[2] + o, b[0] + o, idesc, 1u);
+    tc_mma<true>(tmemC, a[1] + o, b[1] + o, idesc, 1u);
+    tc_mma<true>(tmemC, a[0] + o, b[1] + o, idesc, 1u);
+    tc_mma<true>(tmemC, a[1] + o, b[0] + o, idesc, 1u);
+    tc_mma<true>(tmemD, a[0] + o, b[0] + o, idesc, acc);
+  }
+}
 constexpr int kDwProd = 16; // producer warps of the weight-gradient kernels (their request issue rate paces the kernels: 8 -> 16 measured below)
 // One CTA per SM: 4 epilogue warps (TMEM -> red.global.add), 8 producer warps, 1 MMA warp; a work item is a chunk of
 // one offset's rule list, its partial dW[k] is accumulated in TMEM and added to global memory once.
@@ -1388,18 +1416,20 @@ struct DwParams {
   // (and work-item slots) wStride floats apart; Cin x Cout, rowBytes and wStride = Cin Cout otherwise
   int ldA, ldB, ldW;
   long wStride;
+  long planeA, planeB; // split operands (X3): bytes from the h rows to the m rows and from the m rows to the l rows
 };
 __device__ __forceinline__ uint64_t smem_desc_mn_sw128(uint32_t addr, uint32_t lboBytes) {
   return (uint64_t)((addr >> 4) & 0x3fffu) | ((uint64_t)((lboBytes >> 4) & 0x3fffu) << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
-// BF16: 16-bit operands (kind::f16), fp16 ones with F16 (math mode 5), else TF32
-template <bool BF16, bool F16 = false>
+// BF16: 16-bit operands (kind::f16), fp16 ones with F16 (math mode 5), else TF32.  X3 (with BF16): split operands, three bf16
+// parts h, m, l of each fp32 value, planes P.planeA / P.planeB bytes apart (math mode 3, dw_issue_stage_x3)
+template <bool BF16, bool F16 = false, bool X3 = false>
 __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwParams P) {
   extern __shared__ __align__(1024) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   // `in` rows narrower than 128 channels are zero-padded to M = 128 in shared memory (zero-filled chunks, no traffic)
   const int R = P.R, nBa = max(P.rowBytesA, 256) / 128, nBb = (P.rowBytesB + 127) / 128;
-  const uint32_t blockBytes = (uint32_t)R * 128u, stageBytes = (uint32_t)(nBa + nBb) * blockBytes;
+  const uint32_t blockBytes = (uint32_t)R * 128u, partBytes = (uint32_t)(nBa + nBb) * blockBytes, stageBytes = X3 ? 3u * partBytes : partBytes;
   unsigned char *sStage = smem;
   uint64_t *bars = reinterpret_cast<uint64_t *>(sStage + (size_t)P.S * stageBytes);
   uint64_t *full = bars, *empty = bars + P.S, *accFull = bars + 2 * P.S, *accEmpty = accFull + 2;
@@ -1420,7 +1450,7 @@ __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwPara
   tc_fence_after();
   const uint32_t tmemBase = *tmemSlot;
   const int nItems = P.K * P.nC;
-  const int nMh = (P.Cin + 127) / 128, accCols = nMh * P.Cout;
+  const int nMh = (P.Cin + 127) / 128, accCols = nMh * P.Cout, accStride = X3 ? 2 * accCols : accCols; // (X3: main + correction accumulator)
   // item w -> (list k = w % K, part c = w / K of nC): the rules [len c / nC, len (c + 1) / nC) of list k.  The lists are in row
   // order, so part c of every list covers about the same region of the grid, and the ~148 items in flight at any time are
   // all 27 offsets of a few neighbouring parts: their rows stay in L2 across the offsets.  (List-major order swept the whole grid
@@ -1454,7 +1484,16 @@ __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwPara
         if (mh * 128 + warp * 32 >= P.Cin) continue; // rows of the channel padding (warp-uniform)
         for (int c0 = 0; c0 < P.Cout; c0 += 32) {
           uint32_t v[32];
-          tmem_ld(tmemBase + ((uint32_t)(warp * 32) << 16) + (uint32_t)(a * accCols + mh * P.Cout + c0), v);
+          tmem_ld(tmemBase + ((uint32_t)(warp * 32) << 16) + (uint32_t)(a * accStride + mh * P.Cout + c0), v);
+          if (X3) { // + the correction accumulator, 16 columns at a time (32 more live registers spilled in this epilogue)
+#pragma unroll
+            for (int hf = 0; hf < 32; hf += 16) {
+              uint32_t u[16];
+              tmem_ld(tmemBase + ((uint32_t)(warp * 32) << 16) + (uint32_t)(a * accStride + accCols + c0 + hf), u);
+#pragma unroll
+              for (int j = 0; j < 16; j++) v[hf + j] = __float_as_uint(__uint_as_float(v[hf + j]) + __uint_as_float(u[j]));
+            }
+          }
           if (ci < P.Cin && P.part) {
 #pragma unroll
             for (int j = 0; j < 32; j += 4)
@@ -1492,7 +1531,12 @@ __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwPara
         const int srcId = P.srcIsY ? pr.y : pr.x, dstId = P.srcIsY ? pr.x : pr.y;
         mbar_wait(smem_u32(empty + slot), (round & 1u) ^ 1u);
         const uint32_t sbase = smem_u32(sStage) + slot * stageBytes;
-        if (R == 128) dw_fill_stage<128 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, P.ldA, P.ldB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
+        if (X3) { // the same rows of the three parts (split-operand stages are always 64 rules: launch_conv_dw_tc)
+#pragma unroll 1
+          for (int p = 0; p < 3; p++)
+            dw_fill_stage<64 / kDwProd>(DL, P.a + p * P.planeA, P.b + p * P.planeB, P.rowBytesA, P.rowBytesB, P.ldA, P.ldB, srcId, dstId, sbase + p * partBytes,
+                                        blockBytes, nBa, pw, lane);
+        } else if (R == 128) dw_fill_stage<128 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, P.ldA, P.ldB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
         else dw_fill_stage<64 / kDwProd>(DL, P.a, P.b, P.rowBytesA, P.rowBytesB, P.ldA, P.ldB, srcId, dstId, sbase, blockBytes, nBa, pw, lane);
         cp_async_mbar_arrive_noinc(smem_u32(full + slot));
         if (++slot == (uint32_t)P.S) { slot = 0; round++; }
@@ -1520,8 +1564,9 @@ __global__ void __launch_bounds__(32 * (5 + kDwProd), 1) conv_dw_tc(const DwPara
         tc_fence_after();
         const uint32_t sbase = smem_u32(sStage) + slot * stageBytes;
         if (elect_one()) {
-          if (R == 128) dw_issue_stage<BF16, 128 / kRulesPerMma>(sbase, blockBytes, nBa, nMh, aBlkStride16, tmemBase + (uint32_t)(a * accCols), P.Cout, idesc, base == 0);
-          else dw_issue_stage<BF16, 64 / kRulesPerMma>(sbase, blockBytes, nBa, nMh, aBlkStride16, tmemBase + (uint32_t)(a * accCols), P.Cout, idesc, base == 0);
+          if (X3) dw_issue_stage_x3<64 / kRulesPerMma>(sbase, partBytes, blockBytes, nBa, tmemBase + (uint32_t)(a * accStride), tmemBase + (uint32_t)(a * accStride + accCols), idesc, base == 0);
+          else if (R == 128) dw_issue_stage<BF16, 128 / kRulesPerMma>(sbase, blockBytes, nBa, nMh, aBlkStride16, tmemBase + (uint32_t)(a * accStride), P.Cout, idesc, base == 0);
+          else dw_issue_stage<BF16, 64 / kRulesPerMma>(sbase, blockBytes, nBa, nMh, aBlkStride16, tmemBase + (uint32_t)(a * accStride), P.Cout, idesc, base == 0);
           tc_commit(smem_u32(empty + slot));
         }
         __syncwarp();
@@ -1780,6 +1825,47 @@ bool dw_tc_ok(int Cin, int Cout, int K, int mathMode) {
   if (!half_mode(mathMode) || !tc_available()) return false;
   return dw_shape_ok(Cin, Cout, K);
 }
+// Math mode 3 (split operands): the shapes of one launch, run as blocks of <= 128 x <= 128 channels (launch_conv_dw_tc).  Wider
+// layers and larger filters keep the CUDA-core kernel.  (Not part of dw_tc_ok: that also says whether a layer's rows may be
+// kept as 16-bit copies only, and split operands need the fp32 rows.)
+static bool dw_x3_ok(int Cin, int Cout, int K) { return dw_block_ok(Cin, Cout, K); }
+// fp32 rows of C channels -> three bf16 planes h = rn(x), m = rn(x - h), l = rn(x - h - m), `plane` elements apart, rows zero-padded
+// to Cp channels (Cp % 4 == 0).  Both differences are exact in fp32, and h + m + l = x exactly for normal-range x: h and m take 8
+// significant bits each, the at most 8 that remain fit l.  Where l falls below 2^-126 it is a bf16 subnormal (kept, rounded to the
+// subnormal grid); a finite x that rounds past the largest finite bf16 (|x| >= 3.3962e38) takes h = rz(x), so x - h stays finite.
+__device__ __forceinline__ __nv_bfloat16 split_hi(float x) {
+  const __nv_bfloat16 h = __float2bfloat16_rn(x);
+  return __hisinf(h) ? __float2bfloat16_rz(x) : h;
+}
+__global__ void __launch_bounds__(256) k_split3_bf16(const float *__restrict__ x, uint2 *__restrict__ y, long n, int C, int Cp, long plane) {
+  const long n4 = n * Cp / 4, plane4 = plane / 4;
+  for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
+    float v[4];
+    if (C == Cp) {
+      const float4 q = __ldg(reinterpret_cast<const float4 *>(x) + i);
+      v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+    } else {
+      const long r = i * 4 / Cp;
+      const int c0 = (int)(i * 4 - r * Cp);
+#pragma unroll
+      for (int j = 0; j < 4; j++) v[j] = c0 + j < C ? __ldg(x + r * C + c0 + j) : 0.f;
+    }
+    uint32_t h[2], m[2], l[2];
+#pragma unroll
+    for (int j = 0; j < 4; j += 2) {
+      const __nv_bfloat162 hh = __halves2bfloat162(split_hi(v[j]), split_hi(v[j + 1]));
+      const float r0 = v[j] - __low2float(hh), r1 = v[j + 1] - __high2float(hh);
+      const __nv_bfloat162 mm = __floats2bfloat162_rn(r0, r1);
+      const __nv_bfloat162 ll = __floats2bfloat162_rn(r0 - __low2float(mm), r1 - __high2float(mm));
+      h[j / 2] = *reinterpret_cast<const uint32_t *>(&hh);
+      m[j / 2] = *reinterpret_cast<const uint32_t *>(&mm);
+      l[j / 2] = *reinterpret_cast<const uint32_t *>(&ll);
+    }
+    y[i] = make_uint2(h[0], h[1]);
+    y[plane4 + i] = make_uint2(m[0], m[1]);
+    y[2 * plane4 + i] = make_uint2(l[0], l[1]);
+  }
+}
 template <bool F16>
 __global__ void __launch_bounds__(256) k_from_16(const uint2 *__restrict__ x, float4 *__restrict__ y, long n4) {
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
@@ -1812,10 +1898,12 @@ bool dw_plan_ok(int Cin, int Cout, int K, int mathMode) {
 int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2 *pairs, const int *d_off, const int *offHost, int K, long nInRows,
                       long nOutRows, int Cin, int Cout, int srcIsY, int mathMode, cudaStream_t s, const void *in16, const void *dout16,
                       const int *planNbr, const int *planOutRow, const unsigned long long *planMask, int planPos) {
-  // bf16 / fp16 mode only: with TF32 operands the MN-major product came out as zeros on B200 (unresolved; tf32 mode keeps the CUDA-core kernel)
-  if (!half_mode(mathMode) || !tc_available()) return 1;
+  // bf16 / fp16 mode, and tf32x3 mode with bf16 parts of split operands: with TF32 operands the MN-major product came out as zeros
+  // on B200 (unresolved; tf32 mode keeps the CUDA-core kernel)
+  const bool x3 = mathMode == kModeTF32X3;
+  if (!(half_mode(mathMode) || x3) || !tc_available()) return 1;
   const bool bf16 = true, f16 = mathMode == kModeF16;
-  if (!dw_shape_ok(Cin, Cout, K)) return 1;
+  if (x3 ? !dw_x3_ok(Cin, Cout, K) : !dw_shape_ok(Cin, Cout, K)) return 1;
   const bool wide = Cin > 256 || Cout > 256;
   const int CinP = Cin % 32 == 0 ? Cin : (Cin <= 16 ? 16 : 32); // odd narrow inputs (the 9-channel network input): bf16 rows zero-padded to 16 / 32 channels
   static int planOn = -1;
@@ -1823,7 +1911,7 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
   // (100 % row fill, equal work items) against 0.69 ms with the plan (row fill 89 %, items of unequal cost), all 39 launches of a
   // step 2.6 against 4.2 ms -- the list kernel is the default, SCN_DW_PLAN=1 selects the plan-driven one.
   if (planOn < 0) planOn = getenv("SCN_DW_PLAN") ? atoi(getenv("SCN_DW_PLAN")) : 0;
-  const bool usePlan = planOn && planNbr && planMask && planPos > 0 && !deterministic() && !wide;
+  const bool usePlan = planOn && planNbr && planMask && planPos > 0 && !deterministic() && !wide && !x3;
   SCN_CHECK(usePlan || offHost, "weight gradient: neither a plan nor rule lists");
   const long total = usePlan ? 1 : offHost[K];
   if (total == 0) return 0;
@@ -1831,7 +1919,17 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
   P.pairs = pairs; P.d_off = d_off; P.dW = dW; P.K = K; P.Cin = Cin; P.Cout = Cout; P.srcIsY = srcIsY;
   P.rowBytesA = CinP * (bf16 ? 2 : 4);
   P.rowBytesB = Cout * (bf16 ? 2 : 4);
-  if (bf16) { // operand copies of both row matrices, side by side in the stream's scratch buffer
+  P.planeA = 0; P.planeB = 0;
+  if (x3) { // the three parts of both row matrices: planes h, m, l of `in`, then of `d_out`, in the stream's scratch buffer
+    unsigned char *scr = nullptr;
+    P.planeA = ((long)nInRows * CinP * 2 + 255) & ~255l;
+    P.planeB = ((long)nOutRows * Cout * 2 + 255) & ~255l;
+    SCN_TRY(stream_scratch(s, kScratchDw, 3 * (size_t)(P.planeA + P.planeB) + 16, (void **)&scr));
+    if (nInRows) k_split3_bf16<<<stream_grid(nInRows * CinP / 4, 256), 256, 0, LS(s)>>>(in, reinterpret_cast<uint2 *>(scr), nInRows, Cin, CinP, P.planeA / 2);
+    if (nOutRows) k_split3_bf16<<<stream_grid(nOutRows * Cout / 4, 256), 256, 0, LS(s)>>>(d_out, reinterpret_cast<uint2 *>(scr + 3 * P.planeA), nOutRows, Cout, Cout, P.planeB / 2);
+    SCN_CUDA(cudaGetLastError());
+    P.a = scr; P.b = scr + 3 * P.planeA;
+  } else if (bf16) { // operand copies of both row matrices, side by side in the stream's scratch buffer
     unsigned char *scr = nullptr;
     const bool haveA = in16 && CinP == Cin, haveB = dout16 != nullptr;
     const size_t na = haveA ? 0 : (((size_t)nInRows * CinP * 2 + 255) & ~(size_t)255);
@@ -1850,15 +1948,17 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
   // Channel blocks: Cin in blocks of 256 (two M halves), the rest in one block of <= 128 or 128 + the remainder; Cout in balanced
   // blocks of <= 256 (multiples of 32).  Every block is a shape dw_block_ok takes: one launch each, gathering its channel slice
   // of the same operand rows.  Layers of <= 256 x 256 are one block.
+  // Split operands: three parts per stage, so blocks of <= 128 x <= 128 channels (balanced, multiples of 32 on the Cout side),
+  // whose 64-rule stages fit twice into shared memory.
   std::vector<std::pair<int, int>> bi, bo; // (first channel, channels)
   for (int c = 0; c < Cin;) {
-    const int r = Cin - c, w = !wide || r >= 256 ? std::min(r, 256) : (r <= 128 ? r : 128);
+    const int r = Cin - c, w = x3 ? std::min(r, 128) : !wide || r >= 256 ? std::min(r, 256) : (r <= 128 ? r : 128);
     bi.emplace_back(c, w);
     c += w;
   }
-  const int nOb = wide ? cdiv(Cout, 256) : 1, units = Cout / 32;
+  const int nOb = wide ? cdiv(Cout, 256) : x3 ? cdiv(Cout, 128) : 1, units = Cout / 32;
   for (int i = 0, c = 0; i < nOb; i++) {
-    const int w = wide ? 32 * (units / nOb + (i < units % nOb ? 1 : 0)) : Cout;
+    const int w = wide || x3 ? 32 * (units / nOb + (i < units % nOb ? 1 : 0)) : Cout;
     bo.emplace_back(c, w);
     c += w;
   }
@@ -1869,11 +1969,11 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
     Q.Cin = cinB; Q.Cout = coutB;
     Q.rowBytesA = (cinB == Cin ? CinP : cinB) * 2;
     Q.rowBytesB = coutB * 2;
-    const int nBlocks = std::max(Q.rowBytesA, 256) / 128 + (Q.rowBytesB + 127) / 128;
-    Q.R = (size_t)nBlocks * 128 * 128 * 3 <= budget ? 128 : 64;
+    const int nBlocks = (std::max(Q.rowBytesA, 256) / 128 + (Q.rowBytesB + 127) / 128) * (x3 ? 3 : 1);
+    Q.R = (size_t)nBlocks * 128 * 128 * 3 <= budget && !x3 ? 128 : 64;
     const size_t stageBytes = (size_t)nBlocks * Q.R * 128;
     Q.S = (int)std::min<size_t>(4, budget / stageBytes);
-    Q.nAcc = 2 * ((cinB + 127) / 128) * coutB <= 512 ? 2 : 1;
+    Q.nAcc = 2 * ((cinB + 127) / 128) * coutB * (x3 ? 2 : 1) <= 512 ? 2 : 1; // (split operands: two accumulators per item)
     return stageBytes;
   };
   const size_t stageBytes = shape(P, bi[0].second, bo[0].second);
@@ -1944,6 +2044,7 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
     SCN_CUDA(cudaFuncSetAttribute(conv_dw_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
     SCN_CUDA(cudaFuncSetAttribute(conv_dw_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
     SCN_CUDA(cudaFuncSetAttribute(conv_dw_tc<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
+    SCN_CUDA(cudaFuncSetAttribute(conv_dw_tc<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
     attr = true;
   }
   const int grid = (int)std::min<long>(nItems, kSMs);
@@ -1958,6 +2059,7 @@ int launch_conv_dw_tc(const float *in, const float *d_out, float *dW, const int2
       if (P.part) Q.part = P.part + (size_t)ib.first * Cout + ob.first;
       const size_t smemBytes = (size_t)Q.S * sb + 64 * 8 + 64;
       if (f16) { ++g_counters[kCntF16Launch]; conv_dw_tc<true, true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(Q); }
+      else if (x3) { ++g_counters[kCntDwX3Launch]; conv_dw_tc<true, false, true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(Q); }
       else if (bf16) conv_dw_tc<true><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(Q);
       else conv_dw_tc<false><<<grid, 32 * (5 + kDwProd), smemBytes, LS(s)>>>(Q);
       SCN_CUDA(cudaGetLastError());
